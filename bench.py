@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the sample-stream hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--configs all|none]
+                    [--dump-outputs DIR]
 
 Headline (`value`, `roofline`, `e2e`, `cpu_baseline`) = BASELINE.json configs[1]: batched 1024-point FFT spectrum of
 rtl_tcp-format u8 IQ, 2^28 samples per GPU (fused unpack on load, fftshift + 1/sqrt(N) on store).  A "step" is one
@@ -18,6 +19,11 @@ C3's whole device-resident chain as independent batches.  For N > 1 the halo- an
 (`parity`).
 
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes what the headline workload's last timed step computed (rank 0's outputs) as DIR/<name>.npy,
+so that two builds run with the same arguments can be compared output for output: the inputs come from fixed seeds,
+and a stateful workload (FIR history, PLL, resampler) is reset before the timed steps, so its last step depends on
+--steps alone.  See dump_outputs for the format and the sampling of large outputs.
 """
 import argparse
 import json
@@ -52,6 +58,31 @@ except Exception:
 SEED = 0x5D12B200
 FIR_C64 = {"fir255_c64": (255, 0), "fir64_c64": (64, 0), "fir255_c64_split2": (255, 16), "fir64_c64_split2": (64, 16),
            "fir255_c64_cuda": (255, 2), "fir64_c64_cuda": (64, 2)}
+DUMP_BYTES = 60 << 20  # all --dump-outputs files together, .npy headers included, stay under 64 MB
+DUMP_ROW = 4096        # a 1-D output stream is sampled in blocks of this many samples
+
+
+def sample_rows(n_rows, k):
+    """the fixed, seeded choice of k of n_rows rows that --dump-outputs writes, in row order"""
+    return np.sort(np.random.default_rng(SEED).choice(n_rows, k, replace=False))
+
+
+def dump_outputs(torch, outputs, directory):
+    """Writes every {name: tensor} of `outputs` as directory/<name>.npy in float32: complex values get a trailing
+    (re, im) axis, integer flags become 0.0 / 1.0.  An output larger than its share of DUMP_BYTES is cut into rows (its
+    first axis; a 1-D stream into blocks of DUMP_ROW samples, dropping the tail that fills no block) and only the rows
+    chosen by sample_rows are written."""
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BYTES // len(outputs)
+    for name, t in outputs.items():
+        elem_bytes = 8 if t.is_complex() else 4
+        if t.numel() * elem_bytes > share:
+            if t.dim() == 1:
+                t = t[:t.numel() // DUMP_ROW * DUMP_ROW].view(-1, DUMP_ROW)
+            rows = sample_rows(t.shape[0], max(1, share // (t[0].numel() * elem_bytes)))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        t = torch.view_as_real(t.contiguous()) if t.is_complex() else t.float()
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
 
 
 def measured_peaks():
@@ -392,7 +423,7 @@ def wl_fft1024_u8(cx, log2_samples=28):
 
     return dict(key="c2" if log2_samples == 28 else "c2_small", units=samples, bytes_per_unit=10.0, step=step,
                 e2e_setup=e2e_setup, e2e_step=e2e_step, host=host, h2d=2 * samples, d2h=8 * samples,
-                dtype="f32", kernel="fft1024_warp_kernel<u8iq>")
+                dtype="f32", kernel="fft1024_warp_kernel<u8iq>", outputs=lambda: {"spectrum": out})
 
 
 def wl_fir_u8(cx, key, K=64, D=1, log2_samples=26, complex_taps=False):
@@ -410,9 +441,10 @@ def wl_fir_u8(cx, key, K=64, D=1, log2_samples=26, complex_taps=False):
     n_out = n // D + 1  # the decimation phase carries over between steps
     out = torch.empty(n_out, dtype=torch.complex64, device=dev)
     fir = sdr.Fir(taps, "u8iq", decimation=D, device=dev.index, stream=cx.stream)
+    last = {}
 
     def step():
-        fir.process_dev(mine, n, out, n_out)
+        last["n"] = fir.process_dev(mine, n, out, n_out)
 
     def parity():
         if cx.world == 1:
@@ -451,7 +483,8 @@ def wl_fir_u8(cx, key, K=64, D=1, log2_samples=26, complex_taps=False):
     return dict(key=key, units=n, bytes_per_unit=2.0 + 8.0 / D, step=step, e2e_setup=e2e_setup, e2e_step=e2e_step,
                 host=host, h2d=2 * n, d2h=8 * n_out, dtype="u8 x s8 -> s32 (tcgen05 kind::i8), f32 out",
                 kernel="fir_umma_kernel (tcgen05/TMEM)", parity=parity,
-                sharding="one %d-sample stream, contiguous ranges with a %d-sample halo" % (total, halo))
+                sharding="one %d-sample stream, contiguous ranges with a %d-sample halo" % (total, halo),
+                outputs=lambda: {"filtered": out[:last["n"]]}, reset=fir.reset)
 
 
 def wl_c3_chain(cx, key="c3chain", log2_samples=26, converter=0):
@@ -468,14 +501,20 @@ def wl_c3_chain(cx, key="c3chain", log2_samples=26, converter=0):
     fin = torch.empty(n_fin, dtype=torch.complex64, device=dev)
     fir = sdr.Fir(taps, "u8iq", decimation=D, device=dev.index, stream=cx.stream)
     src = sdr.SampleRate(converter, 2, device=dev.index, stream=cx.stream)
+    last = {}
 
     def step():
         got = fir.process_dev(raw, samples, mid, n_mid)
-        src.process_dev(0.2, mid, got, fin, n_fin)
+        last["n"] = src.process_dev(0.2, mid, got, fin, n_fin)[1]
+
+    def reset():
+        fir.reset()
+        src.reset()
 
     return dict(key=key, units=samples, bytes_per_unit=2.0 + 8.0 / 50, step=step, e2e_setup=None, e2e_step=None,
                 h2d=2 * samples, d2h=8 * n_fin, dtype="u8 x s8 -> s32 (tcgen05), sinc accumulation per DESIGN.md",
-                kernel="fir_umma_poly_kernel + src_sinc kernels", sharding="independent captures per GPU")
+                kernel="fir_umma_poly_kernel + src_sinc kernels", sharding="independent captures per GPU",
+                outputs=lambda: {"resampled": fin[:last["n"]]}, reset=reset)
 
 
 def wl_fft_c64(cx, logn=12, log2_samples=27):
@@ -484,7 +523,8 @@ def wl_fft_c64(cx, logn=12, log2_samples=27):
     samples = 1 << log2_samples
     batches = samples // n
     x = torch.empty((batches, n), dtype=torch.complex64, device=dev)
-    torch.view_as_real(x).uniform_(-1, 1)
+    g = torch.Generator(device=dev).manual_seed(SEED + 5 + cx.rank)
+    torch.view_as_real(x).uniform_(-1, 1, generator=g)
     out = torch.empty_like(x)
     plan = sdr.FftPlan(n, "c64", device=dev.index, stream=cx.stream)
 
@@ -492,7 +532,8 @@ def wl_fft_c64(cx, logn=12, log2_samples=27):
         plan.exec_dev(x, batches, out)
 
     return dict(key="c5_%d" % logn, units=samples, bytes_per_unit=16.0, step=step, e2e_setup=None, e2e_step=None,
-                h2d=8 * samples, d2h=8 * samples, dtype="f32", kernel="fft", sharding="independent batches per GPU")
+                h2d=8 * samples, d2h=8 * samples, dtype="f32", kernel="fft", sharding="independent batches per GPU",
+                outputs=lambda: {"spectrum": out})
 
 
 def wl_fir_c64(cx, key, K=255, total_ch=1024, log2_n=16, flags=0):
@@ -516,7 +557,8 @@ def wl_fir_c64(cx, key, K=255, total_ch=1024, log2_n=16, flags=0):
             2: "fir_rb_kernel (CUDA cores)"}.get(flags, "fir")
     return dict(key=key, units=n_ch * n, bytes_per_unit=16.0, step=step, e2e_setup=None, e2e_step=None,
                 h2d=8 * n_ch * n, d2h=8 * n_ch * n, dtype="bf16 x bf16 -> f32 (tcgen05 kind::f16)" if flags != 2 else "f32",
-                kernel=kern, sharding="%d channels, %d per GPU (shard.unit_range)" % (total_ch, n_ch))
+                kernel=kern, sharding="%d channels, %d per GPU (shard.unit_range)" % (total_ch, n_ch),
+                outputs=lambda: {"filtered": out}, reset=fir.reset)
 
 
 def wl_channelizer(cx, key="c4", total_ch=128, log2_n=16, fast=True):
@@ -560,7 +602,8 @@ def wl_channelizer(cx, key="c4", total_ch=128, log2_n=16, fast=True):
     return dict(key=key, units=n_ch * n, bytes_per_unit=12.125, step=step, e2e_setup=None, e2e_step=None,
                 h2d=8 * n_ch * n, d2h=5 * n_ch * n, dtype="f32", kernel="multi-channel FIR + pll_kernel",
                 parity=parity, bound="latency (PLL dependent chain)",
-                sharding="%d channels, %d per GPU (shard.unit_range)" % (total_ch, n_ch))
+                sharding="%d channels, %d per GPU (shard.unit_range)" % (total_ch, n_ch),
+                outputs=lambda: {"pll_out": out, "locked": lk}, reset=ch.reset)
 
 
 def wl_fm(cx, n_st=128, log2_n=18, fast=True):
@@ -572,13 +615,15 @@ def wl_fm(cx, n_st=128, log2_n=18, fast=True):
     fm = sdr.FmStereo(n_st, 1.8e6, fast_math=fast, device=dev.index, stream=cx.stream)
     cap = fm.max_output(n)
     out = torch.empty((n_st, cap, 2), dtype=torch.float32, device=dev)
+    last = {}
 
     def step():
-        fm.process_dev(raw, n, row, out, cap, cap, end_of_input=False)
+        last["n"] = fm.process_dev(raw, n, row, out, cap, cap, end_of_input=False)
 
     return dict(key="fm", units=n_st * n, bytes_per_unit=2.0 + 8.0 / 37.5, step=step, e2e_setup=None, e2e_step=None,
                 h2d=2 * n_st * n, d2h=8 * n_st * cap, dtype="f32 (f64 atan2/sincos in the PLLs)",
-                kernel="pll_kernel + src_sinc + pll_stereo_kernel + biquad_kernel", bound="latency (PLL dependent chain)")
+                kernel="pll_kernel + src_sinc + pll_stereo_kernel + biquad_kernel", bound="latency (PLL dependent chain)",
+                outputs=lambda: {"audio": out[:, :last["n"]]}, reset=fm.reset)
 
 
 def make_workload(name, cx):
@@ -698,6 +743,7 @@ def bind_to_gpu_cores(local, world_local):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
@@ -709,7 +755,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--configs", default="all", help="all | none | comma list of secondary workloads for the `configs` array")
     ap.add_argument("--config-steps", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the headline workload as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     if args.impl == "reference":
@@ -766,7 +818,11 @@ def main():
         while time.perf_counter() - t_pre < 0.4:
             wl["step"]()
             torch.cuda.synchronize(dev)
+        if wl.get("reset"):  # the pre-roll's step count varies with the clock; the timed steps start from a fresh stream
+            wl["reset"]()
         per_step_ms, launches = cx.time_steps(wl["step"], args.steps, 0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, wl["outputs"](), args.dump_outputs)
     value = world * wl["units"] / (per_step_ms * 1e-3) / 1e9
     achieved = wl["units"] * wl["bytes_per_unit"] / (per_step_ms * 1e-3) / 1e9  # GB/s on this rank's GPU
 
@@ -796,7 +852,8 @@ def main():
     if args.configs != "none":
         names = SECONDARY if args.configs == "all" else [c for c in args.configs.split(",") if c]
         names = [c for c in names if c != args.workload]
-        del wl["step"], wl["e2e_step"], wl["e2e_setup"]
+        for k in ("step", "e2e_step", "e2e_setup", "outputs", "reset"):  # free the headline's device buffers
+            wl.pop(k, None)
         torch.cuda.synchronize(dev)
         torch.cuda.empty_cache()
         for name in names:
