@@ -403,6 +403,52 @@ int sdr_window_fft_process(sdr_window_fft_t *, const void *in, size_t n_in, floa
 int sdr_window_fft_process_dev(sdr_window_fft_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap,
                                size_t *n_windows);
 
+/* ======================================================================================
+ * polyphase filter bank -- one wideband stream cut into M channels, each decimated by D.
+ * Channel k is filter::Fir<Complex<f32>, Complex<f32>> (src/filter/fir.rs:23-32) with taps
+ * g_k[n] = h[n] e^{+2 pi i k n / M} followed by signal::Decimate with wait D (adapters/mod.rs:30-37):
+ *   y_k[m] = sum_{n<L} g_k[n] x[(m+1) D - 1 - n],   x[<0] = 0
+ * Channel k is centred on k * rate / M; k >= M/2 are the negative frequencies.  Computed as the
+ * polyphase form (branch p = taps h[t M + p]) followed by an unnormalised M-point forward DFT
+ * (the sdr_fft plan), so accuracy is the FFT's (DESIGN.md).
+ *   SDR_PFB_SHIFT          row i of a frame is channel (i - M/2) mod M, at sdr_fft_labels(M, rate, 0)[i]
+ *   SDR_PFB_CHANNEL_MAJOR  M rows of frames (what sdr_fir / sdr_pll / sdr_channelizer take as
+ *                          n_channels rows) instead of frames of M channels
+ *   SDR_PFB_GENERAL_KERNEL always the general front end instead of the register-window one (which runs
+ *                          when D divides M and the windows fit in registers); same bits; for testing
+ * Carried state: the last L - 1 inputs and the stream position, so blocks of any size give the same
+ * bits as one call.  Input pointers need only element alignment (2 bytes u8, 8 bytes c64).
+ * ====================================================================================== */
+#define SDR_PFB_SHIFT 1u
+#define SDR_PFB_CHANNEL_MAJOR 2u
+#define SDR_PFB_GENERAL_KERNEL 4u
+
+typedef struct {
+    const float *taps;  /* real prototype lowpass h, n_taps f32 */
+    size_t n_taps;      /* L >= 1 */
+    size_t n_channels;  /* M, 2 <= M <= 65536 (any length the FFT plan accepts) */
+    size_t decimation;  /* D >= 1 (0 is rejected, as for sdr_fir) */
+    int input_format;   /* U8IQ or C64 (F32 is rejected) */
+    unsigned flags;     /* SDR_PFB_* */
+    int device;
+    void *stream;
+} sdr_pfb_config_t;
+
+typedef struct sdr_pfb sdr_pfb_t;
+sdr_pfb_t *sdr_pfb_create(const sdr_pfb_config_t *cfg, int *err);
+void sdr_pfb_destroy(sdr_pfb_t *);
+int sdr_pfb_reset(sdr_pfb_t *);                        /* zero history and stream position */
+sdr_pfb_t *sdr_pfb_clone(const sdr_pfb_t *, int *err);
+/* frames the next n_in input samples complete */
+size_t sdr_pfb_output_count(const sdr_pfb_t *, size_t n_in);
+/* frame-major: out = frames of M c64, frame stride out_stride elements (>= M), capacity out_cap frames;
+ * channel-major: M rows, row stride out_stride elements (>= frames written), out_cap frames per row.
+ * A too-small out_cap returns SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  *n_frames = frames written. */
+int sdr_pfb_process(sdr_pfb_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap, size_t out_stride,
+                    size_t *n_frames);
+int sdr_pfb_process_dev(sdr_pfb_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap, size_t out_stride,
+                        size_t *n_frames);
+
 #ifdef __cplusplus
 }
 #endif

@@ -177,6 +177,52 @@ class Fir {
     const std::vector<C> &coef() const { return coef_; }
 };
 
+// Polyphase filter bank behind sdr_pfb_*: channel k is Fir<Complex, Complex>(h[n] e^{+2 pi i k n / M}) followed by
+// Decimate(D), for k = 0..M-1, computed in one pass over the input.  flags: SDR_PFB_SHIFT, SDR_PFB_CHANNEL_MAJOR.
+class Pfb {
+    sdr_pfb_t *h_ = nullptr;
+    size_t m_ = 0;
+    bool cmajor_ = false;
+
+  public:
+    Pfb(const std::vector<float> &prototype, size_t n_channels, size_t decimation, bool input_u8iq = false,
+        unsigned flags = 0)
+        : m_(n_channels), cmajor_((flags & SDR_PFB_CHANNEL_MAJOR) != 0) {
+        sdr_pfb_config_t cfg{};
+        cfg.taps = prototype.data();
+        cfg.n_taps = prototype.size();
+        cfg.n_channels = n_channels;
+        cfg.decimation = decimation;
+        cfg.input_format = input_u8iq ? SDR_FMT_U8IQ : SDR_FMT_C64;
+        cfg.flags = flags;
+        int err = 0;
+        h_ = sdr_pfb_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Pfb::new");
+    }
+    Pfb(Pfb &&o) noexcept : h_(o.h_), m_(o.m_), cmajor_(o.cmajor_) { o.h_ = nullptr; }
+    Pfb(const Pfb &o) : m_(o.m_), cmajor_(o.cmajor_) {
+        int err = 0;
+        h_ = sdr_pfb_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Pfb::clone");
+    }
+    Pfb &operator=(const Pfb &) = delete;
+    ~Pfb() { sdr_pfb_destroy(h_); }
+    size_t channels() const { return m_; }
+    size_t output_count(size_t n_in) const { return sdr_pfb_output_count(h_, n_in); }
+    // in: n samples (Complex, or 2n bytes when constructed with input_u8iq).  out: frames x M (or M x frames when
+    // channel-major), replaced.  Returns the number of frames.
+    size_t process(const void *in, size_t n, std::vector<Complex> &out) {
+        const size_t nf = output_count(n);
+        out.resize((nf ? nf : 1) * m_);
+        size_t got = 0;
+        check(sdr_pfb_process(h_, in, n, reinterpret_cast<float *>(out.data()), nf, cmajor_ ? nf : m_, &got),
+              "Pfb::process");
+        out.resize(got * m_);
+        return got;
+    }
+    void reset() { check(sdr_pfb_reset(h_), "Pfb::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

@@ -112,6 +112,56 @@ impl<S: Signal, C: GpuCoef> Signal for GpuFilter<S, C> where S::Sample: GpuSampl
     fn rate(&self) -> f32 { self.signal.rate() }
 }
 
+/// Polyphase filter bank: channel k is Fir<Complex<f32>, Complex<f32>> with taps h[n] e^{+2 pi i k n / M} followed by
+/// Decimate(wait), for k = 0..M-1, in one pass over the input.  `process` returns frames of M channels (or M rows of
+/// frames with SDR_PFB_CHANNEL_MAJOR); blocks of any size give the same samples as one call.
+pub struct GpuPfb {
+    h: *mut sdr_pfb_t,
+    m: usize,
+    channel_major: bool,
+}
+unsafe impl Send for GpuPfb {}
+
+impl GpuPfb {
+    pub fn new(prototype: &[f32], channels: usize, wait: usize, input_u8iq: bool, flags: u32) -> Result<Self, Error> {
+        let cfg = sdr_pfb_config_t {
+            taps: prototype.as_ptr(), n_taps: prototype.len(), n_channels: channels, decimation: wait,
+            input_format: if input_u8iq { SDR_FMT_U8IQ } else { SDR_FMT_C64 }, flags, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_pfb_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuPfb { h, m: channels, channel_major: flags & SDR_PFB_CHANNEL_MAJOR != 0 })
+    }
+    /// input: n samples (Complex<f32>, or 2n rtl_tcp bytes); output: replaced by frames x M (or M x frames)
+    pub fn process<T: Copy>(&mut self, input: &[T], n: usize, output: &mut Vec<Complex<f32>>) -> Result<usize, Error> {
+        let nf = unsafe { sdr_pfb_output_count(self.h, n) };
+        output.clear();
+        output.reserve(nf.max(1) * self.m);
+        let mut got = 0usize;
+        let stride = if self.channel_major { nf } else { self.m };
+        check(unsafe {
+            sdr_pfb_process(self.h, input.as_ptr() as *const c_void, n, output.as_mut_ptr() as *mut f32, nf, stride,
+                            &mut got)
+        })?;
+        unsafe { output.set_len(got * self.m) };
+        Ok(got)
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_pfb_reset(self.h) }) }
+}
+impl Clone for GpuPfb {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_pfb_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_pfb_clone failed: {}", Error(err));
+        GpuPfb { h, m: self.m, channel_major: self.channel_major }
+    }
+}
+impl Drop for GpuPfb {
+    fn drop(&mut self) { unsafe { sdr_pfb_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

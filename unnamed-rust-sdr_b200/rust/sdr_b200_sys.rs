@@ -17,6 +17,10 @@ pub const SDR_FFT_NORM: c_uint = 2;
 pub const SDR_FFT_RFFT: c_uint = 4;
 /// sdr_pll_config_t.flags: atan2 / sin / cos evaluated in f64 and rounded to f32 (default: f32 routines within ~1 ulp)
 pub const SDR_PLL_F64_MATH: c_uint = 2;
+/// sdr_pfb_config_t.flags
+pub const SDR_PFB_SHIFT: c_uint = 1;
+pub const SDR_PFB_CHANNEL_MAJOR: c_uint = 2;
+pub const SDR_PFB_GENERAL_KERNEL: c_uint = 4;
 
 pub enum sdr_fir_t {}
 pub enum sdr_fft_t {}
@@ -24,6 +28,7 @@ pub enum sdr_pll_t {}
 pub enum sdr_biquad_t {}
 pub enum sdr_fm_t {}
 pub enum sdr_window_fft_t {}
+pub enum sdr_pfb_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -94,6 +99,18 @@ pub struct sdr_biquad_config_t {
 pub struct sdr_window_fft_config_t {
     pub window: size_t,
     pub hop: size_t,
+    pub input_format: c_int,
+    pub flags: c_uint,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+pub struct sdr_pfb_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_channels: size_t,
+    pub decimation: size_t,
     pub input_format: c_int,
     pub flags: c_uint,
     pub device: c_int,
@@ -180,6 +197,17 @@ extern "C" {
     pub fn sdr_window_fft_output_count(h: *const sdr_window_fft_t, n_in: size_t) -> size_t;
     pub fn sdr_window_fft_process(h: *mut sdr_window_fft_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
                                   out_cap: size_t, n_windows: *mut size_t) -> c_int;
+
+    // polyphase filter bank: M x (Fir(h e^{+2 pi i k n / M}) + Decimate(D)) in one pass
+    pub fn sdr_pfb_create(cfg: *const sdr_pfb_config_t, err: *mut c_int) -> *mut sdr_pfb_t;
+    pub fn sdr_pfb_destroy(h: *mut sdr_pfb_t);
+    pub fn sdr_pfb_reset(h: *mut sdr_pfb_t) -> c_int;
+    pub fn sdr_pfb_clone(h: *const sdr_pfb_t, err: *mut c_int) -> *mut sdr_pfb_t;
+    pub fn sdr_pfb_output_count(h: *const sdr_pfb_t, n_in: size_t) -> size_t;
+    pub fn sdr_pfb_process(h: *mut sdr_pfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float, out_cap: size_t,
+                           out_stride: size_t, n_frames: *mut size_t) -> c_int;
+    pub fn sdr_pfb_process_dev(h: *mut sdr_pfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
+                               out_cap: size_t, out_stride: size_t, n_frames: *mut size_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -12,6 +12,7 @@ FFT_SHIFT, FFT_NORM, FFT_RFFT = 1, 2, 4
 PLL_FAST_MATH = 1
 PLL_F64_MATH = 2
 PLL_GENERAL_KERNEL = 4
+PFB_SHIFT, PFB_CHANNEL_MAJOR, PFB_GENERAL_KERNEL = 1, 2, 4
 BQ_IDENTITY, BQ_LOWPASS, BQ_HIGHPASS, BQ_BANDPASS, BQ_NOTCH, BQ_LR = range(6)
 SRC_SINC_BEST_QUALITY, SRC_SINC_MEDIUM_QUALITY, SRC_SINC_FASTEST, SRC_ZERO_ORDER_HOLD, SRC_LINEAR = range(5)
 
@@ -53,6 +54,11 @@ class FmConfig(C.Structure):
 
 class WindowFftConfig(C.Structure):
     _fields_ = [("window", sz), ("hop", sz), ("input_format", i32), ("flags", C.c_uint), ("device", i32), ("stream", vp)]
+
+
+class PfbConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_channels", sz), ("decimation", sz), ("input_format", i32),
+                ("flags", C.c_uint), ("device", i32), ("stream", vp)]
 
 
 class SrcData(C.Structure):
@@ -103,6 +109,13 @@ PROTOTYPES = {
     "sdr_window_fft_output_count": (sz, [vp, sz]),
     "sdr_window_fft_process": (i32, [vp, vp, sz, vp, sz, C.POINTER(sz)]),
     "sdr_window_fft_process_dev": (i32, [vp, vp, sz, vp, sz, C.POINTER(sz)]),
+    "sdr_pfb_create": (vp, [C.POINTER(PfbConfig), C.POINTER(i32)]),
+    "sdr_pfb_destroy": (None, [vp]),
+    "sdr_pfb_reset": (i32, [vp]),
+    "sdr_pfb_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_pfb_output_count": (sz, [vp, sz]),
+    "sdr_pfb_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_pfb_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -437,6 +437,80 @@ class WindowFft:
     __del__ = close
 
 
+class Pfb:
+    """Polyphase filter bank: one wideband stream -> n_channels channels decimated by `decimation`.  Channel k is
+    Fir(h * exp(+2j pi k n / M)) followed by Decimate(D); channel k is centred on k * rate / M.  shift=True orders the
+    channels like fft::fft's shift (row i = channel (i - M/2) mod M); channel_major=True returns [M, frames] instead of
+    [frames, M].  general=True forces the general front-end kernel (same bits)."""
+
+    def __init__(self, taps, n_channels, decimation, input_format="c64", shift=False, channel_major=False,
+                 general=False, device=0, stream=None, _handle=None, _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        self._taps = np.ascontiguousarray(taps, np.float32)
+        self.n_channels = int(n_channels)
+        self.decimation = int(decimation)
+        self.fmt = _FMT_OF[input_format] if isinstance(input_format, str) else int(input_format)
+        self.channel_major = bool(channel_major)
+        flags = (F.PFB_SHIFT if shift else 0) | (F.PFB_CHANNEL_MAJOR if channel_major else 0) | \
+            (F.PFB_GENERAL_KERNEL if general else 0)
+        cfg = F.PfbConfig(self._taps.ctypes.data, self._taps.size, self.n_channels, self.decimation, self.fmt, flags,
+                          device, _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_pfb_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_pfb_create")
+
+    def output_count(self, n_in):
+        return lib().sdr_pfb_output_count(self.h, n_in)
+
+    def process(self, x):
+        """x: uint8 [2n] (u8iq) or complex64 [n] -> complex64 [frames, M] (or [M, frames] when channel-major)"""
+        if self.fmt == F.FMT_U8IQ:
+            x = np.ascontiguousarray(x, np.uint8)
+            n = x.size // 2
+        else:
+            x = np.ascontiguousarray(x, np.complex64)
+            n = x.size
+        nf = self.output_count(n)
+        M = self.n_channels
+        cap = max(nf, 1)
+        out = np.empty((M, cap) if self.channel_major else (cap, M), np.complex64)
+        got = C.c_size_t(0)
+        check(lib().sdr_pfb_process(self.h, x.ctypes.data if n else None, n, out.ctypes.data, cap,
+                                    cap if self.channel_major else M, C.byref(got)), "sdr_pfb_process")
+        return out[:, :got.value] if self.channel_major else out[:got.value]
+
+    def process_dev(self, d_in, n_in, d_out, out_cap, out_stride=None):
+        """device-resident: d_in n_in samples, d_out frame-major (stride out_stride >= M) or channel-major (M rows of
+        out_stride >= frames); asynchronous on the handle's stream.  Returns the frames written."""
+        if out_stride is None:
+            out_stride = out_cap if self.channel_major else self.n_channels
+        got = C.c_size_t(0)
+        check(lib().sdr_pfb_process_dev(self.h, _ptr(d_in), n_in, _ptr(d_out), out_cap, out_stride, C.byref(got)),
+              "sdr_pfb_process_dev")
+        return got.value
+
+    def reset(self):
+        check(lib().sdr_pfb_reset(self.h), "sdr_pfb_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_pfb_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_pfb_clone")
+        return Pfb(None, 0, 0, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_pfb_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
