@@ -449,6 +449,57 @@ int sdr_pfb_process(sdr_pfb_t *, const void *in, size_t n_in, float *out_c64, si
 int sdr_pfb_process_dev(sdr_pfb_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap, size_t out_stride,
                         size_t *n_frames);
 
+/* ======================================================================================
+ * digital down-converter bank -- C channels at arbitrary centre frequencies of one IQ stream, each
+ * mixed to 0 Hz by its own 64-bit NCO, low-pass filtered by its own real taps and decimated by D.
+ * Channel k restates what the crate builds from a tee'd copy of the stream (Block::clone, adapters/block.rs),
+ * a caller-written oscillator through Signal::map, filter::Fir<Complex<f32>, f32> (src/filter/fir.rs:23-32)
+ * with taps h_k and signal::Decimate with wait D (adapters/mod.rs:30-37):
+ *   z_k[n] = x[n] e^{-2 pi i phi_k(n) / 2^64},   phi_k(n) = (first_sample + n) phase_inc[k]  mod 2^64
+ *   y_k[m] = sum_{j<L} h_k[j] z_k[(m+1) D - 1 - j],   x[<0] = 0 (byte 128 for u8, as fir.rs:15)
+ * n counts the handle's inputs; first_sample only places the NCO phase (exact 64-bit phase accumulator, so the phase
+ * at any stream position is independent of how the stream is cut, across calls and shards).  Channel k is centred on
+ * (int64)phase_inc[k] / 2^64 * rate; sdr_ddc_phase_increment(freq, rate) rounds a frequency to an increment:
+ * nu = freq / rate, nu -= round(nu), phase_inc = llround(nu 2^64), nu = +-0.5 -> 2^63 (0 for non-finite input).
+ * Paths (sdr_ddc_last_path): 2 = tcgen05 integer Toeplitz GEMM for u8 IQ input with D in {1, 2, 4, 8, 16, 32} and
+ * L <= 511 while one channel's table fits in shared memory (all but D = 1 with L > ~430); 1 = CUDA-core kernel for
+ * everything else (c64 input, other D, longer filters) and with SDR_DDC_GENERAL_KERNEL.  Both meet the FIR bar of
+ * 1e-5 of max|y| per channel; they are not bit-equal to each other.
+ * Output: C rows (channel-major, the n_channels rows sdr_fir / sdr_pll / sdr_channelizer take), row stride out_stride
+ * c64 elements (>= outputs written), out_cap outputs per row; a too-small out_cap returns SDR_ERR_OUTPUT_TOO_SMALL
+ * before any state changes.  Carried state: the last L - 1 inputs and the stream position, so blocks of any size from
+ * any element-aligned address give the same bits as one call.
+ * ====================================================================================== */
+#define SDR_DDC_GENERAL_KERNEL 1u /* always the CUDA-core kernel (for testing; results within the same bars) */
+
+typedef struct {
+    const float *taps;         /* n_tap_sets rows of n_taps real f32 */
+    size_t n_taps;             /* L, 1 <= L <= 2^20 */
+    size_t n_tap_sets;         /* 1 (shared) or n_channels */
+    const uint64_t *phase_inc; /* n_channels NCO increments (sdr_ddc_phase_increment) */
+    size_t n_channels;         /* C, 1 <= C <= 256 (SDR_ERR_INVALID_ARG beyond) */
+    size_t decimation;         /* D >= 1 (0 is rejected, as for sdr_fir) */
+    uint64_t first_sample;     /* absolute stream index of the first input this handle sees (NCO phase only) */
+    int input_format;          /* U8IQ or C64 (F32 is rejected) */
+    unsigned flags;            /* SDR_DDC_* */
+    int device;
+    void *stream;
+} sdr_ddc_config_t;
+
+typedef struct sdr_ddc sdr_ddc_t;
+uint64_t sdr_ddc_phase_increment(double freq, double rate); /* host, pure */
+sdr_ddc_t *sdr_ddc_create(const sdr_ddc_config_t *cfg, int *err);
+void sdr_ddc_destroy(sdr_ddc_t *);
+int sdr_ddc_reset(sdr_ddc_t *); /* zero history, position back to first_sample */
+sdr_ddc_t *sdr_ddc_clone(const sdr_ddc_t *, int *err);
+/* outputs per channel that the next n_in input samples complete */
+size_t sdr_ddc_output_count(const sdr_ddc_t *, size_t n_in);
+int sdr_ddc_process(sdr_ddc_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap, size_t out_stride,
+                    size_t *n_out);
+int sdr_ddc_process_dev(sdr_ddc_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap, size_t out_stride,
+                        size_t *n_out);
+int sdr_ddc_last_path(const sdr_ddc_t *); /* path of the last call that produced outputs: 0 none, 1 CUDA-core, 2 tcgen05 */
+
 #ifdef __cplusplus
 }
 #endif

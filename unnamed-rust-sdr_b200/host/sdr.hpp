@@ -223,6 +223,57 @@ class Pfb {
     void reset() { check(sdr_pfb_reset(h_), "Pfb::reset"); }
 };
 
+// Down-converter bank behind sdr_ddc_*: channel k is a tee'd copy of the stream mixed down by a 64-bit NCO
+// (sdr_ddc_phase_increment(freq[k], rate)), Fir<Complex, f32>(h_k) and Decimate(D), computed in one pass over the input.
+// taps: one row of L (shared) or channels rows of L.  Output: channels rows of outputs (channel-major).
+class Ddc {
+    sdr_ddc_t *h_ = nullptr;
+    size_t c_ = 0;
+
+  public:
+    Ddc(const std::vector<float> &taps, size_t n_taps, const std::vector<double> &freqs, double rate, size_t decimation,
+        bool input_u8iq = true, uint64_t first_sample = 0, unsigned flags = 0)
+        : c_(freqs.size()) {
+        std::vector<uint64_t> inc(freqs.size());
+        for (size_t k = 0; k < freqs.size(); ++k) inc[k] = sdr_ddc_phase_increment(freqs[k], rate);
+        sdr_ddc_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.phase_inc = inc.data();
+        cfg.n_channels = freqs.size();
+        cfg.decimation = decimation;
+        cfg.first_sample = first_sample;
+        cfg.input_format = input_u8iq ? SDR_FMT_U8IQ : SDR_FMT_C64;
+        cfg.flags = flags;
+        int err = 0;
+        h_ = sdr_ddc_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Ddc::new");
+    }
+    Ddc(Ddc &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
+    Ddc(const Ddc &o) : c_(o.c_) {
+        int err = 0;
+        h_ = sdr_ddc_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Ddc::clone");
+    }
+    Ddc &operator=(const Ddc &) = delete;
+    ~Ddc() { sdr_ddc_destroy(h_); }
+    size_t channels() const { return c_; }
+    size_t output_count(size_t n_in) const { return sdr_ddc_output_count(h_, n_in); }
+    int last_path() const { return sdr_ddc_last_path(h_); }
+    // in: n samples (Complex, or 2n rtl_tcp bytes when constructed with input_u8iq).  out: channels x outputs,
+    // replaced.  Returns the outputs per channel.
+    size_t process(const void *in, size_t n, std::vector<Complex> &out) {
+        const size_t nf = output_count(n);
+        out.resize((nf ? nf : 1) * c_);
+        size_t got = 0;
+        check(sdr_ddc_process(h_, in, n, reinterpret_cast<float *>(out.data()), nf, nf ? nf : 1, &got), "Ddc::process");
+        out.resize(got * c_);
+        return got;
+    }
+    void reset() { check(sdr_ddc_reset(h_), "Ddc::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

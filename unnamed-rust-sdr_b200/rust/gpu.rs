@@ -162,6 +162,58 @@ impl Drop for GpuPfb {
     fn drop(&mut self) { unsafe { sdr_pfb_destroy(self.h) } }
 }
 
+/// Down-converter bank: channel k is the stream mixed down by a 64-bit NCO at freqs[k] (what a caller writes with
+/// Signal::map over an oscillator), Fir<Complex<f32>, f32>(h_k) and Decimate(wait), for all channels in one pass over
+/// the input.  taps: one row of n_taps (shared) or one row per channel.  `process` returns channels rows of outputs
+/// (channel-major); blocks of any size give the same samples as one call.
+pub struct GpuDdc {
+    h: *mut sdr_ddc_t,
+    c: usize,
+}
+unsafe impl Send for GpuDdc {}
+
+impl GpuDdc {
+    pub fn new(taps: &[f32], n_taps: usize, freqs: &[f64], rate: f64, wait: usize, input_u8iq: bool,
+               first_sample: u64, flags: u32) -> Result<Self, Error> {
+        let inc: Vec<u64> = freqs.iter().map(|&f| unsafe { sdr_ddc_phase_increment(f, rate) }).collect();
+        let cfg = sdr_ddc_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: if n_taps == 0 { 0 } else { taps.len() / n_taps },
+            phase_inc: inc.as_ptr(), n_channels: freqs.len(), decimation: wait, first_sample,
+            input_format: if input_u8iq { SDR_FMT_U8IQ } else { SDR_FMT_C64 }, flags, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_ddc_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuDdc { h, c: freqs.len() })
+    }
+    /// input: n samples (Complex<f32>, or 2n rtl_tcp bytes); output: replaced by channels x outputs
+    pub fn process<T: Copy>(&mut self, input: &[T], n: usize, output: &mut Vec<Complex<f32>>) -> Result<usize, Error> {
+        let nf = unsafe { sdr_ddc_output_count(self.h, n) };
+        output.clear();
+        output.reserve(nf.max(1) * self.c);
+        let mut got = 0usize;
+        check(unsafe {
+            sdr_ddc_process(self.h, input.as_ptr() as *const c_void, n, output.as_mut_ptr() as *mut f32, nf, nf.max(1),
+                            &mut got)
+        })?;
+        unsafe { output.set_len(got * self.c) };
+        Ok(got)
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_ddc_reset(self.h) }) }
+}
+impl Clone for GpuDdc {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_ddc_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_ddc_clone failed: {}", Error(err));
+        GpuDdc { h, c: self.c }
+    }
+}
+impl Drop for GpuDdc {
+    fn drop(&mut self) { unsafe { sdr_ddc_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

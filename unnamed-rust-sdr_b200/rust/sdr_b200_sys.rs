@@ -21,6 +21,8 @@ pub const SDR_PLL_F64_MATH: c_uint = 2;
 pub const SDR_PFB_SHIFT: c_uint = 1;
 pub const SDR_PFB_CHANNEL_MAJOR: c_uint = 2;
 pub const SDR_PFB_GENERAL_KERNEL: c_uint = 4;
+/// sdr_ddc_config_t.flags
+pub const SDR_DDC_GENERAL_KERNEL: c_uint = 1;
 
 pub enum sdr_fir_t {}
 pub enum sdr_fft_t {}
@@ -29,6 +31,7 @@ pub enum sdr_biquad_t {}
 pub enum sdr_fm_t {}
 pub enum sdr_window_fft_t {}
 pub enum sdr_pfb_t {}
+pub enum sdr_ddc_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -111,6 +114,21 @@ pub struct sdr_pfb_config_t {
     pub n_taps: size_t,
     pub n_channels: size_t,
     pub decimation: size_t,
+    pub input_format: c_int,
+    pub flags: c_uint,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+pub struct sdr_ddc_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub phase_inc: *const u64,
+    pub n_channels: size_t,
+    pub decimation: size_t,
+    pub first_sample: u64,
     pub input_format: c_int,
     pub flags: c_uint,
     pub device: c_int,
@@ -208,6 +226,19 @@ extern "C" {
                            out_stride: size_t, n_frames: *mut size_t) -> c_int;
     pub fn sdr_pfb_process_dev(h: *mut sdr_pfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
                                out_cap: size_t, out_stride: size_t, n_frames: *mut size_t) -> c_int;
+
+    // down-converter bank: C x (64-bit NCO mixer + Fir(h_k) + Decimate(D)) in one pass
+    pub fn sdr_ddc_phase_increment(freq: f64, rate: f64) -> u64;
+    pub fn sdr_ddc_create(cfg: *const sdr_ddc_config_t, err: *mut c_int) -> *mut sdr_ddc_t;
+    pub fn sdr_ddc_destroy(h: *mut sdr_ddc_t);
+    pub fn sdr_ddc_reset(h: *mut sdr_ddc_t) -> c_int;
+    pub fn sdr_ddc_clone(h: *const sdr_ddc_t, err: *mut c_int) -> *mut sdr_ddc_t;
+    pub fn sdr_ddc_output_count(h: *const sdr_ddc_t, n_in: size_t) -> size_t;
+    pub fn sdr_ddc_process(h: *mut sdr_ddc_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float, out_cap: size_t,
+                           out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_ddc_process_dev(h: *mut sdr_ddc_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
+                               out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_ddc_last_path(h: *const sdr_ddc_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

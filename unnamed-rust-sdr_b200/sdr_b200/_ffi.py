@@ -13,6 +13,7 @@ PLL_FAST_MATH = 1
 PLL_F64_MATH = 2
 PLL_GENERAL_KERNEL = 4
 PFB_SHIFT, PFB_CHANNEL_MAJOR, PFB_GENERAL_KERNEL = 1, 2, 4
+DDC_GENERAL_KERNEL = 1
 BQ_IDENTITY, BQ_LOWPASS, BQ_HIGHPASS, BQ_BANDPASS, BQ_NOTCH, BQ_LR = range(6)
 SRC_SINC_BEST_QUALITY, SRC_SINC_MEDIUM_QUALITY, SRC_SINC_FASTEST, SRC_ZERO_ORDER_HOLD, SRC_LINEAR = range(5)
 
@@ -59,6 +60,12 @@ class WindowFftConfig(C.Structure):
 class PfbConfig(C.Structure):
     _fields_ = [("taps", vp), ("n_taps", sz), ("n_channels", sz), ("decimation", sz), ("input_format", i32),
                 ("flags", C.c_uint), ("device", i32), ("stream", vp)]
+
+
+class DdcConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phase_inc", vp), ("n_channels", sz),
+                ("decimation", sz), ("first_sample", C.c_uint64), ("input_format", i32), ("flags", C.c_uint),
+                ("device", i32), ("stream", vp)]
 
 
 class SrcData(C.Structure):
@@ -116,6 +123,15 @@ PROTOTYPES = {
     "sdr_pfb_output_count": (sz, [vp, sz]),
     "sdr_pfb_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_pfb_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_ddc_phase_increment": (C.c_uint64, [C.c_double, C.c_double]),
+    "sdr_ddc_create": (vp, [C.POINTER(DdcConfig), C.POINTER(i32)]),
+    "sdr_ddc_destroy": (None, [vp]),
+    "sdr_ddc_reset": (i32, [vp]),
+    "sdr_ddc_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_ddc_output_count": (sz, [vp, sz]),
+    "sdr_ddc_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_ddc_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_ddc_last_path": (i32, [vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -511,6 +511,91 @@ class Pfb:
     __del__ = close
 
 
+def ddc_phase_increment(freq, rate):
+    """the 64-bit NCO increment of a channel centred on `freq` (Hz) in a stream of `rate` samples/s
+    (sdr_ddc_phase_increment: nu = freq / rate folded into [-1/2, 1/2], rounded to nu * 2^64; negative = two's complement)"""
+    return int(lib().sdr_ddc_phase_increment(float(freq), float(rate)))
+
+
+class Ddc:
+    """Digital down-converter bank: channel k of one IQ stream is mixed down by freqs[k] (a 64-bit NCO), filtered by its
+    real taps (taps 1-D: shared; [C, L]: one row per channel) and decimated by `decimation`:
+    y_k[m] = sum_j h_k[j] x[N - j] e^{-2 pi i phi_k(N - j)}, N = (m + 1) D - 1.  first_sample = absolute stream index of
+    the first input (places the NCO phase only).  process returns complex64 [C, outputs] (channel-major rows).
+    general=True forces the CUDA-core kernel."""
+
+    def __init__(self, taps, freqs, rate, decimation, input_format="u8iq", first_sample=0, general=False, device=0,
+                 stream=None, _handle=None, _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        self._taps = t
+        self.phase_inc = np.array([ddc_phase_increment(f, rate) for f in np.atleast_1d(freqs)], np.uint64)
+        self.n_channels = int(self.phase_inc.size)
+        self.decimation = int(decimation)
+        self.fmt = _FMT_OF[input_format] if isinstance(input_format, str) else int(input_format)
+        cfg = F.DdcConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
+                          self.n_channels, self.decimation, int(first_sample), self.fmt,
+                          F.DDC_GENERAL_KERNEL if general else 0, device, _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_ddc_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_ddc_create")
+
+    def output_count(self, n_in):
+        return lib().sdr_ddc_output_count(self.h, n_in)
+
+    @property
+    def last_path(self):
+        """path of the last call that produced outputs: 0 none, 1 CUDA-core kernel, 2 tcgen05 kernel"""
+        return lib().sdr_ddc_last_path(self.h)
+
+    def process(self, x):
+        """x: uint8 [2n] (u8iq) or complex64 [n] -> complex64 [C, outputs]"""
+        if self.fmt == F.FMT_U8IQ:
+            x = np.ascontiguousarray(x, np.uint8)
+            n = x.size // 2
+        else:
+            x = np.ascontiguousarray(x, np.complex64)
+            n = x.size
+        cap = max(self.output_count(n), 1)
+        out = np.empty((self.n_channels, cap), np.complex64)
+        got = C.c_size_t(0)
+        check(lib().sdr_ddc_process(self.h, x.ctypes.data if n else None, n, out.ctypes.data, cap, cap, C.byref(got)),
+              "sdr_ddc_process")
+        return out[:, :got.value]
+
+    def process_dev(self, d_in, n_in, d_out, out_cap, out_stride=None):
+        """device-resident: d_in n_in samples, d_out C rows of out_stride (default out_cap) complex64; asynchronous on
+        the handle's stream.  Returns the outputs written per channel."""
+        got = C.c_size_t(0)
+        check(lib().sdr_ddc_process_dev(self.h, _ptr(d_in), n_in, _ptr(d_out), out_cap,
+                                        out_cap if out_stride is None else out_stride, C.byref(got)),
+              "sdr_ddc_process_dev")
+        return got.value
+
+    def reset(self):
+        check(lib().sdr_ddc_reset(self.h), "sdr_ddc_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_ddc_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_ddc_clone")
+        return Ddc(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_ddc_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
