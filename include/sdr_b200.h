@@ -500,6 +500,60 @@ int sdr_ddc_process_dev(sdr_ddc_t *, const void *in, size_t n_in, float *out_c64
                         size_t *n_out);
 int sdr_ddc_last_path(const sdr_ddc_t *); /* path of the last call that produced outputs: 0 none, 1 CUDA-core, 2 tcgen05 */
 
+/* ======================================================================================
+ * averaged power spectra -- tapered, overlapped |FFT|^2 of one IQ stream, averaged over K frames.  Restates the
+ * crate chain window -> decimate -> map(fft::fft) -> |.|^2 -> mean of K (examples/live.rs:30-39 plus the power
+ * and mean a spectrum display computes): Window (adapters/mod.rs:271-303) and Decimate (mod.rs:14-41) give frame
+ * j = the N samples ending at input sample (j+1) H - 1, x[<0] = 0 (the deque's initial zeros; frames overlap when
+ * H < N and skip samples when H > N), and
+ *   X_j[k] = sum_n w[n] frame_j[n] e^{-2 pi i k n / N}        (times 1/sqrt(N) with SDR_PSD_NORM)
+ *   P_g[k] = (1/K) sum_{j = gK}^{gK+K-1} |X_j[k]|^2           (f32 rows; K = 1 is a waterfall)
+ * Summation order (part of the definition, so outputs are bit-identical however the stream is cut): group g is
+ * split into chunks of 32 consecutive frames anchored on its first frame; a chunk sums |X_j[k]|^2 in f32 in
+ * ascending j; the chunk partials are summed in f64 in chunk order, scaled by 1/K (and 1/N for NORM) in f64 and
+ * rounded to f32 once.
+ *   SDR_PSD_SHIFT          bin order of sdr_fft_labels(N, rate, 0)
+ *   SDR_PSD_NORM           the 1/sqrt(N) of sdr_fft, i.e. rows scaled by 1/N
+ *   SDR_PSD_GENERAL_KERNEL always path 1 (for testing; same bars, not bit-equal to path 2)
+ * Paths (sdr_psd_last_path): 2 = one fused kernel (1024-point warp FFT, |X|^2 accumulated in registers) plus a
+ * small f64 reduce, for N = 1024 and u8 / c64 input; 1 = gather and taper into L2-sized slabs, sdr_fft plan,
+ * accumulate, for every other N (any length sdr_fft_create accepts, Bluestein included).  Both meet the FFT bar
+ * carried through |.|^2: |P - P_f64| <= 2e-5 log2(N) max P per row.
+ * Carried state: the samples of the pending chunk's frames, the open group's f64 accumulator and the stream
+ * position.  The block and the carried tail are read through two pointers (the block is never copied); input
+ * pointers need only element alignment (2 bytes u8, 8 bytes c64).
+ * ====================================================================================== */
+#define SDR_PSD_SHIFT 1u
+#define SDR_PSD_NORM 2u
+#define SDR_PSD_GENERAL_KERNEL 4u
+
+typedef struct {
+    size_t n;             /* N >= 1, any length sdr_fft_create accepts */
+    size_t hop;           /* H >= 1 (0 is rejected, as for Decimate) */
+    size_t average;       /* K >= 1 */
+    const float *window;  /* N real taper values, or NULL = rectangular; copied at create */
+    int input_format;     /* U8IQ or C64 (F32 is rejected) */
+    unsigned flags;       /* SDR_PSD_* */
+    int device;
+    void *stream;
+} sdr_psd_config_t;
+
+typedef struct sdr_psd sdr_psd_t;
+sdr_psd_t *sdr_psd_create(const sdr_psd_config_t *cfg, int *err);
+void sdr_psd_destroy(sdr_psd_t *);
+int sdr_psd_reset(sdr_psd_t *); /* stream position, carried samples and open group back to the start */
+sdr_psd_t *sdr_psd_clone(const sdr_psd_t *, int *err);
+/* spectra the next n_in input samples complete */
+size_t sdr_psd_output_count(const sdr_psd_t *, size_t n_in);
+/* out: spectra of N f32, row stride out_stride floats (>= N), capacity out_cap spectra; a too-small out_cap returns
+ * SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  *n_spectra = spectra written. */
+int sdr_psd_process(sdr_psd_t *, const void *in, size_t n_in, float *out, size_t out_cap, size_t out_stride,
+                    size_t *n_spectra);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_psd_process_dev(sdr_psd_t *, const void *in, size_t n_in, float *out, size_t out_cap, size_t out_stride,
+                        size_t *n_spectra);
+int sdr_psd_last_path(const sdr_psd_t *); /* path of the last call that ran frames: 0 none, 1 plan + slab, 2 fused */
+
 #ifdef __cplusplus
 }
 #endif

@@ -826,6 +826,51 @@ class WindowSpectra {
     }
 };
 
+// window -> decimate -> map(fft::fft) -> |.|^2 -> mean of `average` behind sdr_psd_*: feed blocks of samples, get the
+// averaged power spectra (n floats each, bins shifted like fft::fft, scaled 1/n like its 1/sqrt(n)) back to back.
+// taper: n real values or empty (rectangular).  Copies with sdr_psd_clone.
+class PowerSpectra {
+    sdr_psd_t *h_ = nullptr;
+    size_t n_ = 0;
+
+  public:
+    PowerSpectra(size_t n, size_t hop, size_t average, const std::vector<float> &taper = {}, bool u8iq = false,
+                 unsigned flags = SDR_PSD_SHIFT | SDR_PSD_NORM)
+        : n_(n) {
+        if (!taper.empty() && taper.size() != n) throw Error(SDR_ERR_INVALID_ARG, "PowerSpectra::new");
+        sdr_psd_config_t cfg{};
+        cfg.n = n;
+        cfg.hop = hop;
+        cfg.average = average;
+        cfg.window = taper.empty() ? nullptr : taper.data();
+        cfg.input_format = u8iq ? SDR_FMT_U8IQ : SDR_FMT_C64;
+        cfg.flags = flags;
+        int err = 0;
+        h_ = sdr_psd_create(&cfg, &err);
+        if (!h_) throw Error(err, "PowerSpectra::new");
+    }
+    PowerSpectra(const PowerSpectra &o) : n_(o.n_) {
+        int err = 0;
+        h_ = sdr_psd_clone(o.h_, &err);
+        if (!h_) throw Error(err, "PowerSpectra::clone");
+    }
+    PowerSpectra &operator=(const PowerSpectra &) = delete;
+    ~PowerSpectra() { sdr_psd_destroy(h_); }
+    size_t bins() const { return n_; }
+    int last_path() const { return sdr_psd_last_path(h_); }
+    // in: n samples (Complex, or 2n bytes when constructed with u8iq); returns the number of spectra appended to out
+    size_t process(const void *in, size_t n, std::vector<float> &out) {
+        const size_t ns = sdr_psd_output_count(h_, n);
+        const size_t at = out.size();
+        out.resize(at + ns * n_);
+        size_t got = 0;
+        float dummy;
+        check(sdr_psd_process(h_, in, n, ns ? out.data() + at : &dummy, ns, n_, &got), "PowerSpectra::process");
+        return got;
+    }
+    void reset() { check(sdr_psd_reset(h_), "PowerSpectra::reset"); }
+};
+
 }  // namespace fft
 
 // =========================================================================================

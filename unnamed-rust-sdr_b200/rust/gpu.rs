@@ -214,6 +214,56 @@ impl Drop for GpuDdc {
     fn drop(&mut self) { unsafe { sdr_ddc_destroy(self.h) } }
 }
 
+/// window(n) -> decimate(hop) -> map(fft::fft) -> |.|^2 -> mean of `average` behind sdr_psd_*: averaged power spectra
+/// of n f32 bins (shifted and 1/n-scaled like fft::fft's 1/sqrt(n) with SDR_PSD_SHIFT | SDR_PSD_NORM).  taper: n real
+/// values or empty (rectangular).  `process` appends the spectra the block completes; blocks of any size give the same
+/// bits as one call.
+pub struct GpuPsd {
+    h: *mut sdr_psd_t,
+    n: usize,
+}
+unsafe impl Send for GpuPsd {}
+
+impl GpuPsd {
+    pub fn new(n: usize, hop: usize, average: usize, taper: &[f32], input_u8iq: bool, flags: u32) -> Result<Self, Error> {
+        if !taper.is_empty() && taper.len() != n { return Err(Error(100)); }  // SDR_ERR_INVALID_ARG: the C side copies n values
+        let cfg = sdr_psd_config_t {
+            n, hop, average, window: if taper.is_empty() { std::ptr::null() } else { taper.as_ptr() },
+            input_format: if input_u8iq { SDR_FMT_U8IQ } else { SDR_FMT_C64 }, flags, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_psd_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuPsd { h, n })
+    }
+    /// input: m samples (Complex<f32>, or 2m rtl_tcp bytes); the spectra are appended to output
+    pub fn process<T: Copy>(&mut self, input: &[T], m: usize, output: &mut Vec<f32>) -> Result<usize, Error> {
+        let ns = unsafe { sdr_psd_output_count(self.h, m) };
+        let at = output.len();
+        output.resize(at + ns.max(1) * self.n, 0.0);
+        let mut got = 0usize;
+        check(unsafe {
+            sdr_psd_process(self.h, input.as_ptr() as *const c_void, m, output[at..].as_mut_ptr(), ns, self.n, &mut got)
+        })?;
+        output.truncate(at + got * self.n);
+        Ok(got)
+    }
+    pub fn last_path(&self) -> i32 { unsafe { sdr_psd_last_path(self.h) } }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_psd_reset(self.h) }) }
+}
+impl Clone for GpuPsd {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_psd_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_psd_clone failed: {}", Error(err));
+        GpuPsd { h, n: self.n }
+    }
+}
+impl Drop for GpuPsd {
+    fn drop(&mut self) { unsafe { sdr_psd_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

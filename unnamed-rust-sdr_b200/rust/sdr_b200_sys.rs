@@ -23,6 +23,10 @@ pub const SDR_PFB_CHANNEL_MAJOR: c_uint = 2;
 pub const SDR_PFB_GENERAL_KERNEL: c_uint = 4;
 /// sdr_ddc_config_t.flags
 pub const SDR_DDC_GENERAL_KERNEL: c_uint = 1;
+/// sdr_psd_config_t.flags
+pub const SDR_PSD_SHIFT: c_uint = 1;
+pub const SDR_PSD_NORM: c_uint = 2;
+pub const SDR_PSD_GENERAL_KERNEL: c_uint = 4;
 
 pub enum sdr_fir_t {}
 pub enum sdr_fft_t {}
@@ -32,6 +36,7 @@ pub enum sdr_fm_t {}
 pub enum sdr_window_fft_t {}
 pub enum sdr_pfb_t {}
 pub enum sdr_ddc_t {}
+pub enum sdr_psd_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -129,6 +134,18 @@ pub struct sdr_ddc_config_t {
     pub n_channels: size_t,
     pub decimation: size_t,
     pub first_sample: u64,
+    pub input_format: c_int,
+    pub flags: c_uint,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+pub struct sdr_psd_config_t {
+    pub n: size_t,
+    pub hop: size_t,
+    pub average: size_t,
+    pub window: *const c_float,
     pub input_format: c_int,
     pub flags: c_uint,
     pub device: c_int,
@@ -239,6 +256,16 @@ extern "C" {
     pub fn sdr_ddc_process_dev(h: *mut sdr_ddc_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
                                out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_ddc_last_path(h: *const sdr_ddc_t) -> c_int;
+    pub fn sdr_psd_create(cfg: *const sdr_psd_config_t, err: *mut c_int) -> *mut sdr_psd_t;
+    pub fn sdr_psd_destroy(h: *mut sdr_psd_t);
+    pub fn sdr_psd_reset(h: *mut sdr_psd_t) -> c_int;
+    pub fn sdr_psd_clone(h: *const sdr_psd_t, err: *mut c_int) -> *mut sdr_psd_t;
+    pub fn sdr_psd_output_count(h: *const sdr_psd_t, n_in: size_t) -> size_t;
+    pub fn sdr_psd_process(h: *mut sdr_psd_t, input: *const c_void, n_in: size_t, out: *mut c_float, out_cap: size_t,
+                           out_stride: size_t, n_spectra: *mut size_t) -> c_int;
+    pub fn sdr_psd_process_dev(h: *mut sdr_psd_t, input: *const c_void, n_in: size_t, out: *mut c_float,
+                               out_cap: size_t, out_stride: size_t, n_spectra: *mut size_t) -> c_int;
+    pub fn sdr_psd_last_path(h: *const sdr_psd_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -14,6 +14,7 @@ PLL_F64_MATH = 2
 PLL_GENERAL_KERNEL = 4
 PFB_SHIFT, PFB_CHANNEL_MAJOR, PFB_GENERAL_KERNEL = 1, 2, 4
 DDC_GENERAL_KERNEL = 1
+PSD_SHIFT, PSD_NORM, PSD_GENERAL_KERNEL = 1, 2, 4
 BQ_IDENTITY, BQ_LOWPASS, BQ_HIGHPASS, BQ_BANDPASS, BQ_NOTCH, BQ_LR = range(6)
 SRC_SINC_BEST_QUALITY, SRC_SINC_MEDIUM_QUALITY, SRC_SINC_FASTEST, SRC_ZERO_ORDER_HOLD, SRC_LINEAR = range(5)
 
@@ -65,6 +66,11 @@ class PfbConfig(C.Structure):
 class DdcConfig(C.Structure):
     _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phase_inc", vp), ("n_channels", sz),
                 ("decimation", sz), ("first_sample", C.c_uint64), ("input_format", i32), ("flags", C.c_uint),
+                ("device", i32), ("stream", vp)]
+
+
+class PsdConfig(C.Structure):
+    _fields_ = [("n", sz), ("hop", sz), ("average", sz), ("window", vp), ("input_format", i32), ("flags", C.c_uint),
                 ("device", i32), ("stream", vp)]
 
 
@@ -132,6 +138,14 @@ PROTOTYPES = {
     "sdr_ddc_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_ddc_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_ddc_last_path": (i32, [vp]),
+    "sdr_psd_create": (vp, [C.POINTER(PsdConfig), C.POINTER(i32)]),
+    "sdr_psd_destroy": (None, [vp]),
+    "sdr_psd_reset": (i32, [vp]),
+    "sdr_psd_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_psd_output_count": (sz, [vp, sz]),
+    "sdr_psd_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_psd_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_psd_last_path": (i32, [vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -596,6 +596,82 @@ class Ddc:
     __del__ = close
 
 
+class Psd:
+    """Averaged power spectra (sdr_psd): window(n) -> decimate(hop) -> map(fft::fft) -> |.|^2 -> mean of `average`
+    frames.  Frame j holds the n samples ending at input sample (j + 1) * hop - 1 (x[<0] = 0), tapered by `window`
+    (n real values, None = rectangular); spectrum g is the mean of |X_j|^2 over frames g*average .. g*average +
+    average - 1, as float32 rows of n bins.  shift / norm as for FftPlan (norm scales the rows by 1/n).  average=1 is a
+    waterfall.  general=True forces the plan + slab path (path 1) where the fused 1024-point kernel (path 2) would run."""
+
+    def __init__(self, n, hop, average, window=None, fmt="u8iq", shift=True, norm=True, general=False, device=0,
+                 stream=None, _handle=None, _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        self.n, self.hop, self.average = int(n), int(hop), int(average)
+        self.fmt = _FMT_OF[fmt] if isinstance(fmt, str) else int(fmt)
+        self._window = None if window is None else np.ascontiguousarray(window, np.float32)
+        if self._window is not None and self._window.size != self.n:
+            raise ValueError("window must hold n taper values")
+        flags = (F.PSD_SHIFT if shift else 0) | (F.PSD_NORM if norm else 0) | (F.PSD_GENERAL_KERNEL if general else 0)
+        cfg = F.PsdConfig(self.n, self.hop, self.average, None if self._window is None else self._window.ctypes.data,
+                          self.fmt, flags, device, _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_psd_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_psd_create")
+
+    def output_count(self, n_in):
+        return lib().sdr_psd_output_count(self.h, n_in)
+
+    @property
+    def last_path(self):
+        """path of the last call that ran frames: 0 none, 1 plan + slab, 2 fused 1024-point kernel"""
+        return lib().sdr_psd_last_path(self.h)
+
+    def process(self, x):
+        """x: uint8 [2m] (u8iq) or complex64 [m] -> float32 [spectra, n]"""
+        if self.fmt == F.FMT_U8IQ:
+            x = np.ascontiguousarray(x, np.uint8)
+            m = x.size // 2
+        else:
+            x = np.ascontiguousarray(x, np.complex64)
+            m = x.size
+        cap = max(self.output_count(m), 1)
+        out = np.empty((cap, self.n), np.float32)
+        got = C.c_size_t(0)
+        check(lib().sdr_psd_process(self.h, x.ctypes.data if m else None, m, out.ctypes.data, cap, self.n,
+                                    C.byref(got)), "sdr_psd_process")
+        return out[:got.value]
+
+    def process_dev(self, d_in, n_in, d_out, out_cap, out_stride=None):
+        """device-resident: d_in n_in samples, d_out rows of out_stride (default n) float32; asynchronous on the
+        handle's stream.  Returns the spectra written."""
+        got = C.c_size_t(0)
+        check(lib().sdr_psd_process_dev(self.h, _ptr(d_in), n_in, _ptr(d_out), out_cap,
+                                        self.n if out_stride is None else out_stride, C.byref(got)),
+              "sdr_psd_process_dev")
+        return got.value
+
+    def reset(self):
+        check(lib().sdr_psd_reset(self.h), "sdr_psd_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_psd_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_psd_clone")
+        return Psd(None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_psd_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->

@@ -741,3 +741,26 @@ def window_spectra(signal, duration, fps, block=DEFAULT_BLOCK):
                 yield labels, s
     finally:
         wf.close()
+
+
+def power_spectra(signal, duration, fps, average, window=None, block=DEFAULT_BLOCK):
+    """The power counterpart of window_spectra: signal.window(duration).decimate(fps).map(fft::fft), |.|^2 and the
+    mean of `average` consecutive spectra, as a generator of (labels, power[n_spectra, window]) per input block.
+    window = round(duration * rate), hop = Decimate's wait, as window_spectra; `window` (the taper) is that many real
+    values or None (rectangular).  Raw u8 IQ sources are fed as bytes and unpacked on the device."""
+    rate = float(signal.rate())
+    n = ops.duration_samples(rate, duration)
+    hop = ops.decimate_wait(rate, fps)
+    raw = _has_raw(signal)
+    psd = ops.Psd(n, hop, average, window, "u8iq" if raw else "c64")
+    labels = ops.fft_labels(n, rate)
+    try:
+        while True:
+            b = signal.next_raw(block) if raw else signal.next_block(block)
+            if len(b) == 0:
+                return
+            p = psd.process(b)
+            if len(p):
+                yield labels, p
+    finally:
+        psd.close()
