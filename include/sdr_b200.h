@@ -554,6 +554,62 @@ int sdr_psd_process_dev(sdr_psd_t *, const void *in, size_t n_in, float *out, si
                         size_t *n_spectra);
 int sdr_psd_last_path(const sdr_psd_t *); /* path of the last call that ran frames: 0 none, 1 plan + slab, 2 fused */
 
+/* ======================================================================================
+ * fast-convolution channel bank -- sdr_ddc's channels with one decimation per channel, computed by overlap-save, so
+ * that the cost barely depends on the filter length and is the same for u8 and c64 input.  Channel k restates a tee'd
+ * copy of the stream, a caller-written oscillator (Signal::map), filter::Fir<Complex<f32>, f32> (src/filter/fir.rs:23-32)
+ * with taps h_k and signal::Decimate with wait D_k (adapters/mod.rs:30-37); F = first_sample:
+ *   z_k[n] = x[n] e^{-2 pi i phi_k(F + n) / 2^64},   phi_k(N) = N phase_inc[k]  mod 2^64
+ *   y_k[m] = sum_{j<L} h_k[j] z_k[(m+1) D_k - 1 - j],   x[<0] = 0 (byte 128 for u8, as fir.rs:15)
+ * With every D_k = D this is sdr_ddc's function.  Computed in the rotated-taps form by overlap-save on blocks of the
+ * ABSOLUTE stream grid: Dl = lcm(D_k), N = the smallest power of two >= 1024 with hop P = floor((N - L + 1) / Dl) Dl
+ * >= N / 2 (sdr_fcfb_geometry; SDR_ERR_UNSUPPORTED when N would exceed 2^22).  Block b holds the outputs at absolute
+ * indices [b P + eps, (b+1) P + eps), eps = F mod Dl, and is computed from the N inputs that end at its last output:
+ * one N-point FFT shared by all channels, a per-channel spectral multiply folded by the power-of-two part of D_k, one
+ * small inverse FFT per channel and an exact 64-bit NCO derotation.
+ * Release: a block's outputs are written by the call that delivers its last input, so outputs come up to P - 1 samples
+ * later than sdr_ddc releases them; sdr_fcfb_output_count gives the per-channel counts.  To drain a finite stream, feed
+ * N zeros (the n_fft of sdr_fcfb_geometry) after it and drop the outputs past the stream's end.
+ * Bits: an output depends only on its block's N samples and its absolute position, so blockings (1-sample calls, calls
+ * that end mid-block), addresses and clones give the bits of one call.  A shard gives the same bits when it is cut on a
+ * block boundary of the absolute grid, its halo is at least N - P rounded up to a multiple of Dl, and its first_sample
+ * is the halo's absolute index.  A non-finite sample poisons every output, in every channel, of each block whose span
+ * holds it, and no other output.
+ * Accuracy: per channel |y - y_f64| <= 2e-5 log2(N) max|y_f64| on signals that fill the channel; FFT round-off follows
+ * the block's total power, |y_k - y_f64| <~ 1e-7 log2(N) ||h_k||_2 rms(block) (DESIGN.md K9).
+ * Output: C rows (channel-major), row stride out_stride c64 elements (>= the largest count), out_cap outputs per row;
+ * a too-small out_cap returns SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  *n_out receives C counts.
+ * Carried state: fewer than N raw inputs and the stream position; the block and the carried tail are read through two
+ * pointers (the block is never copied); input pointers need only element alignment (2 bytes u8, 8 bytes c64).
+ * ====================================================================================== */
+typedef struct {
+    const float *taps;         /* n_tap_sets rows of n_taps real f32 */
+    size_t n_taps;             /* L, 1 <= L <= 2^20 */
+    size_t n_tap_sets;         /* 1 (shared) or n_channels */
+    const uint64_t *phase_inc; /* n_channels NCO increments (sdr_ddc_phase_increment) */
+    const size_t *decimation;  /* n_channels decimations D_k >= 1 */
+    size_t n_channels;         /* C, 1 <= C <= 256 */
+    uint64_t first_sample;     /* absolute stream index of the first input: NCO phase and block grid */
+    int input_format;          /* U8IQ or C64 (F32 is rejected) */
+    int device;
+    void *stream;
+} sdr_fcfb_config_t;
+
+typedef struct sdr_fcfb sdr_fcfb_t;
+/* host, pure: the transform size N and hop P the bank uses for these taps and decimations */
+int sdr_fcfb_geometry(size_t n_taps, const size_t *decimation, size_t n_channels, size_t *n_fft, size_t *hop);
+sdr_fcfb_t *sdr_fcfb_create(const sdr_fcfb_config_t *cfg, int *err);
+void sdr_fcfb_destroy(sdr_fcfb_t *);
+int sdr_fcfb_reset(sdr_fcfb_t *); /* carried samples dropped, position back to first_sample */
+sdr_fcfb_t *sdr_fcfb_clone(const sdr_fcfb_t *, int *err);
+/* counts[k] = channel k's outputs in the blocks that the next n_in input samples complete (C entries) */
+int sdr_fcfb_output_count(const sdr_fcfb_t *, size_t n_in, size_t *counts);
+int sdr_fcfb_process(sdr_fcfb_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap, size_t out_stride,
+                     size_t *n_out);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_fcfb_process_dev(sdr_fcfb_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap,
+                         size_t out_stride, size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

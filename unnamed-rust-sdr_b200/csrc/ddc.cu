@@ -32,6 +32,7 @@
 #include <vector>
 
 #include "kernels.h"
+#include "nco.cuh"
 
 using namespace sdr;
 
@@ -101,13 +102,6 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo, uint
 }
 // 64-byte rows: SWIZZLE_64B (the A descriptor's layout type 4)
 __device__ __forceinline__ uint32_t swz64(uint32_t o) { return o ^ (((o >> 7) & 3u) << 4); }
-
-// e^{-2 pi i phi / 2^64} from the exact 64-bit phase (phi read as signed: one turn = 2^64)
-__device__ __forceinline__ float2 nco_rot(uint64_t phi) {
-    double s, c;
-    sincospi((double)(long long)phi * 0x1p-63, &s, &c);
-    return make_float2((float)c, (float)-s);
-}
 
 // stage = the window starts of one tile's 128 rows (64 bytes apart) + the KS * 32-byte halo of the last row
 __host__ __device__ constexpr int ddc_stage_bytes(int KS) { return (64 * 127 + 32 * KS + 1023) / 1024 * 1024; }
@@ -384,11 +378,6 @@ __global__ void __launch_bounds__(256) ddc_general_kernel(DdcSrc src, const floa
         if (c < nc) out[(long long)(c0 + c) * out_stride + m] = cmul(nco_rot(n * __ldg(inc + c0 + c)), make_float2(ar[c], ai[c]));
 }
 
-constexpr double DDC_2PI = 6.283185307179586476925286766559;
-
-// phase in turns, read as signed: (-1/2, 1/2]
-double phase_turns(uint64_t phi) { return (double)(long long)phi * 0x1p-64; }
-
 }  // namespace
 
 extern "C" uint64_t sdr_ddc_phase_increment(double freq, double rate) {
@@ -469,13 +458,7 @@ static bool ddc_tc_geometry(sdr_ddc *h) {
 
 // complex taps g_k[j] = h_k[j] e^{+2 pi i (j Delta_k mod 2^64) / 2^64}, rounded to f32 from f64
 static void ddc_rotated_taps(const sdr_ddc *h, size_t k, std::vector<float> &g) {
-    const float *hk = h->taps.data() + (h->n_sets == 1 ? 0 : k * h->L);
-    g.resize(2 * h->L);
-    for (size_t j = 0; j < h->L; ++j) {
-        const double t = DDC_2PI * phase_turns((uint64_t)j * h->inc[k]);
-        g[2 * j] = (float)((double)hk[j] * std::cos(t));
-        g[2 * j + 1] = (float)((double)hk[j] * std::sin(t));
-    }
+    nco_rotated_taps(h->taps.data() + (h->n_sets == 1 ? 0 : k * h->L), h->L, h->inc[k], g);
 }
 
 // tables, taps and history buffers of a handle whose configuration fields are set
@@ -520,7 +503,7 @@ static int ddc_alloc(sdr_ddc *h, void *user_stream) {
                 }
             chan[k] = DdcChan{{magic[0][0], magic[1][0]}, {magic[0][2], magic[1][2]}, sc[0], sc[2]};
             for (int j = 0; j < TR; ++j) {
-                const double t = DDC_2PI * phase_turns(((uint64_t)h->D * j + h->D - 1) * h->inc[k]);
+                const double t = NCO_2PI * nco_turns(((uint64_t)h->D * j + h->D - 1) * h->inc[k]);
                 rot[2 * (k * TR + j)] = (float)std::cos(t);
                 rot[2 * (k * TR + j) + 1] = (float)-std::sin(t);
             }

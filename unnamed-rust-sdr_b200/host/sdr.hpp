@@ -21,6 +21,7 @@
 // Errors: the reference returns Result and its adaptors unwrap() (panic); here constructors / process
 // throw sdr::Error / sdr::resample::Error, which is the same "abort the pipeline" behaviour.
 #pragma once
+#include <algorithm>
 #include <complex>
 #include <cstdint>
 #include <deque>
@@ -272,6 +273,59 @@ class Ddc {
         return got;
     }
     void reset() { check(sdr_ddc_reset(h_), "Ddc::reset"); }
+};
+
+// Fast-convolution channel bank (sdr_fcfb): Ddc's channels with one decimation per channel, computed by overlap-save.
+// Outputs are released per block of P inputs (sdr_fcfb_geometry); feed N zeros to drain a finite stream.
+class Fcfb {
+    sdr_fcfb_t *h_ = nullptr;
+    size_t c_ = 0;
+
+  public:
+    Fcfb(const std::vector<float> &taps, size_t n_taps, const std::vector<double> &freqs, double rate,
+         const std::vector<size_t> &decimation, bool input_u8iq = true, uint64_t first_sample = 0)
+        : c_(freqs.size()) {
+        std::vector<uint64_t> inc(freqs.size());
+        for (size_t k = 0; k < freqs.size(); ++k) inc[k] = sdr_ddc_phase_increment(freqs[k], rate);
+        if (decimation.size() != freqs.size()) throw sdr::Error(SDR_ERR_INVALID_ARG, "Fcfb::new");
+        sdr_fcfb_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.phase_inc = inc.data();
+        cfg.decimation = decimation.data();
+        cfg.n_channels = freqs.size();
+        cfg.first_sample = first_sample;
+        cfg.input_format = input_u8iq ? SDR_FMT_U8IQ : SDR_FMT_C64;
+        int err = 0;
+        h_ = sdr_fcfb_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Fcfb::new");
+    }
+    Fcfb(Fcfb &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
+    Fcfb(const Fcfb &o) : c_(o.c_) {
+        int err = 0;
+        h_ = sdr_fcfb_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Fcfb::clone");
+    }
+    Fcfb &operator=(const Fcfb &) = delete;
+    ~Fcfb() { sdr_fcfb_destroy(h_); }
+    size_t channels() const { return c_; }
+    std::vector<size_t> output_count(size_t n_in) const {
+        std::vector<size_t> cnt(c_);
+        check(sdr_fcfb_output_count(h_, n_in, cnt.data()), "Fcfb::output_count");
+        return cnt;
+    }
+    // in: n samples (Complex, or 2n rtl_tcp bytes when constructed with input_u8iq).  out: one vector per channel, replaced.
+    void process(const void *in, size_t n, std::vector<std::vector<Complex>> &out) {
+        const std::vector<size_t> cnt = output_count(n);
+        const size_t cap = std::max<size_t>(1, *std::max_element(cnt.begin(), cnt.end()));
+        std::vector<Complex> rows(cap * c_);
+        std::vector<size_t> got(c_);
+        check(sdr_fcfb_process(h_, in, n, reinterpret_cast<float *>(rows.data()), cap, cap, got.data()), "Fcfb::process");
+        out.assign(c_, {});
+        for (size_t k = 0; k < c_; ++k) out[k].assign(rows.begin() + k * cap, rows.begin() + k * cap + got[k]);
+    }
+    void reset() { check(sdr_fcfb_reset(h_), "Fcfb::reset"); }
 };
 
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity

@@ -264,6 +264,61 @@ impl Drop for GpuPsd {
     fn drop(&mut self) { unsafe { sdr_psd_destroy(self.h) } }
 }
 
+/// Fast-convolution channel bank: GpuDdc's channels with one decimation per channel, by overlap-save.  Outputs are
+/// released per block of P inputs (sdr_fcfb_geometry); feed N zeros to drain a finite stream.
+pub struct GpuFcfb {
+    h: *mut sdr_fcfb_t,
+    c: usize,
+}
+unsafe impl Send for GpuFcfb {}
+
+impl GpuFcfb {
+    /// taps: one row of n_taps (shared) or one row per channel; freqs in Hz at `rate`; one decimation per channel
+    pub fn new(taps: &[f32], n_taps: usize, freqs: &[f64], rate: f64, decimation: &[usize], input_u8iq: bool,
+               first_sample: u64) -> Result<Self, Error> {
+        if decimation.len() != freqs.len() || n_taps == 0 { return Err(Error(100)); }
+        let inc: Vec<u64> = freqs.iter().map(|&f| unsafe { sdr_ddc_phase_increment(f, rate) }).collect();
+        let cfg = sdr_fcfb_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: taps.len() / n_taps, phase_inc: inc.as_ptr(),
+            decimation: decimation.as_ptr(), n_channels: freqs.len(), first_sample,
+            input_format: if input_u8iq { SDR_FMT_U8IQ } else { SDR_FMT_C64 }, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_fcfb_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuFcfb { h, c: freqs.len() })
+    }
+    /// input: m samples (Complex<f32>, or 2m rtl_tcp bytes); channel k's released outputs are appended to output[k]
+    pub fn process<T: Copy>(&mut self, input: &[T], m: usize, output: &mut [Vec<Complex<f32>>]) -> Result<(), Error> {
+        let mut cnt = vec![0usize; self.c];
+        check(unsafe { sdr_fcfb_output_count(self.h, m, cnt.as_mut_ptr()) })?;
+        let cap = cnt.iter().copied().max().unwrap_or(0).max(1);
+        let mut rows = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut got = vec![0usize; self.c];
+        check(unsafe {
+            sdr_fcfb_process(self.h, input.as_ptr() as *const c_void, m, rows.as_mut_ptr() as *mut f32, cap, cap,
+                             got.as_mut_ptr())
+        })?;
+        for (k, out) in output.iter_mut().enumerate().take(self.c) {
+            out.extend_from_slice(&rows[k * cap..k * cap + got[k]]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_fcfb_reset(self.h) }) }
+}
+impl Clone for GpuFcfb {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_fcfb_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_fcfb_clone failed: {}", Error(err));
+        GpuFcfb { h, c: self.c }
+    }
+}
+impl Drop for GpuFcfb {
+    fn drop(&mut self) { unsafe { sdr_fcfb_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

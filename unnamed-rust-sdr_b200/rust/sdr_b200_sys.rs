@@ -37,6 +37,7 @@ pub enum sdr_window_fft_t {}
 pub enum sdr_pfb_t {}
 pub enum sdr_ddc_t {}
 pub enum sdr_psd_t {}
+pub enum sdr_fcfb_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -148,6 +149,20 @@ pub struct sdr_psd_config_t {
     pub window: *const c_float,
     pub input_format: c_int,
     pub flags: c_uint,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+pub struct sdr_fcfb_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub phase_inc: *const u64,
+    pub decimation: *const size_t,
+    pub n_channels: size_t,
+    pub first_sample: u64,
+    pub input_format: c_int,
     pub device: c_int,
     pub stream: *mut c_void,
 }
@@ -266,6 +281,17 @@ extern "C" {
     pub fn sdr_psd_process_dev(h: *mut sdr_psd_t, input: *const c_void, n_in: size_t, out: *mut c_float,
                                out_cap: size_t, out_stride: size_t, n_spectra: *mut size_t) -> c_int;
     pub fn sdr_psd_last_path(h: *const sdr_psd_t) -> c_int;
+    pub fn sdr_fcfb_geometry(n_taps: size_t, decimation: *const size_t, n_channels: size_t, n_fft: *mut size_t,
+                             hop: *mut size_t) -> c_int;
+    pub fn sdr_fcfb_create(cfg: *const sdr_fcfb_config_t, err: *mut c_int) -> *mut sdr_fcfb_t;
+    pub fn sdr_fcfb_destroy(h: *mut sdr_fcfb_t);
+    pub fn sdr_fcfb_reset(h: *mut sdr_fcfb_t) -> c_int;
+    pub fn sdr_fcfb_clone(h: *const sdr_fcfb_t, err: *mut c_int) -> *mut sdr_fcfb_t;
+    pub fn sdr_fcfb_output_count(h: *const sdr_fcfb_t, n_in: size_t, counts: *mut size_t) -> c_int;
+    pub fn sdr_fcfb_process(h: *mut sdr_fcfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
+                            out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_fcfb_process_dev(h: *mut sdr_fcfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
+                                out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -74,6 +74,12 @@ class PsdConfig(C.Structure):
                 ("device", i32), ("stream", vp)]
 
 
+class FcfbConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phase_inc", vp), ("decimation", vp),
+                ("n_channels", sz), ("first_sample", C.c_uint64), ("input_format", i32), ("device", i32),
+                ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -146,6 +152,14 @@ PROTOTYPES = {
     "sdr_psd_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_psd_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_psd_last_path": (i32, [vp]),
+    "sdr_fcfb_geometry": (i32, [sz, vp, sz, C.POINTER(sz), C.POINTER(sz)]),
+    "sdr_fcfb_create": (vp, [C.POINTER(FcfbConfig), C.POINTER(i32)]),
+    "sdr_fcfb_destroy": (None, [vp]),
+    "sdr_fcfb_reset": (i32, [vp]),
+    "sdr_fcfb_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_fcfb_output_count": (i32, [vp, sz, vp]),
+    "sdr_fcfb_process": (i32, [vp, vp, sz, vp, sz, sz, vp]),
+    "sdr_fcfb_process_dev": (i32, [vp, vp, sz, vp, sz, sz, vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

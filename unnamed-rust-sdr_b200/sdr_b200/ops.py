@@ -672,6 +672,101 @@ class Psd:
     __del__ = close
 
 
+def fcfb_geometry(n_taps, decimations):
+    """(N, P): the transform size and hop sdr_fcfb uses for n_taps taps and these per-channel decimations"""
+    d = np.ascontiguousarray(np.atleast_1d(decimations), np.uintp)
+    n, p = C.c_size_t(0), C.c_size_t(0)
+    check(lib().sdr_fcfb_geometry(int(n_taps), d.ctypes.data, d.size, C.byref(n), C.byref(p)), "sdr_fcfb_geometry")
+    return n.value, p.value
+
+
+class Fcfb:
+    """Fast-convolution channel bank (sdr_fcfb): channel k of one IQ stream is mixed down by freqs[k] (a 64-bit NCO),
+    filtered by its real taps (taps 1-D: shared; [C, L]: one row per channel) and decimated by decimation[k] (one value
+    or one per channel) -- sdr_ddc's channel with its own D -- computed by overlap-save on blocks of N inputs.  Outputs
+    are released per block of P inputs (see geometry); process returns a list of C complex64 arrays.  To drain a finite
+    stream feed N zeros and drop the outputs past its end."""
+
+    def __init__(self, taps, freqs, rate, decimation, input_format="u8iq", first_sample=0, device=0, stream=None,
+                 _handle=None, _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        self._taps = t
+        self.phase_inc = np.array([ddc_phase_increment(f, rate) for f in np.atleast_1d(freqs)], np.uint64)
+        self.n_channels = int(self.phase_inc.size)
+        d = np.atleast_1d(np.asarray(decimation, np.int64))
+        if d.size == 1:
+            d = np.repeat(d, self.n_channels)
+        if d.size != self.n_channels or (d < 1).any():
+            raise ValueError("decimation: one value >= 1, or one per channel")
+        self.decimation = np.ascontiguousarray(d, np.uintp)
+        self.fmt = _FMT_OF[input_format] if isinstance(input_format, str) else int(input_format)
+        cfg = F.FcfbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
+                           self.decimation.ctypes.data, self.n_channels, int(first_sample), self.fmt, device,
+                           _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_fcfb_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_fcfb_create")
+
+    @property
+    def geometry(self):
+        """(N, P): transform size and hop (inputs per block)"""
+        return fcfb_geometry(self._taps.shape[-1], self.decimation)
+
+    def output_count(self, n_in):
+        """outputs per channel (numpy array of C) of the blocks that the next n_in inputs complete"""
+        cnt = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_fcfb_output_count(self.h, n_in, cnt.ctypes.data), "sdr_fcfb_output_count")
+        return cnt.astype(np.int64)
+
+    def process(self, x):
+        """x: uint8 [2n] (u8iq) or complex64 [n] -> list of C complex64 arrays"""
+        if self.fmt == F.FMT_U8IQ:
+            x = np.ascontiguousarray(x, np.uint8)
+            n = x.size // 2
+        else:
+            x = np.ascontiguousarray(x, np.complex64)
+            n = x.size
+        cap = max(int(self.output_count(n).max()), 1)
+        out = np.empty((self.n_channels, cap), np.complex64)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_fcfb_process(self.h, x.ctypes.data if n else None, n, out.ctypes.data, cap, cap,
+                                     got.ctypes.data), "sdr_fcfb_process")
+        return [out[k, :int(got[k])] for k in range(self.n_channels)]
+
+    def process_dev(self, d_in, n_in, d_out, out_cap, out_stride=None):
+        """device-resident: d_in n_in samples, d_out C rows of out_stride (default out_cap) complex64; asynchronous on
+        the handle's stream.  Returns the outputs written per channel (numpy array of C)."""
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_fcfb_process_dev(self.h, _ptr(d_in), n_in, _ptr(d_out), out_cap,
+                                         out_cap if out_stride is None else out_stride, got.ctypes.data),
+              "sdr_fcfb_process_dev")
+        return got.astype(np.int64)
+
+    def reset(self):
+        check(lib().sdr_fcfb_reset(self.h), "sdr_fcfb_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_fcfb_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_fcfb_clone")
+        return Fcfb(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_fcfb_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
