@@ -610,6 +610,58 @@ int sdr_fcfb_process(sdr_fcfb_t *, const void *in, size_t n_in, float *out_c64, 
 int sdr_fcfb_process_dev(sdr_fcfb_t *, const void *in, size_t n_in, float *out_c64, size_t out_cap,
                          size_t out_stride, size_t *n_out);
 
+/* ======================================================================================
+ * polyphase synthesis filter bank -- M channel streams recombined into one wideband stream at D times
+ * the frame rate; the inverse of sdr_pfb.  Channel k (sample m, k < M) is zero-stuffed by D with sample
+ * m at index (m+1) D - 1, filtered by filter::Fir<Complex<f32>, Complex<f32>> (src/filter/fir.rs:23-32)
+ * with taps f_k[n] = f[n] e^{+2 pi i k n / M}, and all channels are summed:
+ *   xh[t] = sum_m sum_k f_k[t - (m+1) D + 1] y_k[m],   0 <= t - (m+1) D + 1 < L
+ * Computed in polyphase form: V_m[r] = Y_m[(-r) mod M] with Y_m the unnormalised forward M-point DFT of
+ * frame m (the sdr_fft plan), then
+ *   xh[t] = sum_{n < L, n = t+1 (mod D)} f[n] V_{(t+1-n)/D - 1}[n mod M]
+ * as one fmaf chain per component in ascending n (a tap of 0.0 is still multiplied, so NaNs propagate
+ * exactly), frames before the stream being zero.  Accuracy is the FFT's (DESIGN.md).
+ * Release: frame m completes outputs [m D, (m+1) D), so n frames give exactly n D outputs; the filter
+ * tail comes out when ceil((L-1)/D) zero frames follow.  There is no scale: with an analysis prototype
+ * h and a synthesis prototype f of unit DC gain, f must carry a factor D for unit round-trip gain.
+ *   SDR_PFS_SHIFT          row i of a frame is channel (i - M/2) mod M, as SDR_PFB_SHIFT writes it
+ *   SDR_PFS_CHANNEL_MAJOR  M rows of frames, row stride in_stride (>= frames given), as
+ *                          SDR_PFB_CHANNEL_MAJOR writes them; otherwise frames of M, frame stride
+ *                          in_stride (>= M).  Both flags only permute on load: every layout gives the same bits
+ *   SDR_PFS_GENERAL_KERNEL always the general back end instead of the register-window one (which runs when
+ *                          D divides M, M / D <= 8 and ceil(L/D) <= 32); same bits; for testing
+ * Carried state: the transforms of the last ceil((L-1)/D) frames, so calls of any number of frames give
+ * the same bits as one call.  Pointers need c64 (8-byte) alignment.
+ * ====================================================================================== */
+#define SDR_PFS_SHIFT 1u
+#define SDR_PFS_CHANNEL_MAJOR 2u
+#define SDR_PFS_GENERAL_KERNEL 4u
+
+typedef struct {
+    const float *taps;     /* real synthesis prototype f, n_taps f32 */
+    size_t n_taps;         /* L >= 1 */
+    size_t n_channels;     /* M, 2 <= M <= 65536 (any length the FFT plan accepts) */
+    size_t interpolation;  /* D >= 1 (0 is rejected) */
+    unsigned flags;        /* SDR_PFS_* */
+    int device;
+    void *stream;
+} sdr_pfs_config_t;
+
+typedef struct sdr_pfs sdr_pfs_t;
+sdr_pfs_t *sdr_pfs_create(const sdr_pfs_config_t *cfg, int *err);
+void sdr_pfs_destroy(sdr_pfs_t *);
+int sdr_pfs_reset(sdr_pfs_t *);                        /* zero carried frames */
+sdr_pfs_t *sdr_pfs_clone(const sdr_pfs_t *, int *err);
+/* outputs that n_frames frames release: n_frames * D */
+size_t sdr_pfs_output_count(const sdr_pfs_t *, size_t n_frames);
+/* in: n_frames c64 frames, frame-major (frame stride in_stride >= M) or channel-major (M rows, row stride
+ * in_stride >= n_frames).  out: n_frames * D c64 samples, capacity out_cap samples.  A too-small out_cap
+ * returns SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  *n_out = samples written. */
+int sdr_pfs_process(sdr_pfs_t *, const float *in_c64, size_t n_frames, size_t in_stride, float *out_c64,
+                    size_t out_cap, size_t *n_out);
+int sdr_pfs_process_dev(sdr_pfs_t *, const float *in_c64, size_t n_frames, size_t in_stride, float *out_c64,
+                        size_t out_cap, size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

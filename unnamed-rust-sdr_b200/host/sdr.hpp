@@ -224,6 +224,51 @@ class Pfb {
     void reset() { check(sdr_pfb_reset(h_), "Pfb::reset"); }
 };
 
+// Polyphase synthesis bank behind sdr_pfs_*, the inverse of Pfb: channel k is zero-stuffed by D (sample m at index
+// (m+1) D - 1), filtered by Fir<Complex, Complex>(f[n] e^{+2 pi i k n / M}) and summed over k; n frames give n D
+// samples.  flags: SDR_PFS_SHIFT, SDR_PFS_CHANNEL_MAJOR take the layouts Pfb writes with the matching flags.
+class Pfs {
+    sdr_pfs_t *h_ = nullptr;
+    size_t m_ = 0;
+    bool cmajor_ = false;
+
+  public:
+    Pfs(const std::vector<float> &prototype, size_t n_channels, size_t interpolation, unsigned flags = 0)
+        : m_(n_channels), cmajor_((flags & SDR_PFS_CHANNEL_MAJOR) != 0) {
+        sdr_pfs_config_t cfg{};
+        cfg.taps = prototype.data();
+        cfg.n_taps = prototype.size();
+        cfg.n_channels = n_channels;
+        cfg.interpolation = interpolation;
+        cfg.flags = flags;
+        int err = 0;
+        h_ = sdr_pfs_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Pfs::new");
+    }
+    Pfs(Pfs &&o) noexcept : h_(o.h_), m_(o.m_), cmajor_(o.cmajor_) { o.h_ = nullptr; }
+    Pfs(const Pfs &o) : m_(o.m_), cmajor_(o.cmajor_) {
+        int err = 0;
+        h_ = sdr_pfs_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Pfs::clone");
+    }
+    Pfs &operator=(const Pfs &) = delete;
+    ~Pfs() { sdr_pfs_destroy(h_); }
+    size_t channels() const { return m_; }
+    size_t output_count(size_t n_frames) const { return sdr_pfs_output_count(h_, n_frames); }
+    // in: n_frames frames of M (or M rows of n_frames when channel-major).  out: n_frames * D samples, replaced.
+    size_t process(const Complex *in, size_t n_frames, std::vector<Complex> &out) {
+        const size_t n = output_count(n_frames);
+        out.resize(n ? n : 1);
+        size_t got = 0;
+        check(sdr_pfs_process(h_, reinterpret_cast<const float *>(in), n_frames, cmajor_ ? n_frames : m_,
+                              reinterpret_cast<float *>(out.data()), n, &got),
+              "Pfs::process");
+        out.resize(got);
+        return got;
+    }
+    void reset() { check(sdr_pfs_reset(h_), "Pfs::reset"); }
+};
+
 // Down-converter bank behind sdr_ddc_*: channel k is a tee'd copy of the stream mixed down by a 64-bit NCO
 // (sdr_ddc_phase_increment(freq[k], rate)), Fir<Complex, f32>(h_k) and Decimate(D), computed in one pass over the input.
 // taps: one row of L (shared) or channels rows of L.  Output: channels rows of outputs (channel-major).

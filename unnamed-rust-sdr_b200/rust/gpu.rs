@@ -162,6 +162,58 @@ impl Drop for GpuPfb {
     fn drop(&mut self) { unsafe { sdr_pfb_destroy(self.h) } }
 }
 
+/// Polyphase synthesis bank, the inverse of GpuPfb: channel k is zero-stuffed by `interpolation` (D), filtered by
+/// Fir<Complex<f32>, Complex<f32>> with taps f[n] e^{+2 pi i k n / M} and summed over k.  `process` takes frames of M
+/// channels (or M rows of frames with SDR_PFS_CHANNEL_MAJOR) and returns D samples per frame; calls of any number of
+/// frames give the same samples as one call.
+pub struct GpuPfs {
+    h: *mut sdr_pfs_t,
+    m: usize,
+    channel_major: bool,
+}
+unsafe impl Send for GpuPfs {}
+
+impl GpuPfs {
+    pub fn new(prototype: &[f32], channels: usize, interpolation: usize, flags: u32) -> Result<Self, Error> {
+        let cfg = sdr_pfs_config_t {
+            taps: prototype.as_ptr(), n_taps: prototype.len(), n_channels: channels, interpolation, flags, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_pfs_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuPfs { h, m: channels, channel_major: flags & SDR_PFS_CHANNEL_MAJOR != 0 })
+    }
+    /// input: n_frames frames of M (or M rows of n_frames); output: replaced by n_frames * D samples
+    pub fn process(&mut self, input: &[Complex<f32>], n_frames: usize, output: &mut Vec<Complex<f32>>)
+                   -> Result<usize, Error> {
+        assert!(input.len() >= n_frames * self.m);
+        let n = unsafe { sdr_pfs_output_count(self.h, n_frames) };
+        output.clear();
+        output.reserve(n.max(1));
+        let mut got = 0usize;
+        let stride = if self.channel_major { n_frames } else { self.m };
+        check(unsafe {
+            sdr_pfs_process(self.h, input.as_ptr() as *const f32, n_frames, stride, output.as_mut_ptr() as *mut f32, n,
+                            &mut got)
+        })?;
+        unsafe { output.set_len(got) };
+        Ok(got)
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_pfs_reset(self.h) }) }
+}
+impl Clone for GpuPfs {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_pfs_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_pfs_clone failed: {}", Error(err));
+        GpuPfs { h, m: self.m, channel_major: self.channel_major }
+    }
+}
+impl Drop for GpuPfs {
+    fn drop(&mut self) { unsafe { sdr_pfs_destroy(self.h) } }
+}
+
 /// Down-converter bank: channel k is the stream mixed down by a 64-bit NCO at freqs[k] (what a caller writes with
 /// Signal::map over an oscillator), Fir<Complex<f32>, f32>(h_k) and Decimate(wait), for all channels in one pass over
 /// the input.  taps: one row of n_taps (shared) or one row per channel.  `process` returns channels rows of outputs

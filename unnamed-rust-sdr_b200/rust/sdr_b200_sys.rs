@@ -21,6 +21,10 @@ pub const SDR_PLL_F64_MATH: c_uint = 2;
 pub const SDR_PFB_SHIFT: c_uint = 1;
 pub const SDR_PFB_CHANNEL_MAJOR: c_uint = 2;
 pub const SDR_PFB_GENERAL_KERNEL: c_uint = 4;
+/// sdr_pfs_config_t.flags
+pub const SDR_PFS_SHIFT: c_uint = 1;
+pub const SDR_PFS_CHANNEL_MAJOR: c_uint = 2;
+pub const SDR_PFS_GENERAL_KERNEL: c_uint = 4;
 /// sdr_ddc_config_t.flags
 pub const SDR_DDC_GENERAL_KERNEL: c_uint = 1;
 /// sdr_psd_config_t.flags
@@ -38,6 +42,7 @@ pub enum sdr_pfb_t {}
 pub enum sdr_ddc_t {}
 pub enum sdr_psd_t {}
 pub enum sdr_fcfb_t {}
+pub enum sdr_pfs_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -121,6 +126,17 @@ pub struct sdr_pfb_config_t {
     pub n_channels: size_t,
     pub decimation: size_t,
     pub input_format: c_int,
+    pub flags: c_uint,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+pub struct sdr_pfs_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_channels: size_t,
+    pub interpolation: size_t,
     pub flags: c_uint,
     pub device: c_int,
     pub stream: *mut c_void,
@@ -258,6 +274,17 @@ extern "C" {
                            out_stride: size_t, n_frames: *mut size_t) -> c_int;
     pub fn sdr_pfb_process_dev(h: *mut sdr_pfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
                                out_cap: size_t, out_stride: size_t, n_frames: *mut size_t) -> c_int;
+
+    // polyphase synthesis bank: M channel streams -> one stream at D samples per frame (the inverse of sdr_pfb)
+    pub fn sdr_pfs_create(cfg: *const sdr_pfs_config_t, err: *mut c_int) -> *mut sdr_pfs_t;
+    pub fn sdr_pfs_destroy(h: *mut sdr_pfs_t);
+    pub fn sdr_pfs_reset(h: *mut sdr_pfs_t) -> c_int;
+    pub fn sdr_pfs_clone(h: *const sdr_pfs_t, err: *mut c_int) -> *mut sdr_pfs_t;
+    pub fn sdr_pfs_output_count(h: *const sdr_pfs_t, n_frames: size_t) -> size_t;
+    pub fn sdr_pfs_process(h: *mut sdr_pfs_t, in_c64: *const c_float, n_frames: size_t, in_stride: size_t,
+                           out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_pfs_process_dev(h: *mut sdr_pfs_t, in_c64: *const c_float, n_frames: size_t, in_stride: size_t,
+                               out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
 
     // down-converter bank: C x (64-bit NCO mixer + Fir(h_k) + Decimate(D)) in one pass
     pub fn sdr_ddc_phase_increment(freq: f64, rate: f64) -> u64;

@@ -13,6 +13,7 @@ PLL_FAST_MATH = 1
 PLL_F64_MATH = 2
 PLL_GENERAL_KERNEL = 4
 PFB_SHIFT, PFB_CHANNEL_MAJOR, PFB_GENERAL_KERNEL = 1, 2, 4
+PFS_SHIFT, PFS_CHANNEL_MAJOR, PFS_GENERAL_KERNEL = 1, 2, 4
 DDC_GENERAL_KERNEL = 1
 PSD_SHIFT, PSD_NORM, PSD_GENERAL_KERNEL = 1, 2, 4
 BQ_IDENTITY, BQ_LOWPASS, BQ_HIGHPASS, BQ_BANDPASS, BQ_NOTCH, BQ_LR = range(6)
@@ -80,6 +81,11 @@ class FcfbConfig(C.Structure):
                 ("stream", vp)]
 
 
+class PfsConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_channels", sz), ("interpolation", sz), ("flags", C.c_uint),
+                ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -135,6 +141,13 @@ PROTOTYPES = {
     "sdr_pfb_output_count": (sz, [vp, sz]),
     "sdr_pfb_process": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
     "sdr_pfb_process_dev": (i32, [vp, vp, sz, vp, sz, sz, C.POINTER(sz)]),
+    "sdr_pfs_create": (vp, [C.POINTER(PfsConfig), C.POINTER(i32)]),
+    "sdr_pfs_destroy": (None, [vp]),
+    "sdr_pfs_reset": (i32, [vp]),
+    "sdr_pfs_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_pfs_output_count": (sz, [vp, sz]),
+    "sdr_pfs_process": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
+    "sdr_pfs_process_dev": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
     "sdr_ddc_phase_increment": (C.c_uint64, [C.c_double, C.c_double]),
     "sdr_ddc_create": (vp, [C.POINTER(DdcConfig), C.POINTER(i32)]),
     "sdr_ddc_destroy": (None, [vp]),

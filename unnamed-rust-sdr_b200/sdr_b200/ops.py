@@ -517,6 +517,79 @@ def ddc_phase_increment(freq, rate):
     return int(lib().sdr_ddc_phase_increment(float(freq), float(rate)))
 
 
+class Pfs:
+    """Polyphase synthesis filter bank, the inverse of Pfb: frames of n_channels channel samples -> one stream at
+    `interpolation` (D) samples per frame.  Channel k is zero-stuffed by D (sample m at index (m+1) D - 1), filtered by
+    Fir(f * exp(+2j pi k n / M)) and summed over k; frame m releases outputs [m D, (m+1) D).  There is no scale: for
+    unit round-trip gain f carries a factor D.  shift=True / channel_major=True take the layouts Pfb writes with the
+    same flags ([frames, M] with row i = channel (i - M/2) mod M, or [M, frames]).  general=True forces the general
+    back-end kernel (same bits)."""
+
+    def __init__(self, taps, n_channels, interpolation, shift=False, channel_major=False, general=False, device=0,
+                 stream=None, _handle=None, _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        self._taps = np.ascontiguousarray(taps, np.float32)
+        self.n_channels = int(n_channels)
+        self.interpolation = int(interpolation)
+        self.channel_major = bool(channel_major)
+        flags = (F.PFS_SHIFT if shift else 0) | (F.PFS_CHANNEL_MAJOR if channel_major else 0) | \
+            (F.PFS_GENERAL_KERNEL if general else 0)
+        cfg = F.PfsConfig(self._taps.ctypes.data, self._taps.size, self.n_channels, self.interpolation, flags, device,
+                          _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_pfs_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_pfs_create")
+
+    def output_count(self, n_frames):
+        return lib().sdr_pfs_output_count(self.h, n_frames)
+
+    def process(self, frames):
+        """frames: complex64 [n, M] (or [M, n] when channel-major) -> complex64 [n * D]"""
+        y = np.ascontiguousarray(frames, np.complex64)
+        M = self.n_channels
+        if y.ndim != 2 or y.shape[0 if self.channel_major else 1] != M:
+            raise ValueError("frames must be [M, n] (channel-major) or [n, M] with M = %d" % M)
+        n = y.shape[1] if self.channel_major else y.shape[0]
+        cnt = self.output_count(n)
+        out = np.empty(max(cnt, 1), np.complex64)
+        got = C.c_size_t(0)
+        check(lib().sdr_pfs_process(self.h, y.ctypes.data if n else None, n, n if self.channel_major else M,
+                                    out.ctypes.data, cnt, C.byref(got)), "sdr_pfs_process")
+        return out[:got.value]
+
+    def process_dev(self, d_in, n_frames, d_out, out_cap, in_stride=None):
+        """device-resident: d_in n_frames frames, frame-major (stride in_stride >= M) or channel-major (M rows of
+        in_stride >= n_frames); d_out out_cap samples; asynchronous on the handle's stream.  Returns the samples
+        written (n_frames * D)."""
+        if in_stride is None:
+            in_stride = n_frames if self.channel_major else self.n_channels
+        got = C.c_size_t(0)
+        check(lib().sdr_pfs_process_dev(self.h, _ptr(d_in), n_frames, in_stride, _ptr(d_out), out_cap, C.byref(got)),
+              "sdr_pfs_process_dev")
+        return got.value
+
+    def reset(self):
+        check(lib().sdr_pfs_reset(self.h), "sdr_pfs_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_pfs_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_pfs_clone")
+        return Pfs(None, 0, 0, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_pfs_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class Ddc:
     """Digital down-converter bank: channel k of one IQ stream is mixed down by freqs[k] (a 64-bit NCO), filtered by its
     real taps (taps 1-D: shared; [C, L]: one row per channel) and decimated by `decimation`:
