@@ -662,6 +662,59 @@ int sdr_pfs_process(sdr_pfs_t *, const float *in_c64, size_t n_frames, size_t in
 int sdr_pfs_process_dev(sdr_pfs_t *, const float *in_c64, size_t n_frames, size_t in_stride, float *out_c64,
                         size_t out_cap, size_t *n_out);
 
+/* ======================================================================================
+ * digital up-converter bank -- C channel streams, each interpolated by I, mixed up to its own 64-bit-NCO offset and
+ * summed into one IQ stream; the transpose of sdr_ddc.  Channel k restates zero-stuffing on sdr_pfs's grid,
+ * filter::Fir<f32, Complex<f32>> (src/filter/fir.rs:23-32) with real taps h_k, an oscillator through Signal::map and
+ * a sample-by-sample sum; F = first_sample is the absolute stream index of the handle's first OUTPUT:
+ *   s_k[(m+1) I - 1] = y_k[m], 0 elsewhere          (m counts the handle's frames; frames before the stream are 0)
+ *   u_k[n] = sum_{j<L} h_k[j] s_k[n - j]
+ *   x[n]   = sum_k u_k[n] e^{+2 pi i phi_k(F + n) / 2^64},   phi_k(N) = N phase_inc[k]  mod 2^64
+ * The mixer is the conjugate of sdr_ddc's, so baseband in channel k lands at (int64)phase_inc[k] / 2^64 * rate.
+ * Computed with n = q I + c - 1 as u_k[n] = sum_i h_k[c + i I] y_k[q - 1 - i], one fmaf chain per component in
+ * ascending i (a tap of 0.0 is still multiplied, so NaNs propagate), then rotated by the exact integer phase and
+ * accumulated over ascending k.
+ * Release: frame m completes outputs [m I, (m+1) I), so n frames give exactly n I outputs; ceil((L-1)/I) zero frames
+ * drain the tail.  There is no scale: for unit round-trip gain after sdr_ddc the synthesis taps carry the factor I.
+ * Round trip: after sdr_ddc (first_sample F) and a filter cascade that delays the signal by d samples, give this bank
+ * first_sample F - d, or channel k comes back rotated by e^{+2 pi i d phase_inc[k] / 2^64}.
+ * Bits: an output depends only on its frames and on F + n, so blockings, clones and shards give the bits of one call.
+ * A shard primed with the H = ceil((L-1)/I) frames before it, with first_sample the absolute index of the primed
+ * frame's first output, gives one stream's bits after its first H I outputs.
+ * Accuracy: |x - x_f64| <= 1e-5 max|x_f64| (DESIGN.md K11).
+ * Input: C rows of n_frames c64, row stride in_stride elements (>= n_frames when C > 1): the channel-major rows
+ * sdr_ddc and sdr_fcfb write.  Carried state: the last ceil((L-1)/I) frames of every channel and the stream position;
+ * the block and the carried frames are read through two pointers (the block is never copied).  Device pointers need
+ * c64 (8-byte) alignment.
+ * ====================================================================================== */
+typedef struct {
+    const float *taps;         /* n_tap_sets rows of n_taps real f32 */
+    size_t n_taps;             /* L, 1 <= L <= 2^20 */
+    size_t n_tap_sets;         /* 1 (shared) or n_channels */
+    const uint64_t *phase_inc; /* n_channels NCO increments (sdr_ddc_phase_increment) */
+    size_t n_channels;         /* C, 1 <= C <= 256 */
+    size_t interpolation;      /* I >= 1 (0 is rejected) */
+    uint64_t first_sample;     /* absolute stream index of the first OUTPUT (NCO phase only) */
+    unsigned flags;            /* 0 */
+    int device;
+    void *stream;
+} sdr_duc_config_t;
+
+typedef struct sdr_duc sdr_duc_t;
+sdr_duc_t *sdr_duc_create(const sdr_duc_config_t *cfg, int *err);
+void sdr_duc_destroy(sdr_duc_t *);
+int sdr_duc_reset(sdr_duc_t *); /* zero carried frames, position back to first_sample */
+sdr_duc_t *sdr_duc_clone(const sdr_duc_t *, int *err);
+/* outputs that n_frames frames release: n_frames * I */
+size_t sdr_duc_output_count(const sdr_duc_t *, size_t n_frames);
+/* in: C rows of n_frames c64 samples, row stride in_stride.  out: n_frames * I c64 samples, capacity out_cap samples.
+ * A too-small out_cap returns SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  *n_out = samples written. */
+int sdr_duc_process(sdr_duc_t *, const float *in_c64, size_t n_frames, size_t in_stride, float *out_c64,
+                    size_t out_cap, size_t *n_out);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_duc_process_dev(sdr_duc_t *, const float *in_c64, size_t n_frames, size_t in_stride, float *out_c64,
+                        size_t out_cap, size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,5 +1,6 @@
-// nco.cuh -- the 64-bit NCO shared by the down-converter bank (ddc.cu) and the fast-convolution bank (fcfb.cu): the
-// exact derotation e^{-2 pi i phi / 2^64} on the device and the host-side f64 phase and rotated-taps helpers.
+// nco.cuh -- the 64-bit NCO shared by the down-converter bank (ddc.cu), the fast-convolution bank (fcfb.cu) and the
+// up-converter bank (duc.cu, which takes the conjugate of nco_rot): the exact derotation e^{-2 pi i phi / 2^64} on the
+// device and the host-side f64 phase and rotated-taps helpers.
 #pragma once
 #include <cmath>
 #include <vector>

@@ -320,6 +320,56 @@ class Ddc {
     void reset() { check(sdr_ddc_reset(h_), "Ddc::reset"); }
 };
 
+// Up-converter bank behind sdr_duc_*, the transpose of Ddc: channel k is zero-stuffed by I (sample m at index
+// (m+1) I - 1), filtered by Fir<f32, Complex>(h_k), mixed up by a 64-bit NCO (sdr_ddc_phase_increment(freq[k], rate))
+// and the channels are summed.  taps: one row of L (shared) or channels rows of L.  Input: channels rows of frames
+// (channel-major, as Ddc writes them); n frames give n I samples.
+class Duc {
+    sdr_duc_t *h_ = nullptr;
+    size_t c_ = 0;
+
+  public:
+    Duc(const std::vector<float> &taps, size_t n_taps, const std::vector<double> &freqs, double rate,
+        size_t interpolation, uint64_t first_sample = 0)
+        : c_(freqs.size()) {
+        std::vector<uint64_t> inc(freqs.size());
+        for (size_t k = 0; k < freqs.size(); ++k) inc[k] = sdr_ddc_phase_increment(freqs[k], rate);
+        sdr_duc_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.phase_inc = inc.data();
+        cfg.n_channels = freqs.size();
+        cfg.interpolation = interpolation;
+        cfg.first_sample = first_sample;
+        int err = 0;
+        h_ = sdr_duc_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Duc::new");
+    }
+    Duc(Duc &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
+    Duc(const Duc &o) : c_(o.c_) {
+        int err = 0;
+        h_ = sdr_duc_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Duc::clone");
+    }
+    Duc &operator=(const Duc &) = delete;
+    ~Duc() { sdr_duc_destroy(h_); }
+    size_t channels() const { return c_; }
+    size_t output_count(size_t n_frames) const { return sdr_duc_output_count(h_, n_frames); }
+    // in: channels rows of n_frames, row stride in_stride (>= n_frames).  out: n_frames * I samples, replaced.
+    size_t process(const Complex *in, size_t n_frames, size_t in_stride, std::vector<Complex> &out) {
+        const size_t n = output_count(n_frames);
+        out.resize(n ? n : 1);
+        size_t got = 0;
+        check(sdr_duc_process(h_, reinterpret_cast<const float *>(in), n_frames, in_stride,
+                              reinterpret_cast<float *>(out.data()), n, &got),
+              "Duc::process");
+        out.resize(got);
+        return got;
+    }
+    void reset() { check(sdr_duc_reset(h_), "Duc::reset"); }
+};
+
 // Fast-convolution channel bank (sdr_fcfb): Ddc's channels with one decimation per channel, computed by overlap-save.
 // Outputs are released per block of P inputs (sdr_fcfb_geometry); feed N zeros to drain a finite stream.
 class Fcfb {

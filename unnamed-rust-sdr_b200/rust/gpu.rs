@@ -266,6 +266,61 @@ impl Drop for GpuDdc {
     fn drop(&mut self) { unsafe { sdr_ddc_destroy(self.h) } }
 }
 
+/// Up-converter bank, the transpose of GpuDdc: channel k is zero-stuffed by `interpolation` (I; sample m at index
+/// (m+1) I - 1), filtered by Fir<f32, Complex<f32>>(h_k), mixed up by a 64-bit NCO at freqs[k] and the channels are
+/// summed into one stream.  taps: one row of n_taps (shared) or one row per channel.  `process` takes channels rows of
+/// frames (the rows GpuDdc returns) and returns I samples per frame; calls of any number of frames give the same
+/// samples as one call.  first_sample: absolute index of the first output (after GpuDdc, its first_sample minus the
+/// filter cascade's delay).
+pub struct GpuDuc {
+    h: *mut sdr_duc_t,
+    c: usize,
+}
+unsafe impl Send for GpuDuc {}
+
+impl GpuDuc {
+    pub fn new(taps: &[f32], n_taps: usize, freqs: &[f64], rate: f64, interpolation: usize, first_sample: u64)
+               -> Result<Self, Error> {
+        let inc: Vec<u64> = freqs.iter().map(|&f| unsafe { sdr_ddc_phase_increment(f, rate) }).collect();
+        let cfg = sdr_duc_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: if n_taps == 0 { 0 } else { taps.len() / n_taps },
+            phase_inc: inc.as_ptr(), n_channels: freqs.len(), interpolation, first_sample, flags: 0, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_duc_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuDuc { h, c: freqs.len() })
+    }
+    /// input: channels rows of n_frames, row stride `stride` (>= n_frames); output: replaced by n_frames * I samples
+    pub fn process(&mut self, input: &[Complex<f32>], n_frames: usize, stride: usize, output: &mut Vec<Complex<f32>>)
+                   -> Result<usize, Error> {
+        assert!(n_frames == 0 || input.len() >= (self.c - 1) * stride + n_frames);
+        let n = unsafe { sdr_duc_output_count(self.h, n_frames) };
+        output.clear();
+        output.reserve(n.max(1));
+        let mut got = 0usize;
+        check(unsafe {
+            sdr_duc_process(self.h, input.as_ptr() as *const f32, n_frames, stride, output.as_mut_ptr() as *mut f32, n,
+                            &mut got)
+        })?;
+        unsafe { output.set_len(got) };
+        Ok(got)
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_duc_reset(self.h) }) }
+}
+impl Clone for GpuDuc {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_duc_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_duc_clone failed: {}", Error(err));
+        GpuDuc { h, c: self.c }
+    }
+}
+impl Drop for GpuDuc {
+    fn drop(&mut self) { unsafe { sdr_duc_destroy(self.h) } }
+}
+
 /// window(n) -> decimate(hop) -> map(fft::fft) -> |.|^2 -> mean of `average` behind sdr_psd_*: averaged power spectra
 /// of n f32 bins (shifted and 1/n-scaled like fft::fft's 1/sqrt(n) with SDR_PSD_SHIFT | SDR_PSD_NORM).  taper: n real
 /// values or empty (rectangular).  `process` appends the spectra the block completes; blocks of any size give the same

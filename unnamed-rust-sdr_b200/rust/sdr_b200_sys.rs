@@ -43,6 +43,7 @@ pub enum sdr_ddc_t {}
 pub enum sdr_psd_t {}
 pub enum sdr_fcfb_t {}
 pub enum sdr_pfs_t {}
+pub enum sdr_duc_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -152,6 +153,20 @@ pub struct sdr_ddc_config_t {
     pub decimation: size_t,
     pub first_sample: u64,
     pub input_format: c_int,
+    pub flags: c_uint,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+pub struct sdr_duc_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub phase_inc: *const u64,
+    pub n_channels: size_t,
+    pub interpolation: size_t,
+    pub first_sample: u64,
     pub flags: c_uint,
     pub device: c_int,
     pub stream: *mut c_void,
@@ -298,6 +313,17 @@ extern "C" {
     pub fn sdr_ddc_process_dev(h: *mut sdr_ddc_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
                                out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_ddc_last_path(h: *const sdr_ddc_t) -> c_int;
+
+    // up-converter bank: C x (zero-stuff(I) + Fir(h_k) + 64-bit NCO mix up), summed into one stream
+    pub fn sdr_duc_create(cfg: *const sdr_duc_config_t, err: *mut c_int) -> *mut sdr_duc_t;
+    pub fn sdr_duc_destroy(h: *mut sdr_duc_t);
+    pub fn sdr_duc_reset(h: *mut sdr_duc_t) -> c_int;
+    pub fn sdr_duc_clone(h: *const sdr_duc_t, err: *mut c_int) -> *mut sdr_duc_t;
+    pub fn sdr_duc_output_count(h: *const sdr_duc_t, n_frames: size_t) -> size_t;
+    pub fn sdr_duc_process(h: *mut sdr_duc_t, in_c64: *const c_float, n_frames: size_t, in_stride: size_t,
+                           out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_duc_process_dev(h: *mut sdr_duc_t, in_c64: *const c_float, n_frames: size_t, in_stride: size_t,
+                               out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_psd_create(cfg: *const sdr_psd_config_t, err: *mut c_int) -> *mut sdr_psd_t;
     pub fn sdr_psd_destroy(h: *mut sdr_psd_t);
     pub fn sdr_psd_reset(h: *mut sdr_psd_t) -> c_int;

@@ -86,6 +86,12 @@ class PfsConfig(C.Structure):
                 ("device", i32), ("stream", vp)]
 
 
+class DucConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phase_inc", vp), ("n_channels", sz),
+                ("interpolation", sz), ("first_sample", C.c_uint64), ("flags", C.c_uint), ("device", i32),
+                ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -148,6 +154,13 @@ PROTOTYPES = {
     "sdr_pfs_output_count": (sz, [vp, sz]),
     "sdr_pfs_process": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
     "sdr_pfs_process_dev": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
+    "sdr_duc_create": (vp, [C.POINTER(DucConfig), C.POINTER(i32)]),
+    "sdr_duc_destroy": (None, [vp]),
+    "sdr_duc_reset": (i32, [vp]),
+    "sdr_duc_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_duc_output_count": (sz, [vp, sz]),
+    "sdr_duc_process": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
+    "sdr_duc_process_dev": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
     "sdr_ddc_phase_increment": (C.c_uint64, [C.c_double, C.c_double]),
     "sdr_ddc_create": (vp, [C.POINTER(DdcConfig), C.POINTER(i32)]),
     "sdr_ddc_destroy": (None, [vp]),

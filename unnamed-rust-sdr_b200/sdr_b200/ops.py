@@ -669,6 +669,79 @@ class Ddc:
     __del__ = close
 
 
+class Duc:
+    """Digital up-converter bank, the transpose of Ddc: channel k (row k of a [C, n] complex64 array) is zero-stuffed
+    by `interpolation` (I; sample m at index (m+1) I - 1), filtered by its real taps (1-D: shared; [C, L]: one row
+    per channel), mixed UP by freqs[k] (a 64-bit NCO) and all channels are summed:
+    x[n] = sum_k u_k[n] e^{+2 pi i phi_k(first_sample + n)}.  first_sample = absolute stream index of the first
+    OUTPUT (places the NCO phase only).  Frame m releases outputs [m I, (m+1) I).  There is no scale: for unit
+    round-trip gain after Ddc the taps carry the factor I, and first_sample is the Ddc's minus the cascade's delay."""
+
+    def __init__(self, taps, freqs, rate, interpolation, first_sample=0, device=0, stream=None, _handle=None,
+                 _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        self._taps = t
+        self.phase_inc = np.array([ddc_phase_increment(f, rate) for f in np.atleast_1d(freqs)], np.uint64)
+        self.n_channels = int(self.phase_inc.size)
+        self.interpolation = int(interpolation)
+        cfg = F.DucConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
+                          self.n_channels, self.interpolation, int(first_sample) % (1 << 64), 0, device,
+                          _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_duc_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_duc_create")
+
+    def output_count(self, n_frames):
+        return lib().sdr_duc_output_count(self.h, n_frames)
+
+    def process(self, y):
+        """y: complex64 [C, n] (row k = channel k) -> complex64 [n * I]"""
+        y = np.ascontiguousarray(y, np.complex64)
+        if y.ndim == 1 and self.n_channels == 1:
+            y = y[None]
+        if y.ndim != 2 or y.shape[0] != self.n_channels:
+            raise ValueError("y must be [C, n] with C = %d" % self.n_channels)
+        n = y.shape[1]
+        cnt = self.output_count(n)
+        out = np.empty(max(cnt, 1), np.complex64)
+        got = C.c_size_t(0)
+        check(lib().sdr_duc_process(self.h, y.ctypes.data if n else None, n, n, out.ctypes.data, cnt, C.byref(got)),
+              "sdr_duc_process")
+        return out[:got.value]
+
+    def process_dev(self, d_in, n_frames, d_out, out_cap, in_stride=None):
+        """device-resident: d_in C rows of in_stride (default n_frames) complex64, n_frames each; d_out out_cap samples;
+        asynchronous on the handle's stream.  Returns the samples written (n_frames * I)."""
+        got = C.c_size_t(0)
+        check(lib().sdr_duc_process_dev(self.h, _ptr(d_in), n_frames, n_frames if in_stride is None else in_stride,
+                                        _ptr(d_out), out_cap, C.byref(got)), "sdr_duc_process_dev")
+        return got.value
+
+    def reset(self):
+        check(lib().sdr_duc_reset(self.h), "sdr_duc_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_duc_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_duc_clone")
+        return Duc(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_duc_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class Psd:
     """Averaged power spectra (sdr_psd): window(n) -> decimate(hop) -> map(fft::fft) -> |.|^2 -> mean of `average`
     frames.  Frame j holds the n samples ending at input sample (j + 1) * hop - 1 (x[<0] = 0), tapered by `window`
