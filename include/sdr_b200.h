@@ -715,6 +715,67 @@ int sdr_duc_process(sdr_duc_t *, const float *in_c64, size_t n_frames, size_t in
 int sdr_duc_process_dev(sdr_duc_t *, const float *in_c64, size_t n_frames, size_t in_stride, float *out_c64,
                         size_t out_cap, size_t *n_out);
 
+/* ======================================================================================
+ * fast-convolution synthesis bank -- sdr_duc's function with one interpolation per channel, computed by overlap-save,
+ * so that the cost barely depends on the filter length; the inverse of sdr_fcfb.  F = first_sample is the absolute
+ * stream index of the handle's first OUTPUT:
+ *   s_k[(m+1) I_k - 1] = y_k[m], 0 elsewhere          (m counts the handle's frames; frames before the stream are 0)
+ *   u_k[n] = sum_{j<L} h_k[j] s_k[n - j]
+ *   x[n]   = sum_k u_k[n] e^{+2 pi i phi_k(F + n) / 2^64},   phi_k(N) = N phase_inc[k]  mod 2^64
+ * With every I_k = I this is sdr_duc's function.  Computed rotate-first: each frame is rotated by its exact integer
+ * phase, then x = sum_k g_k * w_k with sdr_fcfb's rotated taps g_k[j] = h_k[j] e^{+2 pi i (j phase_inc[k] mod 2^64)
+ * / 2^64}, by overlap-save on sdr_fcfb's geometry (sdr_fcfb_geometry with the interpolations in place of the
+ * decimations): Il = lcm(I_k), N, P.  Block b holds the outputs at absolute indices [b P + eps, (b+1) P + eps),
+ * eps = F mod Il, and is computed from the frames in the N positions that end at its last output: per channel one
+ * small forward FFT of the block's frames, a spectral multiply unfolded by the power-of-two part of I_k and summed over
+ * channels, and one N-point inverse FFT shared by all channels.
+ * Release: a call advances the handle by n_time output positions (a multiple of Il; row k holds n_time / I_k frames)
+ * and writes the outputs of the blocks it completes, up to P - Il positions later than sdr_duc releases them;
+ * sdr_fcsb_output_count gives the count.  To drain a finite stream, feed zero frames covering N positions (rounded up
+ * to a multiple of Il) and drop the outputs past the stream's end.
+ * Bits: an output depends only on its block's frames and its absolute position, so blockings (calls of a single Il,
+ * calls that end mid-block), clones and resets give the bits of one call.  A shard gives the same bits when it is cut
+ * on a block boundary of the absolute grid, is primed with frames covering at least N - P positions (rounded up to a
+ * multiple of Il) and its first_sample is the absolute index of the halo's first output position.  A non-finite frame
+ * poisons every output of each block whose span holds it, and no other output.
+ * Accuracy: |x - x_f64| <= 2e-5 log2(N) max|x_f64| on signals that fill the channels; FFT round-off follows the total
+ * power of the block's frames over all channels, not the level of one channel (DESIGN.md K12).
+ * Scale and round trip as sdr_duc: there is no scale (the synthesis taps carry the factor I_k); after sdr_fcfb
+ * (first_sample F) and a filter cascade that delays the signal by d samples, give this bank first_sample F - d.
+ * sdr_fcfb's per-channel output rows of one call are a valid input of one call at the same stride.
+ * Input: C rows, row k = n_time / I_k c64 frames, row stride in_stride c64 (>= the longest row when C > 1).
+ * Output: one contiguous c64 stream, out_cap samples; a too-small out_cap returns SDR_ERR_OUTPUT_TOO_SMALL before any
+ * state changes.  Carried state: the frames of each channel from the next block's span on (fewer than N + Il
+ * positions) and the stream position; the caller's rows and the carried frames are read through two pointers (the
+ * rows are never copied, except for that tail).  Device pointers need c64 (8-byte) alignment.
+ * ====================================================================================== */
+typedef struct {
+    const float *taps;           /* n_tap_sets rows of n_taps real f32 */
+    size_t n_taps;               /* L, 1 <= L <= 2^20 */
+    size_t n_tap_sets;           /* 1 (shared) or n_channels */
+    const uint64_t *phase_inc;   /* n_channels NCO increments (sdr_ddc_phase_increment) */
+    const size_t *interpolation; /* n_channels I_k >= 1; N, P = sdr_fcfb_geometry(n_taps, interpolation, C) */
+    size_t n_channels;           /* C, 1 <= C <= 256 */
+    uint64_t first_sample;       /* absolute stream index of the first OUTPUT: NCO phase and block grid */
+    int device;
+    void *stream;
+} sdr_fcsb_config_t;
+
+typedef struct sdr_fcsb sdr_fcsb_t;
+sdr_fcsb_t *sdr_fcsb_create(const sdr_fcsb_config_t *cfg, int *err);
+void sdr_fcsb_destroy(sdr_fcsb_t *);
+int sdr_fcsb_reset(sdr_fcsb_t *); /* carried frames dropped, position back to first_sample */
+sdr_fcsb_t *sdr_fcsb_clone(const sdr_fcsb_t *, int *err);
+/* outputs of the blocks that the next n_time output positions complete */
+size_t sdr_fcsb_output_count(const sdr_fcsb_t *, size_t n_time);
+/* in: C rows, row k = n_time / I_k frames, row stride in_stride c64 (>= the longest row when C > 1).  n_time must be a
+ * multiple of lcm(I_k).  *n_out = samples written. */
+int sdr_fcsb_process(sdr_fcsb_t *, const float *in_c64, size_t n_time, size_t in_stride, float *out_c64,
+                     size_t out_cap, size_t *n_out);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_fcsb_process_dev(sdr_fcsb_t *, const float *in_c64, size_t n_time, size_t in_stride, float *out_c64,
+                         size_t out_cap, size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

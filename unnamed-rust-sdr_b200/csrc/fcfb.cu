@@ -151,41 +151,6 @@ __global__ void __launch_bounds__(256) fcfb_store_kernel(const float2 *__restric
     }
 }
 
-// iterative radix-2 f64 DFT in place, a.size() a power of two: X[r] = sum_t a[t] e^{-2 pi i r t / n}
-void fft_f64(std::vector<double> &re, std::vector<double> &im) {
-    const size_t n = re.size();
-    for (size_t i = 1, j = 0; i < n; ++i) {
-        size_t bit = n >> 1;
-        for (; j & bit; bit >>= 1) j ^= bit;
-        j ^= bit;
-        if (i < j) { std::swap(re[i], re[j]); std::swap(im[i], im[j]); }
-    }
-    std::vector<double> wc(n / 2), ws(n / 2);
-    for (size_t k = 0; k < n / 2; ++k) {
-        wc[k] = std::cos(NCO_2PI * (double)k / (double)n);
-        ws[k] = -std::sin(NCO_2PI * (double)k / (double)n);
-    }
-    for (size_t len = 2; len <= n; len <<= 1) {
-        const size_t half = len / 2, step = n / len;
-        for (size_t s = 0; s < n; s += len)
-            for (size_t k = 0; k < half; ++k) {
-                const double c = wc[k * step], d = ws[k * step];
-                const size_t p = s + k, q = p + half;
-                const double tr = re[q] * c - im[q] * d, ti = re[q] * d + im[q] * c;
-                re[q] = re[p] - tr; im[q] = im[p] - ti;
-                re[p] += tr; im[p] += ti;
-            }
-    }
-}
-
-// rho_k = (N - P - 1) mod D_k in [0, D_k): N - P - 1 is -1 when P = N (L = 1), where C++'s % would give -1
-long long fcfb_rho(long long N, long long P, long long D) { return ((N - P - 1) % D + D) % D; }
-
-unsigned long long gcd_u(unsigned long long a, unsigned long long b) {
-    while (b) { const unsigned long long t = a % b; a = b; b = t; }
-    return a;
-}
-
 }  // namespace
 
 extern "C" int sdr_fcfb_geometry(size_t n_taps, const size_t *decimation, size_t n_channels, size_t *n_fft, size_t *hop) {
@@ -295,25 +260,10 @@ static void fcfb_tables(const sdr_fcfb *h, std::vector<float2> &G, std::vector<f
     const long long N = h->N, L = (long long)h->L;
     G.assign((size_t)h->C * N, make_float2(0.f, 0.f));
     tab.assign((size_t)h->C * FCFB_RUN, make_float2(0.f, 0.f));
-    std::vector<double> re, im;
     for (size_t k = 0; k < h->C; ++k) {
         const FcfbChan &c = h->chan[k];
         const float *hk = h->taps.data() + (h->n_sets == 1 ? 0 : k * h->L);
-        re.assign((size_t)N, 0.0);
-        im.assign((size_t)N, 0.0);
-        for (long long j = 0; j < L; ++j) {
-            const double t = NCO_2PI * nco_turns((uint64_t)j * c.inc);
-            re[j] = (double)hk[j] * std::cos(t);
-            im[j] = (double)hk[j] * std::sin(t);
-        }
-        fft_f64(re, im);
-        const long long rho = fcfb_rho(N, h->P, c.D);
-        for (long long r = 0; r < N; ++r) {
-            // e^{+2 pi i r rho / N} with the exact integer angle r rho mod N
-            const long long q = (long long)(((unsigned long long)r * (unsigned long long)rho) % (unsigned long long)N);
-            const double t = NCO_2PI * (double)q / (double)N, cs = std::cos(t), sn = std::sin(t);
-            G[(size_t)k * N + r] = make_float2((float)(re[r] * cs - im[r] * sn), (float)(re[r] * sn + im[r] * cs));
-        }
+        fc_spectrum(hk, L, c.inc, N, fcfb_rho(N, h->P, c.D), +1, G.data() + (size_t)k * N);
         for (int r = 0; r < FCFB_RUN; ++r) {
             const double t = NCO_2PI * nco_turns(((uint64_t)c.D * (uint64_t)r + (uint64_t)c.D - 1) * c.inc);
             tab[(size_t)k * FCFB_RUN + r] = make_float2((float)std::cos(t), (float)-std::sin(t));

@@ -423,6 +423,57 @@ class Fcfb {
     void reset() { check(sdr_fcfb_reset(h_), "Fcfb::reset"); }
 };
 
+// Fast-convolution synthesis bank (sdr_fcsb), the inverse of Fcfb: Duc's channels with one interpolation per channel,
+// computed by overlap-save.  A call advances by n_time output positions (a multiple of lcm(I_k); row k holds
+// n_time / I_k frames) and returns the outputs of the blocks it completes; feed zero frames covering N positions to
+// drain a finite stream.
+class Fcsb {
+    sdr_fcsb_t *h_ = nullptr;
+    size_t c_ = 0;
+
+  public:
+    Fcsb(const std::vector<float> &taps, size_t n_taps, const std::vector<double> &freqs, double rate,
+         const std::vector<size_t> &interpolation, uint64_t first_sample = 0)
+        : c_(freqs.size()) {
+        std::vector<uint64_t> inc(freqs.size());
+        for (size_t k = 0; k < freqs.size(); ++k) inc[k] = sdr_ddc_phase_increment(freqs[k], rate);
+        if (interpolation.size() != freqs.size()) throw sdr::Error(SDR_ERR_INVALID_ARG, "Fcsb::new");
+        sdr_fcsb_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.phase_inc = inc.data();
+        cfg.interpolation = interpolation.data();
+        cfg.n_channels = freqs.size();
+        cfg.first_sample = first_sample;
+        int err = 0;
+        h_ = sdr_fcsb_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Fcsb::new");
+    }
+    Fcsb(Fcsb &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
+    Fcsb(const Fcsb &o) : c_(o.c_) {
+        int err = 0;
+        h_ = sdr_fcsb_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Fcsb::clone");
+    }
+    Fcsb &operator=(const Fcsb &) = delete;
+    ~Fcsb() { sdr_fcsb_destroy(h_); }
+    size_t channels() const { return c_; }
+    size_t output_count(size_t n_time) const { return sdr_fcsb_output_count(h_, n_time); }
+    // in: channels rows, row k = n_time / I_k frames, row stride in_stride (>= the longest row).  out: replaced.
+    size_t process(const Complex *in, size_t n_time, size_t in_stride, std::vector<Complex> &out) {
+        const size_t n = output_count(n_time);
+        out.resize(n ? n : 1);
+        size_t got = 0;
+        check(sdr_fcsb_process(h_, reinterpret_cast<const float *>(in), n_time, in_stride,
+                               reinterpret_cast<float *>(out.data()), n, &got),
+              "Fcsb::process");
+        out.resize(got);
+        return got;
+    }
+    void reset() { check(sdr_fcsb_reset(h_), "Fcsb::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

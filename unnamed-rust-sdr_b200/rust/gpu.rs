@@ -426,6 +426,64 @@ impl Drop for GpuFcfb {
     fn drop(&mut self) { unsafe { sdr_fcfb_destroy(self.h) } }
 }
 
+/// Fast-convolution synthesis bank, the inverse of GpuFcfb: GpuDuc's channels with one interpolation per channel, by
+/// overlap-save.  A call advances by n_time output positions (a multiple of lcm(I_k); row k holds n_time / I_k frames,
+/// the rows GpuFcfb returns) and appends the outputs of the blocks it completes; feed zero frames covering N positions
+/// to drain a finite stream.  first_sample: absolute index of the first output (after GpuFcfb, its first_sample minus
+/// the filter cascade's delay).
+pub struct GpuFcsb {
+    h: *mut sdr_fcsb_t,
+    i: Vec<usize>,
+}
+unsafe impl Send for GpuFcsb {}
+
+impl GpuFcsb {
+    /// taps: one row of n_taps (shared) or one row per channel; freqs in Hz at `rate`; one interpolation per channel
+    pub fn new(taps: &[f32], n_taps: usize, freqs: &[f64], rate: f64, interpolation: &[usize], first_sample: u64)
+               -> Result<Self, Error> {
+        if interpolation.len() != freqs.len() || n_taps == 0 { return Err(Error(100)); }
+        let inc: Vec<u64> = freqs.iter().map(|&f| unsafe { sdr_ddc_phase_increment(f, rate) }).collect();
+        let cfg = sdr_fcsb_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: taps.len() / n_taps, phase_inc: inc.as_ptr(),
+            interpolation: interpolation.as_ptr(), n_channels: freqs.len(), first_sample, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_fcsb_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuFcsb { h, i: interpolation.to_vec() })
+    }
+    /// input: one row per channel, row k n_time / I_k frames at row stride `stride` (>= the longest row); the
+    /// released outputs are appended to output
+    pub fn process(&mut self, input: &[Complex<f32>], n_time: usize, stride: usize, output: &mut Vec<Complex<f32>>)
+                   -> Result<usize, Error> {
+        let last = self.i.len() - 1;
+        assert!(n_time == 0 || input.len() >= last * stride + n_time / self.i[last]);
+        let n = unsafe { sdr_fcsb_output_count(self.h, n_time) };
+        let at = output.len();
+        output.resize(at + n.max(1), Complex::new(0.0, 0.0));
+        let mut got = 0usize;
+        check(unsafe {
+            sdr_fcsb_process(self.h, input.as_ptr() as *const f32, n_time, stride, output[at..].as_mut_ptr() as *mut f32,
+                             n, &mut got)
+        })?;
+        output.truncate(at + got);
+        Ok(got)
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_fcsb_reset(self.h) }) }
+}
+impl Clone for GpuFcsb {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_fcsb_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_fcsb_clone failed: {}", Error(err));
+        GpuFcsb { h, i: self.i.clone() }
+    }
+}
+impl Drop for GpuFcsb {
+    fn drop(&mut self) { unsafe { sdr_fcsb_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

@@ -44,6 +44,7 @@ pub enum sdr_psd_t {}
 pub enum sdr_fcfb_t {}
 pub enum sdr_pfs_t {}
 pub enum sdr_duc_t {}
+pub enum sdr_fcsb_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -199,6 +200,19 @@ pub struct sdr_fcfb_config_t {
 }
 
 #[repr(C)]
+pub struct sdr_fcsb_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub phase_inc: *const u64,
+    pub interpolation: *const size_t,
+    pub n_channels: size_t,
+    pub first_sample: u64,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
     pub rate: c_float,
@@ -345,6 +359,15 @@ extern "C" {
                             out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_fcfb_process_dev(h: *mut sdr_fcfb_t, input: *const c_void, n_in: size_t, out_c64: *mut c_float,
                                 out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_fcsb_create(cfg: *const sdr_fcsb_config_t, err: *mut c_int) -> *mut sdr_fcsb_t;
+    pub fn sdr_fcsb_destroy(h: *mut sdr_fcsb_t);
+    pub fn sdr_fcsb_reset(h: *mut sdr_fcsb_t) -> c_int;
+    pub fn sdr_fcsb_clone(h: *const sdr_fcsb_t, err: *mut c_int) -> *mut sdr_fcsb_t;
+    pub fn sdr_fcsb_output_count(h: *const sdr_fcsb_t, n_time: size_t) -> size_t;
+    pub fn sdr_fcsb_process(h: *mut sdr_fcsb_t, in_c64: *const c_float, n_time: size_t, in_stride: size_t,
+                            out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_fcsb_process_dev(h: *mut sdr_fcsb_t, in_c64: *const c_float, n_time: size_t, in_stride: size_t,
+                                out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

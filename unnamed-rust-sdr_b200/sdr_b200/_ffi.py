@@ -92,6 +92,11 @@ class DucConfig(C.Structure):
                 ("stream", vp)]
 
 
+class FcsbConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phase_inc", vp), ("interpolation", vp),
+                ("n_channels", sz), ("first_sample", C.c_uint64), ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -186,6 +191,13 @@ PROTOTYPES = {
     "sdr_fcfb_output_count": (i32, [vp, sz, vp]),
     "sdr_fcfb_process": (i32, [vp, vp, sz, vp, sz, sz, vp]),
     "sdr_fcfb_process_dev": (i32, [vp, vp, sz, vp, sz, sz, vp]),
+    "sdr_fcsb_create": (vp, [C.POINTER(FcsbConfig), C.POINTER(i32)]),
+    "sdr_fcsb_destroy": (None, [vp]),
+    "sdr_fcsb_reset": (i32, [vp]),
+    "sdr_fcsb_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_fcsb_output_count": (sz, [vp, sz]),
+    "sdr_fcsb_process": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
+    "sdr_fcsb_process_dev": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

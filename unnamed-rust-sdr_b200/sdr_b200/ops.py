@@ -913,6 +913,98 @@ class Fcfb:
     __del__ = close
 
 
+class Fcsb:
+    """Fast-convolution synthesis bank (sdr_fcsb), the inverse of Fcfb: channel k is zero-stuffed by interpolation[k]
+    (I_k, one value or one per channel; frame m at index (m+1) I_k - 1), filtered by its real taps (1-D: shared;
+    [C, L]: one row per channel), mixed UP by freqs[k] (a 64-bit NCO) and all channels are summed -- Duc's function
+    with its own I per channel -- computed by overlap-save on Fcfb's geometry.  first_sample = absolute stream index of
+    the first OUTPUT.  A call advances the handle by n_time output positions (a multiple of lcm(I_k)) and returns the
+    outputs of the blocks it completes (see geometry); to drain a finite stream feed zero frames covering N positions
+    and drop the outputs past its end.  There is no scale: the taps carry the factor I_k."""
+
+    def __init__(self, taps, freqs, rate, interpolation, first_sample=0, device=0, stream=None, _handle=None,
+                 _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        self._taps = t
+        self.phase_inc = np.array([ddc_phase_increment(f, rate) for f in np.atleast_1d(freqs)], np.uint64)
+        self.n_channels = int(self.phase_inc.size)
+        i = np.atleast_1d(np.asarray(interpolation, np.int64))
+        if i.size == 1:
+            i = np.repeat(i, self.n_channels)
+        if i.size != self.n_channels or (i < 1).any():
+            raise ValueError("interpolation: one value >= 1, or one per channel")
+        self.interpolation = np.ascontiguousarray(i, np.uintp)
+        self.lcm = int(np.lcm.reduce(i))
+        cfg = F.FcsbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
+                           self.interpolation.ctypes.data, self.n_channels, int(first_sample) % (1 << 64), device,
+                           _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_fcsb_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_fcsb_create")
+
+    @property
+    def geometry(self):
+        """(N, P): transform size and hop (output positions per block)"""
+        return fcfb_geometry(self._taps.shape[-1], self.interpolation)
+
+    def output_count(self, n_time):
+        """outputs of the blocks that the next n_time output positions complete"""
+        return lib().sdr_fcsb_output_count(self.h, n_time)
+
+    def process(self, rows):
+        """rows: C complex64 arrays (or a [C, n] array when every I_k is equal), row k of n_k frames with the same
+        n_k I_k for every k -> complex64 [released outputs]"""
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n_time = rows[0].size * int(self.interpolation[0])
+        if any(r.size * int(i) != n_time for r, i in zip(rows, self.interpolation)):
+            raise ValueError("rows: n_k I_k must be equal for every channel")
+        stride = max(max(r.size for r in rows), 1)
+        y = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            y[k, :r.size] = r
+        cnt = self.output_count(n_time)
+        out = np.empty(max(cnt, 1), np.complex64)
+        got = C.c_size_t(0)
+        check(lib().sdr_fcsb_process(self.h, y.ctypes.data if n_time else None, n_time, stride, out.ctypes.data, cnt,
+                                     C.byref(got)), "sdr_fcsb_process")
+        return out[:got.value]
+
+    def process_dev(self, d_in, n_time, d_out, out_cap, in_stride=None):
+        """device-resident: d_in C rows of in_stride (default the longest row, n_time / min I_k) complex64, row k
+        n_time / I_k frames; d_out out_cap samples; asynchronous on the handle's stream.  Returns the samples written."""
+        stride = n_time // int(self.interpolation.min()) if in_stride is None else in_stride
+        got = C.c_size_t(0)
+        check(lib().sdr_fcsb_process_dev(self.h, _ptr(d_in), n_time, stride, _ptr(d_out), out_cap, C.byref(got)),
+              "sdr_fcsb_process_dev")
+        return got.value
+
+    def reset(self):
+        check(lib().sdr_fcsb_reset(self.h), "sdr_fcsb_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_fcsb_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_fcsb_clone")
+        return Fcsb(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_fcsb_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
