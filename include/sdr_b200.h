@@ -776,6 +776,60 @@ int sdr_fcsb_process(sdr_fcsb_t *, const float *in_c64, size_t n_time, size_t in
 int sdr_fcsb_process_dev(sdr_fcsb_t *, const float *in_c64, size_t n_time, size_t in_stride, float *out_c64,
                          size_t out_cap, size_t *n_out);
 
+/* ======================================================================================
+ * rational resampler bank -- C independent c64 channel streams, channel k resampled by its own I_k / D_k with its own
+ * real taps h_k: the textbook upfirdn.  Channel k restates sdr_pfs's / sdr_duc's zero-stuffing grid,
+ * filter::Fir<f32, Complex<f32>> (src/filter/fir.rs:23-32) and signal::Decimate (adapters/mod.rs:30-37); m counts the
+ * handle's frames of the channel and frames before the stream are 0:
+ *   s_k[(m+1) I_k - 1] = y_k[m], 0 elsewhere
+ *   u_k[n] = sum_{j<L} h_k[j] s_k[n - j]
+ *   z_k[r] = u_k[(r+1) D_k - 1]
+ * Computed form: with t = (r+1) D_k - 1, q = (t+1) div I_k and c = (t+1) mod I_k,
+ *   z_k[r] = sum_{i < I_c} h_k[c + i I_k] y_k[q - 1 - i],   I_c = ceil((L - c) / I_k)
+ * as one fmaf chain per component in ascending i: a tap of exactly 0.0 is still multiplied (NaNs propagate exactly),
+ * taps with j >= L never are, and an output's bits do not depend on tiling, blocking or launch geometry.
+ * Reduction is exact: with g = gcd(I, D) the chain of (g I', g D') with taps h has the same terms in the same order as
+ * that of (I', D') with taps h[g j]; the bank reduces every channel at create.
+ * Counts: after a channel has received n frames in total it has released floor(n I_k / D_k) outputs (exact integer
+ * arithmetic); a call's count is the difference of two such floors and depends only on that channel's frames.
+ * Shards: a shard cut at frame s with s I_k = 0 (mod D_k) for every channel, primed with H frames, where H is a multiple
+ * of lcm_k(D_k / gcd(I_k, D_k)) and at least max_k ceil(L / I_k), gives one stream's bits after its first H I_k / D_k
+ * outputs per channel.  There is no NCO, and the output grid is relative to the handle, as for sdr_fir's decimation.
+ * Scale: none.  Unit gain needs taps with DC gain I_k, as for sdr_duc.
+ * Accuracy: |z_k - z_k,f64| <= 1e-5 max|z_k,f64| (DESIGN.md K13).
+ * Input: C rows, row k of n_in[k] c64 frames, row stride in_stride c64 (>= the longest row when C > 1): sdr_fcfb's
+ * mixed-rate rows of one call with its counts and out_stride, or sdr_ddc's / sdr_pfb's equal rows with one count
+ * repeated.  Output: C rows of row stride out_stride (>= the largest count when C > 1), out_cap outputs per row; a
+ * too-small out_cap returns SDR_ERR_OUTPUT_TOO_SMALL before any state changes; *n_out receives C counts.
+ * Carried state: the last ceil(L' / I') frames of every channel (L' = ceil(L / g)) and the per-channel frame totals;
+ * the caller's rows and the carried frames are read through two pointers (the rows are never copied).  One compute
+ * launch per call for all channels, and one small launch that updates the carried frames.  Device pointers need c64
+ * (8-byte) alignment.
+ * ====================================================================================== */
+typedef struct {
+    const float *taps;           /* n_tap_sets rows of n_taps real f32 */
+    size_t n_taps;               /* L, 1 <= L <= 2^20 */
+    size_t n_tap_sets;           /* 1 (shared) or n_channels; n_tap_sets * n_taps <= 2^26 */
+    const size_t *interpolation; /* n_channels I_k, 1 <= I_k <= 2^16 */
+    const size_t *decimation;    /* n_channels D_k, 1 <= D_k <= 2^24 */
+    size_t n_channels;           /* C, 1 <= C <= 65536 (sdr_pfb's channel-major rows included) */
+    int device;
+    void *stream;
+} sdr_rrb_config_t;
+
+typedef struct sdr_rrb sdr_rrb_t;
+sdr_rrb_t *sdr_rrb_create(const sdr_rrb_config_t *cfg, int *err);
+void sdr_rrb_destroy(sdr_rrb_t *);
+int sdr_rrb_reset(sdr_rrb_t *); /* carried frames dropped, frame counts back to 0 */
+sdr_rrb_t *sdr_rrb_clone(const sdr_rrb_t *, int *err);
+/* counts[k] = channel k's outputs from its next n_in[k] frames (C entries each) */
+int sdr_rrb_output_count(const sdr_rrb_t *, const size_t *n_in, size_t *counts);
+int sdr_rrb_process(sdr_rrb_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                    size_t out_cap, size_t out_stride, size_t *n_out);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_rrb_process_dev(sdr_rrb_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                        size_t out_cap, size_t out_stride, size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

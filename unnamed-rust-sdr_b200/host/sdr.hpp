@@ -474,6 +474,59 @@ class Fcsb {
     void reset() { check(sdr_fcsb_reset(h_), "Fcsb::reset"); }
 };
 
+// Rational resampler bank (sdr_rrb): channel k zero-stuffed by I_k, filtered by its real taps and decimated by D_k
+// (upfirdn).  After n frames a channel has released floor(n I_k / D_k) outputs; there is no scale (taps carry I_k).
+class Rrb {
+    sdr_rrb_t *h_ = nullptr;
+    size_t c_ = 0;
+
+  public:
+    Rrb(const std::vector<float> &taps, size_t n_taps, const std::vector<size_t> &interpolation,
+        const std::vector<size_t> &decimation)
+        : c_(interpolation.size()) {
+        if (decimation.size() != interpolation.size()) throw sdr::Error(SDR_ERR_INVALID_ARG, "Rrb::new");
+        sdr_rrb_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.interpolation = interpolation.data();
+        cfg.decimation = decimation.data();
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_rrb_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Rrb::new");
+    }
+    Rrb(Rrb &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
+    Rrb(const Rrb &o) : c_(o.c_) {
+        int err = 0;
+        h_ = sdr_rrb_clone(o.h_, &err);
+        if (!h_) throw sdr::Error(err, "Rrb::clone");
+    }
+    Rrb &operator=(const Rrb &) = delete;
+    ~Rrb() { sdr_rrb_destroy(h_); }
+    size_t channels() const { return c_; }
+    std::vector<size_t> output_count(const std::vector<size_t> &n_in) const {
+        std::vector<size_t> cnt(c_);
+        check(sdr_rrb_output_count(h_, n_in.data(), cnt.data()), "Rrb::output_count");
+        return cnt;
+    }
+    // in: channels rows, row k of n_in[k] frames at row stride in_stride (>= the longest row).  out: one vector per
+    // channel, replaced.
+    void process(const Complex *in, const std::vector<size_t> &n_in, size_t in_stride,
+                 std::vector<std::vector<Complex>> &out) {
+        const std::vector<size_t> cnt = output_count(n_in);
+        const size_t cap = std::max<size_t>(1, *std::max_element(cnt.begin(), cnt.end()));
+        std::vector<Complex> rows(cap * c_);
+        std::vector<size_t> got(c_);
+        check(sdr_rrb_process(h_, reinterpret_cast<const float *>(in), n_in.data(), in_stride,
+                              reinterpret_cast<float *>(rows.data()), cap, cap, got.data()),
+              "Rrb::process");
+        out.assign(c_, {});
+        for (size_t k = 0; k < c_; ++k) out[k].assign(rows.begin() + k * cap, rows.begin() + k * cap + got[k]);
+    }
+    void reset() { check(sdr_rrb_reset(h_), "Rrb::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

@@ -484,6 +484,61 @@ impl Drop for GpuFcsb {
     fn drop(&mut self) { unsafe { sdr_fcsb_destroy(self.h) } }
 }
 
+/// Rational resampler bank: channel k zero-stuffed by I_k, filtered by its real taps and decimated by D_k (upfirdn).
+/// After n frames a channel has released floor(n I_k / D_k) outputs; the taps carry the gain I_k.
+pub struct GpuRrb {
+    h: *mut sdr_rrb_t,
+    c: usize,
+}
+unsafe impl Send for GpuRrb {}
+
+impl GpuRrb {
+    /// taps: one row of n_taps (shared) or one row per channel; one interpolation and one decimation per channel
+    pub fn new(taps: &[f32], n_taps: usize, interpolation: &[usize], decimation: &[usize]) -> Result<Self, Error> {
+        if interpolation.len() != decimation.len() || n_taps == 0 { return Err(Error(100)); }
+        let cfg = sdr_rrb_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: taps.len() / n_taps, interpolation: interpolation.as_ptr(),
+            decimation: decimation.as_ptr(), n_channels: interpolation.len(), device: 0, stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_rrb_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuRrb { h, c: interpolation.len() })
+    }
+    /// input: one row per channel, row k of n_in[k] frames at row stride `stride` (>= the longest row); channel k's
+    /// outputs are appended to output[k]
+    pub fn process(&mut self, input: &[Complex<f32>], n_in: &[usize], stride: usize,
+                   output: &mut [Vec<Complex<f32>>]) -> Result<(), Error> {
+        assert!(n_in.len() == self.c);
+        assert!(n_in.iter().enumerate().all(|(k, &n)| n == 0 || input.len() >= k * stride + n));
+        let mut cnt = vec![0usize; self.c];
+        check(unsafe { sdr_rrb_output_count(self.h, n_in.as_ptr(), cnt.as_mut_ptr()) })?;
+        let cap = cnt.iter().copied().max().unwrap_or(0).max(1);
+        let mut rows = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut got = vec![0usize; self.c];
+        check(unsafe {
+            sdr_rrb_process(self.h, input.as_ptr() as *const f32, n_in.as_ptr(), stride, rows.as_mut_ptr() as *mut f32,
+                            cap, cap, got.as_mut_ptr())
+        })?;
+        for (k, out) in output.iter_mut().enumerate().take(self.c) {
+            out.extend_from_slice(&rows[k * cap..k * cap + got[k]]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_rrb_reset(self.h) }) }
+}
+impl Clone for GpuRrb {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_rrb_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_rrb_clone failed: {}", Error(err));
+        GpuRrb { h, c: self.c }
+    }
+}
+impl Drop for GpuRrb {
+    fn drop(&mut self) { unsafe { sdr_rrb_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

@@ -45,6 +45,7 @@ pub enum sdr_fcfb_t {}
 pub enum sdr_pfs_t {}
 pub enum sdr_duc_t {}
 pub enum sdr_fcsb_t {}
+pub enum sdr_rrb_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -213,6 +214,18 @@ pub struct sdr_fcsb_config_t {
 }
 
 #[repr(C)]
+pub struct sdr_rrb_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub interpolation: *const size_t,
+    pub decimation: *const size_t,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
     pub rate: c_float,
@@ -368,6 +381,15 @@ extern "C" {
                             out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_fcsb_process_dev(h: *mut sdr_fcsb_t, in_c64: *const c_float, n_time: size_t, in_stride: size_t,
                                 out_c64: *mut c_float, out_cap: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_rrb_create(cfg: *const sdr_rrb_config_t, err: *mut c_int) -> *mut sdr_rrb_t;
+    pub fn sdr_rrb_destroy(h: *mut sdr_rrb_t);
+    pub fn sdr_rrb_reset(h: *mut sdr_rrb_t) -> c_int;
+    pub fn sdr_rrb_clone(h: *const sdr_rrb_t, err: *mut c_int) -> *mut sdr_rrb_t;
+    pub fn sdr_rrb_output_count(h: *const sdr_rrb_t, n_in: *const size_t, counts: *mut size_t) -> c_int;
+    pub fn sdr_rrb_process(h: *mut sdr_rrb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                           out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_rrb_process_dev(h: *mut sdr_rrb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                               out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -97,6 +97,11 @@ class FcsbConfig(C.Structure):
                 ("n_channels", sz), ("first_sample", C.c_uint64), ("device", i32), ("stream", vp)]
 
 
+class RrbConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("interpolation", vp), ("decimation", vp),
+                ("n_channels", sz), ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -198,6 +203,13 @@ PROTOTYPES = {
     "sdr_fcsb_output_count": (sz, [vp, sz]),
     "sdr_fcsb_process": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
     "sdr_fcsb_process_dev": (i32, [vp, vp, sz, sz, vp, sz, C.POINTER(sz)]),
+    "sdr_rrb_create": (vp, [C.POINTER(RrbConfig), C.POINTER(i32)]),
+    "sdr_rrb_destroy": (None, [vp]),
+    "sdr_rrb_reset": (i32, [vp]),
+    "sdr_rrb_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_rrb_output_count": (i32, [vp, vp, vp]),
+    "sdr_rrb_process": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
+    "sdr_rrb_process_dev": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

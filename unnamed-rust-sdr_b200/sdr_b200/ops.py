@@ -1005,6 +1005,98 @@ class Fcsb:
     __del__ = close
 
 
+class Rrb:
+    """Rational resampler bank (sdr_rrb), the textbook upfirdn per channel: channel k is zero-stuffed by
+    interpolation[k] (I_k; frame m at index (m+1) I_k - 1), filtered by its real taps (1-D: shared; [C, L]: one row per
+    channel) and decimated by decimation[k] (D_k; output r is sample (r+1) D_k - 1).  interpolation and decimation
+    take one value or one per channel.  After n frames a channel has released floor(n I_k / D_k) outputs.  There is no
+    scale: unit gain needs taps with DC gain I_k."""
+
+    def __init__(self, taps, interpolation, decimation, n_channels=None, device=0, stream=None, _handle=None,
+                 _meta=None):
+        if _handle is not None:
+            self.h = _handle
+            self.__dict__.update(_meta)
+            return
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        i = np.atleast_1d(np.asarray(interpolation, np.int64))
+        d = np.atleast_1d(np.asarray(decimation, np.int64))
+        c = int(n_channels) if n_channels is not None else max(i.size, d.size, 1 if t.ndim == 1 else t.shape[0])
+        i = np.repeat(i, c) if i.size == 1 else i
+        d = np.repeat(d, c) if d.size == 1 else d
+        if i.size != c or d.size != c or (i < 1).any() or (d < 1).any():
+            raise ValueError("interpolation / decimation: one value >= 1, or one per channel")
+        self._taps = t
+        self.n_channels = c
+        self.interpolation = np.ascontiguousarray(i, np.uintp)
+        self.decimation = np.ascontiguousarray(d, np.uintp)
+        cfg = F.RrbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.interpolation.ctypes.data,
+                          self.decimation.ctypes.data, c, device, _stream_ptr(stream))
+        err = C.c_int(0)
+        self.h = lib().sdr_rrb_create(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_rrb_create")
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def output_count(self, n_in):
+        """outputs per channel (numpy array of C) from the next n_in frames (an int, or one count per channel)"""
+        n = self._counts(n_in)
+        cnt = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_rrb_output_count(self.h, n.ctypes.data, cnt.ctypes.data), "sdr_rrb_output_count")
+        return cnt.astype(np.int64)
+
+    def process(self, rows):
+        """rows: complex64 [C, n] or a list of C rows of any lengths -> list of C complex64 arrays"""
+        if isinstance(rows, np.ndarray) and rows.ndim == 1 and self.n_channels == 1:
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n = np.array([r.size for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        y = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            y[k, :r.size] = r
+        cnt = self.output_count(n)
+        cap = max(int(cnt.max()), 1)
+        out = np.empty((self.n_channels, cap), np.complex64)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_rrb_process(self.h, y.ctypes.data, n.ctypes.data, stride, out.ctypes.data, cap, cap,
+                                    got.ctypes.data), "sdr_rrb_process")
+        return [out[k, :int(got[k])] for k in range(self.n_channels)]
+
+    def process_dev(self, d_in, n_in, in_stride, d_out, out_cap, out_stride):
+        """device-resident: d_in C rows of in_stride complex64, row k of n_in (an int, or C counts) frames; d_out C rows
+        of out_stride complex64, out_cap outputs each; asynchronous on the handle's stream.  Returns the outputs written
+        per channel (numpy array of C)."""
+        n = self._counts(n_in)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_rrb_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), out_cap, out_stride,
+                                        got.ctypes.data), "sdr_rrb_process_dev")
+        return got.astype(np.int64)
+
+    def reset(self):
+        check(lib().sdr_rrb_reset(self.h), "sdr_rrb_reset")
+
+    def clone(self):
+        err = C.c_int(0)
+        h = lib().sdr_rrb_clone(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_rrb_clone")
+        return Rrb(None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sdr_rrb_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
