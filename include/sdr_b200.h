@@ -156,6 +156,9 @@ void sdr_fft_destroy(sdr_fft_t *);
 /* output elements (c64) per transform: n, or n - n/2 with SDR_FFT_RFFT */
 size_t sdr_fft_output_len(const sdr_fft_t *);
 int sdr_fft_exec(sdr_fft_t *, const void *in, size_t batches, float *out_c64);
+/* device pointers: `in` a multiple of the element size (U8IQ 2, C64 8, F32 4 bytes) and `out_c64` of 8 bytes,
+ * else SDR_ERR_MISALIGNED before anything runs.  Pointers that meet this but are not 16-byte aligned run kernels
+ * without bulk copies. */
 int sdr_fft_exec_dev(sdr_fft_t *, const void *in, size_t batches, float *out_c64);
 /* the frequency labels of fft.rs:14-24: labels[i] = (i - n/2) as f32 * (rate / n as f32);
  * with rfft != 0 only the kept n - n/2 entries are written.  Host-side, pure. */

@@ -688,6 +688,8 @@ extern "C" int sdr_fft_exec_dev(sdr_fft_t *p, const void *in, size_t batches, fl
     if (!p) return SDR_ERR_NULL_HANDLE;
     if (batches == 0) return SDR_OK;
     if (!in || !out) return SDR_ERR_BAD_DATA_PTR;
+    // the kernels load whole elements (u8 IQ pairs as 16-bit words) and store whole c64 values
+    if (((uintptr_t)in % elem_bytes(p->fmt)) != 0 || ((uintptr_t)out % 8) != 0) return SDR_ERR_MISALIGNED;
     DeviceGuard g(p->dev);
     if (!g.ok) return g.status();
     return fft_run_dev(p, in, batches, out);
