@@ -28,16 +28,6 @@ inline size_t f32_as_usize(float v) {
     return (size_t)v;
 }
 
-int check_device(int dev) {
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) {
-        cudaGetLastError();
-        return SDR_ERR_NO_DEVICE;
-    }
-    if (dev < 0 || dev >= n) return SDR_ERR_INVALID_ARG;
-    return SDR_OK;
-}
-
 int copy2d(void *dst, size_t dpitch, const void *src, size_t spitch, size_t width, size_t height, cudaMemcpyKind kind,
            cudaStream_t st) {
     if (width == 0 || height == 0) return SDR_OK;
@@ -53,6 +43,18 @@ struct HostPipe {
     cudaStream_t up = nullptr, down = nullptr;
     cudaEvent_t e_up[2] = {nullptr, nullptr}, e_k[2] = {nullptr, nullptr}, e_down[2] = {nullptr, nullptr};
     bool ready = false;
+    HostPipe() = default;
+    HostPipe(const HostPipe &) = delete;
+    HostPipe &operator=(const HostPipe &) = delete;
+    ~HostPipe() {
+        if (up) cudaStreamDestroy(up);
+        if (down) cudaStreamDestroy(down);
+        for (int i = 0; i < 2; ++i) {
+            if (e_up[i]) cudaEventDestroy(e_up[i]);
+            if (e_k[i]) cudaEventDestroy(e_k[i]);
+            if (e_down[i]) cudaEventDestroy(e_down[i]);
+        }
+    }
     int init() {
         if (ready) return SDR_OK;
         SDR_CUDA_TRY(cudaStreamCreateWithFlags(&up, cudaStreamNonBlocking));
@@ -64,17 +66,6 @@ struct HostPipe {
         }
         ready = true;
         return SDR_OK;
-    }
-    void release() {
-        if (up) cudaStreamDestroy(up);
-        if (down) cudaStreamDestroy(down);
-        for (int i = 0; i < 2; ++i) {
-            if (e_up[i]) cudaEventDestroy(e_up[i]);
-            if (e_k[i]) cudaEventDestroy(e_k[i]);
-            if (e_down[i]) cudaEventDestroy(e_down[i]);
-        }
-        up = down = nullptr;
-        ready = false;
     }
     // before uploading into buffer b: the kernel that last read it must be done
     int begin_upload(int b) { return cuda_status(cudaStreamWaitEvent(up, e_k[b], 0)); }
@@ -173,134 +164,108 @@ extern "C" int sdr_unpack_u8iq(const uint8_t *iq, size_t n, float *out, int devi
     if (!rc) rc = cuda_status(cudaMemcpy(din.p, iq, 2 * n, cudaMemcpyHostToDevice));
     if (!rc) rc = unpack_launch((const uint8_t *)din.p, n, (float *)dout.p, 0);
     if (!rc) rc = cuda_status(cudaMemcpy(out, dout.p, 8 * n, cudaMemcpyDeviceToHost));
-    din.release();
-    dout.release();
     return rc;
 }
 
 // ============================================================================================
 // FIR
 // ============================================================================================
-struct sdr_fir {
+struct FirHost {
     int dev = 0;
-    StreamRef stream;
     int fmt = 0, taps_complex = 0;
     unsigned flags = 0;
     size_t K = 0, Kp = 0, HL = 0, D = 1, n_ch = 1;
     size_t hist_stride = 0;
     std::vector<float> taps;  // padded host copy
-    float *d_taps = nullptr;
-    uint2 *d_tc_tables = nullptr;  // tensor-core Toeplitz tap fragments (u8 input, non-strict)
-    float tc_scale = 1.0f;
-    uint8_t *d_uc_tables = nullptr;  // tcgen05 Toeplitz bf16 tap-term tables (c64 input, real taps, non-strict, D == 1)
-    int uc_ns = 0;
-    uint8_t *d_um_tables = nullptr;  // tcgen05 Toeplitz digit tables (u8 input, non-strict, D == 1)
-    int um_R = 0, um_PC = 0, um_planar = 0, um_magic[2][3] = {{0, 0, 0}, {0, 0, 0}};
-    float um_sc[3] = {0.0f, 0.0f, 0.0f};
-    void *d_hist[2] = {nullptr, nullptr};
-    int cur = 0;
     size_t phase = 0;  // inputs already discarded in the current decimation group
-    DevBuf d_in, d_out, d_in2, d_out2;
-    HostPipe pipe;
     int last_path = 0;
 };
 
-static void fir_free(sdr_fir *f) {
-    if (!f) return;
-    DeviceGuard g(f->dev);
-    if (f->d_taps) cudaFree(f->d_taps);
-    if (f->d_tc_tables) cudaFree(f->d_tc_tables);
-    if (f->d_um_tables) cudaFree(f->d_um_tables);
-    if (f->d_uc_tables) cudaFree(f->d_uc_tables);
-    for (int i = 0; i < 2; ++i)
-        if (f->d_hist[i]) cudaFree(f->d_hist[i]);
-    f->d_in.release();
-    f->d_out.release();
-    f->d_in2.release();
-    f->d_out2.release();
-    f->pipe.release();
-    f->stream.release();
-    delete f;
-}
+struct sdr_fir : FirHost {
+    StreamRef stream;
+    DevBuf d_taps;
+    DevBuf d_tc_tables;  // tensor-core Toeplitz tap fragments (u8 input, non-strict)
+    float tc_scale = 1.0f;
+    DevBuf d_uc_tables;  // tcgen05 Toeplitz bf16 tap-term tables (c64 input, real taps, non-strict, D == 1)
+    int uc_ns = 0;
+    DevBuf d_um_tables;  // tcgen05 Toeplitz digit tables (u8 input, non-strict, D == 1)
+    int um_R = 0, um_PC = 0, um_planar = 0, um_magic[2][3] = {{0, 0, 0}, {0, 0, 0}};
+    float um_sc[3] = {0.0f, 0.0f, 0.0f};
+    DevBuf d_hist[2];
+    int cur = 0;
+    DevBuf d_in, d_out, d_in2, d_out2;
+    HostPipe pipe;
 
-static int fir_alloc(sdr_fir *f, void *user_stream) {
-    int rc = f->stream.init(user_stream);
+    int alloc(void *user_stream, const sdr_fir *);
+    int copy_device(const sdr_fir &src) {
+        return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, n_ch * hist_stride * elem_bytes(fmt),
+                                      cudaMemcpyDeviceToDevice));
+    }
+};
+
+int sdr_fir::alloc(void *user_stream, const sdr_fir *) {
+    int rc = stream.init(user_stream);
     if (rc) return rc;
-    const size_t tap_floats = f->Kp * (f->taps_complex ? 2 : 1);
-    SDR_CUDA_TRY(cudaMalloc(&f->d_taps, tap_floats * sizeof(float)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(f->d_taps, f->taps.data(), tap_floats * sizeof(float), cudaMemcpyHostToDevice, f->stream.s));
-    const size_t hbytes = f->n_ch * f->hist_stride * elem_bytes(f->fmt);
-    for (int i = 0; i < 2; ++i) SDR_CUDA_TRY(cudaMalloc(&f->d_hist[i], hbytes));
-    rc = fir_fill_hist(f->d_hist[0], f->fmt, (long long)(f->n_ch * f->hist_stride), f->stream.s);
+    if ((rc = d_taps.upload(taps.data(), Kp * (taps_complex ? 2 : 1) * sizeof(float), stream.s))) return rc;
+    const size_t hbytes = n_ch * hist_stride * elem_bytes(fmt);
+    for (int i = 0; i < 2; ++i)
+        if ((rc = d_hist[i].alloc(hbytes))) return rc;
+    rc = fir_fill_hist(d_hist[0].p, fmt, (long long)(n_ch * hist_stride), stream.s);
     if (rc) return rc;
-    if (f->fmt == SDR_FMT_U8IQ && !(f->flags & (SDR_FIR_STRICT_ORDER | SDR_FIR_NO_TENSOR)) && f->K <= 4096 && f->D <= 64) {
+    if (fmt == SDR_FMT_U8IQ && !(flags & (SDR_FIR_STRICT_ORDER | SDR_FIR_NO_TENSOR)) && K <= 4096 && D <= 64) {
         std::vector<uint2> tab;
-        f->tc_scale = fir_tc_build_tables(f->taps.data(), (int)f->K, f->taps_complex != 0, (int)f->D, tab);
-        SDR_CUDA_TRY(cudaMalloc(&f->d_tc_tables, tab.size() * sizeof(uint2)));
-        SDR_CUDA_TRY(cudaMemcpyAsync(f->d_tc_tables, tab.data(), tab.size() * sizeof(uint2), cudaMemcpyHostToDevice, f->stream.s));
-        SDR_CUDA_TRY(cudaStreamSynchronize(f->stream.s));
+        tc_scale = fir_tc_build_tables(taps.data(), (int)K, taps_complex != 0, (int)D, tab);
+        if ((rc = d_tc_tables.upload(tab.data(), tab.size() * sizeof(uint2), stream.s))) return rc;
+        SDR_CUDA_TRY(cudaStreamSynchronize(stream.s));
     }
     int R = 0, PC = 0, planar = 0;
-    if (f->fmt == SDR_FMT_U8IQ && !(f->flags & (SDR_FIR_STRICT_ORDER | SDR_FIR_NO_TENSOR | SDR_FIR_NO_TCGEN05)) && f->D <= (1u << 20) &&
-        fir_umma_geometry((int)f->K, (int)f->D, f->taps_complex != 0, (f->flags & SDR_FIR_PLANAR) != 0, &R, &PC, &planar)) {
+    if (fmt == SDR_FMT_U8IQ && !(flags & (SDR_FIR_STRICT_ORDER | SDR_FIR_NO_TENSOR | SDR_FIR_NO_TCGEN05)) && D <= (1u << 20) &&
+        fir_umma_geometry((int)K, (int)D, taps_complex != 0, (flags & SDR_FIR_PLANAR) != 0, &R, &PC, &planar)) {
         std::vector<uint8_t> tab;
-        if (fir_umma_build_tables(f->taps.data(), (int)f->K, f->taps_complex != 0, R, PC, planar, (int)f->D, tab, f->um_magic, f->um_sc)) {
-            f->um_R = R;
-            f->um_PC = PC;
-            f->um_planar = planar;
-            SDR_CUDA_TRY(cudaMalloc(&f->d_um_tables, tab.size()));
-            SDR_CUDA_TRY(cudaMemcpyAsync(f->d_um_tables, tab.data(), tab.size(), cudaMemcpyHostToDevice, f->stream.s));
-            SDR_CUDA_TRY(cudaStreamSynchronize(f->stream.s));
+        if (fir_umma_build_tables(taps.data(), (int)K, taps_complex != 0, R, PC, planar, (int)D, tab, um_magic, um_sc)) {
+            um_R = R;
+            um_PC = PC;
+            um_planar = planar;
+            if ((rc = d_um_tables.upload(tab.data(), tab.size(), stream.s))) return rc;
+            SDR_CUDA_TRY(cudaStreamSynchronize(stream.s));
         }
     }
-    if (f->fmt == SDR_FMT_C64 && !(f->flags & (SDR_FIR_STRICT_ORDER | SDR_FIR_NO_TENSOR | SDR_FIR_NO_TCGEN05))) {
+    if (fmt == SDR_FMT_C64 && !(flags & (SDR_FIR_STRICT_ORDER | SDR_FIR_NO_TENSOR | SDR_FIR_NO_TCGEN05))) {
         // three bf16 terms per operand (the reference's f32 accuracy) when the tables and planes fit in shared memory
         // (K <= 384), two terms (< 1e-5 of max|y|) on request or for longer filters
-        const int ns = ((f->flags & SDR_FIR_SPLIT2) || !fir_umma_c64_applies((int)f->K, (int)f->D, f->taps_complex != 0, 3)) ? 2 : 3;
+        const int ns = ((flags & SDR_FIR_SPLIT2) || !fir_umma_c64_applies((int)K, (int)D, taps_complex != 0, 3)) ? 2 : 3;
         std::vector<uint8_t> tab;
-        if (fir_umma_c64_applies((int)f->K, (int)f->D, f->taps_complex != 0, ns) && f->K >= 8 &&
-            fir_umma_c64_build_tables(f->taps.data(), (int)f->K, ns, tab)) {
-            f->uc_ns = ns;
-            SDR_CUDA_TRY(cudaMalloc(&f->d_uc_tables, tab.size()));
-            SDR_CUDA_TRY(cudaMemcpyAsync(f->d_uc_tables, tab.data(), tab.size(), cudaMemcpyHostToDevice, f->stream.s));
+        if (fir_umma_c64_applies((int)K, (int)D, taps_complex != 0, ns) && K >= 8 &&
+            fir_umma_c64_build_tables(taps.data(), (int)K, ns, tab)) {
+            uc_ns = ns;
+            if ((rc = d_uc_tables.upload(tab.data(), tab.size(), stream.s))) return rc;
         }
     }
-    SDR_CUDA_TRY(cudaStreamSynchronize(f->stream.s));
-    return SDR_OK;
+    return cuda_status(cudaStreamSynchronize(stream.s));
 }
 
 extern "C" sdr_fir_t *sdr_fir_create(const sdr_fir_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->taps || cfg->n_taps == 0 || cfg->decimation == 0 || cfg->n_channels == 0 ||
         cfg->n_taps > (1u << 20) || cfg->input_format < 0 || cfg->input_format > 2 ||
-        (cfg->taps_complex && cfg->input_format == SDR_FMT_F32)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    if ((*err = check_device(cfg->device)) != SDR_OK) return nullptr;
-    sdr_fir *f = new (std::nothrow) sdr_fir;
-    if (!f) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    f->dev = cfg->device;
-    f->fmt = cfg->input_format;
-    f->taps_complex = cfg->taps_complex ? 1 : 0;
-    f->flags = cfg->flags;
-    f->K = cfg->n_taps;
-    f->Kp = round_up(f->K, 8);
-    f->HL = f->Kp;
-    f->hist_stride = f->HL;  // multiple of 8 elements: rows stay 16-byte aligned in every format
-    f->D = cfg->decimation;
-    f->n_ch = cfg->n_channels;
-    const int w = f->taps_complex ? 2 : 1;
-    f->taps.assign(f->Kp * w, 0.0f);
-    std::memcpy(f->taps.data(), cfg->taps, f->K * w * sizeof(float));
-    DeviceGuard g(f->dev);
-    *err = g.ok ? fir_alloc(f, cfg->stream) : g.status();
-    if (*err) { fir_free(f); return nullptr; }
-    return f;
+        (cfg->taps_complex && cfg->input_format == SDR_FMT_F32))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_fir>(err, cfg->device, cfg->stream, [&](sdr_fir &f) {
+        f.fmt = cfg->input_format;
+        f.taps_complex = cfg->taps_complex ? 1 : 0;
+        f.flags = cfg->flags;
+        f.K = cfg->n_taps;
+        f.Kp = round_up(f.K, 8);
+        f.HL = f.Kp;
+        f.hist_stride = f.HL;  // multiple of 8 elements: rows stay 16-byte aligned in every format
+        f.D = cfg->decimation;
+        f.n_ch = cfg->n_channels;
+        const int w = f.taps_complex ? 2 : 1;
+        f.taps.assign(f.Kp * w, 0.0f);
+        std::memcpy(f.taps.data(), cfg->taps, f.K * w * sizeof(float));
+        return SDR_OK;
+    });
 }
-extern "C" void sdr_fir_destroy(sdr_fir_t *f) { fir_free(f); }
+extern "C" void sdr_fir_destroy(sdr_fir_t *f) { destroy_handle(f); }
 
 extern "C" int sdr_fir_reset(sdr_fir_t *f) {
     if (!f) return SDR_ERR_NULL_HANDLE;
@@ -308,30 +273,12 @@ extern "C" int sdr_fir_reset(sdr_fir_t *f) {
     if (!g.ok) return g.status();
     f->phase = 0;
     f->cur = 0;
-    int rc = fir_fill_hist(f->d_hist[0], f->fmt, (long long)(f->n_ch * f->hist_stride), f->stream.s);
+    int rc = fir_fill_hist(f->d_hist[0].p, f->fmt, (long long)(f->n_ch * f->hist_stride), f->stream.s);
     if (rc) return rc;
     return cuda_status(cudaStreamSynchronize(f->stream.s));
 }
 
-extern "C" sdr_fir_t *sdr_fir_clone(const sdr_fir_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_fir *f = new (std::nothrow) sdr_fir;
-    if (!f) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    f->dev = src->dev; f->fmt = src->fmt; f->taps_complex = src->taps_complex; f->flags = src->flags;
-    f->K = src->K; f->Kp = src->Kp; f->HL = src->HL; f->D = src->D; f->n_ch = src->n_ch;
-    f->hist_stride = src->hist_stride; f->taps = src->taps; f->phase = src->phase;
-    DeviceGuard g(f->dev);
-    *err = fir_alloc(f, src->stream.owned ? nullptr : (void *)src->stream.s);
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err)
-        *err = cuda_status(cudaMemcpy(f->d_hist[0], src->d_hist[src->cur],
-                                      f->n_ch * f->hist_stride * elem_bytes(f->fmt), cudaMemcpyDeviceToDevice));
-    if (*err) { fir_free(f); return nullptr; }
-    return f;
-}
+extern "C" sdr_fir_t *sdr_fir_clone(const sdr_fir_t *src, int *err) { return clone_handle<FirHost>(src, err); }
 
 extern "C" size_t sdr_fir_output_count(const sdr_fir_t *f, size_t n_in) {
     if (!f) return 0;
@@ -344,9 +291,9 @@ static int fir_run_dev(sdr_fir *f, const void *in, size_t n_in, size_t in_stride
                        size_t n_out) {
     FirArgs a;
     a.in = in;
-    a.hist = f->d_hist[f->cur];
+    a.hist = f->d_hist[f->cur].p;
     a.out = out;
-    a.taps = f->d_taps;
+    a.taps = (const float *)f->d_taps.p;
     a.n_in = (long long)n_in;
     a.in_stride = (long long)in_stride;
     a.out_stride = (long long)out_stride;
@@ -356,21 +303,22 @@ static int fir_run_dev(sdr_fir *f, const void *in, size_t n_in, size_t in_stride
     a.K = (int)f->K; a.Kp = (int)f->Kp; a.HL = (int)f->HL; a.D = (int)f->D; a.n_ch = (int)f->n_ch;
     const bool strict = (f->flags & SDR_FIR_STRICT_ORDER) != 0;
     int rc = SDR_ERR_UNSUPPORTED;
-    if (f->d_um_tables) {
-        rc = fir_umma_launch(a, f->um_R, f->um_PC, f->um_planar, f->d_um_tables, f->um_magic, f->um_sc, f->stream.s);
+    if (f->d_um_tables.p) {
+        rc = fir_umma_launch(a, f->um_R, f->um_PC, f->um_planar, (const uint8_t *)f->d_um_tables.p, f->um_magic, f->um_sc,
+                             f->stream.s);
         if (rc == SDR_OK) f->last_path = 4;
     }
-    if (rc == SDR_ERR_UNSUPPORTED && f->d_uc_tables) {
-        rc = fir_umma_c64_launch(a, f->uc_ns, f->d_uc_tables, f->stream.s);
+    if (rc == SDR_ERR_UNSUPPORTED && f->d_uc_tables.p) {
+        rc = fir_umma_c64_launch(a, f->uc_ns, (const uint8_t *)f->d_uc_tables.p, f->stream.s);
         if (rc == SDR_OK) f->last_path = 5;
     }
-    if (rc == SDR_ERR_UNSUPPORTED && f->d_tc_tables) {
-        rc = fir_tc_launch(a, f->taps_complex != 0, f->d_tc_tables, f->tc_scale, f->stream.s);
+    if (rc == SDR_ERR_UNSUPPORTED && f->d_tc_tables.p) {
+        rc = fir_tc_launch(a, f->taps_complex != 0, (const uint2 *)f->d_tc_tables.p, f->tc_scale, f->stream.s);
         if (rc == SDR_OK) f->last_path = 3;
     }
     if (rc == SDR_ERR_UNSUPPORTED) rc = fir_launch(a, f->fmt, f->taps_complex != 0, strict, f->stream.s, &f->last_path);
     if (rc) return rc;
-    rc = fir_hist_update(in, f->d_hist[f->cur], f->d_hist[f->cur ^ 1], f->fmt, (int)f->HL, (long long)n_in,
+    rc = fir_hist_update(in, f->d_hist[f->cur].p, f->d_hist[f->cur ^ 1].p, f->fmt, (int)f->HL, (long long)n_in,
                          (long long)in_stride, (long long)f->hist_stride, (int)f->n_ch, f->stream.s);
     if (rc) return rc;
     f->cur ^= 1;
@@ -466,49 +414,38 @@ extern "C" int sdr_fir_process(sdr_fir_t *f, const void *in, size_t n_in, size_t
 // ============================================================================================
 // FFT
 // ============================================================================================
-struct sdr_fft {
+struct FftHost {
     int dev = 0;
-    StreamRef stream;
     size_t n = 0;
     int fmt = 0;
     unsigned flags = 0;
     int mode = 0;  // 0 single-launch pow2 kernels, 1 naive, 2 bluestein, 3 pow2 through convert / four-step / finish
     int log_n = 0;
     float norm = 1.0f;
-    float2 *d_tw = nullptr;     // W_n (pow2 / naive) or W_m (bluestein), when that length is <= 2^16
-    float2 *d_tw1 = nullptr, *d_tw2 = nullptr;  // lengths above 2^16: W tables of the two four-step factors
     // bluestein
     size_t m = 0;
     int log_m = 0;
-    float2 *d_chirp = nullptr, *d_bfft = nullptr;
+};
+
+struct sdr_fft : FftHost {
+    StreamRef stream;
+    DevBuf d_tw;          // W_n (pow2 / naive) or W_m (bluestein), when that length is <= 2^16
+    DevBuf d_tw1, d_tw2;  // lengths above 2^16: W tables of the two four-step factors
+    DevBuf d_chirp, d_bfft;  // bluestein
     DevBuf d_a1, d_a2, d_work, d_h1, d_h2;
     DevBuf d_in, d_out, d_in2, d_out2;
     HostPipe pipe;
+
+    int alloc(void *user_stream, const sdr_fft *);
 };
 
-static void fft_free(sdr_fft *p) {
-    if (!p) return;
-    DeviceGuard g(p->dev);
-    if (p->d_tw) cudaFree(p->d_tw);
-    if (p->d_tw1) cudaFree(p->d_tw1);
-    if (p->d_tw2) cudaFree(p->d_tw2);
-    if (p->d_chirp) cudaFree(p->d_chirp);
-    if (p->d_bfft) cudaFree(p->d_bfft);
-    p->d_a1.release(); p->d_a2.release(); p->d_work.release(); p->d_h1.release(); p->d_h2.release();
-    p->d_in.release(); p->d_out.release(); p->d_in2.release(); p->d_out2.release();
-    p->pipe.release();
-    p->stream.release();
-    delete p;
-}
-
-static int upload_twiddles(float2 **dptr, size_t n, cudaStream_t st) {
+static int upload_twiddles(DevBuf &d, size_t n, cudaStream_t st) {
     std::vector<float2> tw(n);
     const double c = -2.0 * M_PI / (double)n;
     for (size_t k = 0; k < n; ++k) tw[k] = make_float2((float)std::cos(c * (double)k), (float)std::sin(c * (double)k));
-    SDR_CUDA_TRY(cudaMalloc(dptr, n * sizeof(float2)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(*dptr, tw.data(), n * sizeof(float2), cudaMemcpyHostToDevice, st));
-    SDR_CUDA_TRY(cudaStreamSynchronize(st));
-    return SDR_OK;
+    const int rc = d.upload(tw.data(), n * sizeof(float2), st);
+    if (rc) return rc;
+    return cuda_status(cudaStreamSynchronize(st));
 }
 
 static int ilog2_exact(size_t n) {
@@ -522,10 +459,10 @@ constexpr int FFT_MAX_LOG = 27;  // 2^27 c64 = 1 GiB per buffer; the four-step p
 // tables for a plain c64 transform of length 2^l: one table up to 2^16, the two factor tables above
 static int fft_pow2_tables(sdr_fft *p, int l) {
     cudaStream_t st = p->stream.s;
-    if (l <= 16) return upload_twiddles(&p->d_tw, (size_t)1 << l, st);
+    if (l <= 16) return upload_twiddles(p->d_tw, (size_t)1 << l, st);
     const int l1 = l / 2, l2 = l - l1;
-    int rc = upload_twiddles(&p->d_tw1, (size_t)1 << l1, st);
-    if (!rc) rc = upload_twiddles(&p->d_tw2, (size_t)1 << l2, st);
+    int rc = upload_twiddles(p->d_tw1, (size_t)1 << l1, st);
+    if (!rc) rc = upload_twiddles(p->d_tw2, (size_t)1 << l2, st);
     return rc;
 }
 
@@ -534,7 +471,8 @@ static int fft_pow2_c64(sdr_fft *p, const float2 *in, float2 *out, int l, size_t
     cudaStream_t st = p->stream.s;
     if (l <= 16) {
         FftArgs a;
-        a.in = in; a.out = out; a.tw = p->d_tw; a.batches = (long long)batches; a.log_n = l; a.fmt = SDR_FMT_C64;
+        a.in = in; a.out = out; a.tw = (const float2 *)p->d_tw.p; a.batches = (long long)batches; a.log_n = l;
+        a.fmt = SDR_FMT_C64;
         a.flags = 0; a.norm = 1.0f;
         if (l >= 13) {
             const int rc = p->d_work.reserve((batches + 1) * sizeof(int));
@@ -548,7 +486,8 @@ static int fft_pow2_c64(sdr_fft *p, const float2 *in, float2 *out, int l, size_t
     if (!rc) rc = p->d_h2.reserve(bytes);
     if (!rc) rc = p->d_work.reserve(((batches << (l - l / 2)) + 1) * sizeof(int));
     if (rc) return rc;
-    return fft_huge_launch(in, out, (float2 *)p->d_h1.p, (float2 *)p->d_h2.p, p->d_tw1, p->d_tw2, l, (long long)batches,
+    return fft_huge_launch(in, out, (float2 *)p->d_h1.p, (float2 *)p->d_h2.p, (const float2 *)p->d_tw1.p,
+                           (const float2 *)p->d_tw2.p, l, (long long)batches,
                            (int *)p->d_work.p, st);
 }
 
@@ -559,7 +498,7 @@ static int fft_plan_init(sdr_fft *p) {
     if (l2 >= 4 && l2 <= 16 && !((p->flags & SDR_FFT_RFFT) && l2 >= 15)) {
         p->mode = 0;
         p->log_n = l2;
-        return upload_twiddles(&p->d_tw, n, st);
+        return upload_twiddles(p->d_tw, n, st);
     }
     if (l2 >= 15) {  // 2^17 and up, and rfft of 2^15 / 2^16
         if (l2 > FFT_MAX_LOG) return SDR_ERR_UNSUPPORTED;
@@ -569,7 +508,7 @@ static int fft_plan_init(sdr_fft *p) {
     }
     if (n <= 64) {
         p->mode = 1;
-        return upload_twiddles(&p->d_tw, n, st);
+        return upload_twiddles(p->d_tw, n, st);
     }
     // Bluestein: m = smallest power of two >= 2n-1
     p->mode = 2;
@@ -589,40 +528,33 @@ static int fft_plan_init(sdr_fft *p) {
         b[j] = w;
         if (j > 0) b[m - j] = w;
     }
-    SDR_CUDA_TRY(cudaMalloc(&p->d_chirp, n * sizeof(float2)));
-    SDR_CUDA_TRY(cudaMalloc(&p->d_bfft, m * sizeof(float2)));
-    float2 *d_b = nullptr;
-    SDR_CUDA_TRY(cudaMalloc(&d_b, m * sizeof(float2)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(p->d_chirp, chirp.data(), n * sizeof(float2), cudaMemcpyHostToDevice, st));
-    SDR_CUDA_TRY(cudaMemcpyAsync(d_b, b.data(), m * sizeof(float2), cudaMemcpyHostToDevice, st));
-    rc = fft_pow2_c64(p, d_b, p->d_bfft, p->log_m, 1);
-    cudaError_t e = cudaStreamSynchronize(st);
-    cudaFree(d_b);
+    DevBuf d_b;
+    if ((rc = p->d_chirp.upload(chirp.data(), n * sizeof(float2), st)) || (rc = p->d_bfft.alloc(m * sizeof(float2))) ||
+        (rc = d_b.upload(b.data(), m * sizeof(float2), st)))
+        return rc;
+    rc = fft_pow2_c64(p, (const float2 *)d_b.p, (float2 *)p->d_bfft.p, p->log_m, 1);
+    cudaError_t e = cudaStreamSynchronize(st);  // before d_b is freed
     if (rc) return rc;
     return cuda_status(e);
 }
 
-extern "C" sdr_fft_t *sdr_fft_create(const sdr_fft_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!cfg || cfg->n == 0 || cfg->input_format < 0 || cfg->input_format > 2) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    if ((cfg->flags & SDR_FFT_RFFT) && cfg->input_format != SDR_FMT_F32) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    if ((*err = check_device(cfg->device)) != SDR_OK) return nullptr;
-    sdr_fft *p = new (std::nothrow) sdr_fft;
-    if (!p) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    p->dev = cfg->device;
-    p->n = cfg->n;
-    p->fmt = cfg->input_format;
-    p->flags = cfg->flags;
-    p->norm = 1.0f / sqrtf((float)cfg->n);  // fft.rs:16
-    DeviceGuard g(p->dev);
-    *err = g.ok ? p->stream.init(cfg->stream) : g.status();
-    if (!*err) *err = fft_plan_init(p);
-    if (*err) { fft_free(p); return nullptr; }
-    return p;
+int sdr_fft::alloc(void *user_stream, const sdr_fft *) {
+    int rc = stream.init(user_stream);
+    return rc ? rc : fft_plan_init(this);
 }
-extern "C" void sdr_fft_destroy(sdr_fft_t *p) { fft_free(p); }
+
+extern "C" sdr_fft_t *sdr_fft_create(const sdr_fft_config_t *cfg, int *err) {
+    if (!cfg || cfg->n == 0 || cfg->input_format < 0 || cfg->input_format > 2) return fail(err, SDR_ERR_INVALID_ARG);
+    if ((cfg->flags & SDR_FFT_RFFT) && cfg->input_format != SDR_FMT_F32) return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_fft>(err, cfg->device, cfg->stream, [&](sdr_fft &p) {
+        p.n = cfg->n;
+        p.fmt = cfg->input_format;
+        p.flags = cfg->flags;
+        p.norm = 1.0f / sqrtf((float)cfg->n);  // fft.rs:16
+        return SDR_OK;
+    });
+}
+extern "C" void sdr_fft_destroy(sdr_fft_t *p) { destroy_handle(p); }
 extern "C" size_t sdr_fft_output_len(const sdr_fft_t *p) {
     if (!p) return 0;
     return (p->flags & SDR_FFT_RFFT) ? p->n - p->n / 2 : p->n;
@@ -632,7 +564,7 @@ static int fft_run_dev(sdr_fft *p, const void *in, size_t batches, float *out) {
     cudaStream_t st = p->stream.s;
     if (p->mode == 0) {
         FftArgs a;
-        a.in = in; a.out = (float2 *)out; a.tw = p->d_tw; a.batches = (long long)batches; a.log_n = p->log_n;
+        a.in = in; a.out = (float2 *)out; a.tw = (const float2 *)p->d_tw.p; a.batches = (long long)batches; a.log_n = p->log_n;
         a.fmt = p->fmt; a.flags = p->flags; a.norm = p->norm;
         if (p->log_n >= 13) {
             const int rc = p->d_work.reserve((batches + 1) * sizeof(int));
@@ -642,7 +574,7 @@ static int fft_run_dev(sdr_fft *p, const void *in, size_t batches, float *out) {
         return fft_pow2_launch(a, st);
     }
     if (p->mode == 1)
-        return fft_naive_launch(in, (float2 *)out, p->d_tw, (long long)batches, (int)p->n, p->fmt, p->flags, p->norm, st);
+        return fft_naive_launch(in, (float2 *)out, (const float2 *)p->d_tw.p, (long long)batches, (int)p->n, p->fmt, p->flags, p->norm, st);
     const size_t out_len = sdr_fft_output_len(p);
     if (p->mode == 3) {
         // convert -> plain c64 transform -> shift / norm / rfft selection, in slabs that bound the scratch footprint
@@ -669,15 +601,15 @@ static int fft_run_dev(sdr_fft *p, const void *in, size_t batches, float *out) {
         const size_t nb = std::min(slab, batches - b0);
         const char *inb = (const char *)in + b0 * p->n * elem_bytes(p->fmt);
         float2 *a1 = (float2 *)p->d_a1.p, *a2 = (float2 *)p->d_a2.p;
-        rc = bluestein_pre_launch(inb, a1, p->d_chirp, (long long)nb, (int)p->n, (int)p->m, p->fmt, st);
+        rc = bluestein_pre_launch(inb, a1, (const float2 *)p->d_chirp.p, (long long)nb, (int)p->n, (int)p->m, p->fmt, st);
         if (rc) return rc;
         rc = fft_pow2_c64(p, a1, a2, p->log_m, nb);
         if (rc) return rc;
-        rc = bluestein_mul_launch(a2, p->d_bfft, (long long)nb, (int)p->m, st);
+        rc = bluestein_mul_launch(a2, (const float2 *)p->d_bfft.p, (long long)nb, (int)p->m, st);
         if (rc) return rc;
         rc = fft_pow2_c64(p, a2, a1, p->log_m, nb);
         if (rc) return rc;
-        rc = bluestein_post_launch(a1, (float2 *)out + b0 * out_len, p->d_chirp, (long long)nb, (int)p->n, (int)p->m,
+        rc = bluestein_post_launch(a1, (float2 *)out + b0 * out_len, (const float2 *)p->d_chirp.p, (long long)nb, (int)p->n, (int)p->m,
                                    p->flags, p->norm, st);
         if (rc) return rc;
     }
@@ -777,104 +709,71 @@ extern "C" int sdr_biquad_design(const sdr_biquad_design_t *d, float rate, float
     return SDR_OK;
 }
 
-struct sdr_pll {
+struct PllHost {
     int dev = 0;
-    StreamRef stream;
     size_t n_streams = 0, n_designs = 0;
     unsigned flags = 0;
     std::vector<PllParams> params;
     bool any_identity = false;  // some sub-filter is filter::Identity: the kernel keeps its per-filter kind tests
-    PllParams *d_params = nullptr;
-    PllState *d_state = nullptr;
-    DevBuf d_in, d_out, d_lk;
 };
 
-static void pll_free(sdr_pll *p) {
-    if (!p) return;
-    DeviceGuard g(p->dev);
-    if (p->d_params) cudaFree(p->d_params);
-    if (p->d_state) cudaFree(p->d_state);
-    p->d_in.release(); p->d_out.release(); p->d_lk.release();
-    p->stream.release();
-    delete p;
-}
+struct sdr_pll : PllHost {
+    StreamRef stream;
+    DevBuf d_params, d_state;
+    DevBuf d_in, d_out, d_lk;
 
-static int pll_alloc(sdr_pll *p, void *user_stream) {
-    int rc = p->stream.init(user_stream);
-    if (rc) return rc;
-    SDR_CUDA_TRY(cudaMalloc(&p->d_params, p->params.size() * sizeof(PllParams)));
-    SDR_CUDA_TRY(cudaMalloc(&p->d_state, p->n_streams * sizeof(PllState)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(p->d_params, p->params.data(), p->params.size() * sizeof(PllParams),
-                                 cudaMemcpyHostToDevice, p->stream.s));
-    SDR_CUDA_TRY(cudaMemsetAsync(p->d_state, 0, p->n_streams * sizeof(PllState), p->stream.s));  // pll.rs:57-58
-    SDR_CUDA_TRY(cudaStreamSynchronize(p->stream.s));
-    return SDR_OK;
-}
+    int alloc(void *user_stream, const sdr_pll *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        if ((rc = d_params.upload(params.data(), params.size() * sizeof(PllParams), stream.s)) ||
+            (rc = d_state.alloc(n_streams * sizeof(PllState))))
+            return rc;
+        SDR_CUDA_TRY(cudaMemsetAsync(d_state.p, 0, n_streams * sizeof(PllState), stream.s));  // pll.rs:57-58
+        return cuda_status(cudaStreamSynchronize(stream.s));
+    }
+    int copy_device(const sdr_pll &src) {
+        return cuda_status(cudaMemcpy(d_state.p, src.d_state.p, n_streams * sizeof(PllState), cudaMemcpyDeviceToDevice));
+    }
+};
 
 extern "C" sdr_pll_t *sdr_pll_create(const sdr_pll_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->designs || cfg->n_streams == 0 || cfg->n_streams > (1u << 24) ||
-        (cfg->n_designs != 1 && cfg->n_designs != cfg->n_streams)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    if ((*err = check_device(cfg->device)) != SDR_OK) return nullptr;
-    sdr_pll *p = new (std::nothrow) sdr_pll;
-    if (!p) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    p->dev = cfg->device;
-    p->n_streams = cfg->n_streams;
-    p->n_designs = cfg->n_designs;
-    p->flags = cfg->flags;
-    p->params.resize(cfg->n_designs);
-    for (size_t i = 0; i < cfg->n_designs; ++i) {
-        const sdr_pll_design_t &d = cfg->designs[i];
-        PllParams &q = p->params[i];
-        q.reference = d.reference / cfg->rate;  // pll.rs:51
-        q.gain = d.gain;
-        q.rate = cfg->rate;
-        q.lk = d.loopfilter.kind; q.ok = d.outputfilter.kind; q.kk = d.lockfilter.kind;
-        if (q.lk == SDR_BQ_IDENTITY || q.ok == SDR_BQ_IDENTITY || q.kk == SDR_BQ_IDENTITY) p->any_identity = true;
-        // the specialised kernel also assumes |nphase + reference + gain * arg| < 2 (nphase in (-1, 1), |arg| <= pi), so
-        // that f32::fract needs no general trunc; designs with a larger step per sample take the general kernel
-        if (!(std::fabs(q.reference) + 3.1416f * std::fabs(q.gain) < 0.999f)) p->any_identity = true;
-        if (cfg->flags & SDR_PLL_GENERAL_KERNEL) p->any_identity = true;
-        int rc = sdr_biquad_design(&d.loopfilter, cfg->rate, q.lc);
-        if (!rc) rc = sdr_biquad_design(&d.outputfilter, cfg->rate, q.oc);
-        if (!rc) rc = sdr_biquad_design(&d.lockfilter, cfg->rate, q.kc);
-        if (rc) { *err = rc; delete p; return nullptr; }
-    }
-    DeviceGuard g(p->dev);
-    *err = g.ok ? pll_alloc(p, cfg->stream) : g.status();
-    if (*err) { pll_free(p); return nullptr; }
-    return p;
+        (cfg->n_designs != 1 && cfg->n_designs != cfg->n_streams))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_pll>(err, cfg->device, cfg->stream, [&](sdr_pll &p) {
+        p.n_streams = cfg->n_streams;
+        p.n_designs = cfg->n_designs;
+        p.flags = cfg->flags;
+        p.params.resize(cfg->n_designs);
+        for (size_t i = 0; i < cfg->n_designs; ++i) {
+            const sdr_pll_design_t &d = cfg->designs[i];
+            PllParams &q = p.params[i];
+            q.reference = d.reference / cfg->rate;  // pll.rs:51
+            q.gain = d.gain;
+            q.rate = cfg->rate;
+            q.lk = d.loopfilter.kind; q.ok = d.outputfilter.kind; q.kk = d.lockfilter.kind;
+            if (q.lk == SDR_BQ_IDENTITY || q.ok == SDR_BQ_IDENTITY || q.kk == SDR_BQ_IDENTITY) p.any_identity = true;
+            // the specialised kernel also assumes |nphase + reference + gain * arg| < 2 (nphase in (-1, 1), |arg| <= pi), so
+            // that f32::fract needs no general trunc; designs with a larger step per sample take the general kernel
+            if (!(std::fabs(q.reference) + 3.1416f * std::fabs(q.gain) < 0.999f)) p.any_identity = true;
+            if (cfg->flags & SDR_PLL_GENERAL_KERNEL) p.any_identity = true;
+            int rc = sdr_biquad_design(&d.loopfilter, cfg->rate, q.lc);
+            if (!rc) rc = sdr_biquad_design(&d.outputfilter, cfg->rate, q.oc);
+            if (!rc) rc = sdr_biquad_design(&d.lockfilter, cfg->rate, q.kc);
+            if (rc) return rc;
+        }
+        return SDR_OK;
+    });
 }
-extern "C" void sdr_pll_destroy(sdr_pll_t *p) { pll_free(p); }
+extern "C" void sdr_pll_destroy(sdr_pll_t *p) { destroy_handle(p); }
 extern "C" int sdr_pll_reset(sdr_pll_t *p) {
     if (!p) return SDR_ERR_NULL_HANDLE;
     DeviceGuard g(p->dev);
     if (!g.ok) return g.status();
-    SDR_CUDA_TRY(cudaMemsetAsync(p->d_state, 0, p->n_streams * sizeof(PllState), p->stream.s));
+    SDR_CUDA_TRY(cudaMemsetAsync(p->d_state.p, 0, p->n_streams * sizeof(PllState), p->stream.s));
     return cuda_status(cudaStreamSynchronize(p->stream.s));
 }
-extern "C" sdr_pll_t *sdr_pll_clone(const sdr_pll_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_pll *p = new (std::nothrow) sdr_pll;
-    if (!p) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    p->dev = src->dev; p->n_streams = src->n_streams; p->n_designs = src->n_designs; p->flags = src->flags;
-    p->params = src->params;
-    p->any_identity = src->any_identity;
-    DeviceGuard g(p->dev);
-    *err = pll_alloc(p, src->stream.owned ? nullptr : (void *)src->stream.s);
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err) *err = cuda_status(cudaMemcpy(p->d_state, src->d_state, p->n_streams * sizeof(PllState), cudaMemcpyDeviceToDevice));
-    if (*err) { pll_free(p); return nullptr; }
-    return p;
-}
+extern "C" sdr_pll_t *sdr_pll_clone(const sdr_pll_t *src, int *err) { return clone_handle<PllHost>(src, err); }
 
 extern "C" int sdr_pll_process_dev(sdr_pll_t *p, const float *in, size_t n, size_t in_stride, float *out,
                                    uint8_t *locked, size_t out_stride) {
@@ -886,7 +785,7 @@ extern "C" int sdr_pll_process_dev(sdr_pll_t *p, const float *in, size_t n, size
     DeviceGuard g(p->dev);
     if (!g.ok) return g.status();
     return pll_launch((const float2 *)in, (long long)n, (long long)in_stride, out, locked, (long long)out_stride,
-                      p->d_params, p->n_designs == 1, p->d_state, (int)p->n_streams,
+                      (const PllParams *)p->d_params.p, p->n_designs == 1, (PllState *)p->d_state.p, (int)p->n_streams,
                       (p->flags & SDR_PLL_F64_MATH) == 0, p->any_identity, p->stream.s);
 }
 
@@ -908,7 +807,7 @@ extern "C" int sdr_pll_process(sdr_pll_t *p, const float *in, size_t n, size_t i
     rc = copy2d(p->d_in.p, n * 8, in, in_stride * 8, n * 8, S, cudaMemcpyHostToDevice, st);
     if (rc) return rc;
     rc = pll_launch((const float2 *)p->d_in.p, (long long)n, (long long)n, (float *)p->d_out.p, (uint8_t *)p->d_lk.p,
-                    (long long)n, p->d_params, p->n_designs == 1, p->d_state, (int)S,
+                    (long long)n, (const PllParams *)p->d_params.p, p->n_designs == 1, (PllState *)p->d_state.p, (int)S,
                     (p->flags & SDR_PLL_F64_MATH) == 0, p->any_identity, st);
     if (rc) return rc;
     rc = copy2d(out, out_stride * 4, p->d_out.p, n * 4, n * 4, S, cudaMemcpyDeviceToHost, st);
@@ -926,9 +825,9 @@ extern "C" int sdr_pll_stereo_decode_dev(sdr_pll_t *p, const float *v, size_t n,
     if (in_stride < n || out_stride < n) return SDR_ERR_INVALID_ARG;
     DeviceGuard g(p->dev);
     if (!g.ok) return g.status();
-    return pll_stereo_launch(v, (long long)n, (long long)in_stride, out_md, (long long)out_stride, p->d_params,
-                             p->n_designs == 1, p->d_state, (int)p->n_streams, (p->flags & SDR_PLL_F64_MATH) == 0,
-                             p->stream.s);
+    return pll_stereo_launch(v, (long long)n, (long long)in_stride, out_md, (long long)out_stride,
+                             (const PllParams *)p->d_params.p, p->n_designs == 1, (PllState *)p->d_state.p,
+                             (int)p->n_streams, (p->flags & SDR_PLL_F64_MATH) == 0, p->stream.s);
 }
 
 extern "C" int sdr_pll_stereo_decode(sdr_pll_t *p, const float *v, size_t n, size_t in_stride, float *out_md,
@@ -948,7 +847,8 @@ extern "C" int sdr_pll_stereo_decode(sdr_pll_t *p, const float *v, size_t n, siz
     rc = copy2d(p->d_in.p, n * 4, v, in_stride * 4, n * 4, S, cudaMemcpyHostToDevice, st);
     if (rc) return rc;
     rc = pll_stereo_launch((const float *)p->d_in.p, (long long)n, (long long)n, (float *)p->d_out.p, (long long)n,
-                           p->d_params, p->n_designs == 1, p->d_state, (int)S, (p->flags & SDR_PLL_F64_MATH) == 0, st);
+                           (const PllParams *)p->d_params.p, p->n_designs == 1, (PllState *)p->d_state.p, (int)S,
+                           (p->flags & SDR_PLL_F64_MATH) == 0, st);
     if (rc) return rc;
     rc = copy2d(out_md, out_stride * 8, p->d_out.p, n * 8, n * 8, S, cudaMemcpyDeviceToHost, st);
     if (rc) return rc;
@@ -962,7 +862,7 @@ extern "C" int sdr_pll_get_state(sdr_pll_t *p, size_t idx, float *nphase, float 
     if (!g.ok) return g.status();
     PllState s;
     SDR_CUDA_TRY(cudaStreamSynchronize(p->stream.s));
-    SDR_CUDA_TRY(cudaMemcpy(&s, p->d_state + idx, sizeof(s), cudaMemcpyDeviceToHost));
+    SDR_CUDA_TRY(cudaMemcpy(&s, (const PllState *)p->d_state.p + idx, sizeof(s), cudaMemcpyDeviceToHost));
     if (nphase) *nphase = s.nphase;
     if (vre) *vre = s.vre;
     if (vim) *vim = s.vim;
@@ -972,92 +872,61 @@ extern "C" int sdr_pll_get_state(sdr_pll_t *p, size_t idx, float *nphase, float 
 // ============================================================================================
 // Biquad stream filter
 // ============================================================================================
-struct sdr_biquad {
+struct BiquadHost {
     int dev = 0;
-    StreamRef stream;
     size_t n_streams = 0, n_designs = 0;
     int W = 1;
     std::vector<float> coef;  // 5 per design
     std::vector<int> kind;
-    float *d_coef = nullptr, *d_state = nullptr;
-    int *d_kind = nullptr;
-    DevBuf d_in, d_out;
 };
-static void biquad_free(sdr_biquad *b) {
-    if (!b) return;
-    DeviceGuard g(b->dev);
-    if (b->d_coef) cudaFree(b->d_coef);
-    if (b->d_kind) cudaFree(b->d_kind);
-    if (b->d_state) cudaFree(b->d_state);
-    b->d_in.release(); b->d_out.release();
-    b->stream.release();
-    delete b;
-}
-static int biquad_alloc(sdr_biquad *b, void *user_stream) {
-    int rc = b->stream.init(user_stream);
-    if (rc) return rc;
-    const size_t nseq = b->n_streams * b->W;
-    SDR_CUDA_TRY(cudaMalloc(&b->d_coef, b->coef.size() * sizeof(float)));
-    SDR_CUDA_TRY(cudaMalloc(&b->d_kind, b->kind.size() * sizeof(int)));
-    SDR_CUDA_TRY(cudaMalloc(&b->d_state, nseq * 4 * sizeof(float)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(b->d_coef, b->coef.data(), b->coef.size() * sizeof(float), cudaMemcpyHostToDevice, b->stream.s));
-    SDR_CUDA_TRY(cudaMemcpyAsync(b->d_kind, b->kind.data(), b->kind.size() * sizeof(int), cudaMemcpyHostToDevice, b->stream.s));
-    SDR_CUDA_TRY(cudaMemsetAsync(b->d_state, 0, nseq * 4 * sizeof(float), b->stream.s));
-    return cuda_status(cudaStreamSynchronize(b->stream.s));
-}
+
+struct sdr_biquad : BiquadHost {
+    StreamRef stream;
+    DevBuf d_coef, d_kind, d_state;
+    DevBuf d_in, d_out;
+
+    size_t state_bytes() const { return n_streams * W * 4 * sizeof(float); }
+    int alloc(void *user_stream, const sdr_biquad *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        if ((rc = d_coef.upload(coef.data(), coef.size() * sizeof(float), stream.s)) ||
+            (rc = d_kind.upload(kind.data(), kind.size() * sizeof(int), stream.s)) || (rc = d_state.alloc(state_bytes())))
+            return rc;
+        SDR_CUDA_TRY(cudaMemsetAsync(d_state.p, 0, state_bytes(), stream.s));
+        return cuda_status(cudaStreamSynchronize(stream.s));
+    }
+    int copy_device(const sdr_biquad &src) {
+        return cuda_status(cudaMemcpy(d_state.p, src.d_state.p, state_bytes(), cudaMemcpyDeviceToDevice));
+    }
+};
+
 extern "C" sdr_biquad_t *sdr_biquad_create(const sdr_biquad_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->designs || cfg->n_streams == 0 || cfg->n_streams > (1u << 24) ||
-        (cfg->n_designs != 1 && cfg->n_designs != cfg->n_streams)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    if ((*err = check_device(cfg->device)) != SDR_OK) return nullptr;
-    sdr_biquad *b = new (std::nothrow) sdr_biquad;
-    if (!b) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    b->dev = cfg->device;
-    b->n_streams = cfg->n_streams;
-    b->n_designs = cfg->n_designs;
-    b->W = cfg->sample_complex ? 2 : 1;
-    b->coef.resize(5 * cfg->n_designs);
-    b->kind.resize(cfg->n_designs);
-    for (size_t i = 0; i < cfg->n_designs; ++i) {
-        b->kind[i] = cfg->designs[i].kind;
-        const int rc = sdr_biquad_design(&cfg->designs[i], cfg->rate, &b->coef[5 * i]);
-        if (rc) { *err = rc; delete b; return nullptr; }
-    }
-    DeviceGuard g(b->dev);
-    *err = g.ok ? biquad_alloc(b, cfg->stream) : g.status();
-    if (*err) { biquad_free(b); return nullptr; }
-    return b;
+        (cfg->n_designs != 1 && cfg->n_designs != cfg->n_streams))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_biquad>(err, cfg->device, cfg->stream, [&](sdr_biquad &b) {
+        b.n_streams = cfg->n_streams;
+        b.n_designs = cfg->n_designs;
+        b.W = cfg->sample_complex ? 2 : 1;
+        b.coef.resize(5 * cfg->n_designs);
+        b.kind.resize(cfg->n_designs);
+        for (size_t i = 0; i < cfg->n_designs; ++i) {
+            b.kind[i] = cfg->designs[i].kind;
+            const int rc = sdr_biquad_design(&cfg->designs[i], cfg->rate, &b.coef[5 * i]);
+            if (rc) return rc;
+        }
+        return SDR_OK;
+    });
 }
-extern "C" void sdr_biquad_destroy(sdr_biquad_t *b) { biquad_free(b); }
+extern "C" void sdr_biquad_destroy(sdr_biquad_t *b) { destroy_handle(b); }
 extern "C" int sdr_biquad_reset(sdr_biquad_t *b) {
     if (!b) return SDR_ERR_NULL_HANDLE;
     DeviceGuard g(b->dev);
     if (!g.ok) return g.status();
-    SDR_CUDA_TRY(cudaMemsetAsync(b->d_state, 0, b->n_streams * b->W * 4 * sizeof(float), b->stream.s));
+    SDR_CUDA_TRY(cudaMemsetAsync(b->d_state.p, 0, b->state_bytes(), b->stream.s));
     return cuda_status(cudaStreamSynchronize(b->stream.s));
 }
-extern "C" sdr_biquad_t *sdr_biquad_clone(const sdr_biquad_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_biquad *b = new (std::nothrow) sdr_biquad;
-    if (!b) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    b->dev = src->dev; b->n_streams = src->n_streams; b->n_designs = src->n_designs; b->W = src->W;
-    b->coef = src->coef; b->kind = src->kind;
-    DeviceGuard g(b->dev);
-    *err = biquad_alloc(b, src->stream.owned ? nullptr : (void *)src->stream.s);
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err)
-        *err = cuda_status(cudaMemcpy(b->d_state, src->d_state, b->n_streams * b->W * 4 * sizeof(float), cudaMemcpyDeviceToDevice));
-    if (*err) { biquad_free(b); return nullptr; }
-    return b;
-}
+extern "C" sdr_biquad_t *sdr_biquad_clone(const sdr_biquad_t *src, int *err) { return clone_handle<BiquadHost>(src, err); }
 extern "C" int sdr_biquad_process_dev(sdr_biquad_t *b, const float *in, size_t n, size_t in_stride, float *out, size_t out_stride) {
     if (!b) return SDR_ERR_NULL_HANDLE;
     if (n == 0) return SDR_OK;
@@ -1066,8 +935,9 @@ extern "C" int sdr_biquad_process_dev(sdr_biquad_t *b, const float *in, size_t n
     if (in_stride < n || out_stride < n) return SDR_ERR_INVALID_ARG;
     DeviceGuard g(b->dev);
     if (!g.ok) return g.status();
-    return biquad_launch(in, (long long)n, (long long)in_stride, out, (long long)out_stride, b->W, b->d_coef, b->d_kind,
-                         b->n_designs == 1, b->d_state, (int)(b->n_streams * b->W), b->stream.s);
+    return biquad_launch(in, (long long)n, (long long)in_stride, out, (long long)out_stride, b->W,
+                         (const float *)b->d_coef.p, (const int *)b->d_kind.p, b->n_designs == 1, (float *)b->d_state.p,
+                         (int)(b->n_streams * b->W), b->stream.s);
 }
 extern "C" int sdr_biquad_process(sdr_biquad_t *b, const float *in, size_t n, size_t in_stride, float *out, size_t out_stride) {
     if (!b) return SDR_ERR_NULL_HANDLE;
@@ -1085,7 +955,8 @@ extern "C" int sdr_biquad_process(sdr_biquad_t *b, const float *in, size_t n, si
     rc = copy2d(b->d_in.p, n * eb, in, in_stride * eb, n * eb, S, cudaMemcpyHostToDevice, st);
     if (!rc)
         rc = biquad_launch((const float *)b->d_in.p, (long long)n, (long long)n, (float *)b->d_out.p, (long long)n, b->W,
-                           b->d_coef, b->d_kind, b->n_designs == 1, b->d_state, (int)(S * b->W), st);
+                           (const float *)b->d_coef.p, (const int *)b->d_kind.p, b->n_designs == 1, (float *)b->d_state.p,
+                           (int)(S * b->W), st);
     if (!rc) rc = copy2d(out, out_stride * eb, b->d_out.p, n * eb, n * eb, S, cudaMemcpyDeviceToHost, st);
     if (rc) return rc;
     return cuda_status(cudaStreamSynchronize(st));
@@ -1096,51 +967,37 @@ extern "C" int sdr_biquad_process(sdr_biquad_t *b, const float *in, size_t n, si
 // PLL kernel consumes immediately on the same stream.
 // ============================================================================================
 struct sdr_channelizer {
-    sdr_fir *fir = nullptr;
-    sdr_pll *pll = nullptr;
+    Owned<sdr_fir, sdr_fir_destroy> fir;
+    Owned<sdr_pll, sdr_pll_destroy> pll;
     DevBuf mid;
     DevBuf d_in, d_out, d_lk;
 };
 
 extern "C" sdr_channelizer_t *sdr_channelizer_create(const sdr_fir_config_t *fc, const sdr_pll_config_t *pc, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!fc || !pc || fc->n_channels != pc->n_streams || fc->decimation != 1 || fc->input_format == SDR_FMT_F32 ||
-        fc->device != pc->device) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
+        fc->device != pc->device)
+        return fail(err, SDR_ERR_INVALID_ARG);
     sdr_channelizer *c = new (std::nothrow) sdr_channelizer;
-    if (!c) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    c->fir = sdr_fir_create(fc, err);
+    if (!c) return fail(err, SDR_ERR_MALLOC_FAILED);
+    c->fir.reset(sdr_fir_create(fc, err));
     if (c->fir) {
         sdr_pll_config_t pc2 = *pc;
         pc2.stream = (void *)c->fir->stream.s;  // one stream: FIR slab i is followed by PLL slab i
-        c->pll = sdr_pll_create(&pc2, err);
+        c->pll.reset(sdr_pll_create(&pc2, err));
     }
-    if (!c->fir || !c->pll) {
-        sdr_fir_destroy(c->fir);
-        sdr_pll_destroy(c->pll);
-        delete c;
-        return nullptr;
-    }
-    return c;
+    if (c->pll) return c;
+    delete c;
+    return nullptr;
 }
 extern "C" void sdr_channelizer_destroy(sdr_channelizer_t *c) {
     if (!c) return;
-    {
-        DeviceGuard g(c->fir->dev);
-        c->mid.release(); c->d_in.release(); c->d_out.release(); c->d_lk.release();
-    }
-    sdr_pll_destroy(c->pll);
-    sdr_fir_destroy(c->fir);
+    DeviceGuard g(c->fir->dev);
     delete c;
 }
 extern "C" int sdr_channelizer_reset(sdr_channelizer_t *c) {
     if (!c) return SDR_ERR_NULL_HANDLE;
-    int rc = sdr_fir_reset(c->fir);
-    if (!rc) rc = sdr_pll_reset(c->pll);
+    int rc = sdr_fir_reset(c->fir.get());
+    if (!rc) rc = sdr_pll_reset(c->pll.get());
     return rc;
 }
 
@@ -1164,12 +1021,12 @@ extern "C" int sdr_channelizer_process_dev(sdr_channelizer_t *c, const void *in,
     for (size_t s0 = 0; s0 < n; s0 += slab) {
         const size_t cnt = std::min(slab, n - s0);
         size_t used = 0, got = 0;
-        rc = sdr_fir_process_dev(c->fir, (const char *)in + s0 * es, cnt, in_stride, c->mid.p, slab, slab, &used, &got);
+        rc = sdr_fir_process_dev(c->fir.get(), (const char *)in + s0 * es, cnt, in_stride, c->mid.p, slab, slab, &used, &got);
         if (rc) return rc;
         if (C == 1) {
-            rc = sdr_pll_process_dev(c->pll, (const float *)c->mid.p, cnt, cnt, out + s0, locked + s0, cnt);
+            rc = sdr_pll_process_dev(c->pll.get(), (const float *)c->mid.p, cnt, cnt, out + s0, locked + s0, cnt);
         } else {
-            rc = sdr_pll_process_dev(c->pll, (const float *)c->mid.p, cnt, slab, out + s0, locked + s0, out_stride);
+            rc = sdr_pll_process_dev(c->pll.get(), (const float *)c->mid.p, cnt, slab, out + s0, locked + s0, out_stride);
         }
         if (rc) return rc;
     }
@@ -1207,9 +1064,8 @@ extern "C" int sdr_channelizer_process(sdr_channelizer_t *c, const void *in, siz
 // resampler ("sdr-src": see DESIGN.md).  Host side = the position/count state machine; the device
 // holds the carried frames followed by the current input in one contiguous buffer v.
 // ============================================================================================
-struct sdr_src {
+struct SrcHost {
     int dev = 0;
-    StreamRef stream;
     int type = 0, channels = 1;
     double ratio = 0.0;
     bool fresh = true;
@@ -1219,19 +1075,41 @@ struct sdr_src {
     double spos = 0.0;
     long long kept = 0, total_in = 0, origin_abs = 0;
     bool ended = false;
-    float *d_table = nullptr;
+    bool exact = false;  // sdr_src_set_exact: always take the f64 kernels
+};
+
+struct sdr_src : SrcHost {
+    StreamRef stream;
+    DevBuf d_table;
     DevBuf v[2];
     int cur = 0;
     DevBuf carry;  // ZOH / linear: the frame before in[0]
     DevBuf d_out;
     DevBuf coef;   // sinc: per-phase wing coefficients of the polyphase fast path
-    // tensor-core path (integer step, 2 channels): branch filters' Toeplitz tables, phase planes
-    bool exact = false;            // sdr_src_set_exact: always take the f64 kernels
+    // tensor-core path (integer step, 2 channels), built on first use: branch filters' Toeplitz tables, phase planes
     int fast_S = 0, fast_Kb = 0, fast_ns = 0;
     double fast_ratio = 0.0;
-    uint8_t *d_fast_tab = nullptr; // [S][2 deltas][KS][(32 ns) x 32 B]
+    DevBuf d_fast_tab; // [S][2 deltas][KS][(32 ns) x 32 B]
     size_t fast_tab_stride = 0;
     DevBuf fast_planes;
+
+    int alloc(void *user_stream, const sdr_src *) {
+        int rc = stream.init(user_stream);
+        if (rc || type > SDR_SRC_SINC_FASTEST) return rc;
+        const float *tab = nullptr;
+        int inc = 0;
+        const size_t hl = src_sinc_table_host(type, &tab, &inc);
+        return d_table.upload(tab, (hl + 2) * sizeof(float), stream.s);
+    }
+    int copy_device(const sdr_src &o) {
+        const bool zl = type >= SDR_SRC_ZERO_ORDER_HOLD;
+        const size_t bytes = (size_t)(zl ? 1 : kept) * channels * sizeof(float);
+        DevBuf &dst = zl ? carry : v[0];
+        const DevBuf &from = zl ? o.carry : o.v[o.cur];
+        int rc = dst.reserve(std::max<size_t>(bytes, 16));
+        if (!rc && bytes && from.p) rc = cuda_status(cudaMemcpy(dst.p, from.p, bytes, cudaMemcpyDeviceToDevice));
+        return rc;
+    }
 };
 
 static bool bad_ratio(double r) { return !(r >= 1.0 / 256.0 && r <= 256.0); }
@@ -1241,44 +1119,22 @@ static void src_reset_state(sdr_src *s) {
     s->ended = false; s->cur = 0;
 }
 
-static void src_free(sdr_src *s) {
-    if (!s) return;
-    DeviceGuard g(s->dev);
-    if (s->d_table) cudaFree(s->d_table);
-    if (s->d_fast_tab) cudaFree(s->d_fast_tab);
-    s->v[0].release(); s->fast_planes.release(); s->v[1].release(); s->carry.release(); s->d_out.release(); s->coef.release();
-    s->stream.release();
-    delete s;
-}
-
 extern "C" SDR_SRC_STATE *sdr_src_new_on(int type, int channels, int device, void *stream, int *error) {
-    int dummy;
-    if (!error) error = &dummy;
-    *error = SDR_OK;
-    if (channels < 1) { *error = SDR_ERR_BAD_CHANNEL_COUNT; return nullptr; }
-    if (type < 0 || type > 4) { *error = SDR_ERR_BAD_CONVERTER; return nullptr; }
-    if ((*error = check_device(device)) != SDR_OK) return nullptr;
-    sdr_src *s = new (std::nothrow) sdr_src;
-    if (!s) { *error = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    s->dev = device; s->type = type; s->channels = channels;
-    src_reset_state(s);
-    DeviceGuard g(device);
-    *error = g.ok ? s->stream.init(stream) : g.status();
-    if (!*error && type <= SDR_SRC_SINC_FASTEST) {
-        const float *tab = nullptr;
-        int inc = 0;
-        const size_t hl = src_sinc_table_host(type, &tab, &inc);
-        cudaError_t e = cudaMalloc(&s->d_table, (hl + 2) * sizeof(float));
-        if (e == cudaSuccess) e = cudaMemcpy(s->d_table, tab, (hl + 2) * sizeof(float), cudaMemcpyHostToDevice);
-        *error = cuda_status(e);
-    }
-    if (*error) { src_free(s); return nullptr; }
-    return s;
+    if (channels < 1) return fail(error, SDR_ERR_BAD_CHANNEL_COUNT);
+    if (type < 0 || type > 4) return fail(error, SDR_ERR_BAD_CONVERTER);
+    return create_handle<sdr_src>(error, device, stream, [&](sdr_src &s) {
+        s.type = type;
+        s.channels = channels;
+        return SDR_OK;
+    });
 }
 extern "C" SDR_SRC_STATE *sdr_src_new(int type, int channels, int *error) {
     return sdr_src_new_on(type, channels, 0, nullptr, error);
 }
-extern "C" SDR_SRC_STATE *sdr_src_delete(SDR_SRC_STATE *s) { src_free(s); return nullptr; }
+extern "C" SDR_SRC_STATE *sdr_src_delete(SDR_SRC_STATE *s) {
+    destroy_handle(s);
+    return nullptr;
+}
 extern "C" int sdr_src_reset(SDR_SRC_STATE *s) {
     if (!s) return SDR_ERR_BAD_STATE;
     src_reset_state(s);
@@ -1330,26 +1186,8 @@ extern "C" size_t sdr_src_sinc_table(int type, const float **table, int *increme
 }
 
 extern "C" SDR_SRC_STATE *sdr_src_clone(SDR_SRC_STATE *o, int *error) {
-    int dummy;
-    if (!error) error = &dummy;
-    *error = SDR_OK;
-    if (!o) { *error = SDR_ERR_BAD_STATE; return nullptr; }
-    sdr_src *s = sdr_src_new_on(o->type, o->channels, o->dev, o->stream.owned ? nullptr : (void *)o->stream.s, error);
-    if (!s) return nullptr;
-    s->ratio = o->ratio; s->fresh = o->fresh; s->pos = o->pos; s->spos = o->spos; s->kept = o->kept;
-    s->total_in = o->total_in; s->origin_abs = o->origin_abs; s->ended = o->ended; s->cur = 0;
-    s->exact = o->exact;
-    DeviceGuard g(s->dev);
-    const bool zl = (o->type >= SDR_SRC_ZERO_ORDER_HOLD);
-    const size_t bytes = (size_t)(zl ? 1 : o->kept) * o->channels * sizeof(float);
-    DevBuf &dst = zl ? s->carry : s->v[0];
-    const DevBuf &from = zl ? o->carry : o->v[o->cur];
-    *error = dst.reserve(std::max<size_t>(bytes, 16));
-    if (!*error) *error = cuda_status(cudaStreamSynchronize(o->stream.s));
-    if (!*error && bytes && from.p)
-        *error = cuda_status(cudaMemcpy(dst.p, from.p, bytes, cudaMemcpyDeviceToDevice));
-    if (*error) { src_free(s); return nullptr; }
-    return s;
+    if (!o) return fail(error, SDR_ERR_BAD_STATE);
+    return clone_handle<SrcHost>(o, error);
 }
 
 // number of outputs m in [0, cap] such that ok(m') holds for all m' < m, where ok is monotone
@@ -1381,7 +1219,7 @@ static int src_fast_run(sdr_src *s, const SrcLaunch &L, cudaStream_t st) {
     const int ns = fir_umma_c64_applies(Kb, 1, false, 3) ? 3 : 2;
     if (!fir_umma_c64_applies(Kb, 1, false, ns)) return SDR_ERR_UNSUPPORTED;
     const double ratio = 1.0 / step;
-    if (!s->d_fast_tab || s->fast_S != (int)S || s->fast_Kb != Kb || s->fast_ns != ns || s->fast_ratio != ratio) {
+    if (!s->d_fast_tab.p || s->fast_S != (int)S || s->fast_Kb != Kb || s->fast_ns != ns || s->fast_ratio != ratio) {
         // (re)build the branch filters' Toeplitz tables: once per (converter, ratio), reused by every later call
         std::vector<float> br;
         src_fast_taps(s->type, ratio, (int)S, br);
@@ -1390,9 +1228,9 @@ static int src_fast_run(sdr_src *s, const SrcLaunch &L, cudaStream_t st) {
             if (!fir_umma_c64_build_tables(br.data() + (size_t)b * Kb, Kb, ns, one)) return SDR_ERR_UNSUPPORTED;
             all.insert(all.end(), one.begin(), one.end());
         }
-        if (s->d_fast_tab) { cudaStreamSynchronize(st); cudaFree(s->d_fast_tab); s->d_fast_tab = nullptr; }
-        SDR_CUDA_TRY(cudaMalloc(&s->d_fast_tab, all.size()));
-        SDR_CUDA_TRY(cudaMemcpyAsync(s->d_fast_tab, all.data(), all.size(), cudaMemcpyHostToDevice, st));
+        if (s->d_fast_tab.p) cudaStreamSynchronize(st);  // the old tables may still be in use
+        int rc = s->d_fast_tab.upload(all.data(), all.size(), st);
+        if (rc) return rc;
         SDR_CUDA_TRY(cudaStreamSynchronize(st));  // `all` is pageable host memory
         s->fast_tab_stride = one.size();
         s->fast_S = (int)S; s->fast_Kb = Kb; s->fast_ns = ns; s->fast_ratio = ratio;
@@ -1417,7 +1255,7 @@ static int src_fast_run(sdr_src *s, const SrcLaunch &L, cudaStream_t st) {
     a.first = 0;
     a.K = Kb; a.Kp = Kb; a.HL = 0; a.D = 1; a.n_ch = (int)S;
     a.in_step = S; a.in_off = P + L.wc + 1; a.in_limit = L.have;
-    rc = fir_umma_c64_launch(a, ns, s->d_fast_tab, st, S > 1 ? (long long)s->fast_tab_stride : 0);
+    rc = fir_umma_c64_launch(a, ns, (const uint8_t *)s->d_fast_tab.p, st, S > 1 ? (long long)s->fast_tab_stride : 0);
     if (rc) return rc;
     if (S > 1) rc = src_fast_sum(bout, opitch, (int)S, L.out, L.n_out, st);
     return rc;
@@ -1445,7 +1283,7 @@ static int src_process_impl(sdr_src *s, SDR_SRC_DATA *d, bool dev_ptrs) {
 
     SrcLaunch L;
     L.channels = ch; L.type = s->type; L.step = step;
-    L.table = s->d_table; L.half_len = 0; L.rq = 0; L.rho = 0; L.wc = 0;
+    L.table = (const float *)s->d_table.p; L.half_len = 0; L.rq = 0; L.rho = 0; L.wc = 0;
     long long m = 0;
 
     if (s->type >= SDR_SRC_ZERO_ORDER_HOLD) {

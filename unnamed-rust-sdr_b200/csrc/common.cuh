@@ -4,6 +4,9 @@
 #include <stdint.h>
 #include <stddef.h>
 #include <atomic>
+#include <cstddef>
+#include <memory>
+#include <new>
 
 #include "../../include/sdr_b200.h"
 
@@ -58,9 +61,27 @@ inline int current_sm_count() {
     return sms;
 }
 
+// SDR_OK, SDR_ERR_NO_DEVICE when the runtime sees no device, SDR_ERR_INVALID_ARG for an ordinal out of range
+inline int check_device(int dev) {
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) {
+        cudaGetLastError();
+        return SDR_ERR_NO_DEVICE;
+    }
+    if (dev < 0 || dev >= n) return SDR_ERR_INVALID_ARG;
+    return SDR_OK;
+}
+
+// the caller's stream, or one the handle creates and destroys
 struct StreamRef {
     cudaStream_t s = nullptr;
     bool owned = false;
+    StreamRef() = default;
+    StreamRef(const StreamRef &) = delete;
+    StreamRef &operator=(const StreamRef &) = delete;
+    ~StreamRef() {
+        if (owned) cudaStreamDestroy(s);
+    }
     int init(void *user) {
         if (user) {
             s = (cudaStream_t)user;
@@ -71,27 +92,37 @@ struct StreamRef {
         owned = (e == cudaSuccess);
         return cuda_status(e);
     }
-    void release() {
-        if (owned && s) cudaStreamDestroy(s);
-        s = nullptr;
-        owned = false;
-    }
 };
 
-// a grow-only device / pinned-host scratch buffer
+// one device allocation, freed with its owner (on the device current at that point: a DeviceGuard outlives it)
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
+    // grow-only scratch: at least `bytes`, with slack so that slowly growing calls rarely reallocate
     int reserve(size_t bytes) {
         if (bytes <= cap) return SDR_OK;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e != cudaSuccess) return cuda_status(e);
-        cap = want;
+        return alloc(bytes + bytes / 8 + 256);
+    }
+    // exactly `bytes` (tables and state whose size is fixed); the old contents are dropped
+    int alloc(size_t bytes) {
+        release();
+        cudaError_t e = cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) {
+            p = nullptr;
+            return cuda_status(e);
+        }
+        cap = bytes;
         return SDR_OK;
+    }
+    // exactly `bytes`, filled from the host in stream order
+    int upload(const void *host, size_t bytes, cudaStream_t st) {
+        int rc = alloc(bytes);
+        if (rc) return rc;
+        return cuda_status(cudaMemcpyAsync(p, host, bytes, cudaMemcpyHostToDevice, st));
     }
     void release() {
         if (p) cudaFree(p);
@@ -99,6 +130,74 @@ struct DevBuf {
         cap = 0;
     }
 };
+
+// an owned sub-handle, released with the ABI's own destroy function
+template <auto Destroy>
+struct AbiDeleter {
+    template <class T>
+    void operator()(T *h) const { Destroy(h); }
+};
+template <class T, auto Destroy>
+using Owned = std::unique_ptr<T, AbiDeleter<Destroy>>;
+
+// ---- handle lifecycle -------------------------------------------------------------------
+// A handle H derives from a copyable host-state struct (configuration, geometry, host tables, stream position) that
+// holds `int dev`, and adds its device resources: `StreamRef stream` first (destroyed last), then sub-handles, DevBufs.
+// It supplies
+//     int alloc(void *user_stream, const H *src)   stream, tables and buffers for the host state; src: clone source
+//     int copy_device(const H &src)                 the source's carried device state (clone only)
+// and the templates below do the rest.
+
+// *err = code (err may be null); returns the null handle
+inline std::nullptr_t fail(int *err, int code) {
+    if (err) *err = code;
+    return nullptr;
+}
+
+template <class H>
+void destroy_handle(H *h) {
+    if (!h) return;
+    DeviceGuard g(h->dev);
+    delete h;
+}
+
+// after the handle's own argument checks: device check, host state (init(H &) -> error code), then alloc
+template <class H, class Init>
+H *create_handle(int *err, int dev, void *user_stream, Init &&init) {
+    int dummy;
+    if (!err) err = &dummy;
+    if ((*err = check_device(dev)) != SDR_OK) return nullptr;
+    H *h = new (std::nothrow) H;
+    if (!h) return fail(err, SDR_ERR_MALLOC_FAILED);
+    h->dev = dev;
+    DeviceGuard g(dev);
+    *err = init(*h);
+    if (!*err) *err = g.ok ? h->alloc(user_stream, nullptr) : g.status();
+    if (!*err) return h;
+    delete h;
+    return nullptr;
+}
+
+// a handle with the source's host state and a copy of its device state; it allocates on the source's stream when the
+// caller owns that stream, else on a stream of its own
+template <class State, class H>
+H *clone_handle(const H *src, int *err) {
+    int dummy;
+    if (!err) err = &dummy;
+    if (!src) return fail(err, SDR_ERR_NULL_HANDLE);
+    H *h = new (std::nothrow) H;
+    if (!h) return fail(err, SDR_ERR_MALLOC_FAILED);
+    static_cast<State &>(*h) = static_cast<const State &>(*src);
+    DeviceGuard g(h->dev);
+    *err = g.status();
+    // the source's pending work is part of the state it hands over (and alloc may read its device tables)
+    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
+    if (!*err) *err = h->alloc(src->stream.owned ? nullptr : (void *)src->stream.s, src);
+    if (!*err) *err = h->copy_device(*src);
+    if (!*err) return h;
+    delete h;
+    return nullptr;
+}
 
 // ---- device helpers ---------------------------------------------------------------------
 #ifdef __CUDACC__

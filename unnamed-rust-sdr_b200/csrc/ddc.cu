@@ -389,9 +389,8 @@ extern "C" uint64_t sdr_ddc_phase_increment(double freq, double rate) {
     return (uint64_t)std::llround(std::ldexp(nu, 64));  // |nu 2^64| <= 2^63 - 2^10: fits, negative = two's complement
 }
 
-struct sdr_ddc {
+struct DdcHost {
     int dev = 0;
-    StreamRef stream;
     size_t L = 0, C = 0, D = 1, HL = 0, n_sets = 1;
     uint64_t first = 0;
     int fmt = SDR_FMT_U8IQ;
@@ -402,36 +401,30 @@ struct sdr_ddc {
     bool tc = false;
     int PC = 0, KS = 0, Nc8 = 0, Cg = 0, ngroups = 0, Ng = 0, stages = 0;
     size_t smem = 0;
-    DevBuf d_tab, d_chan, d_rot, d_g, d_inc;
     long long total = 0;       // input samples seen
-    DevBuf d_hist[2];          // the last HL inputs before `total`, raw format
-    int cur = 0;
     int last_path = 0;
-    DevBuf d_in, d_out;
 };
 
-static size_t ddc_es(const sdr_ddc *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
+static size_t ddc_es(const DdcHost *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
 
-static void ddc_free(sdr_ddc *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    h->d_tab.release(); h->d_chan.release(); h->d_rot.release(); h->d_g.release(); h->d_inc.release();
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
+struct sdr_ddc : DdcHost {
+    StreamRef stream;
+    DevBuf d_tab, d_chan, d_rot, d_g, d_inc;
+    DevBuf d_hist[2];          // the last HL inputs before `total`, raw format
+    int cur = 0;
+    DevBuf d_in, d_out;
 
-static int ddc_upload(DevBuf &b, const void *src, size_t bytes, cudaStream_t st) {
-    int rc = b.reserve(std::max<size_t>(bytes, 16));
-    if (rc) return rc;
-    return cuda_status(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st));
-}
+    int alloc(void *user_stream, const sdr_ddc *);
+    int copy_device(const sdr_ddc &src) {
+        if (HL == 0) return SDR_OK;
+        return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, HL * ddc_es(this), cudaMemcpyDeviceToDevice));
+    }
+};
 
 // Tensor-path geometry: D | 32, rows 32 samples apart, PC = 32 / D candidates per row and channel (all kept), a channel's
 // 6 PC columns padded to Nc8 (a multiple of 8), Cg channels per group with Ng = Cg Nc8 rounded up to 16 <= 256 columns
 // (two accumulator sets in TMEM) and the group's table plus >= 2 stages in shared memory.  False: the general kernel.
-static bool ddc_tc_geometry(sdr_ddc *h) {
+static bool ddc_tc_geometry(DdcHost *h) {
     if (h->fmt != SDR_FMT_U8IQ || (h->flags & SDR_DDC_GENERAL_KERNEL) || h->D > 32 || 32 % h->D != 0 ||
         h->L > (size_t)DDC_MAX_TC_K)
         return false;
@@ -457,44 +450,43 @@ static bool ddc_tc_geometry(sdr_ddc *h) {
 }
 
 // complex taps g_k[j] = h_k[j] e^{+2 pi i (j Delta_k mod 2^64) / 2^64}, rounded to f32 from f64
-static void ddc_rotated_taps(const sdr_ddc *h, size_t k, std::vector<float> &g) {
+static void ddc_rotated_taps(const DdcHost *h, size_t k, std::vector<float> &g) {
     nco_rotated_taps(h->taps.data() + (h->n_sets == 1 ? 0 : k * h->L), h->L, h->inc[k], g);
 }
 
 // tables, taps and history buffers of a handle whose configuration fields are set
-static int ddc_alloc(sdr_ddc *h, void *user_stream) {
-    int rc = h->stream.init(user_stream);
+int sdr_ddc::alloc(void *user_stream, const sdr_ddc *) {
+    int rc = stream.init(user_stream);
     if (rc) return rc;
-    cudaStream_t st = h->stream.s;
-    const size_t C = h->C, L = h->L;
-    h->tc = ddc_tc_geometry(h);
+    cudaStream_t st = stream.s;
+    tc = ddc_tc_geometry(this);
     std::vector<float> g;
-    if (h->tc) {
+    if (tc) {
         // group tables [delta][group][kk][Ng x 32 B canonical K-major block]; channel cl of a group owns columns
         // cl Nc8 + dg 2PC + 2u + part.  D = 16, 32 take the PC = 4 tables (whose 6 PC column count is a whole number of
         // core matrices) and keep every (8 / PC)-th candidate; their first KS k-steps hold all the kept candidates' taps.
-        const int PC = h->PC, PCb = std::max(PC, 4), sig = PCb / PC, KS = h->KS, Ng = h->Ng;
+        const int PCb = std::max(PC, 4), sig = PCb / PC;
         const size_t blk = (size_t)Ng * 32, grp_bytes = (size_t)KS * blk;
-        std::vector<uint8_t> tab((size_t)8 * h->ngroups * grp_bytes, 0), one;
+        std::vector<uint8_t> tab((size_t)8 * ngroups * grp_bytes, 0), one;
         std::vector<DdcChan> chan(C);
-        const int TR = DDC_TILE / (int)h->D;
+        const int TR = DDC_TILE / (int)D;
         std::vector<float> rot(2 * C * TR);
         for (size_t k = 0; k < C; ++k) {
-            ddc_rotated_taps(h, k, g);
+            ddc_rotated_taps(this, k, g);
             int magic[2][3];
             float sc[3];
-            if (!fir_umma_build_tables(g.data(), (int)L, true, 32, PCb, 0, (int)h->D, one, magic, sc)) return SDR_ERR_INVALID_ARG;
+            if (!fir_umma_build_tables(g.data(), (int)L, true, 32, PCb, 0, (int)D, one, magic, sc)) return SDR_ERR_INVALID_ARG;
             const int KSb = fir_umma_ksteps((int)L, 32, PCb), Nb = 6 * PCb;
-            const size_t grp = k / h->Cg, cl = k % h->Cg;
+            const size_t grp = k / Cg, cl = k % Cg;
             for (int delta = 0; delta < 8; ++delta)
                 for (int kk = 0; kk < KS; ++kk) {
                     const uint8_t *sb = one.data() + ((size_t)delta * KSb + kk) * Nb * 32;
-                    uint8_t *db = tab.data() + ((size_t)delta * h->ngroups + grp) * grp_bytes + (size_t)kk * blk;
+                    uint8_t *db = tab.data() + ((size_t)delta * ngroups + grp) * grp_bytes + (size_t)kk * blk;
                     for (int dg = 0; dg < 3; ++dg)
                         for (int u = 0; u < PC; ++u)
                             for (int part = 0; part < 2; ++part) {
                                 const int ns = dg * 2 * PCb + 2 * sig * u + part;
-                                const int nd = (int)cl * h->Nc8 + dg * 2 * PC + 2 * u + part;
+                                const int nd = (int)cl * Nc8 + dg * 2 * PC + 2 * u + part;
                                 for (int kb = 0; kb < 32; ++kb) {
                                     const int o = (kb / 16) * 128 + kb % 16;
                                     db[(nd / 8) * 256 + (nd % 8) * 16 + o] = sb[(ns / 8) * 256 + (ns % 8) * 16 + o];
@@ -503,69 +495,53 @@ static int ddc_alloc(sdr_ddc *h, void *user_stream) {
                 }
             chan[k] = DdcChan{{magic[0][0], magic[1][0]}, {magic[0][2], magic[1][2]}, sc[0], sc[2]};
             for (int j = 0; j < TR; ++j) {
-                const double t = NCO_2PI * nco_turns(((uint64_t)h->D * j + h->D - 1) * h->inc[k]);
+                const double t = NCO_2PI * nco_turns(((uint64_t)D * j + D - 1) * inc[k]);
                 rot[2 * (k * TR + j)] = (float)std::cos(t);
                 rot[2 * (k * TR + j) + 1] = (float)-std::sin(t);
             }
         }
-        if ((rc = ddc_upload(h->d_tab, tab.data(), tab.size(), st))) return rc;
-        if ((rc = ddc_upload(h->d_chan, chan.data(), chan.size() * sizeof(DdcChan), st))) return rc;
-        if ((rc = ddc_upload(h->d_rot, rot.data(), rot.size() * sizeof(float), st))) return rc;
+        if ((rc = d_tab.upload(tab.data(), tab.size(), st))) return rc;
+        if ((rc = d_chan.upload(chan.data(), chan.size() * sizeof(DdcChan), st))) return rc;
+        if ((rc = d_rot.upload(rot.data(), rot.size() * sizeof(float), st))) return rc;
     } else {
         std::vector<float> all(2 * C * L);
         for (size_t k = 0; k < C; ++k) {
-            ddc_rotated_taps(h, k, g);
+            ddc_rotated_taps(this, k, g);
             std::copy(g.begin(), g.end(), all.begin() + 2 * k * L);
         }
-        if ((rc = ddc_upload(h->d_g, all.data(), all.size() * sizeof(float), st))) return rc;
+        if ((rc = d_g.upload(all.data(), all.size() * sizeof(float), st))) return rc;
     }
-    if ((rc = ddc_upload(h->d_inc, h->inc.data(), C * sizeof(uint64_t), st))) return rc;
+    if ((rc = d_inc.upload(inc.data(), C * sizeof(uint64_t), st))) return rc;
     for (int i = 0; i < 2; ++i)
-        if ((rc = h->d_hist[i].reserve(std::max<size_t>(h->HL, 2) * ddc_es(h)))) return rc;
+        if ((rc = d_hist[i].reserve(std::max<size_t>(HL, 2) * ddc_es(this)))) return rc;
     return cuda_status(cudaStreamSynchronize(st));
 }
 
 extern "C" sdr_ddc_t *sdr_ddc_create(const sdr_ddc_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->taps || !cfg->phase_inc || cfg->n_taps == 0 || cfg->n_taps > ((size_t)1 << 20) ||
         cfg->n_channels == 0 || cfg->n_channels > DDC_MAX_CH ||
         (cfg->n_tap_sets != 1 && cfg->n_tap_sets != cfg->n_channels) || cfg->decimation == 0 ||
         cfg->decimation > ((size_t)1 << 40) || (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) ||
-        (cfg->flags & ~SDR_DDC_GENERAL_KERNEL)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
+        (cfg->flags & ~SDR_DDC_GENERAL_KERNEL))
+        return fail(err, SDR_ERR_INVALID_ARG);
     for (size_t i = 0; i < cfg->n_taps * cfg->n_tap_sets; ++i)
-        if (!std::isfinite(cfg->taps[i])) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    sdr_ddc *h = new (std::nothrow) sdr_ddc;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = cfg->device;
-    h->L = cfg->n_taps;
-    h->C = cfg->n_channels;
-    h->D = cfg->decimation;
-    h->HL = h->L - 1;
-    h->n_sets = cfg->n_tap_sets;
-    h->first = cfg->first_sample;
-    h->fmt = cfg->input_format;
-    h->flags = cfg->flags;
-    h->taps.assign(cfg->taps, cfg->taps + h->L * h->n_sets);
-    h->inc.assign(cfg->phase_inc, cfg->phase_inc + h->C);
-    DeviceGuard g(h->dev);
-    *err = g.ok ? ddc_alloc(h, cfg->stream) : g.status();
-    if (*err) { ddc_free(h); return nullptr; }
-    return h;
+        if (!std::isfinite(cfg->taps[i])) return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_ddc>(err, cfg->device, cfg->stream, [&](sdr_ddc &h) {
+        h.L = cfg->n_taps;
+        h.C = cfg->n_channels;
+        h.D = cfg->decimation;
+        h.HL = h.L - 1;
+        h.n_sets = cfg->n_tap_sets;
+        h.first = cfg->first_sample;
+        h.fmt = cfg->input_format;
+        h.flags = cfg->flags;
+        h.taps.assign(cfg->taps, cfg->taps + h.L * h.n_sets);
+        h.inc.assign(cfg->phase_inc, cfg->phase_inc + h.C);
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_ddc_destroy(sdr_ddc_t *h) { ddc_free(h); }
+extern "C" void sdr_ddc_destroy(sdr_ddc_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_ddc_reset(sdr_ddc_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -575,24 +551,7 @@ extern "C" int sdr_ddc_reset(sdr_ddc_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_ddc_t *sdr_ddc_clone(const sdr_ddc_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_ddc *h = new (std::nothrow) sdr_ddc;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->L = src->L; h->C = src->C; h->D = src->D; h->HL = src->HL; h->n_sets = src->n_sets;
-    h->first = src->first; h->fmt = src->fmt; h->flags = src->flags; h->taps = src->taps; h->inc = src->inc;
-    h->total = src->total; h->last_path = src->last_path;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? ddc_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s) : g.status();
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err && h->HL > 0)
-        *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, h->HL * ddc_es(h), cudaMemcpyDeviceToDevice));
-    if (*err) { ddc_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_ddc_t *sdr_ddc_clone(const sdr_ddc_t *src, int *err) { return clone_handle<DdcHost>(src, err); }
 
 extern "C" size_t sdr_ddc_output_count(const sdr_ddc_t *h, size_t n_in) {
     if (!h) return 0;

@@ -160,94 +160,69 @@ void duc_geometry(size_t I, int *W, long long *T) {
 
 }  // namespace
 
-struct sdr_duc {
+struct DucHost {
     int dev = 0;
-    StreamRef stream;
     size_t L = 0, C = 0, I = 1, H = 0, n_sets = 1;
     uint64_t first = 0;
     int W = 1;
     long long T = 1;
     std::vector<float> taps;    // n_sets x L, as given
     std::vector<uint64_t> inc;
-    DevBuf d_taps, d_inc, d_tab;
     long long total = 0;        // frames seen
+};
+
+struct sdr_duc : DucHost {
+    StreamRef stream;
+    DevBuf d_taps, d_inc, d_tab;
     DevBuf d_hist[2];           // C rows of the H frames before `total`
     int cur = 0;
     DevBuf d_in, d_out;
+
+    // taps, increments, rotation tables (f64 on the host, rounded to f32 once) and history of a handle whose fields are set
+    int alloc(void *user_stream, const sdr_duc *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        cudaStream_t st = stream.s;
+        duc_geometry(I, &W, &T);
+        std::vector<float2> tab((size_t)C * T);
+        for (size_t k = 0; k < C; ++k)
+            for (long long r = 0; r < T; ++r) {
+                const double t = NCO_2PI * nco_turns((uint64_t)r * inc[k]);
+                tab[k * T + r] = make_float2((float)std::cos(t), (float)std::sin(t));
+            }
+        if ((rc = d_taps.upload(taps.data(), taps.size() * sizeof(float), st))) return rc;
+        if ((rc = d_inc.upload(inc.data(), C * sizeof(uint64_t), st))) return rc;
+        if ((rc = d_tab.upload(tab.data(), tab.size() * sizeof(float2), st))) return rc;
+        for (int i = 0; i < 2; ++i)
+            if ((rc = d_hist[i].reserve(std::max<size_t>(H, 1) * C * 8))) return rc;
+        return cuda_status(cudaStreamSynchronize(st));
+    }
+    int copy_device(const sdr_duc &src) {
+        if (H == 0) return SDR_OK;
+        return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, H * C * 8, cudaMemcpyDeviceToDevice));
+    }
 };
 
-static void duc_free(sdr_duc *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    h->d_taps.release(); h->d_inc.release(); h->d_tab.release();
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
-
-static int duc_upload(DevBuf &b, const void *src, size_t bytes, cudaStream_t st) {
-    int rc = b.reserve(std::max<size_t>(bytes, 16));
-    if (rc) return rc;
-    return cuda_status(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st));
-}
-
-// taps, increments, rotation tables (f64 on the host, rounded to f32 once) and history of a handle whose fields are set
-static int duc_alloc(sdr_duc *h, void *user_stream) {
-    int rc = h->stream.init(user_stream);
-    if (rc) return rc;
-    cudaStream_t st = h->stream.s;
-    duc_geometry(h->I, &h->W, &h->T);
-    std::vector<float2> tab((size_t)h->C * h->T);
-    for (size_t k = 0; k < h->C; ++k)
-        for (long long r = 0; r < h->T; ++r) {
-            const double t = NCO_2PI * nco_turns((uint64_t)r * h->inc[k]);
-            tab[k * h->T + r] = make_float2((float)std::cos(t), (float)std::sin(t));
-        }
-    if ((rc = duc_upload(h->d_taps, h->taps.data(), h->taps.size() * sizeof(float), st))) return rc;
-    if ((rc = duc_upload(h->d_inc, h->inc.data(), h->C * sizeof(uint64_t), st))) return rc;
-    if ((rc = duc_upload(h->d_tab, tab.data(), tab.size() * sizeof(float2), st))) return rc;
-    for (int i = 0; i < 2; ++i)
-        if ((rc = h->d_hist[i].reserve(std::max<size_t>(h->H, 1) * h->C * 8))) return rc;
-    return cuda_status(cudaStreamSynchronize(st));
-}
-
 extern "C" sdr_duc_t *sdr_duc_create(const sdr_duc_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->taps || !cfg->phase_inc || cfg->n_taps == 0 || cfg->n_taps > DUC_MAX_TAPS ||
         cfg->n_channels == 0 || cfg->n_channels > DUC_MAX_CH ||
         (cfg->n_tap_sets != 1 && cfg->n_tap_sets != cfg->n_channels) || cfg->interpolation == 0 ||
-        cfg->interpolation > ((size_t)1 << 40) || cfg->flags != 0) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    sdr_duc *h = new (std::nothrow) sdr_duc;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = cfg->device;
-    h->L = cfg->n_taps;
-    h->C = cfg->n_channels;
-    h->I = cfg->interpolation;
-    h->H = (h->L - 1 + h->I - 1) / h->I;
-    h->n_sets = cfg->n_tap_sets;
-    h->first = cfg->first_sample;
-    h->taps.assign(cfg->taps, cfg->taps + h->L * h->n_sets);
-    h->inc.assign(cfg->phase_inc, cfg->phase_inc + h->C);
-    DeviceGuard g(h->dev);
-    *err = g.ok ? duc_alloc(h, cfg->stream) : g.status();
-    if (*err) { duc_free(h); return nullptr; }
-    return h;
+        cfg->interpolation > ((size_t)1 << 40) || cfg->flags != 0)
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_duc>(err, cfg->device, cfg->stream, [&](sdr_duc &h) {
+        h.L = cfg->n_taps;
+        h.C = cfg->n_channels;
+        h.I = cfg->interpolation;
+        h.H = (h.L - 1 + h.I - 1) / h.I;
+        h.n_sets = cfg->n_tap_sets;
+        h.first = cfg->first_sample;
+        h.taps.assign(cfg->taps, cfg->taps + h.L * h.n_sets);
+        h.inc.assign(cfg->phase_inc, cfg->phase_inc + h.C);
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_duc_destroy(sdr_duc_t *h) { duc_free(h); }
+extern "C" void sdr_duc_destroy(sdr_duc_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_duc_reset(sdr_duc_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -257,23 +232,7 @@ extern "C" int sdr_duc_reset(sdr_duc_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_duc_t *sdr_duc_clone(const sdr_duc_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_duc *h = new (std::nothrow) sdr_duc;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->L = src->L; h->C = src->C; h->I = src->I; h->H = src->H; h->n_sets = src->n_sets;
-    h->first = src->first; h->taps = src->taps; h->inc = src->inc; h->total = src->total;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? duc_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s) : g.status();
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err && h->H > 0)
-        *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, h->H * h->C * 8, cudaMemcpyDeviceToDevice));
-    if (*err) { duc_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_duc_t *sdr_duc_clone(const sdr_duc_t *src, int *err) { return clone_handle<DucHost>(src, err); }
 
 extern "C" size_t sdr_duc_output_count(const sdr_duc_t *h, size_t n_frames) {
     if (!h) return 0;

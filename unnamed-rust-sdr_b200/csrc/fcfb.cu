@@ -178,9 +178,8 @@ extern "C" int sdr_fcfb_geometry(size_t n_taps, const size_t *decimation, size_t
     return SDR_ERR_UNSUPPORTED;
 }
 
-struct sdr_fcfb {
+struct FcfbHost {
     int dev = 0;
-    StreamRef stream;
     size_t L = 0, C = 0, n_sets = 1;
     uint64_t first = 0;
     int fmt = SDR_FMT_U8IQ;
@@ -192,32 +191,29 @@ struct sdr_fcfb {
     std::vector<FcfbChan> chan;
     std::vector<std::pair<long long, long long>> groups;  // (M, first channel of the group in `order`)
     std::vector<int> order;          // channels sorted by group
-    sdr_fft_t *fwd = nullptr;
-    std::vector<sdr_fft_t *> inv;    // one per group
-    DevBuf d_G, d_tab, d_chan, d_mlo;
     long long total = 0;             // input samples seen
     long long hist_lo = 0;           // d_hist[cur] holds handle samples hist_lo .. total - 1
+};
+
+using FftPlan = Owned<sdr_fft_t, sdr_fft_destroy>;
+
+struct sdr_fcfb : FcfbHost {
+    StreamRef stream;
+    FftPlan fwd;
+    std::vector<FftPlan> inv;        // one per group
+    DevBuf d_G, d_tab, d_chan, d_mlo;
     DevBuf d_hist[2];
     int cur = 0;
     DevBuf d_x, d_X, d_f, d_y, d_in, d_out;
+
+    int alloc(void *user_stream, const sdr_fcfb *src);
+    int copy_device(const sdr_fcfb &src);
 };
 
-static size_t fcfb_es(const sdr_fcfb *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
-
-static void fcfb_free(sdr_fcfb *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    if (h->fwd) sdr_fft_destroy(h->fwd);
-    for (sdr_fft_t *p : h->inv) sdr_fft_destroy(p);
-    h->d_G.release(); h->d_tab.release(); h->d_chan.release(); h->d_mlo.release();
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_x.release(); h->d_X.release(); h->d_f.release(); h->d_y.release(); h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
+static size_t fcfb_es(const FcfbHost *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
 
 // host-side geometry of a handle whose configuration fields are set: N, P, per-channel fold constants, groups
-static int fcfb_geometry_fields(sdr_fcfb *h) {
+static int fcfb_geometry_fields(FcfbHost *h) {
     size_t n = 0, p = 0;
     int rc = sdr_fcfb_geometry(h->L, h->D.data(), h->C, &n, &p);
     if (rc) return rc;
@@ -256,7 +252,7 @@ static int fcfb_geometry_fields(sdr_fcfb *h) {
 }
 
 // G'_k (C rows of N) and the derotation tables (C rows of FCFB_RUN), f64 on the host, rounded to f32 once
-static void fcfb_tables(const sdr_fcfb *h, std::vector<float2> &G, std::vector<float2> &tab) {
+static void fcfb_tables(const FcfbHost *h, std::vector<float2> &G, std::vector<float2> &tab) {
     const long long N = h->N, L = (long long)h->L;
     G.assign((size_t)h->C * N, make_float2(0.f, 0.f));
     tab.assign((size_t)h->C * FCFB_RUN, make_float2(0.f, 0.f));
@@ -271,13 +267,7 @@ static void fcfb_tables(const sdr_fcfb *h, std::vector<float2> &G, std::vector<f
     }
 }
 
-static int fcfb_upload(DevBuf &b, const void *src, size_t bytes, cudaStream_t st) {
-    int rc = b.reserve(std::max<size_t>(bytes, 16));
-    if (rc) return rc;
-    return cuda_status(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st));
-}
-
-static int fcfb_plan(const sdr_fcfb *h, long long n, sdr_fft_t **out) {
+static int fcfb_plan(const sdr_fcfb *h, long long n, FftPlan &out) {
     sdr_fft_config_t fc;
     fc.n = (size_t)n;
     fc.input_format = SDR_FMT_C64;
@@ -285,84 +275,73 @@ static int fcfb_plan(const sdr_fcfb *h, long long n, sdr_fft_t **out) {
     fc.device = h->dev;
     fc.stream = (void *)h->stream.s;
     int rc = SDR_OK;
-    *out = sdr_fft_create(&fc, &rc);
-    return *out ? SDR_OK : rc;
+    out.reset(sdr_fft_create(&fc, &rc));
+    return out ? SDR_OK : rc;
 }
 
 // plans, tables and history buffers of a handle whose geometry fields are set; src != null copies src's tables
-static int fcfb_alloc(sdr_fcfb *h, void *user_stream, const sdr_fcfb *src) {
-    int rc = h->stream.init(user_stream);
+int sdr_fcfb::alloc(void *user_stream, const sdr_fcfb *src) {
+    int rc = stream.init(user_stream);
     if (rc) return rc;
-    cudaStream_t st = h->stream.s;
-    if ((rc = fcfb_plan(h, h->N, &h->fwd))) return rc;
-    for (const auto &grp : h->groups) {
-        sdr_fft_t *p = nullptr;
-        if ((rc = fcfb_plan(h, grp.first, &p))) return rc;
-        h->inv.push_back(p);
-    }
-    const size_t gbytes = h->C * (size_t)h->N * sizeof(float2), tbytes = h->C * FCFB_RUN * sizeof(float2);
+    cudaStream_t st = stream.s;
+    if ((rc = fcfb_plan(this, N, fwd))) return rc;
+    inv.resize(groups.size());
+    for (size_t q = 0; q < groups.size(); ++q)
+        if ((rc = fcfb_plan(this, groups[q].first, inv[q]))) return rc;
+    const size_t gbytes = C * (size_t)N * sizeof(float2), tbytes = C * FCFB_RUN * sizeof(float2);
     if (src) {
-        if ((rc = h->d_G.reserve(gbytes)) || (rc = h->d_tab.reserve(tbytes))) return rc;
-        SDR_CUDA_TRY(cudaMemcpyAsync(h->d_G.p, src->d_G.p, gbytes, cudaMemcpyDeviceToDevice, st));
-        SDR_CUDA_TRY(cudaMemcpyAsync(h->d_tab.p, src->d_tab.p, tbytes, cudaMemcpyDeviceToDevice, st));
+        if ((rc = d_G.alloc(gbytes)) || (rc = d_tab.alloc(tbytes))) return rc;
+        SDR_CUDA_TRY(cudaMemcpyAsync(d_G.p, src->d_G.p, gbytes, cudaMemcpyDeviceToDevice, st));
+        SDR_CUDA_TRY(cudaMemcpyAsync(d_tab.p, src->d_tab.p, tbytes, cudaMemcpyDeviceToDevice, st));
     } else {
         std::vector<float2> G, tab;
-        fcfb_tables(h, G, tab);
-        if ((rc = fcfb_upload(h->d_G, G.data(), gbytes, st))) return rc;
-        if ((rc = fcfb_upload(h->d_tab, tab.data(), tbytes, st))) return rc;
+        fcfb_tables(this, G, tab);
+        if ((rc = d_G.upload(G.data(), gbytes, st)) || (rc = d_tab.upload(tab.data(), tbytes, st))) return rc;
         SDR_CUDA_TRY(cudaStreamSynchronize(st));  // the host vectors go out of scope
     }
-    if ((rc = fcfb_upload(h->d_chan, h->chan.data(), h->C * sizeof(FcfbChan), st))) return rc;
-    if ((rc = h->d_mlo.reserve(h->C * sizeof(long long)))) return rc;
+    if ((rc = d_chan.upload(chan.data(), C * sizeof(FcfbChan), st))) return rc;
+    if ((rc = d_mlo.reserve(C * sizeof(long long)))) return rc;
     for (int i = 0; i < 2; ++i)
-        if ((rc = h->d_hist[i].reserve(16))) return rc;
+        if ((rc = d_hist[i].reserve(16))) return rc;
     return cuda_status(cudaStreamSynchronize(st));
 }
 
+// the history tail
+int sdr_fcfb::copy_device(const sdr_fcfb &src) {
+    const size_t tail = (size_t)(total - hist_lo) * fcfb_es(this);
+    if (tail == 0) return SDR_OK;
+    int rc = d_hist[0].reserve(tail);
+    if (rc) return rc;
+    return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, tail, cudaMemcpyDeviceToDevice));
+}
+
 extern "C" sdr_fcfb_t *sdr_fcfb_create(const sdr_fcfb_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->taps || !cfg->phase_inc || !cfg->decimation || cfg->n_taps == 0 || cfg->n_taps > FCFB_MAX_TAPS ||
         cfg->n_channels == 0 || cfg->n_channels > FCFB_MAX_CH ||
         (cfg->n_tap_sets != 1 && cfg->n_tap_sets != cfg->n_channels) ||
-        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
+        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64))
+        return fail(err, SDR_ERR_INVALID_ARG);
     for (size_t k = 0; k < cfg->n_channels; ++k)
-        if (cfg->decimation[k] == 0) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
+        if (cfg->decimation[k] == 0) return fail(err, SDR_ERR_INVALID_ARG);
     for (size_t i = 0; i < cfg->n_taps * cfg->n_tap_sets; ++i)
-        if (!std::isfinite(cfg->taps[i])) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
+        if (!std::isfinite(cfg->taps[i])) return fail(err, SDR_ERR_INVALID_ARG);
     size_t n_fft = 0, hop = 0;
-    if ((*err = sdr_fcfb_geometry(cfg->n_taps, cfg->decimation, cfg->n_channels, &n_fft, &hop))) return nullptr;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    sdr_fcfb *h = new (std::nothrow) sdr_fcfb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = cfg->device;
-    h->L = cfg->n_taps;
-    h->C = cfg->n_channels;
-    h->n_sets = cfg->n_tap_sets;
-    h->first = cfg->first_sample;
-    h->fmt = cfg->input_format;
-    h->taps.assign(cfg->taps, cfg->taps + h->L * h->n_sets);
-    h->inc.assign(cfg->phase_inc, cfg->phase_inc + h->C);
-    h->D.assign(cfg->decimation, cfg->decimation + h->C);
-    *err = fcfb_geometry_fields(h);
-    if (*err) { delete h; return nullptr; }
-    DeviceGuard g(h->dev);
-    *err = g.ok ? fcfb_alloc(h, cfg->stream, nullptr) : g.status();
-    if (*err) { fcfb_free(h); return nullptr; }
-    return h;
+    const int rc = sdr_fcfb_geometry(cfg->n_taps, cfg->decimation, cfg->n_channels, &n_fft, &hop);
+    if (rc) return fail(err, rc);
+    return create_handle<sdr_fcfb>(err, cfg->device, cfg->stream, [&](sdr_fcfb &h) {
+        h.L = cfg->n_taps;
+        h.C = cfg->n_channels;
+        h.n_sets = cfg->n_tap_sets;
+        h.first = cfg->first_sample;
+        h.fmt = cfg->input_format;
+        h.taps.assign(cfg->taps, cfg->taps + h.L * h.n_sets);
+        h.inc.assign(cfg->phase_inc, cfg->phase_inc + h.C);
+        h.D.assign(cfg->decimation, cfg->decimation + h.C);
+        return fcfb_geometry_fields(&h);
+    });
 }
 
-extern "C" void sdr_fcfb_destroy(sdr_fcfb_t *h) { fcfb_free(h); }
+extern "C" void sdr_fcfb_destroy(sdr_fcfb_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_fcfb_reset(sdr_fcfb_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -372,29 +351,7 @@ extern "C" int sdr_fcfb_reset(sdr_fcfb_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_fcfb_t *sdr_fcfb_clone(const sdr_fcfb_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_fcfb *h = new (std::nothrow) sdr_fcfb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->L = src->L; h->C = src->C; h->n_sets = src->n_sets; h->first = src->first; h->fmt = src->fmt;
-    h->taps = src->taps; h->inc = src->inc; h->D = src->D;
-    h->N = src->N; h->P = src->P; h->Dl = src->Dl; h->off0 = src->off0; h->rows = src->rows;
-    h->chan = src->chan; h->groups = src->groups; h->order = src->order;
-    h->total = src->total; h->hist_lo = src->hist_lo;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? cuda_status(cudaStreamSynchronize(src->stream.s)) : g.status();
-    if (!*err) *err = fcfb_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s, src);
-    const size_t tail = (size_t)(h->total - h->hist_lo) * fcfb_es(h);
-    if (!*err && tail > 0) {
-        *err = h->d_hist[0].reserve(tail);
-        if (!*err) *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, tail, cudaMemcpyDeviceToDevice));
-    }
-    if (*err) { fcfb_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_fcfb_t *sdr_fcfb_clone(const sdr_fcfb_t *src, int *err) { return clone_handle<FcfbHost>(src, err); }
 
 // blocks completed by the first T inputs, and channel k's outputs among them
 static long long fcfb_blocks(const sdr_fcfb *h, long long T) { return (T + h->off0) / h->P; }
@@ -439,7 +396,7 @@ static int fcfb_blocks_run(sdr_fcfb *h, const FcfbSrc &src, long long jA, long l
             fcfb_gather_kernel<false><<<gg, 256, 0, st>>>(src, N, h->P, h->off0, j0, nb, (float2 *)h->d_x.p);
         count_launch();
         if ((rc = launch_status())) return rc;
-        if ((rc = sdr_fft_exec_dev(h->fwd, h->d_x.p, (size_t)nb, (float *)h->d_X.p))) return rc;
+        if ((rc = sdr_fft_exec_dev(h->fwd.get(), h->d_x.p, (size_t)nb, (float *)h->d_X.p))) return rc;
         dim3 gf((unsigned)((max_m + 255) / 256), (unsigned)h->C, (unsigned)((nb + FCFB_FOLD_BLOCKS - 1) / FCFB_FOLD_BLOCKS));
         fcfb_fold_kernel<<<gf, 256, 0, st>>>((const float2 *)h->d_X.p, (const float2 *)h->d_G.p,
                                              (const FcfbChan *)h->d_chan.p, N, nb, (float2 *)h->d_f.p);
@@ -449,7 +406,7 @@ static int fcfb_blocks_run(sdr_fcfb *h, const FcfbSrc &src, long long jA, long l
             const long long first = h->groups[q].second;
             const long long last = q + 1 < h->groups.size() ? h->groups[q + 1].second : (long long)h->C;
             const size_t off = (size_t)(nb * h->chan[h->order[first]].base);
-            rc = sdr_fft_exec_dev(h->inv[q], (const float2 *)h->d_f.p + off, (size_t)((last - first) * nb),
+            rc = sdr_fft_exec_dev(h->inv[q].get(), (const float2 *)h->d_f.p + off, (size_t)((last - first) * nb),
                                   (float *)((float2 *)h->d_y.p + off));
             if (rc) return rc;
         }

@@ -161,9 +161,8 @@ __global__ void __launch_bounds__(256) fcsb_carry_kernel(FcsbSrc src, const Fcsb
 
 }  // namespace
 
-struct sdr_fcsb {
+struct FcsbHost {
     int dev = 0;
-    StreamRef stream;
     size_t L = 0, C = 0, n_sets = 1;
     uint64_t first = 0;
     std::vector<float> taps;         // n_sets x L, as given
@@ -174,31 +173,28 @@ struct sdr_fcsb {
     std::vector<FcsbChan> chan;
     std::vector<std::pair<long long, long long>> groups;  // (M, first channel of the group in `order`)
     std::vector<int> order;          // channels sorted by group
-    sdr_fft_t *big = nullptr;        // the N-point plan
-    std::vector<sdr_fft_t *> small;  // one per group
-    DevBuf d_G, d_tab, d_chan, d_mb;
     long long total = 0;             // output positions seen (a multiple of Il)
     long long hist_lo = 0;           // d_hist[cur] row k holds channel k's frames from hist_lo / I_k to total / I_k
     long long hist_stride = 0;       // c64 per row of d_hist[cur]
+};
+
+using FftPlan = Owned<sdr_fft_t, sdr_fft_destroy>;
+
+struct sdr_fcsb : FcsbHost {
+    StreamRef stream;
+    FftPlan big;                     // the N-point plan
+    std::vector<FftPlan> small;      // one per group
+    DevBuf d_G, d_tab, d_chan, d_mb;
     DevBuf d_hist[2];
     int cur = 0;
     DevBuf d_v, d_V, d_S, d_X, d_in, d_out;
+
+    int alloc(void *user_stream, const sdr_fcsb *src);
+    int copy_device(const sdr_fcsb &src);
 };
 
-static void fcsb_free(sdr_fcsb *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    if (h->big) sdr_fft_destroy(h->big);
-    for (sdr_fft_t *p : h->small) sdr_fft_destroy(p);
-    h->d_G.release(); h->d_tab.release(); h->d_chan.release(); h->d_mb.release();
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_v.release(); h->d_V.release(); h->d_S.release(); h->d_X.release(); h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
-
 // host-side geometry of a handle whose configuration fields are set: N, P, per-channel constants, groups
-static int fcsb_geometry_fields(sdr_fcsb *h) {
+static int fcsb_geometry_fields(FcsbHost *h) {
     size_t n = 0, p = 0;
     int rc = sdr_fcfb_geometry(h->L, h->I.data(), h->C, &n, &p);
     if (rc) return rc;
@@ -242,7 +238,7 @@ static int fcsb_geometry_fields(sdr_fcsb *h) {
 
 // G'_k (C rows of N, the conjugate rho factor of K9's) and the rotation tables tab[k][r] = e^{+2 pi i r I_k Delta_k}
 // (C rows of FCSB_RUN), f64 on the host, rounded to f32 once
-static void fcsb_tables(const sdr_fcsb *h, std::vector<float2> &G, std::vector<float2> &tab) {
+static void fcsb_tables(const FcsbHost *h, std::vector<float2> &G, std::vector<float2> &tab) {
     const long long N = h->N, L = (long long)h->L;
     G.assign((size_t)h->C * N, make_float2(0.f, 0.f));
     tab.assign((size_t)h->C * FCSB_RUN, make_float2(0.f, 0.f));
@@ -257,13 +253,7 @@ static void fcsb_tables(const sdr_fcsb *h, std::vector<float2> &G, std::vector<f
     }
 }
 
-static int fcsb_upload(DevBuf &b, const void *src, size_t bytes, cudaStream_t st) {
-    int rc = b.reserve(std::max<size_t>(bytes, 16));
-    if (rc) return rc;
-    return cuda_status(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st));
-}
-
-static int fcsb_plan(const sdr_fcsb *h, long long n, sdr_fft_t **out) {
+static int fcsb_plan(const sdr_fcsb *h, long long n, FftPlan &out) {
     sdr_fft_config_t fc;
     fc.n = (size_t)n;
     fc.input_format = SDR_FMT_C64;
@@ -271,84 +261,73 @@ static int fcsb_plan(const sdr_fcsb *h, long long n, sdr_fft_t **out) {
     fc.device = h->dev;
     fc.stream = (void *)h->stream.s;
     int rc = SDR_OK;
-    *out = sdr_fft_create(&fc, &rc);
-    return *out ? SDR_OK : rc;
+    out.reset(sdr_fft_create(&fc, &rc));
+    return out ? SDR_OK : rc;
 }
 
 // plans, tables and history buffers of a handle whose geometry fields are set; src != null copies src's tables
-static int fcsb_alloc(sdr_fcsb *h, void *user_stream, const sdr_fcsb *src) {
-    int rc = h->stream.init(user_stream);
+inline int sdr_fcsb::alloc(void *user_stream, const sdr_fcsb *src) {
+    int rc = stream.init(user_stream);
     if (rc) return rc;
-    cudaStream_t st = h->stream.s;
-    if ((rc = fcsb_plan(h, h->N, &h->big))) return rc;
-    for (const auto &grp : h->groups) {
-        sdr_fft_t *p = nullptr;
-        if ((rc = fcsb_plan(h, grp.first, &p))) return rc;
-        h->small.push_back(p);
-    }
-    const size_t gbytes = h->C * (size_t)h->N * sizeof(float2), tbytes = h->C * FCSB_RUN * sizeof(float2);
+    cudaStream_t st = stream.s;
+    if ((rc = fcsb_plan(this, N, big))) return rc;
+    small.resize(groups.size());
+    for (size_t q = 0; q < groups.size(); ++q)
+        if ((rc = fcsb_plan(this, groups[q].first, small[q]))) return rc;
+    const size_t gbytes = C * (size_t)N * sizeof(float2), tbytes = C * FCSB_RUN * sizeof(float2);
     if (src) {
-        if ((rc = h->d_G.reserve(gbytes)) || (rc = h->d_tab.reserve(tbytes))) return rc;
-        SDR_CUDA_TRY(cudaMemcpyAsync(h->d_G.p, src->d_G.p, gbytes, cudaMemcpyDeviceToDevice, st));
-        SDR_CUDA_TRY(cudaMemcpyAsync(h->d_tab.p, src->d_tab.p, tbytes, cudaMemcpyDeviceToDevice, st));
+        if ((rc = d_G.alloc(gbytes)) || (rc = d_tab.alloc(tbytes))) return rc;
+        SDR_CUDA_TRY(cudaMemcpyAsync(d_G.p, src->d_G.p, gbytes, cudaMemcpyDeviceToDevice, st));
+        SDR_CUDA_TRY(cudaMemcpyAsync(d_tab.p, src->d_tab.p, tbytes, cudaMemcpyDeviceToDevice, st));
     } else {
         std::vector<float2> G, tab;
-        fcsb_tables(h, G, tab);
-        if ((rc = fcsb_upload(h->d_G, G.data(), gbytes, st))) return rc;
-        if ((rc = fcsb_upload(h->d_tab, tab.data(), tbytes, st))) return rc;
+        fcsb_tables(this, G, tab);
+        if ((rc = d_G.upload(G.data(), gbytes, st)) || (rc = d_tab.upload(tab.data(), tbytes, st))) return rc;
         SDR_CUDA_TRY(cudaStreamSynchronize(st));  // the host vectors go out of scope
     }
-    std::vector<longlong2> mb(h->C);
-    for (size_t k = 0; k < h->C; ++k) mb[k] = make_longlong2(h->chan[k].M, h->chan[k].base);
-    if ((rc = fcsb_upload(h->d_chan, h->chan.data(), h->C * sizeof(FcsbChan), st))) return rc;
-    if ((rc = fcsb_upload(h->d_mb, mb.data(), h->C * sizeof(longlong2), st))) return rc;
+    std::vector<longlong2> mb(C);
+    for (size_t k = 0; k < C; ++k) mb[k] = make_longlong2(chan[k].M, chan[k].base);
+    if ((rc = d_chan.upload(chan.data(), C * sizeof(FcsbChan), st))) return rc;
+    if ((rc = d_mb.upload(mb.data(), C * sizeof(longlong2), st))) return rc;
     for (int i = 0; i < 2; ++i)
-        if ((rc = h->d_hist[i].reserve(16))) return rc;
+        if ((rc = d_hist[i].reserve(16))) return rc;
     return cuda_status(cudaStreamSynchronize(st));
 }
 
-extern "C" sdr_fcsb_t *sdr_fcsb_create(const sdr_fcsb_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!cfg || !cfg->taps || !cfg->phase_inc || !cfg->interpolation || cfg->n_taps == 0 ||
-        cfg->n_taps > FCSB_MAX_TAPS || cfg->n_channels == 0 || cfg->n_channels > FCSB_MAX_CH ||
-        (cfg->n_tap_sets != 1 && cfg->n_tap_sets != cfg->n_channels)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    for (size_t k = 0; k < cfg->n_channels; ++k)
-        if (cfg->interpolation[k] == 0) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    for (size_t i = 0; i < cfg->n_taps * cfg->n_tap_sets; ++i)
-        if (!std::isfinite(cfg->taps[i])) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    size_t n_fft = 0, hop = 0;
-    if ((*err = sdr_fcfb_geometry(cfg->n_taps, cfg->interpolation, cfg->n_channels, &n_fft, &hop))) return nullptr;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    sdr_fcsb *h = new (std::nothrow) sdr_fcsb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = cfg->device;
-    h->L = cfg->n_taps;
-    h->C = cfg->n_channels;
-    h->n_sets = cfg->n_tap_sets;
-    h->first = cfg->first_sample;
-    h->taps.assign(cfg->taps, cfg->taps + h->L * h->n_sets);
-    h->inc.assign(cfg->phase_inc, cfg->phase_inc + h->C);
-    h->I.assign(cfg->interpolation, cfg->interpolation + h->C);
-    *err = fcsb_geometry_fields(h);
-    if (*err) { delete h; return nullptr; }
-    DeviceGuard g(h->dev);
-    *err = g.ok ? fcsb_alloc(h, cfg->stream, nullptr) : g.status();
-    if (*err) { fcsb_free(h); return nullptr; }
-    return h;
+// the carried frames
+inline int sdr_fcsb::copy_device(const sdr_fcsb &src) {
+    const size_t bytes = C * (size_t)hist_stride * sizeof(float2);
+    if (bytes == 0) return SDR_OK;
+    int rc = d_hist[0].reserve(bytes);
+    if (rc) return rc;
+    return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, bytes, cudaMemcpyDeviceToDevice));
 }
 
-extern "C" void sdr_fcsb_destroy(sdr_fcsb_t *h) { fcsb_free(h); }
+extern "C" sdr_fcsb_t *sdr_fcsb_create(const sdr_fcsb_config_t *cfg, int *err) {
+    if (!cfg || !cfg->taps || !cfg->phase_inc || !cfg->interpolation || cfg->n_taps == 0 ||
+        cfg->n_taps > FCSB_MAX_TAPS || cfg->n_channels == 0 || cfg->n_channels > FCSB_MAX_CH ||
+        (cfg->n_tap_sets != 1 && cfg->n_tap_sets != cfg->n_channels))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    for (size_t k = 0; k < cfg->n_channels; ++k)
+        if (cfg->interpolation[k] == 0) return fail(err, SDR_ERR_INVALID_ARG);
+    for (size_t i = 0; i < cfg->n_taps * cfg->n_tap_sets; ++i)
+        if (!std::isfinite(cfg->taps[i])) return fail(err, SDR_ERR_INVALID_ARG);
+    size_t n_fft = 0, hop = 0;
+    const int rc = sdr_fcfb_geometry(cfg->n_taps, cfg->interpolation, cfg->n_channels, &n_fft, &hop);
+    if (rc) return fail(err, rc);
+    return create_handle<sdr_fcsb>(err, cfg->device, cfg->stream, [&](sdr_fcsb &h) {
+        h.L = cfg->n_taps;
+        h.C = cfg->n_channels;
+        h.n_sets = cfg->n_tap_sets;
+        h.first = cfg->first_sample;
+        h.taps.assign(cfg->taps, cfg->taps + h.L * h.n_sets);
+        h.inc.assign(cfg->phase_inc, cfg->phase_inc + h.C);
+        h.I.assign(cfg->interpolation, cfg->interpolation + h.C);
+        return fcsb_geometry_fields(&h);
+    });
+}
+
+extern "C" void sdr_fcsb_destroy(sdr_fcsb_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_fcsb_reset(sdr_fcsb_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -358,29 +337,7 @@ extern "C" int sdr_fcsb_reset(sdr_fcsb_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_fcsb_t *sdr_fcsb_clone(const sdr_fcsb_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_fcsb *h = new (std::nothrow) sdr_fcsb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->L = src->L; h->C = src->C; h->n_sets = src->n_sets; h->first = src->first;
-    h->taps = src->taps; h->inc = src->inc; h->I = src->I;
-    h->N = src->N; h->P = src->P; h->Il = src->Il; h->Imin = src->Imin; h->off0 = src->off0; h->rows = src->rows;
-    h->chan = src->chan; h->groups = src->groups; h->order = src->order;
-    h->total = src->total; h->hist_lo = src->hist_lo; h->hist_stride = src->hist_stride;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? cuda_status(cudaStreamSynchronize(src->stream.s)) : g.status();
-    if (!*err) *err = fcsb_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s, src);
-    const size_t bytes = h->C * (size_t)h->hist_stride * sizeof(float2);
-    if (!*err && bytes > 0) {
-        *err = h->d_hist[0].reserve(bytes);
-        if (!*err) *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, bytes, cudaMemcpyDeviceToDevice));
-    }
-    if (*err) { fcsb_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_fcsb_t *sdr_fcsb_clone(const sdr_fcsb_t *src, int *err) { return clone_handle<FcsbHost>(src, err); }
 
 // blocks completed by the first T output positions, and the outputs among them
 static long long fcsb_blocks(const sdr_fcsb *h, long long T) { return (T + h->off0) / h->P; }
@@ -420,7 +377,7 @@ static int fcsb_blocks_run(sdr_fcsb *h, const FcsbSrc &src, long long jA, long l
             const long long first_ch = h->groups[q].second;
             const long long last = q + 1 < h->groups.size() ? h->groups[q + 1].second : (long long)h->C;
             const size_t off = (size_t)(nb * h->chan[h->order[first_ch]].base);
-            rc = sdr_fft_exec_dev(h->small[q], (const float2 *)h->d_v.p + off, (size_t)((last - first_ch) * nb),
+            rc = sdr_fft_exec_dev(h->small[q].get(), (const float2 *)h->d_v.p + off, (size_t)((last - first_ch) * nb),
                                   (float *)((float2 *)h->d_V.p + off));
             if (rc) return rc;
         }
@@ -429,7 +386,7 @@ static int fcsb_blocks_run(sdr_fcsb *h, const FcsbSrc &src, long long jA, long l
                                                (const longlong2 *)h->d_mb.p, (int)h->C, N, nb, (float2 *)h->d_S.p);
         count_launch();
         if ((rc = launch_status())) return rc;
-        if ((rc = sdr_fft_exec_dev(h->big, h->d_S.p, (size_t)nb, (float *)h->d_X.p))) return rc;
+        if ((rc = sdr_fft_exec_dev(h->big.get(), h->d_S.p, (size_t)nb, (float *)h->d_X.p))) return rc;
         dim3 gs((unsigned)((h->P + 255) / 256), (unsigned)nb);
         fcsb_store_kernel<<<gs, 256, 0, st>>>((const float2 *)h->d_X.p, N, h->P, h->off0, j0, n_lo, inv_n, out);
         count_launch();

@@ -20,16 +20,25 @@
 
 using namespace sdr;
 
-struct sdr_fm {
+struct FmHost {
     int dev = 0;
-    StreamRef stream;
     size_t n_st = 0;
     float rate = 0.f, rate_mid = 0.f, rate_out = 0.f;
+    float pilot_hz = 19000.0f;
+    unsigned pll_flags = 0;
     double ratio1 = 0.0, ratio2 = 0.0;
-    sdr_pll_t *demod = nullptr, *pilot = nullptr;
-    std::vector<SDR_SRC_STATE *> src1, src2;
-    sdr_biquad_t *deemph = nullptr;
+};
+
+using SrcHandle = Owned<SDR_SRC_STATE, sdr_src_delete>;
+
+struct sdr_fm : FmHost {
+    StreamRef stream;
+    Owned<sdr_pll_t, sdr_pll_destroy> demod, pilot;
+    std::vector<SrcHandle> src1, src2;
+    Owned<sdr_biquad_t, sdr_biquad_destroy> deemph;
     DevBuf d_iq, d_c64, d_v, d_lk, d_v2, d_md, d_md2, d_out;
+
+    int alloc(void *user_stream, const sdr_fm *);
 };
 
 // A sinc converter withholds the outputs whose right wing it has not seen yet and hands them over in a later call (or
@@ -37,102 +46,74 @@ struct sdr_fm {
 // capacity carries this slack on top of ceil(n * ratio).
 static const size_t kFmSlack = 256;
 
-static void fm_free(sdr_fm *f) {
-    if (!f) return;
-    DeviceGuard g(f->dev);
-    if (f->demod) sdr_pll_destroy(f->demod);
-    if (f->pilot) sdr_pll_destroy(f->pilot);
-    for (auto *s : f->src1) if (s) sdr_src_delete(s);
-    for (auto *s : f->src2) if (s) sdr_src_delete(s);
-    if (f->deemph) sdr_biquad_destroy(f->deemph);
-    f->d_iq.release(); f->d_c64.release(); f->d_v.release(); f->d_lk.release();
-    f->d_v2.release(); f->d_md.release(); f->d_md2.release(); f->d_out.release();
-    f->stream.release();
-    delete f;
-}
-
-extern "C" sdr_fm_t *sdr_fm_create(const sdr_fm_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!cfg || cfg->n_stations == 0 || cfg->n_stations > (1u << 16) || !(cfg->rate >= 144000.0f)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    sdr_fm *f = new (std::nothrow) sdr_fm;
-    if (!f) {
-        *err = SDR_ERR_MALLOC_FAILED;
-        return nullptr;
-    }
-    f->dev = cfg->device;
-    f->n_st = cfg->n_stations;
-    f->rate = cfg->rate;
-    f->rate_mid = 48000.0f * 3.0f;  // main.rs:50
-    f->rate_out = 48000.0f;         // main.rs:73
-    // Resample::new: ratio = rate as f64 / signal.rate() as f64   (adapters/resample.rs:25)
-    f->ratio1 = (double)f->rate_mid / (double)f->rate;
-    f->ratio2 = (double)f->rate_out / (double)f->rate_mid;
-    DeviceGuard g(f->dev);
-    int rc = g.ok ? f->stream.init(cfg->stream) : g.status();
-    if (rc) { *err = rc; fm_free(f); return nullptr; }
-    void *st = (void *)f->stream.s;
+// the stages of one receiver, all on the handle's stream
+int sdr_fm::alloc(void *user_stream, const sdr_fm *) {
+    int rc = stream.init(user_stream);
+    if (rc) return rc;
+    void *st = (void *)stream.s;
 
     sdr_pll_design_t dd;  // main.rs:41-46
     dd.reference = 0.0f; dd.gain = 0.035f;
     dd.loopfilter = {SDR_BQ_LOWPASS, 80000.0f, 0.7f};
     dd.outputfilter = {SDR_BQ_IDENTITY, 0.f, 0.f};
     dd.lockfilter = {SDR_BQ_LOWPASS, 20000.0f, 0.7f};
-    sdr_pll_config_t pc = {&dd, 1, f->n_st, f->rate, cfg->flags & (SDR_PLL_FAST_MATH | SDR_PLL_F64_MATH), f->dev, st};
-    f->demod = sdr_pll_create(&pc, &rc);
-    if (!f->demod) { *err = rc; fm_free(f); return nullptr; }
+    sdr_pll_config_t pc = {&dd, 1, n_st, rate, pll_flags, dev, st};
+    demod.reset(sdr_pll_create(&pc, &rc));
+    if (!demod) return rc;
 
     sdr_pll_design_t pd;  // main.rs:54-60
-    pd.reference = cfg->pilot > 0.f ? cfg->pilot : 19000.0f; pd.gain = 0.0002f;
+    pd.reference = pilot_hz; pd.gain = 0.0002f;
     pd.loopfilter = {SDR_BQ_LOWPASS, 200.0f, 0.7f};
     pd.outputfilter = {SDR_BQ_LOWPASS, 20.0f, 0.7f};
     pd.lockfilter = {SDR_BQ_LOWPASS, 20.0f, 0.7f};
-    sdr_pll_config_t pp = {&pd, 1, f->n_st, f->rate_mid, cfg->flags & (SDR_PLL_FAST_MATH | SDR_PLL_F64_MATH), f->dev, st};
-    f->pilot = sdr_pll_create(&pp, &rc);
-    if (!f->pilot) { *err = rc; fm_free(f); return nullptr; }
+    sdr_pll_config_t pp = {&pd, 1, n_st, rate_mid, pll_flags, dev, st};
+    pilot.reset(sdr_pll_create(&pp, &rc));
+    if (!pilot) return rc;
 
-    f->src1.assign(f->n_st, nullptr);
-    f->src2.assign(f->n_st, nullptr);
-    for (size_t i = 0; i < f->n_st; ++i) {
-        f->src1[i] = sdr_src_new_on(SDR_SRC_SINC_FASTEST, 1, f->dev, st, &rc);                     // main.rs:50
-        if (f->src1[i]) f->src2[i] = sdr_src_new_on(SDR_SRC_SINC_BEST_QUALITY, 2, f->dev, st, &rc);  // main.rs:73
-        if (!f->src1[i] || !f->src2[i]) { *err = rc ? rc : SDR_ERR_MALLOC_FAILED; fm_free(f); return nullptr; }
+    src1.resize(n_st);
+    src2.resize(n_st);
+    for (size_t i = 0; i < n_st; ++i) {
+        src1[i].reset(sdr_src_new_on(SDR_SRC_SINC_FASTEST, 1, dev, st, &rc));                     // main.rs:50
+        if (src1[i]) src2[i].reset(sdr_src_new_on(SDR_SRC_SINC_BEST_QUALITY, 2, dev, st, &rc));  // main.rs:73
+        if (!src1[i] || !src2[i]) return rc ? rc : SDR_ERR_MALLOC_FAILED;
     }
     sdr_biquad_design_t de = {SDR_BQ_LR, 1.0f / (75.0f * 0.001f * 0.001f), 0.f};  // main.rs:52
     sdr_biquad_config_t bc;
-    bc.designs = &de; bc.n_designs = 1; bc.n_streams = f->n_st; bc.rate = f->rate_out;
+    bc.designs = &de; bc.n_designs = 1; bc.n_streams = n_st; bc.rate = rate_out;
     bc.sample_complex = 1;  // (mono, diff) frames: both parts through the same real coefficients (main.rs:74-78)
-    bc.device = f->dev; bc.stream = st;
-    f->deemph = sdr_biquad_create(&bc, &rc);
-    if (!f->deemph) { *err = rc; fm_free(f); return nullptr; }
-    return f;
+    bc.device = dev; bc.stream = st;
+    deemph.reset(sdr_biquad_create(&bc, &rc));
+    return deemph ? SDR_OK : rc;
 }
 
-extern "C" void sdr_fm_destroy(sdr_fm_t *f) { fm_free(f); }
+extern "C" sdr_fm_t *sdr_fm_create(const sdr_fm_config_t *cfg, int *err) {
+    if (!cfg || cfg->n_stations == 0 || cfg->n_stations > (1u << 16) || !(cfg->rate >= 144000.0f))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_fm>(err, cfg->device, cfg->stream, [&](sdr_fm &f) {
+        f.n_st = cfg->n_stations;
+        f.rate = cfg->rate;
+        f.rate_mid = 48000.0f * 3.0f;  // main.rs:50
+        f.rate_out = 48000.0f;         // main.rs:73
+        f.pilot_hz = cfg->pilot > 0.f ? cfg->pilot : 19000.0f;
+        f.pll_flags = cfg->flags & (SDR_PLL_FAST_MATH | SDR_PLL_F64_MATH);
+        // Resample::new: ratio = rate as f64 / signal.rate() as f64   (adapters/resample.rs:25)
+        f.ratio1 = (double)f.rate_mid / (double)f.rate;
+        f.ratio2 = (double)f.rate_out / (double)f.rate_mid;
+        return SDR_OK;
+    });
+}
+
+extern "C" void sdr_fm_destroy(sdr_fm_t *f) { destroy_handle(f); }
 
 extern "C" int sdr_fm_reset(sdr_fm_t *f) {
     if (!f) return SDR_ERR_NULL_HANDLE;
-    int rc = sdr_pll_reset(f->demod);
-    if (!rc) rc = sdr_pll_reset(f->pilot);
+    int rc = sdr_pll_reset(f->demod.get());
+    if (!rc) rc = sdr_pll_reset(f->pilot.get());
     for (size_t i = 0; i < f->n_st && !rc; ++i) {
-        rc = sdr_src_reset(f->src1[i]);
-        if (!rc) rc = sdr_src_reset(f->src2[i]);
+        rc = sdr_src_reset(f->src1[i].get());
+        if (!rc) rc = sdr_src_reset(f->src2[i].get());
     }
-    if (!rc) rc = sdr_biquad_reset(f->deemph);
+    if (!rc) rc = sdr_biquad_reset(f->deemph.get());
     return rc;
 }
 
@@ -147,7 +128,7 @@ extern "C" size_t sdr_fm_max_output(const sdr_fm_t *f, size_t n) {
 // one resampler stage for every station: rows of `n_in` frames -> rows of up to `cap` frames.  All stations see the
 // same counts (they depend on the call history only).  With end_of_input the converter is flushed the way the
 // Resample adaptor does it (empty input => end_of_input, until nothing comes back: adapters/resample.rs:45-65).
-static int fm_resample(std::vector<SDR_SRC_STATE *> &src, double ratio, int ch, const float *in, size_t n_in,
+static int fm_resample(std::vector<SrcHandle> &src, double ratio, int ch, const float *in, size_t n_in,
                        size_t in_stride, float *out, size_t cap, size_t out_stride, int end_of_input, size_t *n_out) {
     size_t gen0 = 0;
     for (size_t i = 0; i < src.size(); ++i) {
@@ -161,7 +142,7 @@ static int fm_resample(std::vector<SDR_SRC_STATE *> &src, double ratio, int ch, 
         d.end_of_input = 0;
         d.src_ratio = ratio;
         if (n_in > 0) {
-            const int rc = sdr_src_process_dev(src[i], &d);
+            const int rc = sdr_src_process_dev(src[i].get(), &d);
             if (rc) return rc;
             if ((size_t)d.input_frames_used != n_in) return SDR_ERR_OUTPUT_TOO_SMALL;
             gen = (size_t)d.output_frames_gen;
@@ -173,7 +154,7 @@ static int fm_resample(std::vector<SDR_SRC_STATE *> &src, double ratio, int ch, 
                 d.input_frames = 0;
                 d.output_frames = (long)(cap - gen);
                 d.end_of_input = 1;
-                const int rc = sdr_src_process_dev(src[i], &d);
+                const int rc = sdr_src_process_dev(src[i].get(), &d);
                 if (rc) return rc;
                 if (d.output_frames_gen == 0) break;
                 gen += (size_t)d.output_frames_gen;
@@ -210,7 +191,7 @@ static int fm_run(sdr_fm *f, const uint8_t *d_iq, size_t n, size_t in_stride, fl
     if (n > 0) {
         for (size_t i = 0; i < S && !rc; ++i)  // rows may be padded on the caller's side
             rc = sdr_unpack_u8iq_dev(d_iq + i * in_stride, n, c64 + 2 * i * nc, f->dev, (void *)st);
-        if (!rc) rc = sdr_pll_process_dev(f->demod, c64, n, nc, v, lk, n);
+        if (!rc) rc = sdr_pll_process_dev(f->demod.get(), c64, n, nc, v, lk, n);
         if (!rc) rc = fm_demod_map_launch(v, lk, v, (long long)(S * n), st);
         if (rc) return rc;
     }
@@ -218,14 +199,14 @@ static int fm_run(sdr_fm *f, const uint8_t *d_iq, size_t n, size_t in_stride, fl
     rc = fm_resample(f->src1, f->ratio1, 1, v, n, n, v2, cap2, cap2, end_of_input, &n2);
     if (rc) return rc;
     if (n2 > 0) {
-        rc = sdr_pll_stereo_decode_dev(f->pilot, v2, n2, cap2, md, cap2);
+        rc = sdr_pll_stereo_decode_dev(f->pilot.get(), v2, n2, cap2, md, cap2);
         if (rc) return rc;
     }
     rc = fm_resample(f->src2, f->ratio2, 2, md, n2, cap2, md2, cap3, cap3, end_of_input, &n3);
     if (rc) return rc;
     if (n3 > out_cap) return SDR_ERR_OUTPUT_TOO_SMALL;
     if (n3 > 0) {
-        rc = sdr_biquad_process_dev(f->deemph, md2, n3, cap3, md2, cap3);
+        rc = sdr_biquad_process_dev(f->deemph.get(), md2, n3, cap3, md2, cap3);
         if (!rc) rc = fm_matrix_launch(md2, (long long)cap3, d_out, (long long)out_stride, (int)S, (long long)n3, st);
         if (rc) return rc;
     }

@@ -179,101 +179,71 @@ bool pfb_launch_reg(int R, int TT, const PfbSrc &s, const float *taps, int M, lo
 
 }  // namespace
 
-struct sdr_pfb {
+struct PfbHost {
     int dev = 0;
-    StreamRef stream;
     size_t L = 0, M = 0, D = 1, T = 0, HL = 0;
     int fmt = SDR_FMT_C64;
     unsigned flags = 0;
     int reg_R = 0, reg_TT = 0;  // register-window geometry, 0 = general kernel
     std::vector<float> taps;    // T * M, zero padded
-    float *d_taps = nullptr;
-    sdr_fft_t *plan = nullptr;
     long long total = 0;        // input samples seen; frames completed = total / D
+};
+
+static size_t pfb_es(const PfbHost *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
+
+struct sdr_pfb : PfbHost {
+    StreamRef stream;
+    Owned<sdr_fft_t, sdr_fft_destroy> plan;
+    DevBuf d_taps;
     DevBuf d_hist[2];           // the last HL inputs before `total`, raw format
     int cur = 0;
     DevBuf d_u, d_y, d_in, d_out;
+
+    // taps, FFT plan and history buffers of a handle whose geometry fields are set
+    int alloc(void *user_stream, const sdr_pfb *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        if ((rc = d_taps.upload(taps.data(), taps.size() * sizeof(float), stream.s))) return rc;
+        for (int i = 0; i < 2; ++i)
+            if ((rc = d_hist[i].reserve(std::max<size_t>(HL, 2) * pfb_es(this)))) return rc;
+        sdr_fft_config_t fc;
+        fc.n = M;
+        fc.input_format = SDR_FMT_C64;
+        fc.flags = (flags & SDR_PFB_SHIFT) ? SDR_FFT_SHIFT : 0u;
+        fc.device = dev;
+        fc.stream = (void *)stream.s;
+        plan.reset(sdr_fft_create(&fc, &rc));
+        if (!plan) return rc;
+        return cuda_status(cudaStreamSynchronize(stream.s));
+    }
+    int copy_device(const sdr_pfb &src) {
+        if (HL == 0) return SDR_OK;
+        return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, HL * pfb_es(this), cudaMemcpyDeviceToDevice));
+    }
 };
 
-static void pfb_free(sdr_pfb *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    if (h->plan) sdr_fft_destroy(h->plan);
-    if (h->d_taps) cudaFree(h->d_taps);
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_u.release(); h->d_y.release(); h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
-
-static size_t pfb_es(const sdr_pfb *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
-
-// taps, FFT plan and history buffers of a handle whose geometry fields are set
-static int pfb_alloc(sdr_pfb *h, void *user_stream) {
-    int rc = h->stream.init(user_stream);
-    if (rc) return rc;
-    SDR_CUDA_TRY(cudaMalloc(&h->d_taps, h->taps.size() * sizeof(float)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(h->d_taps, h->taps.data(), h->taps.size() * sizeof(float), cudaMemcpyHostToDevice,
-                                 h->stream.s));
-    for (int i = 0; i < 2; ++i) {
-        rc = h->d_hist[i].reserve(std::max<size_t>(h->HL, 2) * pfb_es(h));
-        if (rc) return rc;
-    }
-    sdr_fft_config_t fc;
-    fc.n = h->M;
-    fc.input_format = SDR_FMT_C64;
-    fc.flags = (h->flags & SDR_PFB_SHIFT) ? SDR_FFT_SHIFT : 0u;
-    fc.device = h->dev;
-    fc.stream = (void *)h->stream.s;
-    h->plan = sdr_fft_create(&fc, &rc);
-    if (!h->plan) return rc;
-    return cuda_status(cudaStreamSynchronize(h->stream.s));
-}
-
 extern "C" sdr_pfb_t *sdr_pfb_create(const sdr_pfb_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->taps || cfg->n_taps == 0 || cfg->n_taps > ((size_t)1 << 24) || cfg->n_channels < 2 ||
         cfg->n_channels > 65536 || cfg->decimation == 0 || cfg->decimation > ((size_t)1 << 40) ||
-        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) || (cfg->flags & ~PFB_FLAGS)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    sdr_pfb *h = new (std::nothrow) sdr_pfb;
-    if (!h) {
-        *err = SDR_ERR_MALLOC_FAILED;
-        return nullptr;
-    }
-    h->dev = cfg->device;
-    h->L = cfg->n_taps;
-    h->M = cfg->n_channels;
-    h->D = cfg->decimation;
-    h->T = (h->L + h->M - 1) / h->M;
-    h->HL = h->L - 1;
-    h->fmt = cfg->input_format;
-    h->flags = cfg->flags;
-    h->taps.assign(h->T * h->M, 0.0f);
-    std::memcpy(h->taps.data(), cfg->taps, h->L * sizeof(float));
-    if (!(h->flags & SDR_PFB_GENERAL_KERNEL) && !pfb_reg_geometry(h->M, h->D, h->T, &h->reg_R, &h->reg_TT))
-        h->reg_R = h->reg_TT = 0;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? pfb_alloc(h, cfg->stream) : g.status();
-    if (*err) { pfb_free(h); return nullptr; }
-    return h;
+        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) || (cfg->flags & ~PFB_FLAGS))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_pfb>(err, cfg->device, cfg->stream, [&](sdr_pfb &h) {
+        h.L = cfg->n_taps;
+        h.M = cfg->n_channels;
+        h.D = cfg->decimation;
+        h.T = (h.L + h.M - 1) / h.M;
+        h.HL = h.L - 1;
+        h.fmt = cfg->input_format;
+        h.flags = cfg->flags;
+        h.taps.assign(h.T * h.M, 0.0f);
+        std::memcpy(h.taps.data(), cfg->taps, h.L * sizeof(float));
+        if (!(h.flags & SDR_PFB_GENERAL_KERNEL) && !pfb_reg_geometry(h.M, h.D, h.T, &h.reg_R, &h.reg_TT))
+            h.reg_R = h.reg_TT = 0;
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_pfb_destroy(sdr_pfb_t *h) { pfb_free(h); }
+extern "C" void sdr_pfb_destroy(sdr_pfb_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_pfb_reset(sdr_pfb_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -283,24 +253,7 @@ extern "C" int sdr_pfb_reset(sdr_pfb_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_pfb_t *sdr_pfb_clone(const sdr_pfb_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_pfb *h = new (std::nothrow) sdr_pfb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->L = src->L; h->M = src->M; h->D = src->D; h->T = src->T; h->HL = src->HL;
-    h->fmt = src->fmt; h->flags = src->flags; h->reg_R = src->reg_R; h->reg_TT = src->reg_TT;
-    h->taps = src->taps; h->total = src->total;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? pfb_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s) : g.status();
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err && h->HL > 0)
-        *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, h->HL * pfb_es(h), cudaMemcpyDeviceToDevice));
-    if (*err) { pfb_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_pfb_t *sdr_pfb_clone(const sdr_pfb_t *src, int *err) { return clone_handle<PfbHost>(src, err); }
 
 // frames that the next n_in samples complete: frame j needs input sample (j + 1) * D - 1
 extern "C" size_t sdr_pfb_output_count(const sdr_pfb_t *h, size_t n_in) {
@@ -315,6 +268,7 @@ static int pfb_run(sdr_pfb *h, const void *in, size_t n_in, float *out, size_t o
     const size_t M = h->M, es = pfb_es(h);
     const long long D = (long long)h->D;
     const bool cmajor = (h->flags & SDR_PFB_CHANNEL_MAJOR) != 0;
+    const float *taps = (const float *)h->d_taps.p;
     PfbSrc s;
     s.hist = h->d_hist[h->cur].p;
     s.in = in;
@@ -340,26 +294,26 @@ static int pfb_run(sdr_pfb *h, const void *in, size_t n_in, float *out, size_t o
             bool done = false;
             if (h->reg_R) {
                 done = h->fmt == SDR_FMT_U8IQ
-                           ? pfb_launch_reg<true>(h->reg_R, h->reg_TT, s, h->d_taps, (int)M, D, (int)h->L, j0, (long long)cnt, u, st)
-                           : pfb_launch_reg<false>(h->reg_R, h->reg_TT, s, h->d_taps, (int)M, D, (int)h->L, j0, (long long)cnt, u, st);
+                           ? pfb_launch_reg<true>(h->reg_R, h->reg_TT, s, taps, (int)M, D, (int)h->L, j0, (long long)cnt, u, st)
+                           : pfb_launch_reg<false>(h->reg_R, h->reg_TT, s, taps, (int)M, D, (int)h->L, j0, (long long)cnt, u, st);
             }
             if (!done) {
                 dim3 grid((unsigned)((M + 255) / 256), (unsigned)std::min<size_t>(cnt, 65535));
                 if (h->fmt == SDR_FMT_U8IQ)
-                    pfb_front_general_kernel<true><<<grid, 256, 0, st>>>(s, h->d_taps, (int)M, D, (int)h->L, j0, (long long)cnt, u);
+                    pfb_front_general_kernel<true><<<grid, 256, 0, st>>>(s, taps, (int)M, D, (int)h->L, j0, (long long)cnt, u);
                 else
-                    pfb_front_general_kernel<false><<<grid, 256, 0, st>>>(s, h->d_taps, (int)M, D, (int)h->L, j0, (long long)cnt, u);
+                    pfb_front_general_kernel<false><<<grid, 256, 0, st>>>(s, taps, (int)M, D, (int)h->L, j0, (long long)cnt, u);
             }
             count_launch();
             rc = launch_status();
             if (rc) return rc;
             if (direct) {
-                rc = sdr_fft_exec_dev(h->plan, u, cnt, out + f0 * M * 2);
+                rc = sdr_fft_exec_dev(h->plan.get(), u, cnt, out + f0 * M * 2);
                 if (rc) return rc;
                 continue;
             }
             float2 *y = (float2 *)h->d_y.p;
-            rc = sdr_fft_exec_dev(h->plan, u, cnt, (float *)y);
+            rc = sdr_fft_exec_dev(h->plan.get(), u, cnt, (float *)y);
             if (rc) return rc;
             if (cmajor) {
                 pfb_transpose_kernel<<<dim3((unsigned)((M + 31) / 32), (unsigned)((cnt + 31) / 32)), dim3(32, 8), 0, st>>>(

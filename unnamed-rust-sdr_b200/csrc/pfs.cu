@@ -189,95 +189,65 @@ bool pfs_launch_reg(int R, int TT, const PfsSrc &s, const float *taps, int M, in
 
 }  // namespace
 
-struct sdr_pfs {
+struct PfsHost {
     int dev = 0;
-    StreamRef stream;
     size_t L = 0, M = 0, D = 1, H = 0;
     unsigned flags = 0;
     int reg_R = 0, reg_TT = 0;  // register-window geometry, 0 = general kernel
     std::vector<float> taps;
-    float *d_taps = nullptr;
-    sdr_fft_t *plan = nullptr;
     long long total = 0;        // frames seen
+};
+
+struct sdr_pfs : PfsHost {
+    StreamRef stream;
+    Owned<sdr_fft_t, sdr_fft_destroy> plan;
+    DevBuf d_taps;
     DevBuf d_hist[2];           // transforms of the H frames before `total`, frames x M
     int cur = 0;
     DevBuf d_u, d_y, d_in, d_out;
+
+    // taps, FFT plan and history buffers of a handle whose geometry fields are set
+    int alloc(void *user_stream, const sdr_pfs *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        if ((rc = d_taps.upload(taps.data(), taps.size() * sizeof(float), stream.s))) return rc;
+        for (int i = 0; i < 2; ++i)
+            if ((rc = d_hist[i].reserve(std::max<size_t>(H, 1) * M * 8))) return rc;
+        sdr_fft_config_t fc;
+        fc.n = M;
+        fc.input_format = SDR_FMT_C64;
+        fc.flags = 0;
+        fc.device = dev;
+        fc.stream = (void *)stream.s;
+        plan.reset(sdr_fft_create(&fc, &rc));
+        if (!plan) return rc;
+        return cuda_status(cudaStreamSynchronize(stream.s));
+    }
+    int copy_device(const sdr_pfs &src) {
+        if (H == 0) return SDR_OK;
+        return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, H * M * 8, cudaMemcpyDeviceToDevice));
+    }
 };
 
-static void pfs_free(sdr_pfs *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    if (h->plan) sdr_fft_destroy(h->plan);
-    if (h->d_taps) cudaFree(h->d_taps);
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_u.release(); h->d_y.release(); h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
-
-// taps, FFT plan and history buffers of a handle whose geometry fields are set
-static int pfs_alloc(sdr_pfs *h, void *user_stream) {
-    int rc = h->stream.init(user_stream);
-    if (rc) return rc;
-    SDR_CUDA_TRY(cudaMalloc(&h->d_taps, h->taps.size() * sizeof(float)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(h->d_taps, h->taps.data(), h->taps.size() * sizeof(float), cudaMemcpyHostToDevice,
-                                 h->stream.s));
-    for (int i = 0; i < 2; ++i) {
-        rc = h->d_hist[i].reserve(std::max<size_t>(h->H, 1) * h->M * 8);
-        if (rc) return rc;
-    }
-    sdr_fft_config_t fc;
-    fc.n = h->M;
-    fc.input_format = SDR_FMT_C64;
-    fc.flags = 0;
-    fc.device = h->dev;
-    fc.stream = (void *)h->stream.s;
-    h->plan = sdr_fft_create(&fc, &rc);
-    if (!h->plan) return rc;
-    return cuda_status(cudaStreamSynchronize(h->stream.s));
-}
-
 extern "C" sdr_pfs_t *sdr_pfs_create(const sdr_pfs_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || !cfg->taps || cfg->n_taps == 0 || cfg->n_taps > ((size_t)1 << 24) || cfg->n_channels < 2 ||
         cfg->n_channels > 65536 || cfg->interpolation == 0 || cfg->interpolation > ((size_t)1 << 32) ||
-        (cfg->flags & ~PFS_FLAGS)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    sdr_pfs *h = new (std::nothrow) sdr_pfs;
-    if (!h) {
-        *err = SDR_ERR_MALLOC_FAILED;
-        return nullptr;
-    }
-    h->dev = cfg->device;
-    h->L = cfg->n_taps;
-    h->M = cfg->n_channels;
-    h->D = cfg->interpolation;
-    h->H = (h->L - 1 + h->D - 1) / h->D;
-    h->flags = cfg->flags;
-    h->taps.assign(cfg->taps, cfg->taps + h->L);
-    if (!(h->flags & SDR_PFS_GENERAL_KERNEL) && !pfs_reg_geometry(h->M, h->D, h->L, &h->reg_R, &h->reg_TT))
-        h->reg_R = h->reg_TT = 0;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? pfs_alloc(h, cfg->stream) : g.status();
-    if (*err) { pfs_free(h); return nullptr; }
-    return h;
+        (cfg->flags & ~PFS_FLAGS))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_pfs>(err, cfg->device, cfg->stream, [&](sdr_pfs &h) {
+        h.L = cfg->n_taps;
+        h.M = cfg->n_channels;
+        h.D = cfg->interpolation;
+        h.H = (h.L - 1 + h.D - 1) / h.D;
+        h.flags = cfg->flags;
+        h.taps.assign(cfg->taps, cfg->taps + h.L);
+        if (!(h.flags & SDR_PFS_GENERAL_KERNEL) && !pfs_reg_geometry(h.M, h.D, h.L, &h.reg_R, &h.reg_TT))
+            h.reg_R = h.reg_TT = 0;
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_pfs_destroy(sdr_pfs_t *h) { pfs_free(h); }
+extern "C" void sdr_pfs_destroy(sdr_pfs_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_pfs_reset(sdr_pfs_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -287,24 +257,7 @@ extern "C" int sdr_pfs_reset(sdr_pfs_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_pfs_t *sdr_pfs_clone(const sdr_pfs_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_pfs *h = new (std::nothrow) sdr_pfs;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->L = src->L; h->M = src->M; h->D = src->D; h->H = src->H;
-    h->flags = src->flags; h->reg_R = src->reg_R; h->reg_TT = src->reg_TT;
-    h->taps = src->taps; h->total = src->total;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? pfs_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s) : g.status();
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err && h->H > 0)
-        *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, h->H * h->M * 8, cudaMemcpyDeviceToDevice));
-    if (*err) { pfs_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_pfs_t *sdr_pfs_clone(const sdr_pfs_t *src, int *err) { return clone_handle<PfsHost>(src, err); }
 
 extern "C" size_t sdr_pfs_output_count(const sdr_pfs_t *h, size_t n_frames) {
     if (!h) return 0;
@@ -340,7 +293,7 @@ static int pfs_run(sdr_pfs *h, const float2 *in, size_t nf, size_t in_stride, fl
             if ((rc = launch_status())) return rc;
             x = u;
         }
-        if ((rc = sdr_fft_exec_dev(h->plan, x, cnt, (float *)y))) return rc;
+        if ((rc = sdr_fft_exec_dev(h->plan.get(), x, cnt, (float *)y))) return rc;
         PfsSrc s;
         s.hist = (const float2 *)h->d_hist[h->cur].p;
         s.y = y;
@@ -350,10 +303,11 @@ static int pfs_run(sdr_pfs *h, const float2 *in, size_t nf, size_t in_stride, fl
         s.end = h->total + (long long)cnt;
         const long long t0 = h->total * D, nt = (long long)cnt * D;
         float2 *o = out + f0 * (size_t)D;
-        bool done = h->reg_R && pfs_launch_reg(h->reg_R, h->reg_TT, s, h->d_taps, (int)M, (int)D, (int)h->L, t0, nt, o, st);
+        const float *taps = (const float *)h->d_taps.p;
+        bool done = h->reg_R && pfs_launch_reg(h->reg_R, h->reg_TT, s, taps, (int)M, (int)D, (int)h->L, t0, nt, o, st);
         if (!done)
             pfs_back_general_kernel<<<(unsigned)std::min<long long>((nt + 255) / 256, 1 << 20), 256, 0, st>>>(
-                s, h->d_taps, (int)M, D, (int)h->L, t0, nt, o);
+                s, taps, (int)M, D, (int)h->L, t0, nt, o);
         count_launch();
         if ((rc = launch_status())) return rc;
         // history = the transforms of the last H frames of (history, slab)

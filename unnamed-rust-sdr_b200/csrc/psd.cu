@@ -263,120 +263,100 @@ __global__ void psd_reduce_kernel(const float *__restrict__ part, long long gidA
 }  // namespace
 }  // namespace sdr
 
-struct sdr_psd {
+struct PsdHost {
     int dev = 0;
-    StreamRef stream;
     long long N = 0, H = 0, K = 0, cpg = 1;
     int fmt = SDR_FMT_C64;
     unsigned flags = 0;
     bool fused = false;          // path 2
     double scale = 1.0;          // 1/K, and 1/N with NORM
     std::vector<float> taper;
-    float *d_taper = nullptr;
-    float2 *d_tw = nullptr;      // W_1024 (path 2)
-    sdr_fft_t *plan = nullptr;   // path 1
     long long total = 0;         // input samples seen
     long long done = 0;          // frames in finished chunks (a chunk boundary)
     long long hist_lo = 0;       // d_hist[cur] holds stream samples hist_lo .. total - 1
+    int last_path = 0;
+};
+
+static size_t psd_es(const PsdHost *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
+
+struct sdr_psd : PsdHost {
+    StreamRef stream;
+    Owned<sdr_fft_t, sdr_fft_destroy> plan;  // path 1
+    DevBuf d_taper;
+    DevBuf d_tw;                 // W_1024 (path 2)
     DevBuf d_hist[2];
     int cur = 0;
     DevBuf d_acc[2];             // f64 sum of the open group's finished chunks
     int acur = 0;
     DevBuf d_part, d_x, d_y, d_in, d_out;
-    int last_path = 0;
+
+    // taper, twiddles or FFT plan, history and accumulators of a handle whose geometry fields are set
+    int alloc(void *user_stream, const sdr_psd *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        cudaStream_t st = stream.s;
+        if ((rc = d_taper.upload(taper.data(), taper.size() * sizeof(float), st))) return rc;
+        std::vector<float2> tw;
+        if (fused) {
+            // the FFT plans' table: f64 angles rounded to f32
+            tw.resize(1024);
+            for (int k = 0; k < 1024; ++k)
+                tw[k] = make_float2((float)std::cos(-2.0 * M_PI / 1024.0 * k), (float)std::sin(-2.0 * M_PI / 1024.0 * k));
+            if ((rc = d_tw.upload(tw.data(), tw.size() * sizeof(float2), st))) return rc;
+        } else {
+            sdr_fft_config_t fc;
+            fc.n = (size_t)N;
+            fc.input_format = SDR_FMT_C64;  // the gather unpacks and tapers
+            fc.flags = (flags & SDR_PSD_SHIFT) ? SDR_FFT_SHIFT : 0u;  // NORM is applied in f64 at the end
+            fc.device = dev;
+            fc.stream = (void *)st;
+            plan.reset(sdr_fft_create(&fc, &rc));
+            if (!plan) return rc;
+        }
+        for (int i = 0; i < 2; ++i) {
+            rc = d_hist[i].reserve(16);
+            if (!rc) rc = d_acc[i].reserve((size_t)N * sizeof(double));
+            if (rc) return rc;
+        }
+        return cuda_status(cudaStreamSynchronize(st));
+    }
+    // the history tail and the open group's accumulator
+    int copy_device(const sdr_psd &src) {
+        const size_t tail = (size_t)(total - hist_lo) * psd_es(this);
+        int rc = SDR_OK;
+        if (tail > 0) {
+            rc = d_hist[0].reserve(tail);
+            if (!rc) rc = cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, tail, cudaMemcpyDeviceToDevice));
+        }
+        if (!rc)
+            rc = cuda_status(cudaMemcpy(d_acc[0].p, src.d_acc[src.acur].p, (size_t)N * sizeof(double),
+                                        cudaMemcpyDeviceToDevice));
+        return rc;
+    }
 };
 
-static void psd_free(sdr_psd *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    if (h->plan) sdr_fft_destroy(h->plan);
-    if (h->d_taper) cudaFree(h->d_taper);
-    if (h->d_tw) cudaFree(h->d_tw);
-    h->d_hist[0].release(); h->d_hist[1].release(); h->d_acc[0].release(); h->d_acc[1].release();
-    h->d_part.release(); h->d_x.release(); h->d_y.release(); h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
-
-static size_t psd_es(const sdr_psd *h) { return h->fmt == SDR_FMT_U8IQ ? 2 : 8; }
-
-// taper, twiddles or FFT plan, history and accumulators of a handle whose geometry fields are set
-static int psd_alloc(sdr_psd *h, void *user_stream) {
-    int rc = h->stream.init(user_stream);
-    if (rc) return rc;
-    cudaStream_t st = h->stream.s;
-    SDR_CUDA_TRY(cudaMalloc(&h->d_taper, h->taper.size() * sizeof(float)));
-    SDR_CUDA_TRY(cudaMemcpyAsync(h->d_taper, h->taper.data(), h->taper.size() * sizeof(float), cudaMemcpyHostToDevice, st));
-    std::vector<float2> tw;
-    if (h->fused) {
-        // the FFT plans' table: f64 angles rounded to f32
-        tw.resize(1024);
-        for (int k = 0; k < 1024; ++k)
-            tw[k] = make_float2((float)std::cos(-2.0 * M_PI / 1024.0 * k), (float)std::sin(-2.0 * M_PI / 1024.0 * k));
-        SDR_CUDA_TRY(cudaMalloc(&h->d_tw, tw.size() * sizeof(float2)));
-        SDR_CUDA_TRY(cudaMemcpyAsync(h->d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice, st));
-    } else {
-        sdr_fft_config_t fc;
-        fc.n = (size_t)h->N;
-        fc.input_format = SDR_FMT_C64;  // the gather unpacks and tapers
-        fc.flags = (h->flags & SDR_PSD_SHIFT) ? SDR_FFT_SHIFT : 0u;  // NORM is applied in f64 at the end
-        fc.device = h->dev;
-        fc.stream = (void *)st;
-        h->plan = sdr_fft_create(&fc, &rc);
-        if (!h->plan) return rc;
-    }
-    for (int i = 0; i < 2; ++i) {
-        rc = h->d_hist[i].reserve(16);
-        if (!rc) rc = h->d_acc[i].reserve((size_t)h->N * sizeof(double));
-        if (rc) return rc;
-    }
-    return cuda_status(cudaStreamSynchronize(st));
-}
-
 extern "C" sdr_psd_t *sdr_psd_create(const sdr_psd_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || cfg->n == 0 || cfg->n > ((size_t)1 << 26) || cfg->hop == 0 || cfg->hop > ((size_t)1 << 40) ||
         cfg->average == 0 || cfg->average > ((size_t)1 << 40) ||
-        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) || (cfg->flags & ~PSD_FLAGS)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    sdr_psd *h = new (std::nothrow) sdr_psd;
-    if (!h) {
-        *err = SDR_ERR_MALLOC_FAILED;
-        return nullptr;
-    }
-    h->dev = cfg->device;
-    h->N = (long long)cfg->n;
-    h->H = (long long)cfg->hop;
-    h->K = (long long)cfg->average;
-    h->cpg = (h->K + PSD_S - 1) / PSD_S;
-    h->fmt = cfg->input_format;
-    h->flags = cfg->flags;
-    h->fused = h->N == 1024 && !(h->flags & SDR_PSD_GENERAL_KERNEL);
-    h->scale = 1.0 / (double)h->K;
-    if (h->flags & SDR_PSD_NORM) h->scale /= (double)h->N;
-    h->taper.assign((size_t)h->N, 1.0f);
-    if (cfg->window) std::memcpy(h->taper.data(), cfg->window, (size_t)h->N * sizeof(float));
-    DeviceGuard g(h->dev);
-    *err = g.ok ? psd_alloc(h, cfg->stream) : g.status();
-    if (*err) { psd_free(h); return nullptr; }
-    return h;
+        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) || (cfg->flags & ~PSD_FLAGS))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_psd>(err, cfg->device, cfg->stream, [&](sdr_psd &h) {
+        h.N = (long long)cfg->n;
+        h.H = (long long)cfg->hop;
+        h.K = (long long)cfg->average;
+        h.cpg = (h.K + PSD_S - 1) / PSD_S;
+        h.fmt = cfg->input_format;
+        h.flags = cfg->flags;
+        h.fused = h.N == 1024 && !(h.flags & SDR_PSD_GENERAL_KERNEL);
+        h.scale = 1.0 / (double)h.K;
+        if (h.flags & SDR_PSD_NORM) h.scale /= (double)h.N;
+        h.taper.assign((size_t)h.N, 1.0f);
+        if (cfg->window) std::memcpy(h.taper.data(), cfg->window, (size_t)h.N * sizeof(float));
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_psd_destroy(sdr_psd_t *h) { psd_free(h); }
+extern "C" void sdr_psd_destroy(sdr_psd_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_psd_reset(sdr_psd_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -387,30 +367,7 @@ extern "C" int sdr_psd_reset(sdr_psd_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_psd_t *sdr_psd_clone(const sdr_psd_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_psd *h = new (std::nothrow) sdr_psd;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->N = src->N; h->H = src->H; h->K = src->K; h->cpg = src->cpg;
-    h->fmt = src->fmt; h->flags = src->flags; h->fused = src->fused; h->scale = src->scale; h->taper = src->taper;
-    h->total = src->total; h->done = src->done; h->hist_lo = src->hist_lo; h->last_path = src->last_path;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? psd_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s) : g.status();
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    const size_t tail = (size_t)(h->total - h->hist_lo) * psd_es(h);
-    if (!*err && tail > 0) {
-        *err = h->d_hist[0].reserve(tail);
-        if (!*err) *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, tail, cudaMemcpyDeviceToDevice));
-    }
-    if (!*err)
-        *err = cuda_status(cudaMemcpy(h->d_acc[0].p, src->d_acc[src->acur].p, (size_t)h->N * sizeof(double),
-                                      cudaMemcpyDeviceToDevice));
-    if (*err) { psd_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_psd_t *sdr_psd_clone(const sdr_psd_t *src, int *err) { return clone_handle<PsdHost>(src, err); }
 
 // spectra that the next n_in samples complete: frame j needs input sample (j + 1) H - 1, group g frames gK .. gK + K - 1
 extern "C" size_t sdr_psd_output_count(const sdr_psd_t *h, size_t n_in) {
@@ -465,7 +422,8 @@ static int psd_run_fused(sdr_psd *h, const PsdSrc &src, long long gid0, long lon
     for (long long gA = gid0; gA < gid1; gA += step) {
         const long long gB = std::min(gid1, gA + step);
         Psd1kArgs a;
-        a.src = src; a.tw = h->d_tw; a.taper = h->d_taper; a.H = h->H; a.K = h->K; a.cpg = h->cpg;
+        a.src = src; a.tw = (const float2 *)h->d_tw.p; a.taper = (const float *)h->d_taper.p;
+        a.H = h->H; a.K = h->K; a.cpg = h->cpg;
         a.gid0 = gA; a.nchunks = gB - gA; a.part = (float *)h->d_part.p;
         a.out = out + (gA - row_base) * (long long)out_stride;  // cpg == 1: chunk gid is group gid
         a.out_stride = (long long)out_stride; a.scale = h->scale;
@@ -497,12 +455,12 @@ static int psd_run_general(sdr_psd *h, const PsdSrc &src, long long gid0, long l
         const long long fA = psd_frame(h, gA), nf = psd_frame(h, gB) - fA;
         dim3 grid((unsigned)((N + 255) / 256), (unsigned)std::min<long long>(nf, 65535));
         if (h->fmt == SDR_FMT_U8IQ)
-            psd_gather_kernel<true><<<grid, 256, 0, st>>>(src, h->d_taper, N, h->H, fA, nf, (float2 *)h->d_x.p);
+            psd_gather_kernel<true><<<grid, 256, 0, st>>>(src, (const float *)h->d_taper.p, N, h->H, fA, nf, (float2 *)h->d_x.p);
         else
-            psd_gather_kernel<false><<<grid, 256, 0, st>>>(src, h->d_taper, N, h->H, fA, nf, (float2 *)h->d_x.p);
+            psd_gather_kernel<false><<<grid, 256, 0, st>>>(src, (const float *)h->d_taper.p, N, h->H, fA, nf, (float2 *)h->d_x.p);
         count_launch();
         rc = launch_status();
-        if (!rc) rc = sdr_fft_exec_dev(h->plan, h->d_x.p, (size_t)nf, (float *)h->d_y.p);
+        if (!rc) rc = sdr_fft_exec_dev(h->plan.get(), h->d_x.p, (size_t)nf, (float *)h->d_y.p);
         if (rc) return rc;
         grid.y = (unsigned)std::min<long long>(gB - gA, 65535);
         psd_accum_kernel<<<grid, 256, 0, st>>>((const float2 *)h->d_y.p, N, fA, gA, gB - gA, h->K, h->cpg, (float *)h->d_part.p);

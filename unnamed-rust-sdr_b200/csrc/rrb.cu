@@ -169,51 +169,38 @@ unsigned long long gcd_ull(unsigned long long a, unsigned long long b) {
 
 }  // namespace
 
-struct sdr_rrb {
+struct RrbHost {
     int dev = 0;
-    StreamRef stream;
     size_t C = 0;
     std::vector<RrbChan> chans;             // reduced ratios, table and history offsets
     std::vector<unsigned long long> total;  // frames seen, per channel
     std::vector<float> tab;                 // every phase-major table
     size_t hist_len = 0;                    // sum of H_k
+};
+
+struct sdr_rrb : RrbHost {
+    StreamRef stream;
     DevBuf d_tab, d_chans, d_call, d_hist[2];
     int cur = 0;
     std::vector<char> call_host;            // tile0 (C + 1) then C RrbCall, uploaded once per call
     DevBuf d_in, d_out;
+
+    int alloc(void *user_stream, const sdr_rrb *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        if ((rc = d_tab.upload(tab.data(), tab.size() * sizeof(float), stream.s))) return rc;
+        if ((rc = d_chans.upload(chans.data(), C * sizeof(RrbChan), stream.s))) return rc;
+        for (int i = 0; i < 2; ++i)
+            if ((rc = d_hist[i].reserve(std::max<size_t>(hist_len, 1) * 8))) return rc;
+        return cuda_status(cudaStreamSynchronize(stream.s));
+    }
+    int copy_device(const sdr_rrb &src) {
+        if (hist_len == 0) return SDR_OK;
+        return cuda_status(cudaMemcpy(d_hist[0].p, src.d_hist[src.cur].p, hist_len * 8, cudaMemcpyDeviceToDevice));
+    }
 };
 
-static void rrb_free(sdr_rrb *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    h->d_tab.release(); h->d_chans.release(); h->d_call.release();
-    h->d_hist[0].release(); h->d_hist[1].release();
-    h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
-
-static int rrb_upload(DevBuf &b, const void *src, size_t bytes, cudaStream_t st) {
-    int rc = b.reserve(std::max<size_t>(bytes, 16));
-    if (rc) return rc;
-    return cuda_status(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st));
-}
-
-static int rrb_alloc(sdr_rrb *h, void *user_stream) {
-    int rc = h->stream.init(user_stream);
-    if (rc) return rc;
-    cudaStream_t st = h->stream.s;
-    if ((rc = rrb_upload(h->d_tab, h->tab.data(), h->tab.size() * sizeof(float), st))) return rc;
-    if ((rc = rrb_upload(h->d_chans, h->chans.data(), h->C * sizeof(RrbChan), st))) return rc;
-    for (int i = 0; i < 2; ++i)
-        if ((rc = h->d_hist[i].reserve(std::max<size_t>(h->hist_len, 1) * 8))) return rc;
-    return cuda_status(cudaStreamSynchronize(st));
-}
-
 extern "C" sdr_rrb_t *sdr_rrb_create(const sdr_rrb_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     bool ok = cfg && cfg->taps && cfg->interpolation && cfg->decimation && cfg->n_taps >= 1 &&
               cfg->n_taps <= RRB_MAX_TAPS && cfg->n_channels >= 1 && cfg->n_channels <= RRB_MAX_CH &&
               (cfg->n_tap_sets == 1 || cfg->n_tap_sets == cfg->n_channels) &&
@@ -221,56 +208,42 @@ extern "C" sdr_rrb_t *sdr_rrb_create(const sdr_rrb_config_t *cfg, int *err) {
     for (size_t k = 0; ok && k < cfg->n_channels; ++k)
         ok = cfg->interpolation[k] >= 1 && cfg->interpolation[k] <= RRB_MAX_I && cfg->decimation[k] >= 1 &&
              cfg->decimation[k] <= RRB_MAX_D;
-    if (!ok) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) { *err = SDR_ERR_INVALID_ARG; return nullptr; }
-    sdr_rrb *h = new (std::nothrow) sdr_rrb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = cfg->device;
-    h->C = cfg->n_channels;
-    h->chans.resize(h->C);
-    h->total.assign(h->C, 0);
-    const size_t L = cfg->n_taps;
-    // one phase-major table per distinct (tap set, I', g)
-    std::map<std::tuple<size_t, size_t, size_t>, long long> tables;
-    for (size_t k = 0; k < h->C; ++k) {
-        const size_t I = cfg->interpolation[k], D = cfg->decimation[k], g = (size_t)gcd_ull(I, D);
-        const size_t Ir = I / g, Lr = (L + g - 1) / g, set = cfg->n_tap_sets == 1 ? 0 : k;
-        RrbChan &ch = h->chans[k];
-        ch.I = (int)Ir;
-        ch.rI = 1.0 / (double)Ir;
-        ch.D = (long long)(D / g);
-        ch.L = (int)Lr;
-        ch.H = (int)((Lr + Ir - 1) / Ir);
-        ch.pad = 0;
-        ch.hist = (long long)h->hist_len;
-        h->hist_len += (size_t)ch.H;
-        const auto key = std::make_tuple(set, Ir, g);
-        auto it = tables.find(key);
-        if (it == tables.end()) {
-            const float *src = cfg->taps + set * L;
-            const long long at = (long long)h->tab.size();
-            for (size_t c = 0; c < Ir; ++c)
-                for (size_t j = c; j < Lr; j += Ir) h->tab.push_back(src[g * j]);
-            it = tables.emplace(key, at).first;
+    if (!ok) return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_rrb>(err, cfg->device, cfg->stream, [&](sdr_rrb &h) {
+        h.C = cfg->n_channels;
+        h.chans.resize(h.C);
+        h.total.assign(h.C, 0);
+        const size_t L = cfg->n_taps;
+        // one phase-major table per distinct (tap set, I', g)
+        std::map<std::tuple<size_t, size_t, size_t>, long long> tables;
+        for (size_t k = 0; k < h.C; ++k) {
+            const size_t I = cfg->interpolation[k], D = cfg->decimation[k], g = (size_t)gcd_ull(I, D);
+            const size_t Ir = I / g, Lr = (L + g - 1) / g, set = cfg->n_tap_sets == 1 ? 0 : k;
+            RrbChan &ch = h.chans[k];
+            ch.I = (int)Ir;
+            ch.rI = 1.0 / (double)Ir;
+            ch.D = (long long)(D / g);
+            ch.L = (int)Lr;
+            ch.H = (int)((Lr + Ir - 1) / Ir);
+            ch.pad = 0;
+            ch.hist = (long long)h.hist_len;
+            h.hist_len += (size_t)ch.H;
+            const auto key = std::make_tuple(set, Ir, g);
+            auto it = tables.find(key);
+            if (it == tables.end()) {
+                const float *src = cfg->taps + set * L;
+                const long long at = (long long)h.tab.size();
+                for (size_t c = 0; c < Ir; ++c)
+                    for (size_t j = c; j < Lr; j += Ir) h.tab.push_back(src[g * j]);
+                it = tables.emplace(key, at).first;
+            }
+            ch.tab = it->second;
         }
-        ch.tab = it->second;
-    }
-    DeviceGuard g(h->dev);
-    *err = g.ok ? rrb_alloc(h, cfg->stream) : g.status();
-    if (*err) { rrb_free(h); return nullptr; }
-    return h;
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_rrb_destroy(sdr_rrb_t *h) { rrb_free(h); }
+extern "C" void sdr_rrb_destroy(sdr_rrb_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_rrb_reset(sdr_rrb_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -280,23 +253,7 @@ extern "C" int sdr_rrb_reset(sdr_rrb_t *h) {
     return SDR_OK;
 }
 
-extern "C" sdr_rrb_t *sdr_rrb_clone(const sdr_rrb_t *src, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
-    if (!src) { *err = SDR_ERR_NULL_HANDLE; return nullptr; }
-    sdr_rrb *h = new (std::nothrow) sdr_rrb;
-    if (!h) { *err = SDR_ERR_MALLOC_FAILED; return nullptr; }
-    h->dev = src->dev; h->C = src->C; h->chans = src->chans; h->total = src->total; h->tab = src->tab;
-    h->hist_len = src->hist_len;
-    DeviceGuard g(h->dev);
-    *err = g.ok ? rrb_alloc(h, src->stream.owned ? nullptr : (void *)src->stream.s) : g.status();
-    if (!*err) *err = cuda_status(cudaStreamSynchronize(src->stream.s));
-    if (!*err && h->hist_len > 0)
-        *err = cuda_status(cudaMemcpy(h->d_hist[0].p, src->d_hist[src->cur].p, h->hist_len * 8, cudaMemcpyDeviceToDevice));
-    if (*err) { rrb_free(h); return nullptr; }
-    return h;
-}
+extern "C" sdr_rrb_t *sdr_rrb_clone(const sdr_rrb_t *src, int *err) { return clone_handle<RrbHost>(src, err); }
 
 static unsigned long long rrb_released(const RrbChan &ch, unsigned long long frames) {
     return (unsigned long long)((unsigned __int128)frames * (unsigned)ch.I / (unsigned long long)ch.D);
@@ -343,8 +300,9 @@ static int rrb_run(sdr_rrb *h, const float2 *in, const size_t *n_in, size_t in_s
     }
     tile0[C] = tiles;
     if (!any) return SDR_OK;
-    int rc = rrb_upload(h->d_call, h->call_host.data(), h->call_host.size(), st);
+    int rc = h->d_call.reserve(h->call_host.size());
     if (rc) return rc;
+    SDR_CUDA_TRY(cudaMemcpyAsync(h->d_call.p, h->call_host.data(), h->call_host.size(), cudaMemcpyHostToDevice, st));
     const long long *d_tile0 = (const long long *)h->d_call.p;
     const RrbCall *d_calls = (const RrbCall *)(d_tile0 + C + 1);
     const long long stride = C > 1 ? (long long)in_stride : 0;

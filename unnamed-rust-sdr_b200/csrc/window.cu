@@ -34,71 +34,50 @@ __global__ void window_gather_kernel(const void *__restrict__ buf, long long bas
 
 }  // namespace
 
-struct sdr_window_fft {
+struct WindowHost {
     int dev = 0;
-    StreamRef stream;
     size_t N = 0, D = 0;
     int fmt = SDR_FMT_C64;
-    sdr_fft_t *plan = nullptr;
+    unsigned fft_flags = 0;
     long long total = 0;  // input samples seen
     long long kept = 0;   // history samples in d_buf (stream indices total - kept .. total - 1)
     long long emitted = 0;  // windows emitted so far
-    DevBuf d_buf[2], d_win, d_in, d_out;
-    int cur = 0;
 };
 
-static void wf_free(sdr_window_fft *h) {
-    if (!h) return;
-    DeviceGuard g(h->dev);
-    if (h->plan) sdr_fft_destroy(h->plan);
-    h->d_buf[0].release(); h->d_buf[1].release(); h->d_win.release(); h->d_in.release(); h->d_out.release();
-    h->stream.release();
-    delete h;
-}
+struct sdr_window_fft : WindowHost {
+    StreamRef stream;
+    Owned<sdr_fft_t, sdr_fft_destroy> plan;
+    DevBuf d_buf[2], d_win, d_in, d_out;
+    int cur = 0;
+
+    int alloc(void *user_stream, const sdr_window_fft *) {
+        int rc = stream.init(user_stream);
+        if (rc) return rc;
+        sdr_fft_config_t fc;
+        fc.n = N;
+        fc.input_format = SDR_FMT_C64;  // the gather unpacks
+        fc.flags = fft_flags;
+        fc.device = dev;
+        fc.stream = (void *)stream.s;
+        plan.reset(sdr_fft_create(&fc, &rc));
+        return plan ? SDR_OK : rc;
+    }
+};
 
 extern "C" sdr_window_fft_t *sdr_window_fft_create(const sdr_window_fft_config_t *cfg, int *err) {
-    int dummy;
-    if (!err) err = &dummy;
-    *err = SDR_OK;
     if (!cfg || cfg->window == 0 || cfg->hop == 0 || cfg->window > ((size_t)1 << 26) ||
-        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) || (cfg->flags & SDR_FFT_RFFT)) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        *err = SDR_ERR_NO_DEVICE;
-        return nullptr;
-    }
-    if (cfg->device < 0 || cfg->device >= ndev) {
-        *err = SDR_ERR_INVALID_ARG;
-        return nullptr;
-    }
-    sdr_window_fft *h = new (std::nothrow) sdr_window_fft;
-    if (!h) {
-        *err = SDR_ERR_MALLOC_FAILED;
-        return nullptr;
-    }
-    h->dev = cfg->device;
-    h->N = cfg->window;
-    h->D = cfg->hop;
-    h->fmt = cfg->input_format;
-    DeviceGuard g(h->dev);
-    int rc = g.ok ? h->stream.init(cfg->stream) : g.status();
-    if (rc) { *err = rc; wf_free(h); return nullptr; }
-    sdr_fft_config_t fc;
-    fc.n = h->N;
-    fc.input_format = SDR_FMT_C64;  // the gather unpacks
-    fc.flags = cfg->flags;
-    fc.device = h->dev;
-    fc.stream = (void *)h->stream.s;
-    h->plan = sdr_fft_create(&fc, &rc);
-    if (!h->plan) { *err = rc; wf_free(h); return nullptr; }
-    return h;
+        (cfg->input_format != SDR_FMT_U8IQ && cfg->input_format != SDR_FMT_C64) || (cfg->flags & SDR_FFT_RFFT))
+        return fail(err, SDR_ERR_INVALID_ARG);
+    return create_handle<sdr_window_fft>(err, cfg->device, cfg->stream, [&](sdr_window_fft &h) {
+        h.N = cfg->window;
+        h.D = cfg->hop;
+        h.fmt = cfg->input_format;
+        h.fft_flags = cfg->flags;
+        return SDR_OK;
+    });
 }
 
-extern "C" void sdr_window_fft_destroy(sdr_window_fft_t *h) { wf_free(h); }
+extern "C" void sdr_window_fft_destroy(sdr_window_fft_t *h) { destroy_handle(h); }
 
 extern "C" int sdr_window_fft_reset(sdr_window_fft_t *h) {
     if (!h) return SDR_ERR_NULL_HANDLE;
@@ -147,7 +126,7 @@ static int wf_run(sdr_window_fft *h, const void *in, size_t n_in, float *d_out, 
             rc = launch_status();
             if (rc) return rc;
         }
-        rc = sdr_fft_exec_dev(h->plan, h->d_win.p, nw, d_out);
+        rc = sdr_fft_exec_dev(h->plan.get(), h->d_win.p, nw, d_out);
         if (rc) return rc;
     }
     // keep the last N - 1 samples as history for the windows still to come

@@ -48,6 +48,23 @@ inline void check(int rc, const char *what) {
     if (rc != SDR_OK) throw Error(rc, what);
 }
 
+// Owner of one ABI handle for the mirror classes: a move transfers it, a copy clones it (its stream state included)
+// and destruction destroys it.
+template <class T, void (*Destroy)(T *), T *(*Clone)(const T *, int *)>
+class Handle {
+  protected:
+    T *h_ = nullptr;
+    Handle() = default;
+    Handle(Handle &&o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+    Handle(const Handle &o) {
+        int err = 0;
+        h_ = Clone(o.h_, &err);
+        if (!h_) throw Error(err, "clone");
+    }
+    Handle &operator=(const Handle &) = delete;
+    ~Handle() { Destroy(h_); }
+};
+
 template <class A> struct SampleTraits;
 template <> struct SampleTraits<float> { static constexpr int fmt = SDR_FMT_F32; static constexpr int channels = 1; };
 template <> struct SampleTraits<Complex> { static constexpr int fmt = SDR_FMT_C64; static constexpr int channels = 2; };
@@ -129,10 +146,8 @@ namespace filter {
 // Fir<C,A> (src/filter/fir.rs:7-33).  C in {float, Complex}; A in {float, Complex}; also usable with
 // input_u8iq = true, where the samples arrive as rtl_tcp bytes and are unpacked on the GPU.
 template <class C, class A>
-class Fir {
-    sdr_fir_t *h_ = nullptr;
+class Fir : public Handle<sdr_fir_t, sdr_fir_destroy, sdr_fir_clone> {
     std::vector<C> coef_;
-    explicit Fir(sdr_fir_t *h, std::vector<C> c) : h_(h), coef_(std::move(c)) {}
 
   public:
     explicit Fir(std::vector<C> coef, size_t decimation = 1, bool input_u8iq = false, unsigned flags = 0)
@@ -153,13 +168,6 @@ class Fir {
         h_ = sdr_fir_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Fir::new");
     }
-    Fir(Fir &&o) noexcept : h_(o.h_), coef_(std::move(o.coef_)) { o.h_ = nullptr; }
-    Fir(const Fir &o) : coef_(o.coef_) {  // #[derive(Clone)] (fir.rs:6)
-        int err = 0;
-        h_ = sdr_fir_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Fir::clone");
-    }
-    ~Fir() { sdr_fir_destroy(h_); }
 
     // block form of Filter::apply: out gets one element per kept input (all of them when decimation == 1)
     void process(const void *in, size_t n_in, std::vector<A> &out) {
@@ -180,8 +188,7 @@ class Fir {
 
 // Polyphase filter bank behind sdr_pfb_*: channel k is Fir<Complex, Complex>(h[n] e^{+2 pi i k n / M}) followed by
 // Decimate(D), for k = 0..M-1, computed in one pass over the input.  flags: SDR_PFB_SHIFT, SDR_PFB_CHANNEL_MAJOR.
-class Pfb {
-    sdr_pfb_t *h_ = nullptr;
+class Pfb : public Handle<sdr_pfb_t, sdr_pfb_destroy, sdr_pfb_clone> {
     size_t m_ = 0;
     bool cmajor_ = false;
 
@@ -200,14 +207,6 @@ class Pfb {
         h_ = sdr_pfb_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Pfb::new");
     }
-    Pfb(Pfb &&o) noexcept : h_(o.h_), m_(o.m_), cmajor_(o.cmajor_) { o.h_ = nullptr; }
-    Pfb(const Pfb &o) : m_(o.m_), cmajor_(o.cmajor_) {
-        int err = 0;
-        h_ = sdr_pfb_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Pfb::clone");
-    }
-    Pfb &operator=(const Pfb &) = delete;
-    ~Pfb() { sdr_pfb_destroy(h_); }
     size_t channels() const { return m_; }
     size_t output_count(size_t n_in) const { return sdr_pfb_output_count(h_, n_in); }
     // in: n samples (Complex, or 2n bytes when constructed with input_u8iq).  out: frames x M (or M x frames when
@@ -227,8 +226,7 @@ class Pfb {
 // Polyphase synthesis bank behind sdr_pfs_*, the inverse of Pfb: channel k is zero-stuffed by D (sample m at index
 // (m+1) D - 1), filtered by Fir<Complex, Complex>(f[n] e^{+2 pi i k n / M}) and summed over k; n frames give n D
 // samples.  flags: SDR_PFS_SHIFT, SDR_PFS_CHANNEL_MAJOR take the layouts Pfb writes with the matching flags.
-class Pfs {
-    sdr_pfs_t *h_ = nullptr;
+class Pfs : public Handle<sdr_pfs_t, sdr_pfs_destroy, sdr_pfs_clone> {
     size_t m_ = 0;
     bool cmajor_ = false;
 
@@ -245,14 +243,6 @@ class Pfs {
         h_ = sdr_pfs_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Pfs::new");
     }
-    Pfs(Pfs &&o) noexcept : h_(o.h_), m_(o.m_), cmajor_(o.cmajor_) { o.h_ = nullptr; }
-    Pfs(const Pfs &o) : m_(o.m_), cmajor_(o.cmajor_) {
-        int err = 0;
-        h_ = sdr_pfs_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Pfs::clone");
-    }
-    Pfs &operator=(const Pfs &) = delete;
-    ~Pfs() { sdr_pfs_destroy(h_); }
     size_t channels() const { return m_; }
     size_t output_count(size_t n_frames) const { return sdr_pfs_output_count(h_, n_frames); }
     // in: n_frames frames of M (or M rows of n_frames when channel-major).  out: n_frames * D samples, replaced.
@@ -272,8 +262,7 @@ class Pfs {
 // Down-converter bank behind sdr_ddc_*: channel k is a tee'd copy of the stream mixed down by a 64-bit NCO
 // (sdr_ddc_phase_increment(freq[k], rate)), Fir<Complex, f32>(h_k) and Decimate(D), computed in one pass over the input.
 // taps: one row of L (shared) or channels rows of L.  Output: channels rows of outputs (channel-major).
-class Ddc {
-    sdr_ddc_t *h_ = nullptr;
+class Ddc : public Handle<sdr_ddc_t, sdr_ddc_destroy, sdr_ddc_clone> {
     size_t c_ = 0;
 
   public:
@@ -296,14 +285,6 @@ class Ddc {
         h_ = sdr_ddc_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Ddc::new");
     }
-    Ddc(Ddc &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
-    Ddc(const Ddc &o) : c_(o.c_) {
-        int err = 0;
-        h_ = sdr_ddc_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Ddc::clone");
-    }
-    Ddc &operator=(const Ddc &) = delete;
-    ~Ddc() { sdr_ddc_destroy(h_); }
     size_t channels() const { return c_; }
     size_t output_count(size_t n_in) const { return sdr_ddc_output_count(h_, n_in); }
     int last_path() const { return sdr_ddc_last_path(h_); }
@@ -324,8 +305,7 @@ class Ddc {
 // (m+1) I - 1), filtered by Fir<f32, Complex>(h_k), mixed up by a 64-bit NCO (sdr_ddc_phase_increment(freq[k], rate))
 // and the channels are summed.  taps: one row of L (shared) or channels rows of L.  Input: channels rows of frames
 // (channel-major, as Ddc writes them); n frames give n I samples.
-class Duc {
-    sdr_duc_t *h_ = nullptr;
+class Duc : public Handle<sdr_duc_t, sdr_duc_destroy, sdr_duc_clone> {
     size_t c_ = 0;
 
   public:
@@ -346,14 +326,6 @@ class Duc {
         h_ = sdr_duc_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Duc::new");
     }
-    Duc(Duc &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
-    Duc(const Duc &o) : c_(o.c_) {
-        int err = 0;
-        h_ = sdr_duc_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Duc::clone");
-    }
-    Duc &operator=(const Duc &) = delete;
-    ~Duc() { sdr_duc_destroy(h_); }
     size_t channels() const { return c_; }
     size_t output_count(size_t n_frames) const { return sdr_duc_output_count(h_, n_frames); }
     // in: channels rows of n_frames, row stride in_stride (>= n_frames).  out: n_frames * I samples, replaced.
@@ -372,8 +344,7 @@ class Duc {
 
 // Fast-convolution channel bank (sdr_fcfb): Ddc's channels with one decimation per channel, computed by overlap-save.
 // Outputs are released per block of P inputs (sdr_fcfb_geometry); feed N zeros to drain a finite stream.
-class Fcfb {
-    sdr_fcfb_t *h_ = nullptr;
+class Fcfb : public Handle<sdr_fcfb_t, sdr_fcfb_destroy, sdr_fcfb_clone> {
     size_t c_ = 0;
 
   public:
@@ -396,14 +367,6 @@ class Fcfb {
         h_ = sdr_fcfb_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Fcfb::new");
     }
-    Fcfb(Fcfb &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
-    Fcfb(const Fcfb &o) : c_(o.c_) {
-        int err = 0;
-        h_ = sdr_fcfb_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Fcfb::clone");
-    }
-    Fcfb &operator=(const Fcfb &) = delete;
-    ~Fcfb() { sdr_fcfb_destroy(h_); }
     size_t channels() const { return c_; }
     std::vector<size_t> output_count(size_t n_in) const {
         std::vector<size_t> cnt(c_);
@@ -427,8 +390,7 @@ class Fcfb {
 // computed by overlap-save.  A call advances by n_time output positions (a multiple of lcm(I_k); row k holds
 // n_time / I_k frames) and returns the outputs of the blocks it completes; feed zero frames covering N positions to
 // drain a finite stream.
-class Fcsb {
-    sdr_fcsb_t *h_ = nullptr;
+class Fcsb : public Handle<sdr_fcsb_t, sdr_fcsb_destroy, sdr_fcsb_clone> {
     size_t c_ = 0;
 
   public:
@@ -450,14 +412,6 @@ class Fcsb {
         h_ = sdr_fcsb_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Fcsb::new");
     }
-    Fcsb(Fcsb &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
-    Fcsb(const Fcsb &o) : c_(o.c_) {
-        int err = 0;
-        h_ = sdr_fcsb_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Fcsb::clone");
-    }
-    Fcsb &operator=(const Fcsb &) = delete;
-    ~Fcsb() { sdr_fcsb_destroy(h_); }
     size_t channels() const { return c_; }
     size_t output_count(size_t n_time) const { return sdr_fcsb_output_count(h_, n_time); }
     // in: channels rows, row k = n_time / I_k frames, row stride in_stride (>= the longest row).  out: replaced.
@@ -476,8 +430,7 @@ class Fcsb {
 
 // Rational resampler bank (sdr_rrb): channel k zero-stuffed by I_k, filtered by its real taps and decimated by D_k
 // (upfirdn).  After n frames a channel has released floor(n I_k / D_k) outputs; there is no scale (taps carry I_k).
-class Rrb {
-    sdr_rrb_t *h_ = nullptr;
+class Rrb : public Handle<sdr_rrb_t, sdr_rrb_destroy, sdr_rrb_clone> {
     size_t c_ = 0;
 
   public:
@@ -496,14 +449,6 @@ class Rrb {
         h_ = sdr_rrb_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "Rrb::new");
     }
-    Rrb(Rrb &&o) noexcept : h_(o.h_), c_(o.c_) { o.h_ = nullptr; }
-    Rrb(const Rrb &o) : c_(o.c_) {
-        int err = 0;
-        h_ = sdr_rrb_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Rrb::clone");
-    }
-    Rrb &operator=(const Rrb &) = delete;
-    ~Rrb() { sdr_rrb_destroy(h_); }
     size_t channels() const { return c_; }
     std::vector<size_t> output_count(const std::vector<size_t> &n_in) const {
         std::vector<size_t> cnt(c_);
@@ -539,8 +484,7 @@ struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
 
 // Biquad<f32, A> (biquad.rs:5-71) as a block stream filter; BiquadD::design(rate) (biquad.rs:83-154) builds it
 template <class A>
-class Biquad {
-    sdr_biquad_t *h_ = nullptr;
+class Biquad : public Handle<sdr_biquad_t, sdr_biquad_destroy, sdr_biquad_clone> {
 
   public:
     Biquad(const BiquadD &d, float rate) {
@@ -554,13 +498,6 @@ class Biquad {
         h_ = sdr_biquad_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "BiquadD::design");
     }
-    Biquad(Biquad &&o) noexcept : h_(o.h_) { o.h_ = nullptr; }
-    Biquad(const Biquad &o) {
-        int err = 0;
-        h_ = sdr_biquad_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Biquad::clone");
-    }
-    ~Biquad() { sdr_biquad_destroy(h_); }
     void process(const A *in, size_t n, std::vector<A> &out) {
         out.resize(n);
         check(sdr_biquad_process(h_, reinterpret_cast<const float *>(in), n, n, reinterpret_cast<float *>(out.data()), n),
@@ -578,8 +515,7 @@ struct PllDesign {  // pll.rs:4-36
     Pll design(float rate) const;  // FilterDesign::design (pll.rs:48-60)
 };
 
-class Pll {  // pll.rs:13-85 ; Output = Option<f32>
-    sdr_pll_t *h_ = nullptr;
+class Pll : public Handle<sdr_pll_t, sdr_pll_destroy, sdr_pll_clone> {  // pll.rs:13-85 ; Output = Option<f32>
 
   public:
     Pll(const PllDesign &d, float rate, unsigned flags = 0) {
@@ -594,13 +530,6 @@ class Pll {  // pll.rs:13-85 ; Output = Option<f32>
         h_ = sdr_pll_create(&cfg, &err);
         if (!h_) throw sdr::Error(err, "PllDesign::design");
     }
-    Pll(Pll &&o) noexcept : h_(o.h_) { o.h_ = nullptr; }
-    Pll(const Pll &o) {
-        int err = 0;
-        h_ = sdr_pll_clone(o.h_, &err);
-        if (!h_) throw sdr::Error(err, "Pll::clone");
-    }
-    ~Pll() { sdr_pll_destroy(h_); }
     void process(const Complex *in, size_t n, std::vector<std::optional<float>> &out) {
         std::vector<float> v(n);
         std::vector<uint8_t> lk(n);
@@ -1082,8 +1011,7 @@ class WindowSpectra {
 // window -> decimate -> map(fft::fft) -> |.|^2 -> mean of `average` behind sdr_psd_*: feed blocks of samples, get the
 // averaged power spectra (n floats each, bins shifted like fft::fft, scaled 1/n like its 1/sqrt(n)) back to back.
 // taper: n real values or empty (rectangular).  Copies with sdr_psd_clone.
-class PowerSpectra {
-    sdr_psd_t *h_ = nullptr;
+class PowerSpectra : public Handle<sdr_psd_t, sdr_psd_destroy, sdr_psd_clone> {
     size_t n_ = 0;
 
   public:
@@ -1102,13 +1030,6 @@ class PowerSpectra {
         h_ = sdr_psd_create(&cfg, &err);
         if (!h_) throw Error(err, "PowerSpectra::new");
     }
-    PowerSpectra(const PowerSpectra &o) : n_(o.n_) {
-        int err = 0;
-        h_ = sdr_psd_clone(o.h_, &err);
-        if (!h_) throw Error(err, "PowerSpectra::clone");
-    }
-    PowerSpectra &operator=(const PowerSpectra &) = delete;
-    ~PowerSpectra() { sdr_psd_destroy(h_); }
     size_t bins() const { return n_; }
     int last_path() const { return sdr_psd_last_path(h_); }
     // in: n samples (Complex, or 2n bytes when constructed with u8iq); returns the number of spectra appended to out

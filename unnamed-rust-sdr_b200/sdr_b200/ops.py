@@ -80,16 +80,54 @@ _FMT_OF = {"u8iq": F.FMT_U8IQ, "c64": F.FMT_C64, "f32": F.FMT_F32}
 _IN_DTYPE = {F.FMT_U8IQ: np.uint8, F.FMT_C64: np.complex64, F.FMT_F32: np.float32}
 
 
-class Fir:
+class _Handle:
+    """Owner of one C handle of the ABI family sdr_<_abi>_*: create, clone, reset and destroy."""
+    _abi = None
+    h = None
+
+    def _fn(self, verb):
+        return getattr(lib(), "sdr_%s_%s" % (self._abi, verb))
+
+    def _create(self, cfg):
+        err = C.c_int(0)
+        self.h = self._fn("create")(C.byref(cfg), C.byref(err))
+        if not self.h:
+            raise SdrError(err.value, "sdr_%s_create" % self._abi)
+
+    def _adopt(self, h):
+        """a copy of this object that owns handle h"""
+        other = object.__new__(type(self))
+        other.__dict__.update(self.__dict__)
+        other.h = h
+        return other
+
+    def clone(self):
+        err = C.c_int(0)
+        h = self._fn("clone")(self.h, C.byref(err))
+        if not h:
+            raise SdrError(err.value, "sdr_%s_clone" % self._abi)
+        return self._adopt(h)
+
+    def reset(self):
+        check(self._fn("reset")(self.h), "sdr_%s_reset" % self._abi)
+
+    def close(self):
+        if self.h:
+            self._fn("destroy")(self.h)
+            self.h = None
+
+    def __del__(self):
+        self.close()
+
+
+class Fir(_Handle):
     """filter::Fir<C,A> with the signal::Filter (+ optional signal::Decimate) adaptor behaviour:
     a stateful stream filter.  taps float32 -> Fir<f32,A>; complex64 -> Fir<Complex<f32>,Complex<f32>>."""
 
+    _abi = "fir"
+
     def __init__(self, taps, input_format="c64", decimation=1, n_channels=1, strict=False, device=0,
-                 stream=None, flags=0, _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+                 stream=None, flags=0):
         taps = np.asarray(taps)
         self.taps_complex = int(np.iscomplexobj(taps))
         self._taps = np.ascontiguousarray(taps, np.complex64 if self.taps_complex else np.float32)
@@ -100,10 +138,7 @@ class Fir:
         flags = int(flags) | (F.FIR_STRICT_ORDER if strict else 0)
         cfg = F.FirConfig(self._taps.ctypes.data, self._taps.size, self.taps_complex, self.fmt, self.decimation,
                           self.n_channels, flags, device, _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_fir_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_fir_create")
+        self._create(cfg)
 
     @property
     def out_dtype(self):
@@ -132,27 +167,10 @@ class Fir:
                                         out_stride or out_cap, C.byref(used), C.byref(got)), "sdr_fir_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_fir_reset(self.h), "sdr_fir_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_fir_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_fir_clone")
-        meta = {k: v for k, v in self.__dict__.items() if k != "h"}
-        return Fir(None, _handle=h, _meta=meta)
-
     @property
     def last_path(self):
         return lib().sdr_fir_last_path(self.h)
 
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_fir_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
 class FftPlan:
@@ -249,15 +267,13 @@ class BiquadD:
 Identity = BiquadD.Identity
 
 
-class Biquad:
+class Biquad(_Handle):
     """filter::Biquad<f32, A> as a stream filter (biquad.rs:40-56): n_streams independent streams of f32 or
     Complex<f32> samples; designs = one BiquadD shared by all streams, or one per stream."""
 
-    def __init__(self, designs, rate, n_streams=1, complex_samples=False, device=0, stream=None, _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+    _abi = "biquad"
+
+    def __init__(self, designs, rate, n_streams=1, complex_samples=False, device=0, stream=None):
         if isinstance(designs, BiquadD):
             designs = [designs]
         self.n_streams, self.complex_samples = int(n_streams), bool(complex_samples)
@@ -265,10 +281,7 @@ class Biquad:
         self._arr = arr
         cfg = F.BiquadConfig(C.cast(arr, C.c_void_p), len(designs), self.n_streams, rate, int(self.complex_samples),
                              device, _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_biquad_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_biquad_create")
+        self._create(cfg)
 
     def process(self, x):
         dt = np.complex64 if self.complex_samples else np.float32
@@ -283,22 +296,6 @@ class Biquad:
         check(lib().sdr_biquad_process_dev(self.h, _ptr(d_in), n, in_stride or n, _ptr(d_out), out_stride or n),
               "sdr_biquad_process_dev")
 
-    def reset(self):
-        check(lib().sdr_biquad_reset(self.h), "sdr_biquad_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_biquad_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_biquad_clone")
-        return Biquad(None, 0, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k not in ("h", "_arr")})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_biquad_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
 class PllDesign:
@@ -315,24 +312,20 @@ class PllDesign:
         return PllBatch([self], n_streams, rate, **kw)
 
 
-class PllBatch:
+class PllBatch(_Handle):
     """n_streams independent filter::Pll instances (pll.rs:13-85)."""
 
-    def __init__(self, designs, n_streams, rate, fast_math=True, device=0, stream=None, _handle=None, general=False):
+    _abi = "pll"
+
+    def __init__(self, designs, n_streams, rate, fast_math=True, device=0, stream=None, general=False):
         self.n_streams = int(n_streams)
-        if _handle is not None:
-            self.h = _handle
-            return
         arr = (F.PllDesign * len(designs))(*[d._c() for d in designs])
         self._arr = arr
         cfg = F.PllConfig(C.cast(arr, C.c_void_p), len(designs), self.n_streams, rate,
                           (0 if fast_math else F.PLL_F64_MATH) | (F.PLL_GENERAL_KERNEL if general else 0), device,
                           _stream_ptr(stream))
         self._cfg = cfg
-        err = C.c_int(0)
-        self.h = lib().sdr_pll_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_pll_create")
+        self._create(cfg)
 
     def process(self, x):
         """x: complex64 [n] or [n_streams, n] -> (out f32, locked u8) of the same shape."""
@@ -370,22 +363,6 @@ class PllBatch:
         check(lib().sdr_pll_get_state(self.h, idx, C.byref(a), C.byref(b), C.byref(c)), "sdr_pll_get_state")
         return a.value, complex(b.value, c.value)
 
-    def reset(self):
-        check(lib().sdr_pll_reset(self.h), "sdr_pll_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_pll_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_pll_clone")
-        return PllBatch(None, self.n_streams, 0.0, _handle=h)
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_pll_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
 class WindowFft:
@@ -437,18 +414,16 @@ class WindowFft:
     __del__ = close
 
 
-class Pfb:
+class Pfb(_Handle):
     """Polyphase filter bank: one wideband stream -> n_channels channels decimated by `decimation`.  Channel k is
     Fir(h * exp(+2j pi k n / M)) followed by Decimate(D); channel k is centred on k * rate / M.  shift=True orders the
     channels like fft::fft's shift (row i = channel (i - M/2) mod M); channel_major=True returns [M, frames] instead of
     [frames, M].  general=True forces the general front-end kernel (same bits)."""
 
+    _abi = "pfb"
+
     def __init__(self, taps, n_channels, decimation, input_format="c64", shift=False, channel_major=False,
-                 general=False, device=0, stream=None, _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+                 general=False, device=0, stream=None):
         self._taps = np.ascontiguousarray(taps, np.float32)
         self.n_channels = int(n_channels)
         self.decimation = int(decimation)
@@ -458,10 +433,7 @@ class Pfb:
             (F.PFB_GENERAL_KERNEL if general else 0)
         cfg = F.PfbConfig(self._taps.ctypes.data, self._taps.size, self.n_channels, self.decimation, self.fmt, flags,
                           device, _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_pfb_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_pfb_create")
+        self._create(cfg)
 
     def output_count(self, n_in):
         return lib().sdr_pfb_output_count(self.h, n_in)
@@ -493,22 +465,6 @@ class Pfb:
               "sdr_pfb_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_pfb_reset(self.h), "sdr_pfb_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_pfb_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_pfb_clone")
-        return Pfb(None, 0, 0, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_pfb_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
 def ddc_phase_increment(freq, rate):
@@ -517,7 +473,7 @@ def ddc_phase_increment(freq, rate):
     return int(lib().sdr_ddc_phase_increment(float(freq), float(rate)))
 
 
-class Pfs:
+class Pfs(_Handle):
     """Polyphase synthesis filter bank, the inverse of Pfb: frames of n_channels channel samples -> one stream at
     `interpolation` (D) samples per frame.  Channel k is zero-stuffed by D (sample m at index (m+1) D - 1), filtered by
     Fir(f * exp(+2j pi k n / M)) and summed over k; frame m releases outputs [m D, (m+1) D).  There is no scale: for
@@ -525,12 +481,10 @@ class Pfs:
     same flags ([frames, M] with row i = channel (i - M/2) mod M, or [M, frames]).  general=True forces the general
     back-end kernel (same bits)."""
 
+    _abi = "pfs"
+
     def __init__(self, taps, n_channels, interpolation, shift=False, channel_major=False, general=False, device=0,
-                 stream=None, _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+                 stream=None):
         self._taps = np.ascontiguousarray(taps, np.float32)
         self.n_channels = int(n_channels)
         self.interpolation = int(interpolation)
@@ -539,10 +493,7 @@ class Pfs:
             (F.PFS_GENERAL_KERNEL if general else 0)
         cfg = F.PfsConfig(self._taps.ctypes.data, self._taps.size, self.n_channels, self.interpolation, flags, device,
                           _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_pfs_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_pfs_create")
+        self._create(cfg)
 
     def output_count(self, n_frames):
         return lib().sdr_pfs_output_count(self.h, n_frames)
@@ -572,37 +523,19 @@ class Pfs:
               "sdr_pfs_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_pfs_reset(self.h), "sdr_pfs_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_pfs_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_pfs_clone")
-        return Pfs(None, 0, 0, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_pfs_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
-class Ddc:
+class Ddc(_Handle):
     """Digital down-converter bank: channel k of one IQ stream is mixed down by freqs[k] (a 64-bit NCO), filtered by its
     real taps (taps 1-D: shared; [C, L]: one row per channel) and decimated by `decimation`:
     y_k[m] = sum_j h_k[j] x[N - j] e^{-2 pi i phi_k(N - j)}, N = (m + 1) D - 1.  first_sample = absolute stream index of
     the first input (places the NCO phase only).  process returns complex64 [C, outputs] (channel-major rows).
     general=True forces the CUDA-core kernel."""
 
+    _abi = "ddc"
+
     def __init__(self, taps, freqs, rate, decimation, input_format="u8iq", first_sample=0, general=False, device=0,
-                 stream=None, _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+                 stream=None):
         t = np.ascontiguousarray(taps, np.float32)
         if t.ndim not in (1, 2):
             raise ValueError("taps must be 1-D (shared) or [channels, taps]")
@@ -614,10 +547,7 @@ class Ddc:
         cfg = F.DdcConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
                           self.n_channels, self.decimation, int(first_sample), self.fmt,
                           F.DDC_GENERAL_KERNEL if general else 0, device, _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_ddc_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_ddc_create")
+        self._create(cfg)
 
     def output_count(self, n_in):
         return lib().sdr_ddc_output_count(self.h, n_in)
@@ -651,25 +581,9 @@ class Ddc:
               "sdr_ddc_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_ddc_reset(self.h), "sdr_ddc_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_ddc_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_ddc_clone")
-        return Ddc(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_ddc_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
-class Duc:
+class Duc(_Handle):
     """Digital up-converter bank, the transpose of Ddc: channel k (row k of a [C, n] complex64 array) is zero-stuffed
     by `interpolation` (I; sample m at index (m+1) I - 1), filtered by its real taps (1-D: shared; [C, L]: one row
     per channel), mixed UP by freqs[k] (a 64-bit NCO) and all channels are summed:
@@ -677,12 +591,9 @@ class Duc:
     OUTPUT (places the NCO phase only).  Frame m releases outputs [m I, (m+1) I).  There is no scale: for unit
     round-trip gain after Ddc the taps carry the factor I, and first_sample is the Ddc's minus the cascade's delay."""
 
-    def __init__(self, taps, freqs, rate, interpolation, first_sample=0, device=0, stream=None, _handle=None,
-                 _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+    _abi = "duc"
+
+    def __init__(self, taps, freqs, rate, interpolation, first_sample=0, device=0, stream=None):
         t = np.ascontiguousarray(taps, np.float32)
         if t.ndim not in (1, 2):
             raise ValueError("taps must be 1-D (shared) or [channels, taps]")
@@ -693,10 +604,7 @@ class Duc:
         cfg = F.DucConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
                           self.n_channels, self.interpolation, int(first_sample) % (1 << 64), 0, device,
                           _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_duc_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_duc_create")
+        self._create(cfg)
 
     def output_count(self, n_frames):
         return lib().sdr_duc_output_count(self.h, n_frames)
@@ -724,37 +632,19 @@ class Duc:
                                         _ptr(d_out), out_cap, C.byref(got)), "sdr_duc_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_duc_reset(self.h), "sdr_duc_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_duc_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_duc_clone")
-        return Duc(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_duc_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
-class Psd:
+class Psd(_Handle):
     """Averaged power spectra (sdr_psd): window(n) -> decimate(hop) -> map(fft::fft) -> |.|^2 -> mean of `average`
     frames.  Frame j holds the n samples ending at input sample (j + 1) * hop - 1 (x[<0] = 0), tapered by `window`
     (n real values, None = rectangular); spectrum g is the mean of |X_j|^2 over frames g*average .. g*average +
     average - 1, as float32 rows of n bins.  shift / norm as for FftPlan (norm scales the rows by 1/n).  average=1 is a
     waterfall.  general=True forces the plan + slab path (path 1) where the fused 1024-point kernel (path 2) would run."""
 
+    _abi = "psd"
+
     def __init__(self, n, hop, average, window=None, fmt="u8iq", shift=True, norm=True, general=False, device=0,
-                 stream=None, _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+                 stream=None):
         self.n, self.hop, self.average = int(n), int(hop), int(average)
         self.fmt = _FMT_OF[fmt] if isinstance(fmt, str) else int(fmt)
         self._window = None if window is None else np.ascontiguousarray(window, np.float32)
@@ -763,10 +653,7 @@ class Psd:
         flags = (F.PSD_SHIFT if shift else 0) | (F.PSD_NORM if norm else 0) | (F.PSD_GENERAL_KERNEL if general else 0)
         cfg = F.PsdConfig(self.n, self.hop, self.average, None if self._window is None else self._window.ctypes.data,
                           self.fmt, flags, device, _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_psd_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_psd_create")
+        self._create(cfg)
 
     def output_count(self, n_in):
         return lib().sdr_psd_output_count(self.h, n_in)
@@ -800,22 +687,6 @@ class Psd:
               "sdr_psd_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_psd_reset(self.h), "sdr_psd_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_psd_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_psd_clone")
-        return Psd(None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_psd_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
 def fcfb_geometry(n_taps, decimations):
@@ -826,19 +697,16 @@ def fcfb_geometry(n_taps, decimations):
     return n.value, p.value
 
 
-class Fcfb:
+class Fcfb(_Handle):
     """Fast-convolution channel bank (sdr_fcfb): channel k of one IQ stream is mixed down by freqs[k] (a 64-bit NCO),
     filtered by its real taps (taps 1-D: shared; [C, L]: one row per channel) and decimated by decimation[k] (one value
     or one per channel) -- sdr_ddc's channel with its own D -- computed by overlap-save on blocks of N inputs.  Outputs
     are released per block of P inputs (see geometry); process returns a list of C complex64 arrays.  To drain a finite
     stream feed N zeros and drop the outputs past its end."""
 
-    def __init__(self, taps, freqs, rate, decimation, input_format="u8iq", first_sample=0, device=0, stream=None,
-                 _handle=None, _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+    _abi = "fcfb"
+
+    def __init__(self, taps, freqs, rate, decimation, input_format="u8iq", first_sample=0, device=0, stream=None):
         t = np.ascontiguousarray(taps, np.float32)
         if t.ndim not in (1, 2):
             raise ValueError("taps must be 1-D (shared) or [channels, taps]")
@@ -855,10 +723,7 @@ class Fcfb:
         cfg = F.FcfbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
                            self.decimation.ctypes.data, self.n_channels, int(first_sample), self.fmt, device,
                            _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_fcfb_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_fcfb_create")
+        self._create(cfg)
 
     @property
     def geometry(self):
@@ -895,25 +760,9 @@ class Fcfb:
               "sdr_fcfb_process_dev")
         return got.astype(np.int64)
 
-    def reset(self):
-        check(lib().sdr_fcfb_reset(self.h), "sdr_fcfb_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_fcfb_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_fcfb_clone")
-        return Fcfb(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_fcfb_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
-class Fcsb:
+class Fcsb(_Handle):
     """Fast-convolution synthesis bank (sdr_fcsb), the inverse of Fcfb: channel k is zero-stuffed by interpolation[k]
     (I_k, one value or one per channel; frame m at index (m+1) I_k - 1), filtered by its real taps (1-D: shared;
     [C, L]: one row per channel), mixed UP by freqs[k] (a 64-bit NCO) and all channels are summed -- Duc's function
@@ -922,12 +771,9 @@ class Fcsb:
     outputs of the blocks it completes (see geometry); to drain a finite stream feed zero frames covering N positions
     and drop the outputs past its end.  There is no scale: the taps carry the factor I_k."""
 
-    def __init__(self, taps, freqs, rate, interpolation, first_sample=0, device=0, stream=None, _handle=None,
-                 _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+    _abi = "fcsb"
+
+    def __init__(self, taps, freqs, rate, interpolation, first_sample=0, device=0, stream=None):
         t = np.ascontiguousarray(taps, np.float32)
         if t.ndim not in (1, 2):
             raise ValueError("taps must be 1-D (shared) or [channels, taps]")
@@ -944,10 +790,7 @@ class Fcsb:
         cfg = F.FcsbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phase_inc.ctypes.data,
                            self.interpolation.ctypes.data, self.n_channels, int(first_sample) % (1 << 64), device,
                            _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_fcsb_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_fcsb_create")
+        self._create(cfg)
 
     @property
     def geometry(self):
@@ -987,37 +830,18 @@ class Fcsb:
               "sdr_fcsb_process_dev")
         return got.value
 
-    def reset(self):
-        check(lib().sdr_fcsb_reset(self.h), "sdr_fcsb_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_fcsb_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_fcsb_clone")
-        return Fcsb(None, None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_fcsb_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
-class Rrb:
+class Rrb(_Handle):
     """Rational resampler bank (sdr_rrb), the textbook upfirdn per channel: channel k is zero-stuffed by
     interpolation[k] (I_k; frame m at index (m+1) I_k - 1), filtered by its real taps (1-D: shared; [C, L]: one row per
     channel) and decimated by decimation[k] (D_k; output r is sample (r+1) D_k - 1).  interpolation and decimation
     take one value or one per channel.  After n frames a channel has released floor(n I_k / D_k) outputs.  There is no
     scale: unit gain needs taps with DC gain I_k."""
 
-    def __init__(self, taps, interpolation, decimation, n_channels=None, device=0, stream=None, _handle=None,
-                 _meta=None):
-        if _handle is not None:
-            self.h = _handle
-            self.__dict__.update(_meta)
-            return
+    _abi = "rrb"
+
+    def __init__(self, taps, interpolation, decimation, n_channels=None, device=0, stream=None):
         t = np.ascontiguousarray(taps, np.float32)
         if t.ndim not in (1, 2):
             raise ValueError("taps must be 1-D (shared) or [channels, taps]")
@@ -1034,10 +858,7 @@ class Rrb:
         self.decimation = np.ascontiguousarray(d, np.uintp)
         cfg = F.RrbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.interpolation.ctypes.data,
                           self.decimation.ctypes.data, c, device, _stream_ptr(stream))
-        err = C.c_int(0)
-        self.h = lib().sdr_rrb_create(C.byref(cfg), C.byref(err))
-        if not self.h:
-            raise SdrError(err.value, "sdr_rrb_create")
+        self._create(cfg)
 
     def _counts(self, n_in):
         return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
@@ -1079,22 +900,6 @@ class Rrb:
                                         got.ctypes.data), "sdr_rrb_process_dev")
         return got.astype(np.int64)
 
-    def reset(self):
-        check(lib().sdr_rrb_reset(self.h), "sdr_rrb_reset")
-
-    def clone(self):
-        err = C.c_int(0)
-        h = lib().sdr_rrb_clone(self.h, C.byref(err))
-        if not h:
-            raise SdrError(err.value, "sdr_rrb_clone")
-        return Rrb(None, None, None, _handle=h, _meta={k: v for k, v in self.__dict__.items() if k != "h"})
-
-    def close(self):
-        if getattr(self, "h", None):
-            lib().sdr_rrb_destroy(self.h)
-            self.h = None
-
-    __del__ = close
 
 
 class FmStereo:
@@ -1215,14 +1020,13 @@ class ResampleError(RuntimeError):
         super().__init__(msg.decode() if msg else "Unknown(%d)" % code)
 
 
-class SampleRate:
+class SampleRate(_Handle):
     """resample::SampleRate<A> (src/resample.rs:11-110).  channels: 1 for f32, 2 for Complex<f32>."""
 
-    def __init__(self, typ, channels, device=0, stream=None, _handle=None):
+    _abi = "src"
+
+    def __init__(self, typ, channels, device=0, stream=None):
         self.channels = int(channels)
-        if _handle is not None:
-            self.h = _handle
-            return
         err = C.c_int(0)
         self.h = lib().sdr_src_new_on(int(typ), self.channels, device, _stream_ptr(stream), C.byref(err))
         if not self.h:
@@ -1260,7 +1064,7 @@ class SampleRate:
         h = lib().sdr_src_clone(self.h, C.byref(err))
         if not h:
             raise ResampleError(err.value)
-        return SampleRate(0, self.channels, _handle=h)
+        return self._adopt(h)
 
     def set_ratio(self, ratio):
         rc = lib().sdr_src_set_ratio(self.h, ratio)
@@ -1281,11 +1085,9 @@ class SampleRate:
             raise ResampleError(rc)
 
     def close(self):
-        if getattr(self, "h", None):
+        if self.h:
             lib().sdr_src_delete(self.h)
             self.h = None
-
-    __del__ = close
 
 
 def sinc_table(typ):
