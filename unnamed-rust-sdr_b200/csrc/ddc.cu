@@ -33,6 +33,7 @@
 
 #include "kernels.h"
 #include "nco.cuh"
+#include "ptx.cuh"
 
 using namespace sdr;
 
@@ -49,59 +50,6 @@ constexpr int DDC_THREADS = (DDC_PROD_WARPS + 1 + 16) * 32;
 constexpr int DDC_ACC_COLS = 256;                    // TMEM columns per accumulator set (two sets fill the 512)
 constexpr size_t DDC_SMEM_MAX = 220 * 1024;
 constexpr size_t DDC_SLAB_BYTES = (size_t)32 << 20;  // host-memory calls: input chunk size
-
-// ---- PTX wrappers (the subset of fir_umma.cu's that this kernel uses) ----------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done)
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cp_async16_s(uint32_t dst, const void *src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_arrive_noinc(uint32_t bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-template <bool ACC>
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
-    if (ACC)
-        asm volatile("{\n .reg .pred p;\n setp.eq.u32 p, 1, 1;\n tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-                     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-    else
-        asm volatile("{\n .reg .pred p;\n setp.eq.u32 p, 1, 0;\n tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-                     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t *v) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n .reg .pred p;\n elect.sync _|p, 0xffffffff;\n selp.u32 %0, 1, 0, p;\n}\n" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46) | ((uint64_t)layout << 61);
-}
-// 64-byte rows: SWIZZLE_64B (the A descriptor's layout type 4)
-__device__ __forceinline__ uint32_t swz64(uint32_t o) { return o ^ (((o >> 7) & 3u) << 4); }
 
 // stage = the window starts of one tile's 128 rows (64 bytes apart) + the KS * 32-byte halo of the last row
 __host__ __device__ constexpr int ddc_stage_bytes(int KS) { return (64 * 127 + 32 * KS + 1023) / 1024 * 1024; }
@@ -165,11 +113,10 @@ __global__ void __launch_bounds__(DDC_THREADS, 1) ddc_tc_kernel(const DdcTcArgs 
     if (tid == 0) {
         for (int s = 0; s < DDC_STAGES; ++s) { mbar_init(full_bar(s), 32 * DDC_PROD_WARPS); mbar_init(empty_bar(s), 1); }
         for (int s = 0; s < 2; ++s) { mbar_init(accf_bar(s), 1); mbar_init(acce_bar(s), 8); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == DDC_MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_base_s)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<512>(smem_u32(&tmem_base_s));
     }
     fence_proxy_async();
     tc_fence_before();
@@ -191,11 +138,11 @@ __global__ void __launch_bounds__(DDC_THREADS, 1) ddc_tc_kernel(const DdcTcArgs 
             if (w0 >= 0 && w0 + 8LL * nchunks <= a.n_in) {
                 const uint8_t *src = a.in + 2 * w0;
 #pragma unroll 4
-                for (int c = ptid; c < nchunks; c += 32 * DDC_PROD_WARPS) cp_async16_s(sbase + swz64(16u * (uint32_t)c), src + 16 * c);
+                for (int c = ptid; c < nchunks; c += 32 * DDC_PROD_WARPS) cp_async16_s(sbase + SmemLayout<64>::swz(16u * (uint32_t)c), src + 16 * c);
             } else {
                 for (int c = ptid; c < nchunks; c += 32 * DDC_PROD_WARPS) {
                     const long long s0 = w0 + 8LL * c;
-                    const uint32_t off = swz64(16u * (uint32_t)c);
+                    const uint32_t off = SmemLayout<64>::swz(16u * (uint32_t)c);
                     if (s0 >= 0 && s0 + 8 <= a.n_in) {
                         cp_async16_s(sbase + off, a.in + 2 * s0);
                     } else if (s0 < a.n_in) {
@@ -222,10 +169,10 @@ __global__ void __launch_bounds__(DDC_THREADS, 1) ddc_tc_kernel(const DdcTcArgs 
             cp_async_arrive_noinc(full_bar(stage));
             if (++stage == NST) { stage = 0; ph ^= 1u; }
         }
-        asm volatile("cp.async.wait_all;" ::: "memory");
+        cp_async_wait_all();
     } else if (warp == DDC_MMA_WARP) {
         // ================= MMA issuer =================
-        const uint32_t idesc = (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(Ng >> 3) << 17) | ((128u >> 4) << 24);
+        const uint32_t idesc = idesc_u8s8_s32(128, Ng);
         const uint64_t bdesc0 = smem_desc(tab_s, 128, 256, 0);
         int stage = 0, as = 0;
         uint32_t ph = 0, aph = 0;
@@ -234,7 +181,7 @@ __global__ void __launch_bounds__(DDC_THREADS, 1) ddc_tc_kernel(const DdcTcArgs 
             mbar_wait(acce_bar(as), aph ^ 1u);
             tc_fence_after();
             if (elect_one()) {
-                uint64_t ad = smem_desc(stage0 + (uint32_t)stage * SB, 16, 8 * 64, 4);
+                uint64_t ad = smem_desc(stage0 + (uint32_t)stage * SB, 16, 8 * 64, SmemLayout<64>::type);
                 uint64_t bd = bdesc0;
                 const uint32_t d0 = tmem + (uint32_t)(as * DDC_ACC_COLS);
                 umma_i8<false>(d0, ad, bd, idesc);
@@ -288,11 +235,11 @@ __global__ void __launch_bounds__(DDC_THREADS, 1) ddc_tc_kernel(const DdcTcArgs 
                     uint32_t v[24];
                     if constexpr (PC <= 2) {
                         // the channel's 8 (PC = 1) or 16 (PC = 2) columns hold (dg, u, part) at dg * 2 PC + 2u + part
-                        tmem_ld8(col0, v);
-                        if constexpr (PC == 2) tmem_ld8(col0 + 8, v + 8);
+                        tmem_ld_32x32b_x8(col0, v);
+                        if constexpr (PC == 2) tmem_ld_32x32b_x8(col0 + 8, v + 8);
                     } else {
 #pragma unroll
-                        for (int dg = 0; dg < 3; ++dg) tmem_ld8(col0 + dg * 2 * PC + 2 * k0, v + 8 * dg);
+                        for (int dg = 0; dg < 3; ++dg) tmem_ld_32x32b_x8(col0 + dg * 2 * PC + 2 * k0, v + 8 * dg);
                     }
                     tmem_ld_wait();
 #pragma unroll
@@ -320,7 +267,7 @@ __global__ void __launch_bounds__(DDC_THREADS, 1) ddc_tc_kernel(const DdcTcArgs 
     __syncthreads();
     if (warp == DDC_MMA_WARP) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+        tmem_dealloc<512>(tmem);
     }
 }
 

@@ -14,10 +14,10 @@
 //                      FFTs with the W_n^{k r} twiddle folded into the load.  The intermediate is
 //                      written in place in the output buffer.
 #include <cstdlib>
-#include <cuda.h>  // CUtensorMap and the cuTensorMapEncodeTiled prototype only: the entry point is resolved at run time
 
 #include "kernels.h"
 #include "fft_core.cuh"
+#include "ptx.cuh"
 
 namespace sdr {
 
@@ -143,7 +143,6 @@ __host__ __device__ constexpr size_t w1k_smem(int fmt) {
 // per-(warp, buffer) mbarrier, instead of four LDGSTS per lane and a wait_group: the same bytes over the same path into
 // shared memory, 128 fewer issued instructions per transform in an issue-bound kernel.  TMA = false keeps the cp.async
 // loader (A/B switch SDR_FFT_NO_TMA=1).
-__device__ __forceinline__ uint32_t w1k_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 template <int FMT, int SHIFT, bool TMA = false>
 __global__ void __launch_bounds__(W1K_WARPS * 32, 2) fft1024_warp_kernel(FftArgs a) {
     constexpr int N = 1024;
@@ -169,17 +168,16 @@ __global__ void __launch_bounds__(W1K_WARPS * 32, 2) fft1024_warp_kernel(FftArgs
     const unsigned char *in8 = reinterpret_cast<const unsigned char *>(a.in);
     int buf = 0;
     uint32_t tph = 0;  // bit i = parity of buffer i's mbarrier
-    const uint32_t bar_s = w1k_smem_u32(&tma_bar[warp][0]), raw_s = w1k_smem_u32(raw);
+    const uint32_t bar_s = smem_u32(&tma_bar[warp][0]), raw_s = smem_u32(raw);
     auto tma_load = [&](long long bb, int bf) {  // lane 0 only
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], 2048;" ::"r"(bar_s + 8u * bf) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], 2048, [%2];"
-                     ::"r"(raw_s + 2048u * bf), "l"(in8 + bb * 2048), "r"(bar_s + 8u * bf) : "memory");
+        mbar_arrive_expect_tx(bar_s + 8u * bf, 2048);
+        tma_bulk_g2s(raw_s + 2048u * bf, in8 + bb * 2048, 2048, bar_s + 8u * bf);
     };
     if (FMT == SDR_FMT_U8IQ && TMA) {
         if (lane == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_s));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_s + 8u));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            mbar_init(bar_s, 1);
+            mbar_init(bar_s + 8u, 1);
+            mbar_init_fence();
             if (b < a.batches) tma_load(b, 0);
         }
         __syncwarp();
@@ -195,10 +193,7 @@ __global__ void __launch_bounds__(W1K_WARPS * 32, 2) fft1024_warp_kernel(FftArgs
             if (TMA) {
                 // buffer buf ^ 1 was last read one iteration ago, before that iteration's closing __syncwarp
                 if (lane == 0 && nb < a.batches) tma_load(nb, buf ^ 1);
-                uint32_t done = 0;
-                while (!done)
-                    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-                                 : "=r"(done) : "r"(bar_s + 8u * buf), "r"((tph >> buf) & 1u) : "memory");
+                mbar_wait(bar_s + 8u * buf, (tph >> buf) & 1u);
                 tph ^= 1u << buf;
             } else if (nb < a.batches) {
 #pragma unroll
@@ -908,17 +903,6 @@ int launch_l2w(const FftArgs &a, cudaStream_t st) {
 // Forward progress: as for fft_l2w_kernel -- a CTA walks its items in increasing global order, a STEP 1 copy waits only
 // for STEP 0 items at least lag 2S - S items older, and lag 2S > G + 3S makes those older than anything this CTA has
 // not yet signalled; the launcher keeps the whole grid resident.
-__device__ __forceinline__ void tma_tile_3d(uint32_t dst, const CUtensorMap *tm, int c0, int c1, int c2, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_parity(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done)
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-
 template <int LOGN2, int FMT>
 __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, long long total_items,
                                                          const __grid_constant__ CUtensorMap map_in,
@@ -937,9 +921,9 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
     for (int i = tid; i < 15 * 16; i += 288) tw0[i] = __ldg(a.tw + (long long)((i / 16 + 1) * (i % 16)) * (n / 256));
     for (int i = tid; i < (R2 - 1) * 16; i += 288) tw1[i] = __ldg(a.tw + (long long)((i / 16 + 1) * (i % 16)) * 256);
     if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(w1k_smem_u32(&full_bar[0])));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(w1k_smem_u32(&full_bar[1])));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(smem_u32(&full_bar[0]), 1);
+        mbar_init(smem_u32(&full_bar[1]), 1);
+        mbar_init_fence();
         cnt[0] = 0;
         cnt[1] = 0;
     }
@@ -972,19 +956,19 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
         bool step1; long long b; int tile;
         decode(item, step1, b, tile);
         if (b < 0) return true;
-        const uint32_t bar = w1k_smem_u32(&full_bar[s]), dst = w1k_smem_u32(sm + (size_t)s * STAGE);
+        const uint32_t bar = smem_u32(&full_bar[s]), dst = smem_u32(sm + (size_t)s * STAGE);
         if (!step1) {
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(4096 * ES) : "memory");
-            tma_tile_3d(dst, &map_in, 16 * tile, 0, (int)b, bar);
+            mbar_arrive_expect_tx(bar, 4096 * ES);
+            tma_load_3d(dst, &map_in, 16 * tile, 0, (int)b, bar);
         } else {
             while (ld_acquire_gpu(flags + b) < S) {
                 if (try_only) return false;
                 __nanosleep(64);
             }
             // the STEP 0 stores (generic proxy, other SMs; acquired above) before this thread's async-proxy reads of them
-            asm volatile("fence.proxy.async;" ::: "memory");
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(4096 * 8) : "memory");
-            tma_tile_3d(dst, &map_scr, NC * tile, 0, (int)b, bar);
+            fence_proxy_async_all();
+            mbar_arrive_expect_tx(bar, 4096 * 8);
+            tma_load_3d(dst, &map_scr, NC * tile, 0, (int)b, bar);
         }
         return true;
     };
@@ -994,12 +978,12 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
     auto cnt_arrive = [&](int which) {
         __syncwarp();  // orders the other lanes' accesses before lane 0's release
         if ((tid & 31) == 0)
-            asm volatile("red.release.cta.shared::cta.add.u32 [%0], 1;" ::"r"(w1k_smem_u32(&cnt[which])) : "memory");
+            asm volatile("red.release.cta.shared::cta.add.u32 [%0], 1;" ::"r"(smem_u32(&cnt[which])) : "memory");
     };
     auto cnt_wait = [&](int which, unsigned target) {
         unsigned v;
         for (;;) {
-            asm volatile("ld.acquire.cta.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(w1k_smem_u32(&cnt[which])) : "memory");
+            asm volatile("ld.acquire.cta.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(smem_u32(&cnt[which])) : "memory");
             if (v >= target) break;
             __nanosleep(32);
         }
@@ -1042,7 +1026,7 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
         float2 v[16];
         if (b >= 0) {
             if (!step1) {
-                mbar_wait_parity(w1k_smem_u32(&full_bar[s]), (ph >> s) & 1u);
+                mbar_wait(smem_u32(&full_bar[s]), (ph >> s) & 1u);
                 const int c = tid & 15, rr = tid >> 4;
                 const unsigned char *raw = reinterpret_cast<const unsigned char *>(st);
 #pragma unroll
@@ -1052,7 +1036,7 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
                 const int k = NC * tile + c;
                 // a_e = W_n^{k (t + e TC)} = w0 * ws^e (the two table loads are in flight while the tile lands)
                 const float2 w0 = __ldg(a.tw + k * t), p1 = __ldg(a.tw + k * TC);
-                mbar_wait_parity(w1k_smem_u32(&full_bar[s]), (ph >> s) & 1u);
+                mbar_wait(smem_u32(&full_bar[s]), (ph >> s) & 1u);
 #pragma unroll
                 for (int e = 0; e < 16; ++e) v[e] = st[(t + TC * e) * NC + c];
                 const float2 p2 = cmul(p1, p1), p4 = cmul(p2, p2), p8 = cmul(p4, p4);
@@ -1082,7 +1066,7 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
             const float2 *srcs = st + col * PL::SSTRIDE0;
 #pragma unroll
             for (int e = 0; e < 16; ++e) v[e] = srcs[t + 17 * e];  // pad(t + 16 e) = t + 17 e for t < 16
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // these accesses before the stage's next tensor copy
+            fence_proxy_async();  // these accesses before the stage's next tensor copy
             cnt_arrive(0);
 #pragma unroll
             for (int q = 1; q < 16; ++q) v[q] = cmul(v[q], tw0[(q - 1) * 16 + t]);
@@ -1100,7 +1084,7 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
             asm volatile("bar.sync 2, 256;" ::: "memory");  // (B)
 #pragma unroll
             for (int e = 0; e < 16; ++e) v[e] = col[pad(t + e * TC)];
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async();
             cnt_arrive(0);
 #pragma unroll
             for (int vi = 0; vi < NB2; ++vi) {
@@ -1125,25 +1109,9 @@ __global__ void __launch_bounds__(288, 3) fft_l2t_kernel(FftArgs a, int lag, lon
     }
 }
 
-// cuTensorMapEncodeTiled, resolved through the runtime (no link-time dependency on libcuda); null = not available
-typedef CUresult (*FftEncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                     const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-inline FftEncodeTiledFn fft_encode_tiled_fn() {
-    static FftEncodeTiledFn fn = []() -> FftEncodeTiledFn {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        return (FftEncodeTiledFn)p;
-    }();
-    return fn;
-}
 // {cols, rows, transforms} view of `batches` transforms of rows x cols elements of `es` bytes; box = cols_box x rows x 1
 inline bool fft_tile_map(CUtensorMap *tm, const void *base, int es, int cols, int rows, long long batches, int cols_box) {
-    FftEncodeTiledFn enc = fft_encode_tiled_fn();
+    EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) return false;
     const CUtensorMapDataType dt = es == 8 ? CU_TENSOR_MAP_DATA_TYPE_UINT64 : es == 4 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT16;
     cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)batches};

@@ -1,5 +1,5 @@
 // fft_core.cuh -- register-resident FFT building blocks shared by the FFT kernels (fft.cu) and the fused power-spectrum
-// kernel (psd.cu): radix 2/4/8/16 butterflies, the 32-point DFT of the 1024-point warp kernel, cp.async helpers.
+// kernel (psd.cu): radix 2/4/8/16 butterflies and the 32-point DFT of the 1024-point warp kernel.
 #pragma once
 #include "common.cuh"
 
@@ -97,13 +97,6 @@ __device__ __forceinline__ void dft32(float2 (&v)[32], float2 (&w)[32]) {
         w[r + 16] = csub_t<PK>(u0, t);
     }
 }
-
-__device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) {
-    const unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem_src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
 }  // namespace
 

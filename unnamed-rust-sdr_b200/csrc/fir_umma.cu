@@ -45,9 +45,8 @@
 #include <cstring>
 #include <vector>
 
-#include <cuda.h>  // CUtensorMap and the cuTensorMapEncodeTiled prototype only: the entry point is resolved at run time
-
 #include "kernels.h"
+#include "ptx.cuh"
 
 namespace sdr {
 
@@ -79,85 +78,6 @@ struct UmArgs {
     int tma_need = 0;    // window rows a tile really reads (the boxes are rounded up to multiples of 8 rows)
     long long tma_rows_total = 0;  // rows of the map: a tile whose needed rows reach beyond it is staged by cp.async
 };
-
-// ---- PTX wrappers ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done)
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cp_async16_s(uint32_t dst, const void *src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_arrive_noinc(uint32_t bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// TMA, non-tensor form: one bulk copy global -> shared, completion (bytes) on an mbarrier.  SASS: UBLKCP.
-__device__ __forceinline__ void tma_bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-// TMA tensor copies global -> shared (SASS: UTMALDG), completion in bytes on an mbarrier
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *tm, int c0, int c1, int c2, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap *tm, int c0, int c1, int c2, int c3, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-                 ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// D[tmem] (+)= A[smem desc] * B[smem desc], u8 x s8 -> s32; the accumulate flag is fixed at compile time (no setp on
-// the issuing thread's critical path)
-template <bool ACC>
-__device__ __forceinline__ void umma_i8c(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
-    if (ACC)
-        asm volatile("{\n .reg .pred p;\n setp.eq.u32 p, 1, 1;\n tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-                     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-    else
-        asm volatile("{\n .reg .pred p;\n setp.eq.u32 p, 1, 0;\n tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-                     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_16x256b_x2(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr) : "memory");
-}
-// one lane of a converged warp (elect.sync): unlike `lane == 0`, ptxas KNOWS a single thread follows the branch, so the
-// tcgen05.mma operands stay in uniform registers and no per-instruction election loop is emitted around them
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n .reg .pred p;\n elect.sync _|p, 0xffffffff;\n selp.u32 %0, 1, 0, p;\n}\n" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// shared-memory matrix descriptor (K-major): start address, leading / stride byte offsets (16-byte units), version 1
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46) | ((uint64_t)layout << 61);
-}
-
-template <int P> struct UmLayout;
-template <> struct UmLayout<8>  { static constexpr uint32_t type = 0; __device__ static uint32_t swz(uint32_t o) { return o; } };
-template <> struct UmLayout<16> { static constexpr uint32_t type = 6; __device__ static uint32_t swz(uint32_t o) { return o ^ (((o >> 7) & 1u) << 4); } };
-template <> struct UmLayout<32> { static constexpr uint32_t type = 4; __device__ static uint32_t swz(uint32_t o) { return o ^ (((o >> 7) & 3u) << 4); } };
 
 // one stage holds the 128*MB window starts of a tile, R samples apart, plus the KS*32-byte halo of the last row
 __host__ __device__ constexpr int um_stage_bytes(int R, int PC, int KS) {
@@ -212,11 +132,10 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_kernel(const UmArgs a,
     if (tid == 0) {
         for (int s = 0; s < UM_STAGES; ++s) { mbar_init(full_bar(s), 32 * UM_PROD_WARPS); mbar_init(empty_bar(s), 1); }
         for (int s = 0; s < 2; ++s) { mbar_init(accf_bar(s), 1); mbar_init(acce_bar(s), 8); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == UM_MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_base_s)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<512>(smem_u32(&tmem_base_s));
     }
     fence_proxy_async();  // the tap tables were written through the generic proxy, tcgen05.mma reads through the async one
     tc_fence_before();
@@ -269,11 +188,11 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_kernel(const UmArgs a,
                 const unsigned char *src = in + 2 * w0;
 #pragma unroll 4
                 for (int c = ptid; c < nchunks; c += 32 * UM_PROD_WARPS)
-                    cp_async16_s(sbase + UmLayout<P>::swz(16u * (uint32_t)c), src + 16 * c);
+                    cp_async16_s(sbase + SmemLayout<ROWB>::swz(16u * (uint32_t)c), src + 16 * c);
             } else {
                 for (int c = ptid; c < nchunks; c += 32 * UM_PROD_WARPS) {
                     const long long s0 = w0 + 8LL * c;
-                    const uint32_t off = UmLayout<P>::swz(16u * (uint32_t)c);
+                    const uint32_t off = SmemLayout<ROWB>::swz(16u * (uint32_t)c);
                     if (s0 >= 0 && s0 + 8 <= f.n_in) {
                         cp_async16_s(sbase + off, in + 2 * s0);
                     } else if (s0 < f.n_in) {
@@ -300,10 +219,10 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_kernel(const UmArgs a,
             cp_async_arrive_noinc(full_bar(stage));
             if (++stage == NST) { stage = 0; ph ^= 1u; }
         }
-        asm volatile("cp.async.wait_all;" ::: "memory");
+        cp_async_wait_all();
     } else if (warp == UM_MMA_WARP) {
         // ================= MMA issuer =================
-        const uint32_t idesc = (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((128u >> 4) << 24);
+        const uint32_t idesc = idesc_u8s8_s32(128, N);
         const uint64_t bdesc0 = smem_desc(tab_s, 128, 256, 0);
         int stage = 0, as = 0;
         uint32_t ph = 0, aph = 0;
@@ -314,16 +233,16 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_kernel(const UmArgs a,
             if (elect_one()) {
                 // running descriptors: the issuing thread's uniform-datapath work per MMA is two 64-bit adds of
                 // constants (recomputing them from kk cost ~130 cycles per MMA: the real limit of MMA-heavy tiles)
-                uint64_t ad = smem_desc(stage0 + (uint32_t)stage * SB, 16, 8 * ROWB, UmLayout<P>::type);
+                uint64_t ad = smem_desc(stage0 + (uint32_t)stage * SB, 16, 8 * ROWB, SmemLayout<ROWB>::type);
                 uint64_t bd = bdesc0;
                 const uint32_t d0 = tmem + (uint32_t)(as * UM_ACC_COLS);
 #pragma unroll
-                for (int mb = 0; mb < MB; ++mb) umma_i8c<false>(d0 + mb * N, ad + (uint64_t)((mb * 128 * ROWB) >> 4), bd, idesc);
+                for (int mb = 0; mb < MB; ++mb) umma_i8<false>(d0 + mb * N, ad + (uint64_t)((mb * 128 * ROWB) >> 4), bd, idesc);
                 for (int kk = 1; kk < KS; ++kk) {
                     ad += 2;               // 32 bytes along the window
                     bd += (N * 32) >> 4;   // next tap block
 #pragma unroll
-                    for (int mb = 0; mb < MB; ++mb) umma_i8c<true>(d0 + mb * N, ad + (uint64_t)((mb * 128 * ROWB) >> 4), bd, idesc);
+                    for (int mb = 0; mb < MB; ++mb) umma_i8<true>(d0 + mb * N, ad + (uint64_t)((mb * 128 * ROWB) >> 4), bd, idesc);
                 }
                 umma_commit(empty_bar(stage));  // the stage may be refilled once these MMAs have read it
                 umma_commit(accf_bar(as));      // ... and the accumulator set is complete
@@ -449,7 +368,7 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_kernel(const UmArgs a,
     __syncthreads();
     if (warp == UM_MMA_WARP) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+        tmem_dealloc<512>(tmem);
     }
 }
 
@@ -468,16 +387,6 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_kernel(const UmArgs a,
 // and the producers share; the raw-ring -> plane conversion adds 17 KB per tile to it and puts an LDS on the
 // producers' critical path.  C1 392 vs 490, C3 483 vs 588, 255 taps D=1 343 vs 321-377 Gsamples/s: it stays opt-in.
 // =====================================================================================================================
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr) : "memory");
-}
-template <int PITCH> struct PitchLayout;  // row pitch in bytes
-template <> struct PitchLayout<16> { static constexpr uint32_t type = 0; __device__ static uint32_t swz(uint32_t o) { return o; } };
-template <> struct PitchLayout<32> { static constexpr uint32_t type = 6; __device__ static uint32_t swz(uint32_t o) { return o ^ (((o >> 7) & 1u) << 4); } };
-template <> struct PitchLayout<64> { static constexpr uint32_t type = 4; __device__ static uint32_t swz(uint32_t o) { return o ^ (((o >> 7) & 3u) << 4); } };
-
 // one plane of a stage: the 128*MB window starts R bytes apart + the KS*32-byte halo, 1024-aligned
 __host__ __device__ constexpr int um_plane_bytes(int R, int PC, int KS) {
     return (R * (128 * (32 / PC) - 1) + 32 * KS + 1023) / 1024 * 1024;
@@ -523,11 +432,10 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
     if (tid == 0) {
         for (int s = 0; s < UM_STAGES; ++s) { mbar_init(full_bar(s), 32 * UM_PROD_WARPS); mbar_init(empty_bar(s), 1); }
         for (int s = 0; s < 2; ++s) { mbar_init(accf_bar(s), 1); mbar_init(acce_bar(s), 8); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == UM_MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(&tmem_base_s)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<512>(smem_u32(&tmem_base_s));
     }
     fence_proxy_async();
     tc_fence_before();
@@ -584,7 +492,7 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
                     }
                 }
             }
-            asm volatile("cp.async.commit_group;" ::: "memory");
+            cp_async_commit();
         };
         issue(blockIdx.x, 0);
         issue(blockIdx.x + wstride, 1);
@@ -594,7 +502,7 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
             int s2 = slot + 2;
             if (s2 >= UM_RAW_SLOTS) s2 -= UM_RAW_SLOTS;
             issue(w + 2 * wstride, s2);
-            asm volatile("cp.async.wait_group 2;" ::: "memory");  // this lane's chunks of tile w have landed
+            cp_async_wait<2>();  // this lane's chunks of tile w have landed
             mbar_wait(empty_bar(stage), ph ^ 1u);
             uint8_t *pI = gen + (size_t)stage * SB, *pQ = pI + PB;
             const uint8_t *rs = raw0 + (size_t)slot * RAWB;
@@ -603,7 +511,7 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
                 const uint4 q = *reinterpret_cast<const uint4 *>(rs + 16 * c);  // words = I0 Q0 I1 Q1
                 const uint32_t i_lo = __byte_perm(q.x, q.y, 0x6420), i_hi = __byte_perm(q.z, q.w, 0x6420);
                 const uint32_t q_lo = __byte_perm(q.x, q.y, 0x7531), q_hi = __byte_perm(q.z, q.w, 0x7531);
-                const uint32_t off = PitchLayout<R>::swz((8u * (uint32_t)c) & ~15u) | ((8u * (uint32_t)c) & 8u);
+                const uint32_t off = SmemLayout<R>::swz((8u * (uint32_t)c) & ~15u) | ((8u * (uint32_t)c) & 8u);
                 *reinterpret_cast<uint2 *>(pI + off) = make_uint2(i_lo, i_hi);
                 *reinterpret_cast<uint2 *>(pQ + off) = make_uint2(q_lo, q_hi);
             }
@@ -612,10 +520,10 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
             if (++stage == NST) { stage = 0; ph ^= 1u; }
             if (++slot == UM_RAW_SLOTS) slot = 0;
         }
-        asm volatile("cp.async.wait_all;" ::: "memory");
+        cp_async_wait_all();
     } else if (warp == UM_MMA_WARP) {
         // ================= MMA issuer =================
-        const uint32_t idesc = (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((128u >> 4) << 24);
+        const uint32_t idesc = idesc_u8s8_s32(128, N);
         const uint64_t bdesc0 = smem_desc(tab_s, 128, 256, 0);
         int stage = 0, as = 0;
         uint32_t ph = 0, aph = 0;
@@ -624,22 +532,22 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
             mbar_wait(acce_bar(as), aph ^ 1u);
             tc_fence_after();
             if (elect_one()) {
-                uint64_t aI = smem_desc(stage0 + (uint32_t)stage * SB, 16, 8 * R, PitchLayout<R>::type);
-                uint64_t aQ = smem_desc(stage0 + (uint32_t)stage * SB + PB, 16, 8 * R, PitchLayout<R>::type);
+                uint64_t aI = smem_desc(stage0 + (uint32_t)stage * SB, 16, 8 * R, SmemLayout<R>::type);
+                uint64_t aQ = smem_desc(stage0 + (uint32_t)stage * SB + PB, 16, 8 * R, SmemLayout<R>::type);
                 uint64_t bd = bdesc0;
                 const uint32_t d0 = tmem + (uint32_t)(as * UM_ACC_COLS);
 #pragma unroll
                 for (int mb = 0; mb < MB; ++mb) {
-                    umma_i8c<false>(d0 + mb * 2 * N, aI + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
-                    umma_i8c<false>(d0 + mb * 2 * N + N, aQ + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
+                    umma_i8<false>(d0 + mb * 2 * N, aI + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
+                    umma_i8<false>(d0 + mb * 2 * N + N, aQ + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
                 }
                 for (int kk = 1; kk < KS; ++kk) {
                     aI += 2; aQ += 2;
                     bd += (N * 32) >> 4;
 #pragma unroll
                     for (int mb = 0; mb < MB; ++mb) {
-                        umma_i8c<true>(d0 + mb * 2 * N, aI + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
-                        umma_i8c<true>(d0 + mb * 2 * N + N, aQ + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
+                        umma_i8<true>(d0 + mb * 2 * N, aI + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
+                        umma_i8<true>(d0 + mb * 2 * N + N, aQ + (uint64_t)((mb * 128 * R) >> 4), bd, idesc);
                     }
                 }
                 umma_commit(empty_bar(stage));
@@ -682,8 +590,8 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
                     const uint32_t col = tbase + (uint32_t)(mb * 2 * N + 8 * pc);
 #pragma unroll
                     for (int dg = 0; dg < 3; ++dg) {
-                        tmem_ld8(col + dg * PC, dI[dg]);
-                        tmem_ld8(col + N + dg * PC, dQ[dg]);
+                        tmem_ld_32x32b_x8(col + dg * PC, dI[dg]);
+                        tmem_ld_32x32b_x8(col + N + dg * PC, dQ[dg]);
                     }
                     tmem_ld_wait();
                 }
@@ -785,7 +693,7 @@ __global__ void __launch_bounds__(UM_THREADS, 1) fir_umma_planar_kernel(const Um
     __syncthreads();
     if (warp == UM_MMA_WARP) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+        tmem_dealloc<512>(tmem);
     }
 }
 
@@ -839,10 +747,10 @@ static_assert(UP_EPI_WARP0 % 4 == 0, "epilogue warps must start on a TMEM lane-q
 template <int D, int KS>
 __device__ __forceinline__ void up_issue_tile(uint32_t d0, uint64_t ap, uint64_t bd, uint32_t idesc) {
     constexpr uint64_t PSTEP = 128 + 2 * KS, BSTEP = (48 * 32) >> 4;
-    umma_i8c<false>(d0, ap, bd, idesc);
+    umma_i8<false>(d0, ap, bd, idesc);
 #pragma unroll
     for (int j = 1; j < D * KS; ++j)
-        umma_i8c<true>(d0, ap + (uint64_t)(j / KS) * PSTEP + 2 * (uint64_t)(j % KS), bd + (uint64_t)j * BSTEP, idesc);
+        umma_i8<true>(d0, ap + (uint64_t)(j / KS) * PSTEP + 2 * (uint64_t)(j % KS), bd + (uint64_t)j * BSTEP, idesc);
 }
 
 template <int D>
@@ -874,11 +782,10 @@ __global__ void __launch_bounds__(UP_THREADS, 1) fir_umma_poly_kernel(const UmAr
         for (int s = 0; s < UP_SETS; ++s) { mbar_init(accf_bar(s), 1); mbar_init(acce_bar(s), 4); }
         for (int s = 0; s < UP_RAW; ++s) { mbar_init(rawfull_bar(s), 1); mbar_init(rawfree_bar(s), UP_CONV_WARPS); }
         mbar_init(tab_bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == UP_MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(&tmem_base_s)) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<256>(smem_u32(&tmem_base_s));
     }
     fence_proxy_async();
     tc_fence_before();
@@ -992,7 +899,7 @@ __global__ void __launch_bounds__(UP_THREADS, 1) fir_umma_poly_kernel(const UmAr
     } else if (warp < UP_EPI_WARP0) {
         // ================= MMA issuers: warp j takes tiles j, j + 2, ...; D phases x KS k-steps into one set =================
         const int mw = warp - UP_MMA_WARP;
-        const uint32_t idesc = (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((128u >> 4) << 24);
+        const uint32_t idesc = idesc_u8s8_s32(128, N);
         const uint64_t bdesc0 = smem_desc(tab_s, 128, 256, 0);
         {
             // the tap tables arrive by one bulk copy while the first raw tile is loaded and converted
@@ -1081,7 +988,7 @@ __global__ void __launch_bounds__(UP_THREADS, 1) fir_umma_poly_kernel(const UmAr
     __syncthreads();
     if (warp == UP_MMA_WARP) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
+        tmem_dealloc<256>(tmem);
     }
 }
 
@@ -1291,23 +1198,6 @@ static int fir_umma_poly_launch(const FirArgs &f, const uint8_t *d_tables, const
         case 12: return go(fir_umma_poly_kernel<12>);
     }
     return SDR_ERR_UNSUPPORTED;
-}
-
-// cuTensorMapEncodeTiled, resolved through the runtime (no link-time dependency on libcuda); null = not available
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn() {
-    static EncodeTiledFn fn = []() -> EncodeTiledFn {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        return (EncodeTiledFn)p;
-    }();
-    return fn;
 }
 
 // Tensor map over the raw byte stream for fir_umma_kernel's stages: {ROWB bytes, ROWB/16 sub-offsets (stride 16 B),

@@ -36,6 +36,7 @@
 #include <cuda_bf16.h>
 
 #include "kernels.h"
+#include "ptx.cuh"
 
 namespace sdr {
 
@@ -67,60 +68,6 @@ struct UcArgs {
     long long tab_stride; // 0 = all channels share `tab`
 };
 
-// ---- PTX wrappers (same conventions as fir_umma.cu) ----------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done)
-        asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// TMA, non-tensor form: one bulk copy global -> shared, completion (bytes) on an mbarrier.  SASS: UBLKCP.
-__device__ __forceinline__ void tma_bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// D[tmem] (+)= A[smem desc] * B[smem desc], bf16 x bf16 -> f32
-template <bool ACC>
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc) {
-    if (ACC)
-        asm volatile("{\n .reg .pred p;\n setp.eq.u32 p, 1, 1;\n tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n"
-                     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-    else
-        asm volatile("{\n .reg .pred p;\n setp.eq.u32 p, 1, 0;\n tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n"
-                     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_16x256b_x2(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n .reg .pred p;\n elect.sync _|p, 0xffffffff;\n selp.u32 %0, 1, 0, p;\n}\n" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo, uint32_t layout) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | ((uint64_t)1 << 46) | ((uint64_t)layout << 61);
-}
-__device__ __forceinline__ uint32_t swz64(uint32_t o) { return o ^ (((o >> 7) & 3u) << 4); }  // SWIZZLE_64B
 __device__ __forceinline__ void prod_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(UC_PROD_WARPS * 32) : "memory"); }
 
 // split 8 f32 values (4 pairs; pair i belongs to word (i + rot) & 3 of the 16-byte chunk) into bf16 terms, round to
@@ -203,11 +150,10 @@ __global__ void __launch_bounds__(UC_THREADS, 1) fir_umma_c64_kernel(const UcArg
         for (int s = 0; s < UC_MAX_STAGES; ++s) { mbar_init(full_bar(s), 32 * UC_PROD_WARPS); mbar_init(empty_bar(s), 1); }
         for (int s = 0; s < 2; ++s) { mbar_init(accf_bar(s), 1); mbar_init(acce_bar(s), 8); }
         for (int s = 0; s < UC_RAW; ++s) mbar_init(raw_bar(s), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == UC_MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "n"(TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<TMEM_COLS>(smem_u32(&tmem_base_s));
     }
     fence_proxy_async();  // the tap tables were written through the generic proxy, tcgen05.mma reads through the async one
     tc_fence_before();
@@ -287,10 +233,10 @@ __global__ void __launch_bounds__(UC_THREADS, 1) fir_umma_c64_kernel(const UcArg
                 for (int e = ptid; e < NEL; e += 32 * UC_PROD_WARPS) {
                     const long long j = j0 + f.in_step * e;
                     const bool ok = j >= 0 && j < f.in_limit;
-                    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(rs_s + 8u * (uint32_t)e), "l"(ok ? in + j : in), "r"(ok ? 8 : 0) : "memory");
+                    cp_async8_zfill(rs_s + 8u * (uint32_t)e, ok ? in + j : in, ok ? 8 : 0);
                 }
-                asm volatile("cp.async.commit_group;" ::: "memory");
-                asm volatile("cp.async.wait_group 0;" ::: "memory");
+                cp_async_commit();
+                cp_async_wait<0>();
                 prod_bar_sync();
             } else if (e_hi - e_lo < NEL) {
                 int ch; long long wt;
@@ -330,7 +276,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) fir_umma_c64_kernel(const UcArg
                     const float4 q = *reinterpret_cast<const float4 *>(src + 16 * ((i + rot) & 3));
                     re[2 * i] = q.x; im[2 * i] = q.y; re[2 * i + 1] = q.z; im[2 * i + 1] = q.w;
                 }
-                const uint32_t off = swz64(16u * (uint32_t)c);
+                const uint32_t off = SmemLayout<64>::swz(16u * (uint32_t)c);
                 split_store<NS>(re, st_g, PB, off, rot);
                 split_store<NS>(im, st_g + (size_t)NS * PB, PB, off, rot);
             }
@@ -343,7 +289,6 @@ __global__ void __launch_bounds__(UC_THREADS, 1) fir_umma_c64_kernel(const UcArg
         }
     } else if (warp == UC_MMA_WARP) {
         // ================= MMA issuer =================
-        constexpr uint32_t IDESC0 = (1u << 4) | (1u << 7) | (1u << 10) | ((128u >> 4) << 24);  // f32 += bf16 x bf16, M = 128
         const uint64_t bdesc0 = smem_desc(tab_s, 128, 256, 0);
         int stage = 0, as = 0;
         uint32_t ph = 0, aph = 0;
@@ -358,18 +303,18 @@ __global__ void __launch_bounds__(UC_THREADS, 1) fir_umma_c64_kernel(const UcArg
                     const uint32_t d0 = tmem + (uint32_t)(as * SETC + part * NCOL);
                     uint64_t ad[NS];
 #pragma unroll
-                    for (int s = 0; s < NS; ++s) ad[s] = smem_desc(sbase + (uint32_t)((part * NS + s) * PB), 16, 8 * 64, 4);
+                    for (int s = 0; s < NS; ++s) ad[s] = smem_desc(sbase + (uint32_t)((part * NS + s) * PB), 16, 8 * 64, SmemLayout<64>::type);
                     uint64_t bd = bdesc0;
                     // k-step 0 initialises all NCOL columns; everything after accumulates
-                    umma_bf16<false>(d0, ad[0], bd, IDESC0 | ((uint32_t)(NCOL >> 3) << 17));
+                    umma_bf16<false>(d0, ad[0], bd, idesc_bf16_f32(128, NCOL));
 #pragma unroll
-                    for (int s = 1; s < NS; ++s) umma_bf16<true>(d0, ad[s], bd, IDESC0 | ((uint32_t)((32 * (NS - s)) >> 3) << 17));
+                    for (int s = 1; s < NS; ++s) umma_bf16<true>(d0, ad[s], bd, idesc_bf16_f32(128, 32 * (NS - s)));
                     for (int kk = 1; kk < KS; ++kk) {
                         bd += (NCOL * 32) >> 4;
 #pragma unroll
                         for (int s = 0; s < NS; ++s) {
                             ad[s] += 2;  // 32 bytes = 16 samples along the window
-                            umma_bf16<true>(d0, ad[s], bd, IDESC0 | ((uint32_t)((32 * (NS - s)) >> 3) << 17));
+                            umma_bf16<true>(d0, ad[s], bd, idesc_bf16_f32(128, 32 * (NS - s)));
                         }
                     }
                 }
@@ -452,7 +397,7 @@ __global__ void __launch_bounds__(UC_THREADS, 1) fir_umma_c64_kernel(const UcArg
     __syncthreads();
     if (warp == UC_MMA_WARP) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(TMEM_COLS) : "memory");
+        tmem_dealloc<TMEM_COLS>(tmem);
     }
 }
 

@@ -15,6 +15,7 @@
 // Data movement: a warp moves [32 streams x 32 samples] tiles between HBM and shared memory with
 // 256-byte row segments, so the lane-per-stream inner loop reads shared memory, not strided HBM.
 #include "kernels.h"
+#include "ptx.cuh"
 
 namespace sdr {
 
@@ -237,13 +238,6 @@ __device__ __forceinline__ Biquad1 make_bq(const float *c, int kind) {
     b.kind = kind;
     return b;
 }
-
-__device__ __forceinline__ void cp_async8(void *smem_dst, const void *gmem_src) {
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(sa), "l"(gmem_src));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
 // A CTA of two warps owns 32 streams, one lane of each warp per stream.
 //   warp 0 (main)   steps the recurrence, nothing else: per sample one shared load (prefetched) and one shared store

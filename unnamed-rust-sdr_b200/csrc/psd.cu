@@ -20,6 +20,7 @@
 
 #include "kernels.h"
 #include "fft_core.cuh"
+#include "ptx.cuh"
 
 using namespace sdr;
 
@@ -106,12 +107,11 @@ __global__ void __launch_bounds__(P1K_WARPS * 32, 2) psd1024_kernel(Psd1kArgs a)
     auto bulk = [&](long long s) { return U8 && s >= a.src.in_lo && ((in_mis + 2u * (uint32_t)(s - a.src.in_lo)) & 15u) == 0; };
     int buf = 0;
     uint32_t tph = 0;  // bit i = parity of buffer i's mbarrier
-    const uint32_t bar_s = (uint32_t)__cvta_generic_to_shared(&tma_bar[warp][0]);
-    const uint32_t raw_s = (uint32_t)__cvta_generic_to_shared(raw);
+    const uint32_t bar_s = smem_u32(&tma_bar[warp][0]);
+    const uint32_t raw_s = smem_u32(raw);
     auto tma_load = [&](long long s, int bf) {  // lane 0 only
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], 2048;" ::"r"(bar_s + 8u * bf) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], 2048, [%2];"
-                     ::"r"(raw_s + 2048u * bf), "l"(in8 + 2 * (s - a.src.in_lo)), "r"(bar_s + 8u * bf) : "memory");
+        mbar_arrive_expect_tx(bar_s + 8u * bf, 2048);
+        tma_bulk_g2s(raw_s + 2048u * bf, in8 + 2 * (s - a.src.in_lo), 2048, bar_s + 8u * bf);
     };
     // the current frame: number i of nf in chunk c, first sample s0
     long long f0, nfl, s0;
@@ -120,9 +120,9 @@ __global__ void __launch_bounds__(P1K_WARPS * 32, 2) psd1024_kernel(Psd1kArgs a)
     int i = 0, nf = (int)nfl;
     if (U8) {
         if (lane == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_s));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_s + 8u));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            mbar_init(bar_s, 1);
+            mbar_init(bar_s + 8u, 1);
+            mbar_init_fence();
             if (bulk(s0)) tma_load(s0, 0);
         }
         __syncwarp();
@@ -149,10 +149,7 @@ __global__ void __launch_bounds__(P1K_WARPS * 32, 2) psd1024_kernel(Psd1kArgs a)
                 if (more && bulk(ns)) tma_load(ns, buf ^ 1);
             }
             if (bulk(s0)) {
-                uint32_t done = 0;
-                while (!done)
-                    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
-                                 : "=r"(done) : "r"(bar_s + 8u * buf), "r"((tph >> buf) & 1u) : "memory");
+                mbar_wait(bar_s + 8u * buf, (tph >> buf) & 1u);
                 tph ^= 1u << buf;
                 const unsigned short *r16 = reinterpret_cast<const unsigned short *>(raw + buf * 2048);
 #pragma unroll
