@@ -833,6 +833,78 @@ int sdr_rrb_process(sdr_rrb_t *, const float *in_c64, const size_t *n_in, size_t
 int sdr_rrb_process_dev(sdr_rrb_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
                         size_t out_cap, size_t out_stride, size_t *n_out);
 
+/* ======================================================================================
+ * arbitrary-ratio resampler bank -- C independent c64 channel streams, channel k resampled by its own step sigma_k
+ * (input frames per output; any ratio, not only small rationals) on an exact time base, with real taps h_k of length L
+ * designed at P times the input rate (P a power of two): GNU Radio's pfb_arb_resampler idea, a polyphase prototype
+ * with linear interpolation between adjacent phases.  Positions are exact in units of 2^-64 frames (sdr_arb_time_t);
+ * m counts the handle's frames of the channel and frames before the stream are 0:
+ *   tau_k(r) = tau_k(0) + r sigma_k                                              (exact integer arithmetic)
+ *   H_k(t) = (1 - a) h_k[j] + a h_k[j+1],  j = floor(t P), a = t P - j,  0 <= j < L (h_k[L] = 0); 0 otherwise
+ *   z_k[r] = sum_{0 <= m <= floor(tau_k(r))} H_k(tau_k(r) - m) y_k[m]
+ * Computed form: n0 = floor(tau), f = its 64-bit fraction, p = log2 P, ip = f >> (64 - p) (0 when P = 1),
+ * a = ((f << p) >> 40) 2^-24 (exact in f32: the weight sees the position truncated to 2^-(24+p) frames), the table
+ * d_k[j] = f32(h_k[j+1] - h_k[j]) computed in f64 at create, c_i = fmaf(a, d_k[iP + ip], h_k[iP + ip]), and
+ *   acc = fmaf(c_i, y_k[n0 - i], acc)   for i = 0, 1, ... while iP + ip < L
+ * as one fmaf chain per component: frames before the stream are 0 and still multiplied (NaNs propagate exactly), taps
+ * past L never are, and an output's bits depend only on its inputs and its absolute position -- not on tiling,
+ * blocking or launch geometry.
+ * Counts: output r depends on frames <= floor(tau(r)), so after n frames a channel has released #{r : tau(r) < n} =
+ * ceil((n - tau(0)) / sigma) when n > tau(0), else 0 (exact integer arithmetic); a call's count is the difference of two
+ * such values and depends only on that channel's frames.
+ * Relation to sdr_rrb: with P = I, sigma = D / I, r0 = ceil(I / D) - 1 and tau(0) = ((r0+1) D - I) / I, the outputs are
+ * sdr_rrb's outputs r >= r0 bit for bit (a = 0); an output whose tau lies in (n-1, n) is released one frame earlier.
+ * Retuning: sdr_arb_set_steps gives every channel a new step from its next unreleased output R on,
+ * tau(R + e) = tau_old(R) + e sigma_new; released outputs do not change.  reset restores the creation positions and
+ * steps, clone copies the current ones.
+ * Shards are anchored on outputs: for any R0_k and a common frame f <= min_k(floor(tau_k(R0_k)) - ceil(L / P) + 1), a
+ * handle fed the stream from frame f with first positions tau_k(R0_k) - f and the same steps produces outputs R0_k,
+ * R0_k + 1, ... of the whole stream bit for bit.
+ * Limits: 2^-16 <= sigma <= 2^24, P <= 2^16, L <= 2^20, n_tap_sets L <= 2^26, C <= 65536; position whole parts, frame
+ * totals and per-call counts stay below 2^62, else SDR_ERR_INVALID_ARG.
+ * Scale: none.  Unit gain needs sum h = P.
+ * Accuracy: |z_k - z_k,f64| <= 1e-5 max|z_k,f64| at exact positions (DESIGN.md K14).
+ * Input and output rows are sdr_rrb's: C rows, row k of n_in[k] c64 frames, row stride in_stride (>= the longest row
+ * when C > 1); C output rows of out_stride (>= the largest count when C > 1), out_cap outputs per row; a too-small
+ * out_cap returns SDR_ERR_OUTPUT_TOO_SMALL before any state changes; *n_out receives C counts.
+ * Carried state: the last ceil(L / P) frames of every channel, the frame totals and the time base.  One compute launch
+ * per call for all channels and one small launch that updates the carried frames.  Device pointers need c64 (8-byte)
+ * alignment.
+ * ====================================================================================== */
+typedef struct {
+    uint64_t whole, frac; /* whole + frac / 2^64 input frames */
+} sdr_arb_time_t;
+
+typedef struct {
+    const float *taps;           /* n_tap_sets rows of n_taps real f32: the prototype at P times the input rate */
+    size_t n_taps;               /* L, 1 <= L <= 2^20 */
+    size_t n_tap_sets;           /* 1 (shared) or n_channels; n_tap_sets * n_taps <= 2^26 */
+    size_t phases;               /* P, a power of two, 1 <= P <= 2^16 */
+    const sdr_arb_time_t *step;  /* n_channels steps, 2^-16 <= sigma <= 2^24 */
+    const sdr_arb_time_t *first; /* n_channels first positions (whole part < 2^62), or NULL = all 0 */
+    size_t n_channels;           /* C, 1 <= C <= 65536 */
+    int device;
+    void *stream;
+} sdr_arb_config_t;
+
+typedef struct sdr_arb sdr_arb_t;
+/* host, pure: rate_in / rate_out rounded to the nearest 2^-64 (ties to even); SDR_ERR_INVALID_ARG for a non-finite or
+ * non-positive rate or a result outside [2^-16, 2^24] */
+int sdr_arb_step(double rate_in, double rate_out, sdr_arb_time_t *step);
+sdr_arb_t *sdr_arb_create(const sdr_arb_config_t *cfg, int *err);
+void sdr_arb_destroy(sdr_arb_t *);
+int sdr_arb_reset(sdr_arb_t *); /* creation positions and steps, frame counts back to 0 */
+sdr_arb_t *sdr_arb_clone(const sdr_arb_t *, int *err);
+/* n_channels new steps, from each channel's next unreleased output on */
+int sdr_arb_set_steps(sdr_arb_t *, const sdr_arb_time_t *steps);
+/* counts[k] = channel k's outputs from its next n_in[k] frames (C entries each) */
+int sdr_arb_output_count(const sdr_arb_t *, const size_t *n_in, size_t *counts);
+int sdr_arb_process(sdr_arb_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                    size_t out_cap, size_t out_stride, size_t *n_out);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_arb_process_dev(sdr_arb_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                        size_t out_cap, size_t out_stride, size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

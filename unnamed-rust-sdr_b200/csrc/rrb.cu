@@ -18,6 +18,7 @@
 #include <tuple>
 #include <vector>
 
+#include "bank.cuh"
 #include "kernels.h"
 
 using namespace sdr;
@@ -101,15 +102,7 @@ __global__ void __launch_bounds__(RRB_THREADS) rrb_kernel(const float *__restric
                                                           float2 *__restrict__ out, long long out_stride) {
     __shared__ int k_s;
     for (long long t = blockIdx.x; t < tiles; t += gridDim.x) {
-        if (threadIdx.x == 0) {  // the channel whose tiles hold t: tile0[k] <= t < tile0[k + 1]
-            int a = 0, b = C;
-            while (b - a > 1) {
-                const int m = (a + b) >> 1;
-                if (__ldg(tile0 + m) <= t) a = m;
-                else b = m;
-            }
-            k_s = a;
-        }
+        if (threadIdx.x == 0) k_s = bank_tile_channel(tile0, C, t);
         __syncthreads();
         const int k = k_s;
         __syncthreads();
@@ -150,12 +143,7 @@ __global__ void __launch_bounds__(RRB_THREADS) rrb_carry_kernel(const RrbChan *_
                                                                 float2 *__restrict__ hist_new) {
     const int k = blockIdx.x;
     const RrbChan ch = chans[k];
-    const long long n = calls[k].n;
-    const float2 *y = in + k * in_stride;
-    for (int j = threadIdx.x; j < ch.H; j += blockDim.x) {
-        const long long s = n - ch.H + j;
-        hist_new[ch.hist + j] = s >= 0 ? __ldg(y + s) : __ldg(hist_old + ch.hist + ch.H + s);
-    }
+    bank_carry(hist_old, in + k * in_stride, calls[k].n, ch.H, ch.hist, hist_new);
 }
 
 unsigned long long gcd_ull(unsigned long long a, unsigned long long b) {

@@ -472,6 +472,63 @@ class Rrb : public Handle<sdr_rrb_t, sdr_rrb_destroy, sdr_rrb_clone> {
     void reset() { check(sdr_rrb_reset(h_), "Rrb::reset"); }
 };
 
+// Arbitrary-ratio resampler bank (sdr_arb): channel k resampled by its own step (input frames per output, exact in
+// units of 2^-64) with real taps designed at P times the input rate, interpolated between adjacent phases.  After n
+// frames a channel has released #{r : tau(r) < n} outputs; there is no scale (unit gain needs sum h = P).
+class Arb : public Handle<sdr_arb_t, sdr_arb_destroy, sdr_arb_clone> {
+    size_t c_ = 0;
+
+  public:
+    // rate_in / rate_out to the nearest 2^-64
+    static sdr_arb_time_t step(double rate_in, double rate_out) {
+        sdr_arb_time_t t{};
+        check(sdr_arb_step(rate_in, rate_out, &t), "Arb::step");
+        return t;
+    }
+    // first: empty (all 0) or one position per channel
+    Arb(const std::vector<float> &taps, size_t n_taps, size_t phases, const std::vector<sdr_arb_time_t> &steps,
+        const std::vector<sdr_arb_time_t> &first = {})
+        : c_(steps.size()) {
+        if (!first.empty() && first.size() != steps.size()) throw sdr::Error(SDR_ERR_INVALID_ARG, "Arb::new");
+        sdr_arb_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.phases = phases;
+        cfg.step = steps.data();
+        cfg.first = first.empty() ? nullptr : first.data();
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_arb_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Arb::new");
+    }
+    size_t channels() const { return c_; }
+    void set_steps(const std::vector<sdr_arb_time_t> &steps) {
+        if (steps.size() != c_) throw sdr::Error(SDR_ERR_INVALID_ARG, "Arb::set_steps");
+        check(sdr_arb_set_steps(h_, steps.data()), "Arb::set_steps");
+    }
+    std::vector<size_t> output_count(const std::vector<size_t> &n_in) const {
+        std::vector<size_t> cnt(c_);
+        check(sdr_arb_output_count(h_, n_in.data(), cnt.data()), "Arb::output_count");
+        return cnt;
+    }
+    // in: channels rows, row k of n_in[k] frames at row stride in_stride (>= the longest row).  out: one vector per
+    // channel, replaced.
+    void process(const Complex *in, const std::vector<size_t> &n_in, size_t in_stride,
+                 std::vector<std::vector<Complex>> &out) {
+        const std::vector<size_t> cnt = output_count(n_in);
+        const size_t cap = std::max<size_t>(1, *std::max_element(cnt.begin(), cnt.end()));
+        std::vector<Complex> rows(cap * c_);
+        std::vector<size_t> got(c_);
+        check(sdr_arb_process(h_, reinterpret_cast<const float *>(in), n_in.data(), in_stride,
+                              reinterpret_cast<float *>(rows.data()), cap, cap, got.data()),
+              "Arb::process");
+        out.assign(c_, {});
+        for (size_t k = 0; k < c_; ++k) out[k].assign(rows.begin() + k * cap, rows.begin() + k * cap + got[k]);
+    }
+    void reset() { check(sdr_arb_reset(h_), "Arb::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

@@ -539,6 +539,76 @@ impl Drop for GpuRrb {
     fn drop(&mut self) { unsafe { sdr_rrb_destroy(self.h) } }
 }
 
+/// Arbitrary-ratio resampler bank: channel k resampled by its own step (input frames per output, exact in units of
+/// 2^-64) with real taps designed at `phases` times the input rate, interpolated between adjacent phases.  After n
+/// frames a channel has released #{r : tau(r) < n} outputs; unit gain needs taps summing to `phases`.
+pub struct GpuArb {
+    h: *mut sdr_arb_t,
+    c: usize,
+}
+unsafe impl Send for GpuArb {}
+
+impl GpuArb {
+    /// rate_in / rate_out to the nearest 2^-64
+    pub fn step(rate_in: f64, rate_out: f64) -> Result<sdr_arb_time_t, Error> {
+        let mut t = sdr_arb_time_t::default();
+        check(unsafe { sdr_arb_step(rate_in, rate_out, &mut t) })?;
+        Ok(t)
+    }
+    /// taps: one row of n_taps (shared) or one row per channel; one step per channel; first: empty (all 0) or one
+    /// position per channel
+    pub fn new(taps: &[f32], n_taps: usize, phases: usize, steps: &[sdr_arb_time_t], first: &[sdr_arb_time_t])
+               -> Result<Self, Error> {
+        if n_taps == 0 || (!first.is_empty() && first.len() != steps.len()) { return Err(Error(100)); }
+        let cfg = sdr_arb_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: taps.len() / n_taps, phases, step: steps.as_ptr(),
+            first: if first.is_empty() { std::ptr::null() } else { first.as_ptr() }, n_channels: steps.len(),
+            device: 0, stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_arb_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuArb { h, c: steps.len() })
+    }
+    /// new steps from each channel's next unreleased output on
+    pub fn set_steps(&mut self, steps: &[sdr_arb_time_t]) -> Result<(), Error> {
+        assert!(steps.len() == self.c);
+        check(unsafe { sdr_arb_set_steps(self.h, steps.as_ptr()) })
+    }
+    /// input: one row per channel, row k of n_in[k] frames at row stride `stride` (>= the longest row); channel k's
+    /// outputs are appended to output[k]
+    pub fn process(&mut self, input: &[Complex<f32>], n_in: &[usize], stride: usize,
+                   output: &mut [Vec<Complex<f32>>]) -> Result<(), Error> {
+        assert!(n_in.len() == self.c);
+        assert!(n_in.iter().enumerate().all(|(k, &n)| n == 0 || input.len() >= k * stride + n));
+        let mut cnt = vec![0usize; self.c];
+        check(unsafe { sdr_arb_output_count(self.h, n_in.as_ptr(), cnt.as_mut_ptr()) })?;
+        let cap = cnt.iter().copied().max().unwrap_or(0).max(1);
+        let mut rows = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut got = vec![0usize; self.c];
+        check(unsafe {
+            sdr_arb_process(self.h, input.as_ptr() as *const f32, n_in.as_ptr(), stride, rows.as_mut_ptr() as *mut f32,
+                            cap, cap, got.as_mut_ptr())
+        })?;
+        for (k, out) in output.iter_mut().enumerate().take(self.c) {
+            out.extend_from_slice(&rows[k * cap..k * cap + got[k]]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_arb_reset(self.h) }) }
+}
+impl Clone for GpuArb {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_arb_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_arb_clone failed: {}", Error(err));
+        GpuArb { h, c: self.c }
+    }
+}
+impl Drop for GpuArb {
+    fn drop(&mut self) { unsafe { sdr_arb_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

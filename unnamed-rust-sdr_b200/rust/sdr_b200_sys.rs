@@ -46,6 +46,7 @@ pub enum sdr_pfs_t {}
 pub enum sdr_duc_t {}
 pub enum sdr_fcsb_t {}
 pub enum sdr_rrb_t {}
+pub enum sdr_arb_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -225,6 +226,27 @@ pub struct sdr_rrb_config_t {
     pub stream: *mut c_void,
 }
 
+/// whole + frac / 2^64 input frames
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default, PartialEq, Eq)]
+pub struct sdr_arb_time_t {
+    pub whole: u64,
+    pub frac: u64,
+}
+
+#[repr(C)]
+pub struct sdr_arb_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub phases: size_t,
+    pub step: *const sdr_arb_time_t,
+    pub first: *const sdr_arb_time_t,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
 #[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
@@ -389,6 +411,17 @@ extern "C" {
     pub fn sdr_rrb_process(h: *mut sdr_rrb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
                            out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_rrb_process_dev(h: *mut sdr_rrb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                               out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_arb_step(rate_in: c_double, rate_out: c_double, step: *mut sdr_arb_time_t) -> c_int;
+    pub fn sdr_arb_create(cfg: *const sdr_arb_config_t, err: *mut c_int) -> *mut sdr_arb_t;
+    pub fn sdr_arb_destroy(h: *mut sdr_arb_t);
+    pub fn sdr_arb_reset(h: *mut sdr_arb_t) -> c_int;
+    pub fn sdr_arb_clone(h: *const sdr_arb_t, err: *mut c_int) -> *mut sdr_arb_t;
+    pub fn sdr_arb_set_steps(h: *mut sdr_arb_t, steps: *const sdr_arb_time_t) -> c_int;
+    pub fn sdr_arb_output_count(h: *const sdr_arb_t, n_in: *const size_t, counts: *mut size_t) -> c_int;
+    pub fn sdr_arb_process(h: *mut sdr_arb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                           out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_arb_process_dev(h: *mut sdr_arb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
                                out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs

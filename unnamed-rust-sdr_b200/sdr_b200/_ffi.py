@@ -102,6 +102,15 @@ class RrbConfig(C.Structure):
                 ("n_channels", sz), ("device", i32), ("stream", vp)]
 
 
+class ArbTime(C.Structure):
+    _fields_ = [("whole", C.c_uint64), ("frac", C.c_uint64)]
+
+
+class ArbConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phases", sz), ("step", vp), ("first", vp),
+                ("n_channels", sz), ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -210,6 +219,15 @@ PROTOTYPES = {
     "sdr_rrb_output_count": (i32, [vp, vp, vp]),
     "sdr_rrb_process": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
     "sdr_rrb_process_dev": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
+    "sdr_arb_step": (i32, [C.c_double, C.c_double, C.POINTER(ArbTime)]),
+    "sdr_arb_create": (vp, [C.POINTER(ArbConfig), C.POINTER(i32)]),
+    "sdr_arb_destroy": (None, [vp]),
+    "sdr_arb_reset": (i32, [vp]),
+    "sdr_arb_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_arb_set_steps": (i32, [vp, vp]),
+    "sdr_arb_output_count": (i32, [vp, vp, vp]),
+    "sdr_arb_process": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
+    "sdr_arb_process_dev": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -902,6 +902,99 @@ class Rrb(_Handle):
 
 
 
+_ONE = 1 << 64  # one input frame in the units of Arb's steps and positions
+
+
+def _arb_times(v, c, what):
+    """ints in units of 2^-64 frames (one, or one per channel) -> ctypes array of c ArbTime"""
+    v = [int(x) for x in (v if hasattr(v, "__len__") else [v])]
+    v = v * c if len(v) == 1 else v
+    if len(v) != c or any(x < 0 or x >> 128 for x in v):
+        raise ValueError("%s: one value in [0, 2^128), or one per channel, in units of 2^-64 frames" % what)
+    return (F.ArbTime * c)(*[F.ArbTime(x >> 64, x & (_ONE - 1)) for x in v])
+
+
+def arb_step(rate_in, rate_out):
+    """rate_in / rate_out rounded to the nearest 2^-64 (ties to even), as an int in units of 2^-64 frames"""
+    t = F.ArbTime()
+    check(lib().sdr_arb_step(float(rate_in), float(rate_out), C.byref(t)), "sdr_arb_step")
+    return (t.whole << 64) | t.frac
+
+
+class Arb(_Handle):
+    """Arbitrary-ratio resampler bank (sdr_arb): channel k resampled by its own step sigma_k (input frames per output)
+    on an exact time base, with real taps designed at `phases` (P, a power of two) times the input rate (1-D: shared;
+    [C, L]: one row per channel), linearly interpolated between adjacent phases.  Output r sits at
+    tau_k(r) = first_k + r sigma_k.  steps and first are Python ints in units of 2^-64 frames (arb_step converts a rate
+    pair), one value or one per channel; first defaults to 0.  After n frames a channel has released
+    #{r : tau(r) < n} outputs.  There is no scale: unit gain needs sum(taps) = P."""
+
+    _abi = "arb"
+
+    def __init__(self, taps, phases, steps, first=None, n_channels=None, device=0, stream=None):
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        ns = len(steps) if hasattr(steps, "__len__") else 1
+        nf = len(first) if hasattr(first, "__len__") else 1
+        c = int(n_channels) if n_channels is not None else max(ns, nf, 1 if t.ndim == 1 else t.shape[0])
+        self._taps = t
+        self.n_channels = c
+        self.phases = int(phases)
+        self._steps = _arb_times(steps, c, "steps")
+        self._first = None if first is None else _arb_times(first, c, "first")
+        cfg = F.ArbConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phases,
+                          C.addressof(self._steps), None if self._first is None else C.addressof(self._first), c,
+                          device, _stream_ptr(stream))
+        self._create(cfg)
+
+    def set_steps(self, steps):
+        """new steps (ints in units of 2^-64, one or one per channel) from each channel's next unreleased output on"""
+        s = _arb_times(steps, self.n_channels, "steps")
+        check(lib().sdr_arb_set_steps(self.h, C.addressof(s)), "sdr_arb_set_steps")
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def output_count(self, n_in):
+        """outputs per channel (numpy array of C) from the next n_in frames (an int, or one count per channel)"""
+        n = self._counts(n_in)
+        cnt = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_arb_output_count(self.h, n.ctypes.data, cnt.ctypes.data), "sdr_arb_output_count")
+        return cnt.astype(np.int64)
+
+    def process(self, rows):
+        """rows: complex64 [C, n] or a list of C rows of any lengths -> list of C complex64 arrays"""
+        if isinstance(rows, np.ndarray) and rows.ndim == 1 and self.n_channels == 1:
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n = np.array([r.size for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        y = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            y[k, :r.size] = r
+        cnt = self.output_count(n)
+        cap = max(int(cnt.max()), 1)
+        out = np.empty((self.n_channels, cap), np.complex64)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_arb_process(self.h, y.ctypes.data, n.ctypes.data, stride, out.ctypes.data, cap, cap,
+                                    got.ctypes.data), "sdr_arb_process")
+        return [out[k, :int(got[k])] for k in range(self.n_channels)]
+
+    def process_dev(self, d_in, n_in, in_stride, d_out, out_cap, out_stride):
+        """device-resident: d_in C rows of in_stride complex64, row k of n_in (an int, or C counts) frames; d_out C rows
+        of out_stride complex64, out_cap outputs each; asynchronous on the handle's stream.  Returns the outputs written
+        per channel (numpy array of C)."""
+        n = self._counts(n_in)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_arb_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), out_cap, out_stride,
+                                        got.ctypes.data), "sdr_arb_process_dev")
+        return got.astype(np.int64)
+
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
