@@ -905,6 +905,86 @@ int sdr_arb_process(sdr_arb_t *, const float *in_c64, const size_t *n_in, size_t
 int sdr_arb_process_dev(sdr_arb_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
                         size_t out_cap, size_t out_stride, size_t *n_out);
 
+/* ======================================================================================
+ * symbol timing recovery bank -- C independent c64 channel streams, each with a Gardner timing loop that steers
+ * sdr_arb's interpolator on the same exact time base.  Channel k has real taps h_k of length L designed at P = 2^p
+ * times the input rate (typically the matched filter, e.g. a root-raised cosine), a nominal symbol period T_k in input
+ * frames (sdr_arb_time_t: sdr_arb_step(rate, symbol_rate) gives it), a first on-time position tau_k(0) and a loop
+ * {kp, ki, err_max, max_dev}.  Positions are 64.64 values in units of 2^-64 frames; loop quantities are int64 in
+ * units of 2^-40 frames, q(x) = (int64) rint(x 2^40) for an f32 x (exact scaling; create guarantees it fits), and
+ * V = floor(max_dev T) in those units, exact from the double's binary value.
+ * A(t) is sdr_arb's computed form at absolute position t, bit for bit: the same (h, d) table, the same 2^-24-truncated
+ * weight and the same fmaf chain; frames before the stream are 0.  With v_0 = 0 and y_{-1} = 0, for s = 0, 1, 2, ...:
+ *   T_s       = T + 2^24 v_s                                     (units of 2^-64; |v_s| <= V)
+ *   y_s       = A(tau_s)                                         (the output symbol)
+ *   m_s       = A(tau_s - floor(T_s / 2))                        (mid-symbol sample, s >= 1)
+ *   g         = fl(fl(fl(y_s.re - y_{s-1}.re) m_s.re) + fl(fl(y_s.im - y_{s-1}.im) m_s.im))
+ *   e_s       = 0 for s = 0 or a non-finite g, else min(max(g, -err_max), err_max)
+ *   v_{s+1}   = clamp(v_s - q(fl(ki e_s)), -V, V)
+ *   tau_{s+1} = tau_s + T + 2^24 v_{s+1} - 2^24 q(fl(kp e_s))
+ * e_s is Gardner's detector Re{(y_s - y_{s-1}) conj(m_s)}: e > 0 means the on-time sample is late, so both corrections
+ * subtract.  Every f32 operation is rounded on its own (nothing is contracted into an FMA), so a float32 restatement
+ * reproduces e, v and tau exactly.  A NaN frame makes the symbols whose chains read it NaN; their errors count as 0,
+ * so positions stay finite and deterministic.
+ * Validity at create, with D = 2^24 q(fl(kp err_max)): 2 D < T - V, so every step tau_{s+1} - tau_s is at least
+ * T_min = T - V - D > 0 and every mid sample m_{s+1} lies after tau_s.  Also rejected (SDR_ERR_INVALID_ARG): max_dev
+ * outside [0, 0.25], negative or non-finite kp / ki, err_max <= 0 or non-finite, T outside [1, 2^20] frames,
+ * fl(ki err_max) >= 2^22 frames, sdr_arb's limits on P, L, C and tap sets, first whole parts >= 2^62.
+ * Release: symbol s is released by the first call after which the channel's frame total n satisfies
+ * floor(tau_s) < n (its mid sample lies earlier), so with kp = ki = 0 the counts are sdr_arb's #{r : tau(r) < n}.
+ * Counts depend on the data: sdr_tsync_max_output gives the host-computable bound ceil(n_in 2^64 / T_min) per channel
+ * (every unreleased tau is >= the previous frame total); a call whose out_cap is below the largest bound returns
+ * SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  This is the one bank whose counts come from the device:
+ * sdr_tsync_process_dev enqueues its work, copies the C counts back and synchronises the handle's stream.
+ * Rows are sdr_arb's: C input rows of n_in[k] frames at in_stride (>= the longest row when C > 1), C output rows of
+ * out_stride (>= the largest bound when C > 1); pos (the exact tau_s) and err (e_s) share that stride and may be NULL.
+ * Outputs of sdr_ddc, sdr_fcfb and sdr_arb (and sdr_pfb's channel-major rows) feed it unchanged.
+ * Carried state per channel: the last ceil(L / P) + ceil((T + V) / 2) + 1 frames, tau of the next unreleased symbol,
+ * v, y_{s-1} and the frame total.  reset restores the creation state; clone copies the current one, device part
+ * included.  A call is at most 2 launches (compute, carry) and one small copy of the counts back.
+ * Not shardable by range: the loop is a recurrence, so the bank shards by channel only.
+ * Device pointers need c64 (8-byte) alignment for rows and positions, 4 bytes for err.
+ * ====================================================================================== */
+typedef struct {
+    float kp, ki;   /* proportional and integral gains, frames per unit of e (sdr_tsync_loop_design) */
+    float err_max;  /* the detector output is clamped to [-err_max, err_max] */
+    double max_dev; /* |v| <= max_dev T, 0 <= max_dev <= 0.25 */
+} sdr_tsync_loop_t;
+
+typedef struct {
+    const float *taps;             /* as sdr_arb_config_t: n_tap_sets rows of n_taps real f32 at P times the rate */
+    size_t n_taps, n_tap_sets, phases;
+    const sdr_arb_time_t *period;  /* n_channels nominal periods T_k, 1 <= T_k <= 2^20 frames */
+    const sdr_arb_time_t *first;   /* n_channels first positions (whole part < 2^62), or NULL = all 0 */
+    const sdr_tsync_loop_t *loops; /* n_loops loop parameter sets */
+    size_t n_loops;                /* 1 (shared) or n_channels */
+    size_t n_channels;             /* C, 1 <= C <= 65536 */
+    int device;
+    void *stream;
+} sdr_tsync_config_t;
+
+typedef struct sdr_tsync sdr_tsync_t;
+/* host, pure: gains of the standard second-order (PI, type-2) loop for a noise bandwidth bn_t (normalised to the
+ * symbol rate), damping zeta, detector slope ted_gain (mean e per symbol period of timing error) and a period of
+ * period_frames input frames:
+ *   theta = bn_t / (zeta + 1 / (4 zeta)),  delta = 1 + 2 zeta theta + theta^2,
+ *   kp = 4 zeta theta / (delta ted_gain) period_frames,  ki = 4 theta^2 / (delta ted_gain) period_frames
+ * in frames per unit of e (this bank's units); SDR_ERR_INVALID_ARG unless every argument is positive and finite */
+int sdr_tsync_loop_design(double bn_t, double zeta, double ted_gain, double period_frames, float *kp, float *ki);
+sdr_tsync_t *sdr_tsync_create(const sdr_tsync_config_t *cfg, int *err);
+void sdr_tsync_destroy(sdr_tsync_t *);
+int sdr_tsync_reset(sdr_tsync_t *); /* creation positions, v = 0, y_{-1} = 0, frame totals back to 0 */
+sdr_tsync_t *sdr_tsync_clone(const sdr_tsync_t *, int *err);
+/* caps[k] = ceil(n_in[k] 2^64 / T_min_k): the most symbols channel k can release from its next n_in[k] frames */
+int sdr_tsync_max_output(const sdr_tsync_t *, const size_t *n_in, size_t *caps);
+int sdr_tsync_process(sdr_tsync_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *sym_c64,
+                      sdr_arb_time_t *pos, float *err, size_t out_cap, size_t out_stride, size_t *n_out);
+/* device pointers; returns after the counts are copied back (synchronises the handle's stream) */
+int sdr_tsync_process_dev(sdr_tsync_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *sym_c64,
+                          sdr_arb_time_t *pos, float *err, size_t out_cap, size_t out_stride, size_t *n_out);
+/* the next unreleased position and the period offset v (2^-40 frames) of one channel; synchronises */
+int sdr_tsync_get_state(sdr_tsync_t *, size_t channel, sdr_arb_time_t *next, int64_t *v);
+
 #ifdef __cplusplus
 }
 #endif

@@ -18,6 +18,7 @@
 #include <new>
 #include <vector>
 
+#include "arb_core.cuh"
 #include "bank.cuh"
 #include "kernels.h"
 
@@ -51,30 +52,6 @@ struct ArbCall {                  // per channel and call; frames are relative t
     long long lo;                 // frames below lo lie before the stream and read as 0
     long long pad;
 };
-
-// frame j of a channel: hist[j] for j < 0 (hist points one past the carried frames), y[j] for 0 <= j < n, else 0
-__device__ __forceinline__ float2 arb_load(const float2 *hist, const float2 *y, long long j, long long lo) {
-    if (j < lo) return make_float2(0.f, 0.f);
-    if (j < 0) return __ldg(hist + j);
-    return __ldg(y + j);
-}
-
-// the chain of one output: T terms, frame n0 - i and table entry tb[i P] (tb = the table at ip).  CHECK = false when
-// every frame read lies in the caller's row.
-template <bool CHECK>
-__device__ __forceinline__ float2 arb_chain(const float2 *__restrict__ tb, int T, int P, float a, const float2 *hist,
-                                            const float2 *y, long long n0, long long lo) {
-    float2 acc = make_float2(0.f, 0.f);
-#pragma unroll 4
-    for (int i = 0; i < T; ++i) {
-        const float2 hd = __ldg(tb + (long long)i * P);
-        const float c = __fmaf_rn(a, hd.y, hd.x);
-        const float2 v = CHECK ? arb_load(hist, y, n0 - i, lo) : __ldg(y + (n0 - i));
-        acc.x = __fmaf_rn(c, v.x, acc.x);
-        acc.y = __fmaf_rn(c, v.y, acc.y);
-    }
-    return acc;
-}
 
 // One CTA per tile of ARB_THREADS consecutive outputs over the flattened (channel, output) space: channel k owns tiles
 // [tile0[k], tile0[k+1]).  Lane e of a tile takes output e, so a warp's frame loads span about 32 sigma frames.

@@ -529,6 +529,82 @@ class Arb : public Handle<sdr_arb_t, sdr_arb_destroy, sdr_arb_clone> {
     void reset() { check(sdr_arb_reset(h_), "Arb::reset"); }
 };
 
+// Symbol timing recovery bank (sdr_tsync): a Gardner loop per channel steering sdr_arb's interpolator on the exact
+// 64.64 time base.  Channel k: matched filter taps at P times the input rate, a nominal period (Arb::step(rate,
+// symbol_rate)), a first position and loop parameters {kp, ki, err_max, max_dev}; each call returns the released symbols
+// with their exact positions and detector outputs.  Counts come from the device, so every call synchronises.
+class Tsync : public Handle<sdr_tsync_t, sdr_tsync_destroy, sdr_tsync_clone> {
+    size_t c_ = 0;
+
+  public:
+    struct Out {
+        std::vector<std::vector<Complex>> sym;
+        std::vector<std::vector<sdr_arb_time_t>> pos;
+        std::vector<std::vector<float>> err;
+    };
+    // kp, ki in frames per unit of detector output for a noise bandwidth bn_t, damping zeta and detector slope ted_gain
+    static std::pair<float, float> loop_design(double bn_t, double zeta, double ted_gain, double period_frames) {
+        float kp = 0, ki = 0;
+        check(sdr_tsync_loop_design(bn_t, zeta, ted_gain, period_frames, &kp, &ki), "Tsync::loop_design");
+        return {kp, ki};
+    }
+    // loops: one (shared) or one per channel; first: empty (all 0) or one position per channel
+    Tsync(const std::vector<float> &taps, size_t n_taps, size_t phases, const std::vector<sdr_arb_time_t> &periods,
+          const std::vector<sdr_tsync_loop_t> &loops, const std::vector<sdr_arb_time_t> &first = {})
+        : c_(periods.size()) {
+        if (!first.empty() && first.size() != periods.size()) throw sdr::Error(SDR_ERR_INVALID_ARG, "Tsync::new");
+        sdr_tsync_config_t cfg{};
+        cfg.taps = taps.data();
+        cfg.n_taps = n_taps;
+        cfg.n_tap_sets = n_taps ? taps.size() / n_taps : 0;
+        cfg.phases = phases;
+        cfg.period = periods.data();
+        cfg.first = first.empty() ? nullptr : first.data();
+        cfg.loops = loops.data();
+        cfg.n_loops = loops.size();
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_tsync_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Tsync::new");
+    }
+    size_t channels() const { return c_; }
+    std::vector<size_t> max_output(const std::vector<size_t> &n_in) const {
+        std::vector<size_t> cap(c_);
+        check(sdr_tsync_max_output(h_, n_in.data(), cap.data()), "Tsync::max_output");
+        return cap;
+    }
+    // next unreleased position and v (units of 2^-40 frames) of one channel
+    std::pair<sdr_arb_time_t, int64_t> state(size_t k) {
+        sdr_arb_time_t t{};
+        int64_t v = 0;
+        check(sdr_tsync_get_state(h_, k, &t, &v), "Tsync::state");
+        return {t, v};
+    }
+    // in: channels rows, row k of n_in[k] frames at row stride in_stride (>= the longest row)
+    Out process(const Complex *in, const std::vector<size_t> &n_in, size_t in_stride) {
+        const std::vector<size_t> caps = max_output(n_in);
+        const size_t cap = std::max<size_t>(1, *std::max_element(caps.begin(), caps.end()));
+        std::vector<Complex> sym(cap * c_);
+        std::vector<sdr_arb_time_t> pos(cap * c_);
+        std::vector<float> err(cap * c_);
+        std::vector<size_t> got(c_);
+        check(sdr_tsync_process(h_, reinterpret_cast<const float *>(in), n_in.data(), in_stride,
+                                reinterpret_cast<float *>(sym.data()), pos.data(), err.data(), cap, cap, got.data()),
+              "Tsync::process");
+        Out o;
+        o.sym.resize(c_);
+        o.pos.resize(c_);
+        o.err.resize(c_);
+        for (size_t k = 0; k < c_; ++k) {
+            o.sym[k].assign(sym.begin() + k * cap, sym.begin() + k * cap + got[k]);
+            o.pos[k].assign(pos.begin() + k * cap, pos.begin() + k * cap + got[k]);
+            o.err[k].assign(err.begin() + k * cap, err.begin() + k * cap + got[k]);
+        }
+        return o;
+    }
+    void reset() { check(sdr_tsync_reset(h_), "Tsync::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

@@ -609,6 +609,84 @@ impl Drop for GpuArb {
     fn drop(&mut self) { unsafe { sdr_arb_destroy(self.h) } }
 }
 
+/// Symbol timing recovery bank: a Gardner loop per channel steering `GpuArb`'s interpolator on the exact 64.64 time
+/// base.  Channel k: matched-filter taps at `phases` times the input rate, a nominal period (`GpuArb::step(rate,
+/// symbol_rate)`), a first position and loop parameters; each call appends the released symbols, their exact positions
+/// and the detector outputs.  Counts come from the device, so every call synchronises.
+pub struct GpuTsync {
+    h: *mut sdr_tsync_t,
+    c: usize,
+}
+unsafe impl Send for GpuTsync {}
+
+impl GpuTsync {
+    /// (kp, ki) of the second-order loop for noise bandwidth bn_t, damping zeta and detector slope ted_gain
+    pub fn loop_design(bn_t: f64, zeta: f64, ted_gain: f64, period_frames: f64) -> Result<(f32, f32), Error> {
+        let (mut kp, mut ki) = (0.0f32, 0.0f32);
+        check(unsafe { sdr_tsync_loop_design(bn_t, zeta, ted_gain, period_frames, &mut kp, &mut ki) })?;
+        Ok((kp, ki))
+    }
+    /// taps: one row of n_taps (shared) or one row per channel; one period per channel; loops: one (shared) or one per
+    /// channel; first: empty (all 0) or one position per channel
+    pub fn new(taps: &[f32], n_taps: usize, phases: usize, periods: &[sdr_arb_time_t], loops: &[sdr_tsync_loop_t],
+               first: &[sdr_arb_time_t]) -> Result<Self, Error> {
+        if n_taps == 0 || (!first.is_empty() && first.len() != periods.len()) { return Err(Error(100)); }
+        let cfg = sdr_tsync_config_t {
+            taps: taps.as_ptr(), n_taps, n_tap_sets: taps.len() / n_taps, phases, period: periods.as_ptr(),
+            first: if first.is_empty() { std::ptr::null() } else { first.as_ptr() }, loops: loops.as_ptr(),
+            n_loops: loops.len(), n_channels: periods.len(), device: 0, stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_tsync_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuTsync { h, c: periods.len() })
+    }
+    /// next unreleased position and period offset v (units of 2^-40 frames) of one channel
+    pub fn state(&mut self, k: usize) -> Result<(sdr_arb_time_t, i64), Error> {
+        let mut t = sdr_arb_time_t::default();
+        let mut v = 0i64;
+        check(unsafe { sdr_tsync_get_state(self.h, k, &mut t, &mut v) })?;
+        Ok((t, v))
+    }
+    /// input: one row per channel, row k of n_in[k] frames at row stride `stride` (>= the longest row); channel k's
+    /// symbols, positions and errors are appended to sym[k], pos[k] and err[k]
+    pub fn process(&mut self, input: &[Complex<f32>], n_in: &[usize], stride: usize, sym: &mut [Vec<Complex<f32>>],
+                   pos: &mut [Vec<sdr_arb_time_t>], err: &mut [Vec<f32>]) -> Result<(), Error> {
+        assert!(n_in.len() == self.c);
+        assert!(n_in.iter().enumerate().all(|(k, &n)| n == 0 || input.len() >= k * stride + n));
+        let mut caps = vec![0usize; self.c];
+        check(unsafe { sdr_tsync_max_output(self.h, n_in.as_ptr(), caps.as_mut_ptr()) })?;
+        let cap = caps.iter().copied().max().unwrap_or(0).max(1);
+        let mut s = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut p = vec![sdr_arb_time_t::default(); cap * self.c];
+        let mut e = vec![0.0f32; cap * self.c];
+        let mut got = vec![0usize; self.c];
+        check(unsafe {
+            sdr_tsync_process(self.h, input.as_ptr() as *const f32, n_in.as_ptr(), stride, s.as_mut_ptr() as *mut f32,
+                              p.as_mut_ptr(), e.as_mut_ptr(), cap, cap, got.as_mut_ptr())
+        })?;
+        for k in 0..self.c {
+            let r = k * cap..k * cap + got[k];
+            sym[k].extend_from_slice(&s[r.clone()]);
+            pos[k].extend_from_slice(&p[r.clone()]);
+            err[k].extend_from_slice(&e[r]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_tsync_reset(self.h) }) }
+}
+impl Clone for GpuTsync {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_tsync_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_tsync_clone failed: {}", Error(err));
+        GpuTsync { h, c: self.c }
+    }
+}
+impl Drop for GpuTsync {
+    fn drop(&mut self) { unsafe { sdr_tsync_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

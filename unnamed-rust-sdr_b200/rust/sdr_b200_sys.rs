@@ -47,6 +47,7 @@ pub enum sdr_duc_t {}
 pub enum sdr_fcsb_t {}
 pub enum sdr_rrb_t {}
 pub enum sdr_arb_t {}
+pub enum sdr_tsync_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -248,6 +249,30 @@ pub struct sdr_arb_config_t {
 }
 
 #[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct sdr_tsync_loop_t {
+    pub kp: c_float,
+    pub ki: c_float,
+    pub err_max: c_float,
+    pub max_dev: c_double,
+}
+
+#[repr(C)]
+pub struct sdr_tsync_config_t {
+    pub taps: *const c_float,
+    pub n_taps: size_t,
+    pub n_tap_sets: size_t,
+    pub phases: size_t,
+    pub period: *const sdr_arb_time_t,
+    pub first: *const sdr_arb_time_t,
+    pub loops: *const sdr_tsync_loop_t,
+    pub n_loops: size_t,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
     pub rate: c_float,
@@ -423,6 +448,20 @@ extern "C" {
                            out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_arb_process_dev(h: *mut sdr_arb_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
                                out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_tsync_loop_design(bn_t: c_double, zeta: c_double, ted_gain: c_double, period_frames: c_double,
+                                 kp: *mut c_float, ki: *mut c_float) -> c_int;
+    pub fn sdr_tsync_create(cfg: *const sdr_tsync_config_t, err: *mut c_int) -> *mut sdr_tsync_t;
+    pub fn sdr_tsync_destroy(h: *mut sdr_tsync_t);
+    pub fn sdr_tsync_reset(h: *mut sdr_tsync_t) -> c_int;
+    pub fn sdr_tsync_clone(h: *const sdr_tsync_t, err: *mut c_int) -> *mut sdr_tsync_t;
+    pub fn sdr_tsync_max_output(h: *const sdr_tsync_t, n_in: *const size_t, caps: *mut size_t) -> c_int;
+    pub fn sdr_tsync_process(h: *mut sdr_tsync_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                             sym_c64: *mut c_float, pos: *mut sdr_arb_time_t, err: *mut c_float, out_cap: size_t,
+                             out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_tsync_process_dev(h: *mut sdr_tsync_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                                 sym_c64: *mut c_float, pos: *mut sdr_arb_time_t, err: *mut c_float, out_cap: size_t,
+                                 out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_tsync_get_state(h: *mut sdr_tsync_t, channel: size_t, next: *mut sdr_arb_time_t, v: *mut i64) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -111,6 +111,15 @@ class ArbConfig(C.Structure):
                 ("n_channels", sz), ("device", i32), ("stream", vp)]
 
 
+class TsyncLoop(C.Structure):
+    _fields_ = [("kp", C.c_float), ("ki", C.c_float), ("err_max", C.c_float), ("max_dev", C.c_double)]
+
+
+class TsyncConfig(C.Structure):
+    _fields_ = [("taps", vp), ("n_taps", sz), ("n_tap_sets", sz), ("phases", sz), ("period", vp), ("first", vp),
+                ("loops", vp), ("n_loops", sz), ("n_channels", sz), ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -228,6 +237,16 @@ PROTOTYPES = {
     "sdr_arb_output_count": (i32, [vp, vp, vp]),
     "sdr_arb_process": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
     "sdr_arb_process_dev": (i32, [vp, vp, vp, sz, vp, sz, sz, vp]),
+    "sdr_tsync_loop_design": (i32, [C.c_double, C.c_double, C.c_double, C.c_double, C.POINTER(C.c_float),
+                                    C.POINTER(C.c_float)]),
+    "sdr_tsync_create": (vp, [C.POINTER(TsyncConfig), C.POINTER(i32)]),
+    "sdr_tsync_destroy": (None, [vp]),
+    "sdr_tsync_reset": (i32, [vp]),
+    "sdr_tsync_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_tsync_max_output": (i32, [vp, vp, vp]),
+    "sdr_tsync_process": (i32, [vp, vp, vp, sz, vp, vp, vp, sz, sz, vp]),
+    "sdr_tsync_process_dev": (i32, [vp, vp, vp, sz, vp, vp, vp, sz, sz, vp]),
+    "sdr_tsync_get_state": (i32, [vp, sz, C.POINTER(ArbTime), C.POINTER(C.c_int64)]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

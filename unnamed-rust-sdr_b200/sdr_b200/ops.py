@@ -994,6 +994,102 @@ class Arb(_Handle):
         return got.astype(np.int64)
 
 
+def tsync_loop_design(bn_t, zeta, ted_gain, period_frames):
+    """(kp, ki) of the standard second-order loop, in frames per unit of detector output: noise bandwidth bn_t
+    (normalised to the symbol rate), damping zeta, detector slope ted_gain (mean e per symbol period of timing error)"""
+    kp, ki = C.c_float(), C.c_float()
+    check(lib().sdr_tsync_loop_design(float(bn_t), float(zeta), float(ted_gain), float(period_frames), C.byref(kp),
+                                      C.byref(ki)), "sdr_tsync_loop_design")
+    return kp.value, ki.value
+
+
+def _positions(a):
+    """[n, 2] uint64 (whole, frac) -> list of Python ints in units of 2^-64 frames"""
+    return [(int(w) << 64) | int(f) for w, f in a]
+
+
+class Tsync(_Handle):
+    """Symbol timing recovery bank (sdr_tsync): a Gardner loop per channel that steers sdr_arb's interpolator.  taps:
+    the matched filter at `phases` (P, a power of two) times the input rate (1-D: shared; [C, L]: one row per channel);
+    periods and first: Python ints in units of 2^-64 frames (arb_step(rate, symbol_rate) gives a period), one value or
+    one per channel, first defaulting to 0; loops: one (kp, ki, err_max, max_dev) or one per channel.  process returns
+    the symbols y_s, their exact positions tau_s and the detector outputs e_s; see include/sdr_b200.h for the
+    recurrence."""
+
+    _abi = "tsync"
+
+    def __init__(self, taps, phases, periods, loops, first=None, n_channels=None, device=0, stream=None):
+        t = np.ascontiguousarray(taps, np.float32)
+        if t.ndim not in (1, 2):
+            raise ValueError("taps must be 1-D (shared) or [channels, taps]")
+        lp = [loops] if np.ndim(loops[0]) == 0 else list(loops)
+        ns = len(periods) if hasattr(periods, "__len__") else 1
+        nf = len(first) if hasattr(first, "__len__") else 1
+        c = int(n_channels) if n_channels is not None else max(ns, nf, len(lp), 1 if t.ndim == 1 else t.shape[0])
+        self._taps = t
+        self.n_channels = c
+        self.phases = int(phases)
+        self._periods = _arb_times(periods, c, "periods")
+        self._first = None if first is None else _arb_times(first, c, "first")
+        self._loops = (F.TsyncLoop * len(lp))(*[F.TsyncLoop(*map(float, x)) for x in lp])
+        cfg = F.TsyncConfig(t.ctypes.data, t.shape[-1], 1 if t.ndim == 1 else t.shape[0], self.phases,
+                            C.addressof(self._periods), None if self._first is None else C.addressof(self._first),
+                            C.addressof(self._loops), len(lp), c, device, _stream_ptr(stream))
+        self._create(cfg)
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def max_output(self, n_in):
+        """the most symbols per channel (numpy array of C) the next n_in frames (an int, or one per channel) release"""
+        n = self._counts(n_in)
+        cap = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_tsync_max_output(self.h, n.ctypes.data, cap.ctypes.data), "sdr_tsync_max_output")
+        return cap.astype(np.int64)
+
+    def state(self, k):
+        """(next unreleased position as an int in units of 2^-64 frames, v in units of 2^-40 frames) of channel k"""
+        t, v = F.ArbTime(), C.c_int64()
+        check(lib().sdr_tsync_get_state(self.h, int(k), C.byref(t), C.byref(v)), "sdr_tsync_get_state")
+        return (t.whole << 64) | t.frac, v.value
+
+    def process(self, rows):
+        """rows: complex64 [C, n] or a list of C rows of any lengths -> (symbols, positions, errors): lists of C
+        complex64 arrays, C lists of Python ints (units of 2^-64 frames) and C float32 arrays"""
+        if isinstance(rows, np.ndarray) and rows.ndim == 1 and self.n_channels == 1:
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n = np.array([r.size for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        y = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            y[k, :r.size] = r
+        cap = max(int(self.max_output(n).max()), 1)
+        sym = np.empty((self.n_channels, cap), np.complex64)
+        pos = np.empty((self.n_channels, cap, 2), np.uint64)
+        err = np.empty((self.n_channels, cap), np.float32)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_tsync_process(self.h, y.ctypes.data, n.ctypes.data, stride, sym.ctypes.data, pos.ctypes.data,
+                                      err.ctypes.data, cap, cap, got.ctypes.data), "sdr_tsync_process")
+        g = [int(x) for x in got]
+        return ([sym[k, :g[k]] for k in range(self.n_channels)],
+                [_positions(pos[k, :g[k]]) for k in range(self.n_channels)],
+                [err[k, :g[k]] for k in range(self.n_channels)])
+
+    def process_dev(self, d_in, n_in, in_stride, d_sym, out_cap, out_stride, d_pos=None, d_err=None):
+        """device-resident: d_in C rows of in_stride complex64, row k of n_in (an int, or C counts) frames; d_sym C rows
+        of out_stride complex64 (out_cap >= max_output); d_pos (int64 [C, out_stride, 2]: whole, frac) and d_err
+        (float32 [C, out_stride]) may be None.  Returns the symbols written per channel (numpy array of C) once they
+        are known, which synchronises the handle's stream."""
+        n = self._counts(n_in)
+        got = np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_tsync_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_sym), _ptr(d_pos),
+                                          _ptr(d_err), out_cap, out_stride, got.ctypes.data), "sdr_tsync_process_dev")
+        return got.astype(np.int64)
+
+
 
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
