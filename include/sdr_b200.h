@@ -985,6 +985,70 @@ int sdr_tsync_process_dev(sdr_tsync_t *, const float *in_c64, const size_t *n_in
 /* the next unreleased position and the period offset v (2^-40 frames) of one channel; synchronises */
 int sdr_tsync_get_state(sdr_tsync_t *, size_t channel, sdr_arb_time_t *next, int64_t *v);
 
+/* ======================================================================================
+ * carrier recovery bank -- C independent c64 symbol streams (one sample per symbol, e.g. sdr_tsync's output rows with
+ * its counts as n_in), each with a decision-directed Costas loop that removes the carrier frequency and phase left
+ * after down-conversion.  State per channel: the phase phi, a uint64 in units of 2^-64 turn (the NCO convention of
+ * sdr_ddc), and the frequency nu, an int64 in units of 2^-40 turn per symbol with |nu| <= V = floor(max_freq 2^40)
+ * (exact).  q(x) = (int64) rint(x 2^40) for an f32 x.  From phi_0 and nu_0 (config, default 0), for s = 0, 1, 2, ...:
+ *   r_s       = nco_rot_fast(phi_s) ~ e^{-2 pi i phi_s / 2^64}
+ *   z_s       = (fl(fl(x.re r.re) - fl(x.im r.im)), fl(fl(x.re r.im) + fl(x.im r.re)))     (the output symbol)
+ *   e_s       = 0 for a non-finite g = D_M(z_s), else min(max(g, -err_max), err_max)
+ *   nu_{s+1}  = clamp(nu_s + q(fl(ki e_s)), -V, V)
+ *   phi_{s+1} = phi_s + 2^24 (nu_{s+1} + q(fl(kp e_s)))                                    (mod 2^64)
+ * nco_rot_fast(phi): f = fl((float)(int64) phi 2^-64), (s, c) = an f32 sincos of fl(f 6.2831855f) (quadrant from f),
+ * r = (c, -s); within a few 1e-7 of the exact rotation.
+ * Detectors, with a = sgn(z.re) z.im and b = sgn(z.im) z.re (exact; sgn(x) = +1 for x >= 0, -0 included, else -1) and
+ * K = f32(sqrt 2 - 1) -- GNU Radio's order-2/4/8 Costas detectors, order 2 decision-directed:
+ *   M = 2  (+-1):                 D = a                                                     slope K_d = A
+ *   M = 4  ((+-1 +- i)/sqrt 2):   D = fl(a - b)                                             K_d = sqrt(2) A
+ *   M = 8  (e^{i pi (2k+1)/8}):   D = |z.re| >= |z.im| ? fl(a - fl(K b)) : fl(fl(K a) - b)   K_d = A / cos(pi/8)
+ * (K_d: mean D per radian of phase error at amplitude A).  e > 0 means z leads its decision, so both corrections add.
+ * Every f32 operation is rounded on its own (nothing is contracted into an FMA): a float32 restatement gives e_s from
+ * the reported z_s bit for bit, and integer arithmetic every phi_s and nu_s from the reported e_s.  A non-finite x_s
+ * gives a non-finite z_s and e_s = 0: nu stays and phi advances by 2^24 nu, so the state stays finite.
+ * Loop design: sdr_tsync_loop_design(bn_t, zeta, K_d, 1 / (2 pi)) gives kp and ki in turns per unit of e (the same
+ * type-2 loop; 1 / (2 pi) turns per radian takes the place of the period).
+ * Validity at create (SDR_ERR_INVALID_ARG): order not 2, 4 or 8; kp or ki negative or non-finite; err_max <= 0 or
+ * non-finite; fl(kp err_max) or fl(ki err_max) >= 1 / (2 M) turn (one correction stays within half a decision sector);
+ * max_freq outside [0, 1 / (2 M)]; |nu_0| > V; C outside [1, 65536]; n_loops not 1 or C.
+ * One symbol out per symbol in: the counts are n_in, so sdr_csync_process_dev copies nothing back and does not
+ * synchronise.  Rows: C input rows of n_in[k] symbols at in_stride, C output rows z at out_stride (both >= the longest
+ * row when C > 1); phase (phi_s) and err (e_s) rows share out_stride and may be NULL.  out may equal in with the same
+ * stride (in place).  reset restores the creation phases and frequencies; clone copies the current ones.  A call is one
+ * launch and one small upload of the counts.  The loop is a recurrence, so the bank shards by channel only.
+ * Device pointers need 8-byte alignment for rows and phases, 4 bytes for err.
+ * ====================================================================================== */
+typedef struct {
+    unsigned order;  /* M: 2, 4 or 8 (the constellations above) */
+    float kp, ki;    /* turns per unit of e: sdr_tsync_loop_design(bn_t, zeta, K_d, 1 / (2 pi)) */
+    float err_max;   /* e is clamped to [-err_max, err_max] */
+    double max_freq; /* |nu| <= V = floor(max_freq 2^40), 0 <= max_freq <= 1 / (2 M) turns per symbol */
+} sdr_csync_loop_t;
+
+typedef struct {
+    const sdr_csync_loop_t *loops; /* n_loops loop parameter sets */
+    size_t n_loops;                /* 1 (shared) or n_channels */
+    const uint64_t *phase;         /* n_channels phi_0 in 2^-64 turns, or NULL = 0 */
+    const int64_t *freq;           /* n_channels nu_0 in 2^-40 turns per symbol, or NULL = 0 */
+    size_t n_channels;             /* C, 1 <= C <= 65536 */
+    int device;
+    void *stream;
+} sdr_csync_config_t;
+
+typedef struct sdr_csync sdr_csync_t;
+sdr_csync_t *sdr_csync_create(const sdr_csync_config_t *cfg, int *err);
+void sdr_csync_destroy(sdr_csync_t *);
+int sdr_csync_reset(sdr_csync_t *); /* the creation phases and frequencies */
+sdr_csync_t *sdr_csync_clone(const sdr_csync_t *, int *err);
+int sdr_csync_process(sdr_csync_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                      uint64_t *phase, float *err, size_t out_stride);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_csync_process_dev(sdr_csync_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                          uint64_t *phase, float *err, size_t out_stride);
+/* phi and nu of one channel's next symbol; synchronises */
+int sdr_csync_get_state(sdr_csync_t *, size_t channel, uint64_t *phase, int64_t *freq);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,7 +1,8 @@
 // nco.cuh -- the 64-bit NCO shared by the down-converter bank (ddc.cu), the fast-convolution banks (fcfb.cu, fcsb.cu)
 // and the up-converter bank (duc.cu; duc.cu and fcsb.cu take the conjugate of nco_rot): the exact derotation
 // e^{-2 pi i phi / 2^64} on the device and the host-side f64 phase and rotated-taps helpers, plus the f64 DFT and the
-// G' table builder of the two fast-convolution banks.
+// G' table builder of the two fast-convolution banks.  The f32 sincos of the PLL (pll.cu) and the carrier recovery
+// bank's rotation built on it (csync.cu) live here too.
 #pragma once
 #include <cmath>
 #include <utility>
@@ -16,6 +17,36 @@ __device__ __forceinline__ float2 nco_rot(uint64_t phi) {
     double s, c;
     sincospi((double)(long long)phi * 0x1p-63, &s, &c);
     return make_float2((float)c, (float)-s);
+}
+
+// xf = fl(2 pi f) with f = the fractional phase in (-1, 1): the quadrant k = rint(4 f) is taken from f, beside the
+// multiplication that forms xf (one operation less on the chain than rint(xf * 2/pi); the two agree except within an ulp of
+// a quadrant boundary, where either k leaves |r| <= pi/4 + 1e-6)
+__device__ __forceinline__ void sincos_fast(float xf, float f, float &sn, float &cs) {
+    const float kb = __fmaf_rn(f, 4.0f, 12582912.0f);
+    const float kf = kb - 12582912.0f;
+    const int q = __float_as_int(kb);  // low two bits = k mod 4
+    float r = __fmaf_rn(-kf, 1.57079637050628662109375f, xf);
+    r = __fmaf_rn(-kf, -4.37113882867379e-8f, r);
+    const float s = r * r, s2 = s * s, rs = r * s;
+    const float ps = __fmaf_rn(__fmaf_rn(2.7417770525062224e-06f, s, -0.00019841655739583075f), s2,
+                               __fmaf_rn(0.008333335630595684f, s, -0.1666666716337204f));
+    const float pc = __fmaf_rn(__fmaf_rn(2.4507638954673894e-05f, s, -0.0013888041721656919f), s2,
+                               __fmaf_rn(0.0416666641831398f, s, -0.5f));
+    const float sr = __fmaf_rn(rs, ps, r), cr = __fmaf_rn(s, pc, 1.0f);
+    const float a = (q & 1) ? cr : sr, b = (q & 1) ? sr : cr;
+    sn = __int_as_float(__float_as_int(a) ^ ((q & 2) << 30));
+    cs = __int_as_float(__float_as_int(b) ^ (((q + 1) & 2) << 30));
+}
+
+// e^{-2 pi i phi / 2^64} in f32 from sincos_fast (the carrier loop's rotation, csync.cu): f = fl(phi 2^-64) with phi
+// read as signed, so f in [-1/2, 1/2] carries at most 2^-25 turn of rounding; the result is within a few 1e-7 of the
+// exact rotation
+__device__ __forceinline__ float2 nco_rot_fast(uint64_t phi) {
+    const float f = __fmul_rn(__ll2float_rn((long long)phi), 0x1p-64f);
+    float s, c;
+    sincos_fast(__fmul_rn(f, 6.2831855f), f, s, c);
+    return make_float2(c, -s);
 }
 
 constexpr double NCO_2PI = 6.283185307179586476925286766559;

@@ -15,6 +15,7 @@
 // Data movement: a warp moves [32 streams x 32 samples] tiles between HBM and shared memory with
 // 256-byte row segments, so the lane-per-stream inner loop reads shared memory, not strided HBM.
 #include "kernels.h"
+#include "nco.cuh"
 #include "ptx.cuh"
 
 namespace sdr {
@@ -163,26 +164,6 @@ __device__ __forceinline__ float atan2_fast(float yf, float xf) {
     const float r = __fmaf_rn(tz, A, t);
     return __fmaf_rn(S, r, C);
 }
-// xf = fl(2 pi f) with f = the fractional phase in (-1, 1): the quadrant k = rint(4 f) is taken from f, beside the
-// multiplication that forms xf (one operation less on the chain than rint(xf * 2/pi); the two agree except within an ulp of
-// a quadrant boundary, where either k leaves |r| <= pi/4 + 1e-6)
-__device__ __forceinline__ void sincos_fast(float xf, float f, float &sn, float &cs) {
-    const float kb = __fmaf_rn(f, 4.0f, 12582912.0f);
-    const float kf = kb - 12582912.0f;
-    const int q = __float_as_int(kb);  // low two bits = k mod 4
-    float r = __fmaf_rn(-kf, 1.57079637050628662109375f, xf);
-    r = __fmaf_rn(-kf, -4.37113882867379e-8f, r);
-    const float s = r * r, s2 = s * s, rs = r * s;
-    const float ps = __fmaf_rn(__fmaf_rn(2.7417770525062224e-06f, s, -0.00019841655739583075f), s2,
-                               __fmaf_rn(0.008333335630595684f, s, -0.1666666716337204f));
-    const float pc = __fmaf_rn(__fmaf_rn(2.4507638954673894e-05f, s, -0.0013888041721656919f), s2,
-                               __fmaf_rn(0.0416666641831398f, s, -0.5f));
-    const float sr = __fmaf_rn(rs, ps, r), cr = __fmaf_rn(s, pc, 1.0f);
-    const float a = (q & 1) ? cr : sr, b = (q & 1) ? sr : cr;
-    sn = __int_as_float(__float_as_int(a) ^ ((q & 2) << 30));
-    cs = __int_as_float(__float_as_int(b) ^ (((q + 1) & 2) << 30));
-}
-
 // The recurrence (pll.rs:71-76): everything the NEXT sample depends on.  Returns c.re and phasedif for the two filters
 // that do not feed back (lock, output), which a helper warp applies one tile later.
 template <bool FAST, bool GEN>

@@ -605,6 +605,66 @@ class Tsync : public Handle<sdr_tsync_t, sdr_tsync_destroy, sdr_tsync_clone> {
     void reset() { check(sdr_tsync_reset(h_), "Tsync::reset"); }
 };
 
+// Carrier recovery bank (sdr_csync): a decision-directed Costas loop per channel on an exact 64-bit phase.  Channel k:
+// loop parameters {order, kp, ki, err_max, max_freq} (kp, ki from Tsync::loop_design(bn_t, zeta, K_d, 1 / (2 pi))), a
+// first phase (2^-64 turn) and frequency (2^-40 turn per symbol); each call returns one derotated symbol per input
+// symbol with its phase and detector output.
+class Csync : public Handle<sdr_csync_t, sdr_csync_destroy, sdr_csync_clone> {
+    size_t c_ = 0;
+
+  public:
+    struct Out {
+        std::vector<std::vector<Complex>> sym;
+        std::vector<std::vector<uint64_t>> phase;
+        std::vector<std::vector<float>> err;
+    };
+    // loops: one (shared) or one per channel; phase, freq: empty (all 0) or one per channel
+    Csync(size_t channels, const std::vector<sdr_csync_loop_t> &loops, const std::vector<uint64_t> &phase = {},
+          const std::vector<int64_t> &freq = {})
+        : c_(channels) {
+        if ((!phase.empty() && phase.size() != channels) || (!freq.empty() && freq.size() != channels))
+            throw sdr::Error(SDR_ERR_INVALID_ARG, "Csync::new");
+        sdr_csync_config_t cfg{};
+        cfg.loops = loops.data();
+        cfg.n_loops = loops.size();
+        cfg.phase = phase.empty() ? nullptr : phase.data();
+        cfg.freq = freq.empty() ? nullptr : freq.data();
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_csync_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Csync::new");
+    }
+    size_t channels() const { return c_; }
+    // phase (2^-64 turn) and frequency (2^-40 turn per symbol) of one channel's next symbol
+    std::pair<uint64_t, int64_t> state(size_t k) {
+        uint64_t ph = 0;
+        int64_t f = 0;
+        check(sdr_csync_get_state(h_, k, &ph, &f), "Csync::state");
+        return {ph, f};
+    }
+    // in: channels rows, row k of n_in[k] symbols at row stride in_stride (>= the longest row)
+    Out process(const Complex *in, const std::vector<size_t> &n_in, size_t in_stride) {
+        const size_t cap = std::max<size_t>(1, *std::max_element(n_in.begin(), n_in.end()));
+        std::vector<Complex> sym(cap * c_);
+        std::vector<uint64_t> ph(cap * c_);
+        std::vector<float> err(cap * c_);
+        check(sdr_csync_process(h_, reinterpret_cast<const float *>(in), n_in.data(), in_stride,
+                                reinterpret_cast<float *>(sym.data()), ph.data(), err.data(), cap),
+              "Csync::process");
+        Out o;
+        o.sym.resize(c_);
+        o.phase.resize(c_);
+        o.err.resize(c_);
+        for (size_t k = 0; k < c_; ++k) {
+            o.sym[k].assign(sym.begin() + k * cap, sym.begin() + k * cap + n_in[k]);
+            o.phase[k].assign(ph.begin() + k * cap, ph.begin() + k * cap + n_in[k]);
+            o.err[k].assign(err.begin() + k * cap, err.begin() + k * cap + n_in[k]);
+        }
+        return o;
+    }
+    void reset() { check(sdr_csync_reset(h_), "Csync::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

@@ -687,6 +687,75 @@ impl Drop for GpuTsync {
     fn drop(&mut self) { unsafe { sdr_tsync_destroy(self.h) } }
 }
 
+/// Carrier recovery bank: a decision-directed Costas loop per channel on an exact 64-bit phase.  Channel k: loop
+/// parameters {order, kp, ki, err_max, max_freq} (kp, ki from `GpuTsync::loop_design(bn_t, zeta, K_d, 1 / (2 pi))`), a
+/// first phase (2^-64 turn) and frequency (2^-40 turn per symbol); each call appends one derotated symbol per input
+/// symbol with its phase and detector output.
+pub struct GpuCsync {
+    h: *mut sdr_csync_t,
+    c: usize,
+}
+unsafe impl Send for GpuCsync {}
+
+impl GpuCsync {
+    /// loops: one (shared) or one per channel; phase, freq: empty (all 0) or one per channel
+    pub fn new(channels: usize, loops: &[sdr_csync_loop_t], phase: &[u64], freq: &[i64]) -> Result<Self, Error> {
+        if (!phase.is_empty() && phase.len() != channels) || (!freq.is_empty() && freq.len() != channels) {
+            return Err(Error(100));
+        }
+        let cfg = sdr_csync_config_t {
+            loops: loops.as_ptr(), n_loops: loops.len(),
+            phase: if phase.is_empty() { std::ptr::null() } else { phase.as_ptr() },
+            freq: if freq.is_empty() { std::ptr::null() } else { freq.as_ptr() },
+            n_channels: channels, device: 0, stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_csync_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuCsync { h, c: channels })
+    }
+    /// phase (2^-64 turn) and frequency (2^-40 turn per symbol) of one channel's next symbol
+    pub fn state(&mut self, k: usize) -> Result<(u64, i64), Error> {
+        let (mut ph, mut f) = (0u64, 0i64);
+        check(unsafe { sdr_csync_get_state(self.h, k, &mut ph, &mut f) })?;
+        Ok((ph, f))
+    }
+    /// input: one row per channel, row k of n_in[k] symbols at row stride `stride` (>= the longest row); channel k's
+    /// symbols, phases and errors are appended to sym[k], phase[k] and err[k]
+    pub fn process(&mut self, input: &[Complex<f32>], n_in: &[usize], stride: usize, sym: &mut [Vec<Complex<f32>>],
+                   phase: &mut [Vec<u64>], err: &mut [Vec<f32>]) -> Result<(), Error> {
+        assert!(n_in.len() == self.c);
+        assert!(n_in.iter().enumerate().all(|(k, &n)| n == 0 || input.len() >= k * stride + n));
+        let cap = n_in.iter().copied().max().unwrap_or(0).max(1);
+        let mut s = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut p = vec![0u64; cap * self.c];
+        let mut e = vec![0.0f32; cap * self.c];
+        check(unsafe {
+            sdr_csync_process(self.h, input.as_ptr() as *const f32, n_in.as_ptr(), stride, s.as_mut_ptr() as *mut f32,
+                              p.as_mut_ptr(), e.as_mut_ptr(), cap)
+        })?;
+        for k in 0..self.c {
+            let r = k * cap..k * cap + n_in[k];
+            sym[k].extend_from_slice(&s[r.clone()]);
+            phase[k].extend_from_slice(&p[r.clone()]);
+            err[k].extend_from_slice(&e[r]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_csync_reset(self.h) }) }
+}
+impl Clone for GpuCsync {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_csync_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_csync_clone failed: {}", Error(err));
+        GpuCsync { h, c: self.c }
+    }
+}
+impl Drop for GpuCsync {
+    fn drop(&mut self) { unsafe { sdr_csync_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

@@ -48,6 +48,7 @@ pub enum sdr_fcsb_t {}
 pub enum sdr_rrb_t {}
 pub enum sdr_arb_t {}
 pub enum sdr_tsync_t {}
+pub enum sdr_csync_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -273,6 +274,27 @@ pub struct sdr_tsync_config_t {
 }
 
 #[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct sdr_csync_loop_t {
+    pub order: c_uint,
+    pub kp: c_float,
+    pub ki: c_float,
+    pub err_max: c_float,
+    pub max_freq: c_double,
+}
+
+#[repr(C)]
+pub struct sdr_csync_config_t {
+    pub loops: *const sdr_csync_loop_t,
+    pub n_loops: size_t,
+    pub phase: *const u64,
+    pub freq: *const i64,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
     pub rate: c_float,
@@ -462,6 +484,16 @@ extern "C" {
                                  sym_c64: *mut c_float, pos: *mut sdr_arb_time_t, err: *mut c_float, out_cap: size_t,
                                  out_stride: size_t, n_out: *mut size_t) -> c_int;
     pub fn sdr_tsync_get_state(h: *mut sdr_tsync_t, channel: size_t, next: *mut sdr_arb_time_t, v: *mut i64) -> c_int;
+    pub fn sdr_csync_create(cfg: *const sdr_csync_config_t, err: *mut c_int) -> *mut sdr_csync_t;
+    pub fn sdr_csync_destroy(h: *mut sdr_csync_t);
+    pub fn sdr_csync_reset(h: *mut sdr_csync_t) -> c_int;
+    pub fn sdr_csync_clone(h: *const sdr_csync_t, err: *mut c_int) -> *mut sdr_csync_t;
+    pub fn sdr_csync_process(h: *mut sdr_csync_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                             out_c64: *mut c_float, phase: *mut u64, err: *mut c_float, out_stride: size_t) -> c_int;
+    pub fn sdr_csync_process_dev(h: *mut sdr_csync_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                                 out_c64: *mut c_float, phase: *mut u64, err: *mut c_float, out_stride: size_t)
+                                 -> c_int;
+    pub fn sdr_csync_get_state(h: *mut sdr_csync_t, channel: size_t, phase: *mut u64, freq: *mut i64) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

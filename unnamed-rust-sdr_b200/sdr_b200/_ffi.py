@@ -120,6 +120,16 @@ class TsyncConfig(C.Structure):
                 ("loops", vp), ("n_loops", sz), ("n_channels", sz), ("device", i32), ("stream", vp)]
 
 
+class CsyncLoop(C.Structure):
+    _fields_ = [("order", C.c_uint), ("kp", C.c_float), ("ki", C.c_float), ("err_max", C.c_float),
+                ("max_freq", C.c_double)]
+
+
+class CsyncConfig(C.Structure):
+    _fields_ = [("loops", vp), ("n_loops", sz), ("phase", vp), ("freq", vp), ("n_channels", sz), ("device", i32),
+                ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -247,6 +257,13 @@ PROTOTYPES = {
     "sdr_tsync_process": (i32, [vp, vp, vp, sz, vp, vp, vp, sz, sz, vp]),
     "sdr_tsync_process_dev": (i32, [vp, vp, vp, sz, vp, vp, vp, sz, sz, vp]),
     "sdr_tsync_get_state": (i32, [vp, sz, C.POINTER(ArbTime), C.POINTER(C.c_int64)]),
+    "sdr_csync_create": (vp, [C.POINTER(CsyncConfig), C.POINTER(i32)]),
+    "sdr_csync_destroy": (None, [vp]),
+    "sdr_csync_reset": (i32, [vp]),
+    "sdr_csync_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_csync_process": (i32, [vp, vp, vp, sz, vp, vp, vp, sz]),
+    "sdr_csync_process_dev": (i32, [vp, vp, vp, sz, vp, vp, vp, sz]),
+    "sdr_csync_get_state": (i32, [vp, sz, C.POINTER(C.c_uint64), C.POINTER(C.c_int64)]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -1090,6 +1090,79 @@ class Tsync(_Handle):
         return got.astype(np.int64)
 
 
+class Csync(_Handle):
+    """Carrier recovery bank (sdr_csync): a decision-directed Costas loop per channel on an exact 64-bit phase.  loops:
+    one (order, kp, ki, err_max, max_freq) or one per channel, order M in {2, 4, 8} (BPSK, QPSK, 8PSK), kp and ki in
+    turns per unit of detector output (tsync_loop_design(bn_t, zeta, K_d, 1 / (2 pi))), max_freq in turns per symbol;
+    phase (units of 2^-64 turn) and freq (units of 2^-40 turn per symbol): Python ints, one value or one per channel,
+    defaulting to 0.  process returns the derotated symbols z_s, their phases phi_s and the detector outputs e_s; see
+    include/sdr_b200.h for the recurrence."""
+
+    _abi = "csync"
+
+    def __init__(self, loops, n_channels=None, phase=None, freq=None, device=0, stream=None):
+        lp = [loops] if np.ndim(loops[0]) == 0 else list(loops)
+        npd = len(phase) if hasattr(phase, "__len__") else 1
+        nfq = len(freq) if hasattr(freq, "__len__") else 1
+        c = int(n_channels) if n_channels is not None else max(len(lp), npd, nfq)
+        self.n_channels = c
+        self._loops = (F.CsyncLoop * len(lp))(*[F.CsyncLoop(int(x[0]), *map(float, x[1:])) for x in lp])
+        self._phase = None if phase is None else (C.c_uint64 * c)(*self._per_channel(phase, c, 0, 1 << 64, "phase"))
+        self._freq = None if freq is None else (C.c_int64 * c)(*self._per_channel(freq, c, -(1 << 63), 1 << 63,
+                                                                                  "freq"))
+        cfg = F.CsyncConfig(C.addressof(self._loops), len(lp),
+                            None if self._phase is None else C.addressof(self._phase),
+                            None if self._freq is None else C.addressof(self._freq), c, device, _stream_ptr(stream))
+        self._create(cfg)
+
+    @staticmethod
+    def _per_channel(v, c, lo, hi, what):
+        v = [int(x) for x in (v if hasattr(v, "__len__") else [v])]
+        v = v * c if len(v) == 1 else v
+        if len(v) != c or any(x < lo or x >= hi for x in v):
+            raise ValueError("%s: one value in [%d, %d), or one per channel" % (what, lo, hi))
+        return v
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def state(self, k):
+        """(phase in units of 2^-64 turn, freq in units of 2^-40 turn per symbol) of channel k's next symbol"""
+        ph, fr = C.c_uint64(), C.c_int64()
+        check(lib().sdr_csync_get_state(self.h, int(k), C.byref(ph), C.byref(fr)), "sdr_csync_get_state")
+        return ph.value, fr.value
+
+    def process(self, rows):
+        """rows: complex64 [C, n] or a list of C rows of any lengths -> (symbols, phases, errors): lists of C complex64,
+        uint64 (units of 2^-64 turn) and float32 arrays, as long as the rows"""
+        if isinstance(rows, np.ndarray) and rows.ndim == 1 and self.n_channels == 1:
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n = np.array([r.size for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        y = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            y[k, :r.size] = r
+        z = np.empty_like(y)
+        ph = np.empty((self.n_channels, stride), np.uint64)
+        err = np.empty((self.n_channels, stride), np.float32)
+        check(lib().sdr_csync_process(self.h, y.ctypes.data, n.ctypes.data, stride, z.ctypes.data, ph.ctypes.data,
+                                      err.ctypes.data, stride), "sdr_csync_process")
+        g = [int(x) for x in n]
+        return ([z[k, :g[k]] for k in range(self.n_channels)], [ph[k, :g[k]] for k in range(self.n_channels)],
+                [err[k, :g[k]] for k in range(self.n_channels)])
+
+    def process_dev(self, d_in, n_in, in_stride, d_out, out_stride, d_phase=None, d_err=None):
+        """device-resident: d_in C rows of in_stride complex64, row k of n_in (an int, or C counts) symbols; d_out C rows
+        of out_stride complex64 (may be d_in with the same stride); d_phase (int64 or uint64 [C, out_stride]) and d_err
+        (float32 [C, out_stride]) may be None.  Asynchronous on the handle's stream: row k gets n_in[k] symbols."""
+        n = self._counts(n_in)
+        check(lib().sdr_csync_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), _ptr(d_phase),
+                                          _ptr(d_err), out_stride), "sdr_csync_process_dev")
+
+
 
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
