@@ -1049,6 +1049,73 @@ int sdr_csync_process_dev(sdr_csync_t *, const float *in_c64, const size_t *n_in
 /* phi and nu of one channel's next symbol; synchronises */
 int sdr_csync_get_state(sdr_csync_t *, size_t channel, uint64_t *phase, int64_t *freq);
 
+/* ======================================================================================
+ * adaptive equalizer bank -- C independent c64 symbol streams (one sample per symbol, e.g. sdr_tsync's output rows with
+ * its counts as n_in), each through an N-tap FIR whose complex weights adapt by blind CMA and then decision-directed
+ * LMS, to remove the intersymbol interference of multipath and filter mismatch.  One tap count N for the handle,
+ * 1 <= N <= 64.  Channel k carries the weights w[0..N), a delay line x_{s-j} (zeros before the stream), a symbol total
+ * s and an adaptation set {M, mu, a, err_max, S}: M in {2, 4, 8} (sdr_csync's constellations +-1, (+-1 +- i)/sqrt 2 and
+ * e^{i pi (2k+1)/8}, scaled to radius a), the step mu >= 0, the radius a > 0 with R = fl(a a), err_max > 0, and S:
+ * symbols s < S adapt by CMA and s >= S by DD (S = UINT64_MAX: CMA only; S = 0: DD only).  For each symbol s:
+ *   P_j = w[j] x_{s-j} = (fl(fl(w.re x.re) - fl(w.im x.im)), fl(fl(w.re x.im) + fl(w.im x.re)))
+ *   W   = 2^ceil(log2 min(N, 32)) lanes; p_l = P_l for l < min(N, W), 0 for N <= l < W;
+ *         N > 32: p_l = fl(P_l + P_{l+32}) where l + 32 < N, else P_l
+ *   y_s = pairwise tree over p_0..p_{W-1}: for o = W/2, ..., 1: p_l <- fl(p_l + p_{l+o});  y_s = p_0
+ *   CMA: eps = fl(fl(fl(y.re y.re) + fl(y.im y.im)) - R),  g = (fl(eps y.re), fl(eps y.im))
+ *   DD:  d = D_M(y) at radius a, g = (fl(y.re - d.re), fl(y.im - d.im)), with sgn(-0) = +1:
+ *        M = 2: (+-a, 0);  M = 4: (+-c, +-c), c = f32(a / sqrt 2);
+ *        M = 8: |y.re| >= |y.im| ? (+-p, +-q) : (+-q, +-p), p = f32(a cos pi/8), q = f32(a sin pi/8)
+ *        (c, p and q computed in double at create and rounded once)
+ *   y or g not finite: e_s = 0 and the taps do not change (no update is computed: a NaN in the delay line cannot
+ *   reach w); else e_s = each component of g clamped to [-err_max, err_max],  u = (fl(mu e.re), fl(mu e.im)),
+ *   w[j] <- (fl(w.re - fl(fl(u.re x.re) + fl(u.im x.im))), fl(w.im - fl(fl(u.im x.re) - fl(u.re x.im))))
+ *   (w <- w - mu e conj(x), x = x_{s-j}: the gradient of E(|y|^2 - R)^2 and of E|y - d|^2)
+ * Every f32 operation is rounded on its own (nothing is contracted into an FMA) and the summation order is part of the
+ * definition, so a numpy float32 restatement reproduces every y_s, every e_s and the final taps bit for bit.
+ * Initial taps: n_tap_sets rows of N c64 (1 shared, or C), or n_tap_sets = 0 for the centre spike
+ * w[floor((N-1)/2)] = 1, which delays the output by that many symbols; the weights must be finite.
+ * Validity at create (SDR_ERR_INVALID_ARG): N outside [1, 64]; C outside [1, 65536]; n_adapt not 1 or C; n_tap_sets
+ * not 0, 1 or C; NULL taps with n_tap_sets > 0, or non-finite taps; M not 2, 4 or 8; mu negative or non-finite; a <= 0,
+ * non-finite, or with R = fl(a a) not finite; err_max <= 0 or non-finite.
+ * One symbol out per symbol in: the counts are n_in, so sdr_eq_process_dev copies nothing back and does not
+ * synchronise.  Rows: C input rows of n_in[k] symbols at in_stride, C output rows y and C error rows e (c64, may be
+ * NULL) at out_stride (both strides >= the longest row when C > 1).  out may equal in with the same stride (in place).
+ * reset restores the creation taps, zeroes the delay lines and sets s = 0; clone copies the current state.  A call is
+ * one launch and one small upload of the counts: the taps, the last N - 1 symbols and s live on the device between
+ * calls.  The equalizer is a recurrence, so the bank shards by channel only.  Device rows need 8-byte alignment.
+ * ====================================================================================== */
+typedef struct {
+    unsigned order;        /* M: 2, 4 or 8 (the DD decisions above) */
+    float mu;              /* step, >= 0 */
+    float radius;          /* a > 0: the CMA modulus R = fl(a a) and the DD constellation's radius */
+    float err_max;         /* each component of e is clamped to [-err_max, err_max] */
+    uint64_t cma_symbols;  /* S: symbols s < S adapt by CMA, s >= S by DD */
+} sdr_eq_adapt_t;
+
+typedef struct {
+    size_t n_taps;                /* N, 1 <= N <= 64 */
+    const float *taps;            /* n_tap_sets rows of N c64, or NULL with n_tap_sets = 0 */
+    size_t n_tap_sets;            /* 0 (centre spike), 1 (shared) or n_channels */
+    const sdr_eq_adapt_t *adapt;  /* n_adapt adaptation sets */
+    size_t n_adapt;               /* 1 (shared) or n_channels */
+    size_t n_channels;            /* C, 1 <= C <= 65536 */
+    int device;
+    void *stream;
+} sdr_eq_config_t;
+
+typedef struct sdr_eq sdr_eq_t;
+sdr_eq_t *sdr_eq_create(const sdr_eq_config_t *cfg, int *err);
+void sdr_eq_destroy(sdr_eq_t *);
+int sdr_eq_reset(sdr_eq_t *); /* the creation taps, zero delay lines, s = 0 */
+sdr_eq_t *sdr_eq_clone(const sdr_eq_t *, int *err);
+int sdr_eq_process(sdr_eq_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                   float *err_c64, size_t out_stride);
+/* device pointers, asynchronous on the handle's stream */
+int sdr_eq_process_dev(sdr_eq_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                       float *err_c64, size_t out_stride);
+/* the N c64 taps of one channel for its next symbol; synchronises */
+int sdr_eq_get_taps(sdr_eq_t *, size_t channel, float *taps_c64);
+
 #ifdef __cplusplus
 }
 #endif

@@ -665,6 +665,60 @@ class Csync : public Handle<sdr_csync_t, sdr_csync_destroy, sdr_csync_clone> {
     void reset() { check(sdr_csync_reset(h_), "Csync::reset"); }
 };
 
+// Adaptive equalizer bank (sdr_eq): an N-tap FIR per channel whose complex weights adapt by blind CMA and then
+// decision-directed LMS.  Channel k: an adaptation set {order, mu, radius, err_max, cma_symbols} (symbols s <
+// cma_symbols adapt by CMA, later ones by DD) and initial taps (none: the centre spike); each call returns one
+// equalized symbol per input symbol with its error.
+class Eq : public Handle<sdr_eq_t, sdr_eq_destroy, sdr_eq_clone> {
+    size_t c_ = 0, n_ = 0;
+
+  public:
+    struct Out {
+        std::vector<std::vector<Complex>> sym;
+        std::vector<std::vector<Complex>> err;
+    };
+    // adapt: one (shared) or one per channel; taps: empty (centre spike), n_taps (shared) or channels * n_taps
+    Eq(size_t n_taps, size_t channels, const std::vector<sdr_eq_adapt_t> &adapt, const std::vector<Complex> &taps = {})
+        : c_(channels), n_(n_taps) {
+        if (n_taps == 0 || taps.size() % n_taps != 0) throw sdr::Error(SDR_ERR_INVALID_ARG, "Eq::new");
+        sdr_eq_config_t cfg{};
+        cfg.n_taps = n_;
+        cfg.taps = taps.empty() ? nullptr : reinterpret_cast<const float *>(taps.data());
+        cfg.n_tap_sets = taps.size() / n_taps;
+        cfg.adapt = adapt.data();
+        cfg.n_adapt = adapt.size();
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_eq_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Eq::new");
+    }
+    size_t channels() const { return c_; }
+    size_t taps_per_channel() const { return n_; }
+    // the taps of one channel for its next symbol
+    std::vector<Complex> taps(size_t k) {
+        std::vector<Complex> w(n_);
+        check(sdr_eq_get_taps(h_, k, reinterpret_cast<float *>(w.data())), "Eq::taps");
+        return w;
+    }
+    // in: channels rows, row k of n_in[k] symbols at row stride in_stride (>= the longest row)
+    Out process(const Complex *in, const std::vector<size_t> &n_in, size_t in_stride) {
+        const size_t cap = std::max<size_t>(1, *std::max_element(n_in.begin(), n_in.end()));
+        std::vector<Complex> sym(cap * c_), err(cap * c_);
+        check(sdr_eq_process(h_, reinterpret_cast<const float *>(in), n_in.data(), in_stride,
+                             reinterpret_cast<float *>(sym.data()), reinterpret_cast<float *>(err.data()), cap),
+              "Eq::process");
+        Out o;
+        o.sym.resize(c_);
+        o.err.resize(c_);
+        for (size_t k = 0; k < c_; ++k) {
+            o.sym[k].assign(sym.begin() + k * cap, sym.begin() + k * cap + n_in[k]);
+            o.err[k].assign(err.begin() + k * cap, err.begin() + k * cap + n_in[k]);
+        }
+        return o;
+    }
+    void reset() { check(sdr_eq_reset(h_), "Eq::reset"); }
+};
+
 struct BiquadD {  // biquad.rs:74-81 + simple.rs Identity
     sdr_biquad_design_t d;
     static BiquadD LowPass(float f, float q) { return {{SDR_BQ_LOWPASS, f, q}}; }

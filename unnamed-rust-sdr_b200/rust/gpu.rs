@@ -756,6 +756,71 @@ impl Drop for GpuCsync {
     fn drop(&mut self) { unsafe { sdr_csync_destroy(self.h) } }
 }
 
+/// Adaptive equalizer bank: an N-tap FIR per channel whose complex weights adapt by blind CMA and then decision-directed
+/// LMS.  Channel k: an adaptation set {order, mu, radius, err_max, cma_symbols} (symbols s < cma_symbols adapt by CMA,
+/// later ones by DD) and initial taps (empty: the centre spike); each call appends one equalized symbol per input
+/// symbol and its error.
+pub struct GpuEq {
+    h: *mut sdr_eq_t,
+    c: usize,
+    n: usize,
+}
+unsafe impl Send for GpuEq {}
+
+impl GpuEq {
+    /// adapt: one (shared) or one per channel; taps: empty (centre spike), n_taps (shared) or channels * n_taps
+    pub fn new(n_taps: usize, channels: usize, adapt: &[sdr_eq_adapt_t], taps: &[Complex<f32>]) -> Result<Self, Error> {
+        if n_taps == 0 || taps.len() % n_taps != 0 { return Err(Error(100)); }
+        let cfg = sdr_eq_config_t {
+            n_taps, taps: if taps.is_empty() { std::ptr::null() } else { taps.as_ptr() as *const f32 },
+            n_tap_sets: taps.len() / n_taps, adapt: adapt.as_ptr(), n_adapt: adapt.len(), n_channels: channels,
+            device: 0, stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_eq_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuEq { h, c: channels, n: n_taps })
+    }
+    /// the taps of one channel for its next symbol
+    pub fn taps(&mut self, k: usize) -> Result<Vec<Complex<f32>>, Error> {
+        let mut w = vec![Complex::new(0.0f32, 0.0); self.n];
+        check(unsafe { sdr_eq_get_taps(self.h, k, w.as_mut_ptr() as *mut f32) })?;
+        Ok(w)
+    }
+    /// input: one row per channel, row k of n_in[k] symbols at row stride `stride` (>= the longest row); channel k's
+    /// symbols and errors are appended to sym[k] and err[k]
+    pub fn process(&mut self, input: &[Complex<f32>], n_in: &[usize], stride: usize, sym: &mut [Vec<Complex<f32>>],
+                   err: &mut [Vec<Complex<f32>>]) -> Result<(), Error> {
+        assert!(n_in.len() == self.c);
+        assert!(n_in.iter().enumerate().all(|(k, &n)| n == 0 || input.len() >= k * stride + n));
+        let cap = n_in.iter().copied().max().unwrap_or(0).max(1);
+        let mut s = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut e = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        check(unsafe {
+            sdr_eq_process(self.h, input.as_ptr() as *const f32, n_in.as_ptr(), stride, s.as_mut_ptr() as *mut f32,
+                           e.as_mut_ptr() as *mut f32, cap)
+        })?;
+        for k in 0..self.c {
+            let r = k * cap..k * cap + n_in[k];
+            sym[k].extend_from_slice(&s[r.clone()]);
+            err[k].extend_from_slice(&e[r]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_eq_reset(self.h) }) }
+}
+impl Clone for GpuEq {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_eq_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_eq_clone failed: {}", Error(err));
+        GpuEq { h, c: self.c, n: self.n }
+    }
+}
+impl Drop for GpuEq {
+    fn drop(&mut self) { unsafe { sdr_eq_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

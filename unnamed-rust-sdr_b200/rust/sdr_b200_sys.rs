@@ -49,6 +49,7 @@ pub enum sdr_rrb_t {}
 pub enum sdr_arb_t {}
 pub enum sdr_tsync_t {}
 pub enum sdr_csync_t {}
+pub enum sdr_eq_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -295,6 +296,28 @@ pub struct sdr_csync_config_t {
 }
 
 #[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct sdr_eq_adapt_t {
+    pub order: c_uint,
+    pub mu: c_float,
+    pub radius: c_float,
+    pub err_max: c_float,
+    pub cma_symbols: u64,
+}
+
+#[repr(C)]
+pub struct sdr_eq_config_t {
+    pub n_taps: size_t,
+    pub taps: *const c_float,
+    pub n_tap_sets: size_t,
+    pub adapt: *const sdr_eq_adapt_t,
+    pub n_adapt: size_t,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
     pub rate: c_float,
@@ -494,6 +517,15 @@ extern "C" {
                                  out_c64: *mut c_float, phase: *mut u64, err: *mut c_float, out_stride: size_t)
                                  -> c_int;
     pub fn sdr_csync_get_state(h: *mut sdr_csync_t, channel: size_t, phase: *mut u64, freq: *mut i64) -> c_int;
+    pub fn sdr_eq_create(cfg: *const sdr_eq_config_t, err: *mut c_int) -> *mut sdr_eq_t;
+    pub fn sdr_eq_destroy(h: *mut sdr_eq_t);
+    pub fn sdr_eq_reset(h: *mut sdr_eq_t) -> c_int;
+    pub fn sdr_eq_clone(h: *const sdr_eq_t, err: *mut c_int) -> *mut sdr_eq_t;
+    pub fn sdr_eq_process(h: *mut sdr_eq_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                          out_c64: *mut c_float, err_c64: *mut c_float, out_stride: size_t) -> c_int;
+    pub fn sdr_eq_process_dev(h: *mut sdr_eq_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                              out_c64: *mut c_float, err_c64: *mut c_float, out_stride: size_t) -> c_int;
+    pub fn sdr_eq_get_taps(h: *mut sdr_eq_t, channel: size_t, taps_c64: *mut c_float) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -130,6 +130,16 @@ class CsyncConfig(C.Structure):
                 ("stream", vp)]
 
 
+class EqAdapt(C.Structure):
+    _fields_ = [("order", C.c_uint), ("mu", C.c_float), ("radius", C.c_float), ("err_max", C.c_float),
+                ("cma_symbols", C.c_uint64)]
+
+
+class EqConfig(C.Structure):
+    _fields_ = [("n_taps", sz), ("taps", vp), ("n_tap_sets", sz), ("adapt", vp), ("n_adapt", sz), ("n_channels", sz),
+                ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -264,6 +274,13 @@ PROTOTYPES = {
     "sdr_csync_process": (i32, [vp, vp, vp, sz, vp, vp, vp, sz]),
     "sdr_csync_process_dev": (i32, [vp, vp, vp, sz, vp, vp, vp, sz]),
     "sdr_csync_get_state": (i32, [vp, sz, C.POINTER(C.c_uint64), C.POINTER(C.c_int64)]),
+    "sdr_eq_create": (vp, [C.POINTER(EqConfig), C.POINTER(i32)]),
+    "sdr_eq_destroy": (None, [vp]),
+    "sdr_eq_reset": (i32, [vp]),
+    "sdr_eq_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_eq_process": (i32, [vp, vp, vp, sz, vp, vp, sz]),
+    "sdr_eq_process_dev": (i32, [vp, vp, vp, sz, vp, vp, sz]),
+    "sdr_eq_get_taps": (i32, [vp, sz, vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

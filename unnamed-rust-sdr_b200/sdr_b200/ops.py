@@ -1163,6 +1163,70 @@ class Csync(_Handle):
                                           _ptr(d_err), out_stride), "sdr_csync_process_dev")
 
 
+class Eq(_Handle):
+    """Adaptive equalizer bank (sdr_eq): an n_taps-tap FIR per channel whose complex weights adapt by blind CMA and then
+    decision-directed LMS.  adapt: one (order, mu, radius, err_max, cma_symbols) or one per channel, order M in
+    {2, 4, 8} (the DD decisions: BPSK, QPSK, 8PSK at the radius), cma_symbols S: symbols s < S adapt by CMA, later ones
+    by DD (None or 2**64 - 1: CMA only; 0: DD only).  taps: None (the centre spike), N complex taps shared, or [C, N];
+    n_channels defaults to the number of adaptation or tap sets.  process returns the equalized symbols y_s and the
+    errors e_s; see include/sdr_b200.h for the recurrence."""
+
+    _abi = "eq"
+
+    def __init__(self, n_taps, adapt, n_channels=None, taps=None, device=0, stream=None):
+        ad = [adapt] if np.ndim(adapt[0]) == 0 else list(adapt)
+        N = int(n_taps)
+        t = None if taps is None else np.ascontiguousarray(np.asarray(taps, np.complex64).reshape(-1, N))
+        c = int(n_channels) if n_channels is not None else max(len(ad), 1 if t is None else len(t))
+        self.n_channels, self.n_taps = c, N
+
+        def one(a):
+            S = (1 << 64) - 1 if a[4] is None else int(a[4])
+            return F.EqAdapt(int(a[0]), float(a[1]), float(a[2]), float(a[3]), S)
+        self._adapt = (F.EqAdapt * len(ad))(*[one(a) for a in ad])
+        self._taps = t
+        cfg = F.EqConfig(N, None if t is None else t.ctypes.data, 0 if t is None else len(t), C.addressof(self._adapt),
+                         len(ad), c, device, _stream_ptr(stream))
+        self._create(cfg)
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def taps(self, k):
+        """channel k's N complex64 taps for its next symbol"""
+        w = np.empty(self.n_taps, np.complex64)
+        check(lib().sdr_eq_get_taps(self.h, int(k), w.ctypes.data), "sdr_eq_get_taps")
+        return w
+
+    def process(self, rows):
+        """rows: complex64 [C, n] or a list of C rows of any lengths -> (y, e): lists of C complex64 arrays, as long as
+        the rows"""
+        if isinstance(rows, np.ndarray) and rows.ndim == 1 and self.n_channels == 1:
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n = np.array([r.size for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        x = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            x[k, :r.size] = r
+        y = np.empty_like(x)
+        e = np.empty_like(x)
+        check(lib().sdr_eq_process(self.h, x.ctypes.data, n.ctypes.data, stride, y.ctypes.data, e.ctypes.data,
+                                   stride), "sdr_eq_process")
+        g = [int(v) for v in n]
+        return [y[k, :g[k]] for k in range(self.n_channels)], [e[k, :g[k]] for k in range(self.n_channels)]
+
+    def process_dev(self, d_in, n_in, in_stride, d_out, out_stride, d_err=None):
+        """device-resident: d_in C rows of in_stride complex64, row k of n_in (an int, or C counts) symbols; d_out C
+        rows of out_stride complex64 (may be d_in with the same stride); d_err (complex64 [C, out_stride]) may be None.
+        Asynchronous on the handle's stream: row k gets n_in[k] symbols."""
+        n = self._counts(n_in)
+        check(lib().sdr_eq_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), _ptr(d_err),
+                                       out_stride), "sdr_eq_process_dev")
+
+
 
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
