@@ -1116,6 +1116,70 @@ int sdr_eq_process_dev(sdr_eq_t *, const float *in_c64, const size_t *n_in, size
 /* the N c64 taps of one channel for its next symbol; synchronises */
 int sdr_eq_get_taps(sdr_eq_t *, size_t channel, float *taps_c64);
 
+/* ======================================================================================
+ * Viterbi decoder bank -- C independent soft-decision streams of one convolutional code, e.g. sdr_csync's output rows
+ * (Gray QPSK at rate 1/2: one c64 symbol is one step, I -> c_0, Q -> c_1, in_stride counted in steps).
+ * Code: constraint length K, 3 <= K <= 9, S = 2^(K-1) states; rate 1/n, 2 <= n <= 4; generators g_0 .. g_{n-1}, each
+ * in [1, 2^K), in the usual octal convention where the MSB taps the current input (802.11: K = 7, (0133, 0171)).
+ * Encoder the decoder inverts: the state s_{t-1} holds the K - 1 previous inputs, u_{t-1} at bit K - 2;
+ *   r_t = (u_t << (K-1)) | s_{t-1},  c_{t,j} = popcount(r_t & g_j) mod 2,  s_t = r_t >> 1.
+ * Soft input: step t reads n f32 values x[t n + j]; a positive value favours bit 0 (BPSK 0 -> +1).  With the scale
+ * sigma_k of channel k: a non-finite x gives q = 0 (an erasure), else q = rint(clamp(fl(x sigma_k), -127, 127)),
+ * rounding half to even; a product that overflows saturates.  Erasures are how callers depuncture: they insert zeros.
+ * Branch cost: sum_j (c_j ? 127 + q_j : 127 - q_j), an integer in [0, 254 n].
+ * Add-compare-select: the new state s' has predecessors p_b = ((s' << 1) & (S-1)) | b; m'(s') = min_b m(p_b) + cost;
+ * the decision d = 1 only when the b = 1 sum is strictly smaller (ties take b = 0).
+ * Start metrics: zero start m(0) = 0 and every other state I = (K-1) 254 n + 1 (after K - 1 steps every survivor
+ * descends from state 0); uniform start: every state 0, for a stream picked up mid-way.
+ * Release: L is the decision depth, a multiple of 32, 32 <= L <= 512.  At every per-channel step total T = 32 j with
+ * T >= L + 32: the best state after step T - 1 (least metric, ties to the lowest index), a traceback through steps
+ * T - 1 .. T - L - 32 (step i's bit is s >> (K-2), the previous state ((s << 1) & (S-1)) | d_i(s)), and the bits of
+ * steps [T - L - 32, T - L) are released.  After T steps since create, reset or finish E(T) = max(0, 32 floor(T/32) - L)
+ * bits are out, so a call's count per channel is E(T + n_in) - E(T): the host knows it without asking the device
+ * (sdr_vit_output_count), and sdr_vit_process_dev does not synchronise.
+ * Finish: for the channels in `which` (C bytes, nonzero = listed; NULL: all) the T - E(T) <= L + 31 remaining bits by
+ * one traceback from state 0 (terminated != 0) or from the best state; the channel then returns to its creation state.
+ * Metrics are exact integers (never renormalised); the spread max m - min m never exceeds (2K - 3) 254 n + 1, so the
+ * device holds them in 32 bits and compares modulo 2^32 with the same decisions.
+ * Validity at create (SDR_ERR_INVALID_ARG): K, n, L or C out of range; a generator 0 or >= 2^K; a scale <= 0 or
+ * non-finite; n_scales not 1 and not C.
+ * Rows: C input rows of n_in[k] steps (n f32 each) at in_stride steps (>= the longest row when C > 1); C output rows
+ * of one byte per decoded bit (0 or 1) at out_stride bytes (>= the largest count when C > 1); n_out receives C counts.
+ * Device rows need 4-byte alignment (out_stride a multiple of 4 when C > 1).  reset returns every channel to its
+ * creation state; clone copies the current state.  A call is one launch and one small upload of the counts: the
+ * metrics, the undecoded decisions and T live on the device.  The decoder is a recurrence, so the bank shards by
+ * channel only.
+ * ====================================================================================== */
+typedef struct {
+    unsigned constraint;  /* K, 3..9 */
+    const uint32_t *gens; /* n generators, octal convention above */
+    size_t n_gens;        /* n, 2..4 */
+    size_t depth;         /* L: multiple of 32, 32..512 */
+    const float *scale;   /* n_scales soft-value scales sigma_k > 0, finite */
+    size_t n_scales;      /* 1 (shared) or n_channels */
+    int zero_start;       /* 1: the encoder starts in state 0; 0: uniform start */
+    size_t n_channels;    /* C, 1..65536 */
+    int device;
+    void *stream;
+} sdr_vit_config_t;
+
+typedef struct sdr_vit sdr_vit_t;
+sdr_vit_t *sdr_vit_create(const sdr_vit_config_t *cfg, int *err);
+void sdr_vit_destroy(sdr_vit_t *);
+int sdr_vit_reset(sdr_vit_t *); /* every channel to its creation state, T = 0 */
+sdr_vit_t *sdr_vit_clone(const sdr_vit_t *, int *err);
+/* host only, no device work: n_out[k] = E(T_k + n_in[k]) - E(T_k) */
+int sdr_vit_output_count(const sdr_vit_t *, const size_t *n_in, size_t *n_out);
+int sdr_vit_process(sdr_vit_t *, const float *in, const size_t *n_in, size_t in_stride, uint8_t *out,
+                    size_t out_stride, size_t *n_out);
+/* device pointers, asynchronous on the handle's stream; n_out is filled on the host */
+int sdr_vit_process_dev(sdr_vit_t *, const float *in, const size_t *n_in, size_t in_stride, uint8_t *out,
+                        size_t out_stride, size_t *n_out);
+int sdr_vit_finish(sdr_vit_t *, const uint8_t *which, int terminated, uint8_t *out, size_t out_stride, size_t *n_out);
+/* device out, asynchronous; n_out is filled on the host */
+int sdr_vit_finish_dev(sdr_vit_t *, const uint8_t *which, int terminated, uint8_t *out, size_t out_stride,
+                       size_t *n_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -48,6 +48,9 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src)
 __device__ __forceinline__ void cp_async8(void *smem_dst, const void *gmem_src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
 }
+__device__ __forceinline__ void cp_async4(void *smem_dst, const void *gmem_src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
+}
 // reads src_bytes (0 or 8) bytes and zero-fills the rest of the 8
 __device__ __forceinline__ void cp_async8_zfill(uint32_t dst, const void *src, uint32_t src_bytes) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");

@@ -1295,6 +1295,69 @@ class PowerSpectra : public Handle<sdr_psd_t, sdr_psd_destroy, sdr_psd_clone> {
 }  // namespace fft
 
 // =========================================================================================
+namespace fec {
+
+// Viterbi decoder bank (sdr_vit): soft-decision decoding of C streams of one rate-1/n convolutional code (constraint
+// length K, generators in the octal convention, decision depth L).  Each call takes n floats per step (positive
+// favours bit 0) and returns the bits it releases, one byte (0 or 1) each; finish releases the rest.
+class Vit : public Handle<sdr_vit_t, sdr_vit_destroy, sdr_vit_clone> {
+    size_t c_ = 0, n_ = 0, l_ = 0;
+
+    static std::vector<std::vector<uint8_t>> rows(const std::vector<uint8_t> &buf, size_t stride,
+                                                  const std::vector<size_t> &got) {
+        std::vector<std::vector<uint8_t>> o(got.size());
+        for (size_t k = 0; k < got.size(); ++k) o[k].assign(buf.begin() + k * stride, buf.begin() + k * stride + got[k]);
+        return o;
+    }
+
+  public:
+    // scale: one (shared) or one per channel
+    Vit(unsigned K, const std::vector<uint32_t> &gens, size_t depth, const std::vector<float> &scale, size_t channels,
+        bool zero_start = true)
+        : c_(channels), n_(gens.size()), l_(depth) {
+        sdr_vit_config_t cfg{};
+        cfg.constraint = K;
+        cfg.gens = gens.data();
+        cfg.n_gens = gens.size();
+        cfg.depth = depth;
+        cfg.scale = scale.data();
+        cfg.n_scales = scale.size();
+        cfg.zero_start = zero_start ? 1 : 0;
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_vit_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Vit::new");
+    }
+    size_t channels() const { return c_; }
+    // the bits a call of n_in steps per channel releases
+    std::vector<size_t> output_count(const std::vector<size_t> &n_in) const {
+        std::vector<size_t> o(c_);
+        check(sdr_vit_output_count(h_, n_in.data(), o.data()), "Vit::output_count");
+        return o;
+    }
+    // in: channels rows, row k of n_in[k] steps of n floats at a row stride of in_stride steps (>= the longest row)
+    std::vector<std::vector<uint8_t>> process(const float *in, const std::vector<size_t> &n_in, size_t in_stride) {
+        const std::vector<size_t> cnt = output_count(n_in);
+        const size_t cap = (std::max<size_t>(4, *std::max_element(cnt.begin(), cnt.end())) + 3) & ~(size_t)3;
+        std::vector<uint8_t> buf(cap * c_);
+        std::vector<size_t> got(c_);
+        check(sdr_vit_process(h_, in, n_in.data(), in_stride, buf.data(), cap, got.data()), "Vit::process");
+        return rows(buf, cap, got);
+    }
+    // the remaining bits of every channel (traced back from state 0 when terminated); the bank returns to its start
+    std::vector<std::vector<uint8_t>> finish(bool terminated) {
+        const size_t cap = l_ + 32;
+        std::vector<uint8_t> buf(cap * c_);
+        std::vector<size_t> got(c_);
+        check(sdr_vit_finish(h_, nullptr, terminated ? 1 : 0, buf.data(), cap, got.data()), "Vit::finish");
+        return rows(buf, cap, got);
+    }
+    void reset() { check(sdr_vit_reset(h_), "Vit::reset"); }
+};
+
+}  // namespace fec
+
+// =========================================================================================
 namespace app {
 
 // The receiver of src/main.rs:32-81 as one device-resident pipeline (sdr_fm_*): rtl_tcp bytes in, 48 kHz

@@ -821,6 +821,76 @@ impl Drop for GpuEq {
     fn drop(&mut self) { unsafe { sdr_eq_destroy(self.h) } }
 }
 
+/// Viterbi decoder bank: soft-decision decoding of C streams of one rate-1/n convolutional code (constraint length K,
+/// generators in the octal convention, decision depth L).  Each call takes n floats per step (positive favours bit 0)
+/// and appends the bits it releases, one byte (0 or 1) each; finish appends the rest.
+pub struct GpuVit {
+    h: *mut sdr_vit_t,
+    c: usize,
+    l: usize,
+}
+unsafe impl Send for GpuVit {}
+
+impl GpuVit {
+    /// scale: one (shared) or one per channel
+    pub fn new(k: u32, gens: &[u32], depth: usize, scale: &[f32], channels: usize, zero_start: bool)
+               -> Result<Self, Error> {
+        let cfg = sdr_vit_config_t {
+            constraint: k, gens: gens.as_ptr(), n_gens: gens.len(), depth, scale: scale.as_ptr(),
+            n_scales: scale.len(), zero_start: zero_start as i32, n_channels: channels, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_vit_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuVit { h, c: channels, l: depth })
+    }
+    /// the bits a call of n_in steps per channel releases
+    pub fn output_count(&self, n_in: &[usize]) -> Result<Vec<usize>, Error> {
+        assert!(n_in.len() == self.c);
+        let mut o = vec![0usize; self.c];
+        check(unsafe { sdr_vit_output_count(self.h, n_in.as_ptr(), o.as_mut_ptr()) })?;
+        Ok(o)
+    }
+    /// input: one row per channel, row k of n_in[k] steps of n floats at a row stride of `stride` steps (>= the
+    /// longest row); channel k's released bits are appended to bits[k]
+    pub fn process(&mut self, input: &[f32], n_in: &[usize], stride: usize, bits: &mut [Vec<u8>])
+                   -> Result<(), Error> {
+        let cnt = self.output_count(n_in)?;
+        let cap = (cnt.iter().copied().max().unwrap_or(0).max(4) + 3) & !3;
+        let mut out = vec![0u8; cap * self.c];
+        let mut got = vec![0usize; self.c];
+        check(unsafe {
+            sdr_vit_process(self.h, input.as_ptr(), n_in.as_ptr(), stride, out.as_mut_ptr(), cap, got.as_mut_ptr())
+        })?;
+        for k in 0..self.c { bits[k].extend_from_slice(&out[k * cap..k * cap + got[k]]); }
+        Ok(())
+    }
+    /// the remaining bits of every channel (traced back from state 0 when terminated); the bank returns to its start
+    pub fn finish(&mut self, terminated: bool, bits: &mut [Vec<u8>]) -> Result<(), Error> {
+        let cap = self.l + 32;
+        let mut out = vec![0u8; cap * self.c];
+        let mut got = vec![0usize; self.c];
+        check(unsafe {
+            sdr_vit_finish(self.h, std::ptr::null(), terminated as i32, out.as_mut_ptr(), cap, got.as_mut_ptr())
+        })?;
+        for k in 0..self.c { bits[k].extend_from_slice(&out[k * cap..k * cap + got[k]]); }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_vit_reset(self.h) }) }
+}
+impl Clone for GpuVit {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_vit_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_vit_clone failed: {}", Error(err));
+        GpuVit { h, c: self.c, l: self.l }
+    }
+}
+impl Drop for GpuVit {
+    fn drop(&mut self) { unsafe { sdr_vit_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

@@ -50,6 +50,7 @@ pub enum sdr_arb_t {}
 pub enum sdr_tsync_t {}
 pub enum sdr_csync_t {}
 pub enum sdr_eq_t {}
+pub enum sdr_vit_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -318,6 +319,20 @@ pub struct sdr_eq_config_t {
 }
 
 #[repr(C)]
+pub struct sdr_vit_config_t {
+    pub constraint: c_uint,
+    pub gens: *const u32,
+    pub n_gens: size_t,
+    pub depth: size_t,
+    pub scale: *const c_float,
+    pub n_scales: size_t,
+    pub zero_start: c_int,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
     pub rate: c_float,
@@ -526,6 +541,19 @@ extern "C" {
     pub fn sdr_eq_process_dev(h: *mut sdr_eq_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
                               out_c64: *mut c_float, err_c64: *mut c_float, out_stride: size_t) -> c_int;
     pub fn sdr_eq_get_taps(h: *mut sdr_eq_t, channel: size_t, taps_c64: *mut c_float) -> c_int;
+    pub fn sdr_vit_create(cfg: *const sdr_vit_config_t, err: *mut c_int) -> *mut sdr_vit_t;
+    pub fn sdr_vit_destroy(h: *mut sdr_vit_t);
+    pub fn sdr_vit_reset(h: *mut sdr_vit_t) -> c_int;
+    pub fn sdr_vit_clone(h: *const sdr_vit_t, err: *mut c_int) -> *mut sdr_vit_t;
+    pub fn sdr_vit_output_count(h: *const sdr_vit_t, n_in: *const size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_vit_process(h: *mut sdr_vit_t, input: *const c_float, n_in: *const size_t, in_stride: size_t,
+                           out: *mut u8, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_vit_process_dev(h: *mut sdr_vit_t, input: *const c_float, n_in: *const size_t, in_stride: size_t,
+                               out: *mut u8, out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_vit_finish(h: *mut sdr_vit_t, which: *const u8, terminated: c_int, out: *mut u8, out_stride: size_t,
+                          n_out: *mut size_t) -> c_int;
+    pub fn sdr_vit_finish_dev(h: *mut sdr_vit_t, which: *const u8, terminated: c_int, out: *mut u8,
+                              out_stride: size_t, n_out: *mut size_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -140,6 +140,11 @@ class EqConfig(C.Structure):
                 ("device", i32), ("stream", vp)]
 
 
+class VitConfig(C.Structure):
+    _fields_ = [("constraint", C.c_uint), ("gens", vp), ("n_gens", sz), ("depth", sz), ("scale", vp), ("n_scales", sz),
+                ("zero_start", i32), ("n_channels", sz), ("device", i32), ("stream", vp)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -281,6 +286,15 @@ PROTOTYPES = {
     "sdr_eq_process": (i32, [vp, vp, vp, sz, vp, vp, sz]),
     "sdr_eq_process_dev": (i32, [vp, vp, vp, sz, vp, vp, sz]),
     "sdr_eq_get_taps": (i32, [vp, sz, vp]),
+    "sdr_vit_create": (vp, [C.POINTER(VitConfig), C.POINTER(i32)]),
+    "sdr_vit_destroy": (None, [vp]),
+    "sdr_vit_reset": (i32, [vp]),
+    "sdr_vit_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_vit_output_count": (i32, [vp, vp, vp]),
+    "sdr_vit_process": (i32, [vp, vp, vp, sz, vp, sz, vp]),
+    "sdr_vit_process_dev": (i32, [vp, vp, vp, sz, vp, sz, vp]),
+    "sdr_vit_finish": (i32, [vp, vp, i32, vp, sz, vp]),
+    "sdr_vit_finish_dev": (i32, [vp, vp, i32, vp, sz, vp]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -1226,6 +1226,96 @@ class Eq(_Handle):
         check(lib().sdr_eq_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), _ptr(d_err),
                                        out_stride), "sdr_eq_process_dev")
 
+class Vit(_Handle):
+    """Viterbi decoder bank (sdr_vit): soft-decision decoding of C streams of one rate-1/n convolutional code.
+    K: constraint length (3..9); gens: n generators in the octal convention (the MSB taps the current input, e.g.
+    (0o133, 0o171)); depth: the decision depth L (a multiple of 32, 32..512); scale: sigma, one or one per channel (soft
+    values are quantised as rint(clamp(x sigma, -127, 127)), positive favouring bit 0); zero_start: the encoder starts
+    in state 0 (else every state is equally likely).  A step is n f32 values; complex64 rows at n = 2 are one step per
+    symbol (I -> c_0, Q -> c_1).  process returns the released bits, one uint8 (0 or 1) each; after T steps
+    max(0, 32 floor(T/32) - L) bits are out, and finish releases the rest.  See include/sdr_b200.h."""
+
+    _abi = "vit"
+
+    def __init__(self, K, gens, depth, scale=1.0, n_channels=None, zero_start=True, device=0, stream=None):
+        self._gens = np.ascontiguousarray(gens, np.uint32).ravel()
+        self._scale = np.ascontiguousarray(np.atleast_1d(np.asarray(scale, np.float32)))
+        self.K, self.n, self.depth = int(K), int(self._gens.size), int(depth)
+        self.n_channels = int(n_channels) if n_channels is not None else int(self._scale.size)
+        cfg = F.VitConfig(self.K, self._gens.ctypes.data, self._gens.size, self.depth, self._scale.ctypes.data,
+                          self._scale.size, int(bool(zero_start)), self.n_channels, device, _stream_ptr(stream))
+        self._create(cfg)
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def output_count(self, n_in):
+        """bits the next call of n_in steps (an int, or C counts) releases per channel; no device work"""
+        n = self._counts(n_in)
+        out = np.empty(self.n_channels, np.uintp)
+        check(lib().sdr_vit_output_count(self.h, n.ctypes.data, out.ctypes.data), "sdr_vit_output_count")
+        return out.astype(np.int64)
+
+    def process(self, rows):
+        """rows: f32 [C, steps, n] or [C, steps * n], complex64 [C, steps] at n = 2, or a list of C such rows of any
+        lengths -> a list of C uint8 arrays of released bits"""
+        if isinstance(rows, np.ndarray) and self.n_channels == 1 and (rows.ndim == 1 or (
+                rows.ndim == 2 and rows.shape[1] == self.n and rows.dtype != np.complex64)):
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r).view(np.float32).ravel() if np.iscomplexobj(r)
+                else np.ascontiguousarray(r, np.float32).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        if any(r.size % self.n for r in rows):
+            raise ValueError("rows: whole steps of %d values expected" % self.n)
+        n = np.array([r.size // self.n for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        x = np.zeros((self.n_channels, stride * self.n), np.float32)
+        for k, r in enumerate(rows):
+            x[k, :r.size] = r
+        cnt = self.output_count(n)
+        ostride = max(int(cnt.max()), 4)
+        ostride += -ostride % 4
+        y = np.empty((self.n_channels, ostride), np.uint8)
+        got = np.empty(self.n_channels, np.uintp)
+        check(lib().sdr_vit_process(self.h, x.ctypes.data, n.ctypes.data, stride, y.ctypes.data, ostride,
+                                    got.ctypes.data), "sdr_vit_process")
+        return [y[k, :int(got[k])].copy() for k in range(self.n_channels)]
+
+    def process_dev(self, d_in, n_in, in_stride, d_out, out_stride):
+        """device-resident: d_in C rows of in_stride steps (n f32 each), row k of n_in (an int, or C counts) steps;
+        d_out C rows of out_stride bytes (a multiple of 4 when C > 1).  Asynchronous on the handle's stream; returns the
+        C bit counts written, known on the host"""
+        n = self._counts(n_in)
+        got = np.empty(self.n_channels, np.uintp)
+        check(lib().sdr_vit_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), out_stride,
+                                        got.ctypes.data), "sdr_vit_process_dev")
+        return got.astype(np.int64)
+
+    def _which(self, which):
+        return None if which is None else np.ascontiguousarray(np.broadcast_to(
+            np.asarray(which, bool), (self.n_channels,)), np.uint8)
+
+    def finish(self, which=None, terminated=True):
+        """the remaining bits of the channels in `which` (C booleans; None: all), traced back from state 0
+        (terminated) or from the best state; those channels return to their creation state.  A list of C uint8 arrays
+        (empty for channels not listed)"""
+        w = self._which(which)
+        cap = self.depth + 32
+        y = np.empty((self.n_channels, cap), np.uint8)
+        got = np.empty(self.n_channels, np.uintp)
+        check(lib().sdr_vit_finish(self.h, None if w is None else w.ctypes.data, int(bool(terminated)), y.ctypes.data,
+                                   cap, got.ctypes.data), "sdr_vit_finish")
+        return [y[k, :int(got[k])].copy() for k in range(self.n_channels)]
+
+    def finish_dev(self, d_out, out_stride, which=None, terminated=True):
+        """finish into device rows d_out (C rows of out_stride bytes, >= depth + 31); asynchronous; returns the C
+        counts"""
+        w = self._which(which)
+        got = np.empty(self.n_channels, np.uintp)
+        check(lib().sdr_vit_finish_dev(self.h, None if w is None else w.ctypes.data, int(bool(terminated)),
+                                       _ptr(d_out), out_stride, got.ctypes.data), "sdr_vit_finish_dev")
+        return got.astype(np.int64)
 
 
 class FmStereo:
