@@ -1180,6 +1180,129 @@ int sdr_vit_finish(sdr_vit_t *, const uint8_t *which, int terminated, uint8_t *o
 int sdr_vit_finish_dev(sdr_vit_t *, const uint8_t *which, int terminated, uint8_t *out, size_t out_stride,
                        size_t *n_out);
 
+/* ======================================================================================
+ * frame synchronizer bank -- C independent c64 symbol streams (e.g. sdr_csync's output rows), each carrying frames of
+ * F symbols that start with a known sync word.  The bank finds the word by correlation, tracks frames with a
+ * search -> verify -> lock -> flywheel state machine, reads the constellation's phase ambiguity (sdr_csync locks up to
+ * a rotation by 2 pi / M, CMA leaves any phase) from the phase of each frame's correlation, and emits each frame's
+ * payload derotated: the input sdr_vit needs, from the library alone.
+ * Sync word: one length Lp per handle, 8 <= Lp <= 1024; n_words rows of Lp c64 (1 shared, or C), finite, with
+ * E_p > 0 and finite.  Parameters {F, M, th_search, th_check, V, max_miss, W}, 1 set or C: F the frame period in
+ * symbols (word included), Lp + 2 W < F <= 2^24; M in {2, 4, 8} (sdr_csync's constellations); th_search, th_check in
+ * (0, 1]; V <= 8 verifications before lock; 1 <= max_miss <= 255; W <= 32 the check window half-width.
+ * Symbols z_t are numbered from 0 since create or reset; position s reads z_s .. z_{s+Lp-1}.  Every f32 operation is
+ * rounded on its own (nothing is contracted):
+ *   P_j  = conj(p_j) z_{s+j} = (fl(fl(p.re z.re) + fl(p.im z.im)), fl(fl(p.re z.im) - fl(p.im z.re)))
+ *   c_s  = P_0, then c_s <- fl(c_s + P_j) for j = 1 .. Lp-1, componentwise and in that order
+ *   E_s  = the same sequential sum of fl(fl(z.re z.re) + fl(z.im z.im)); E_p the same over the word, once
+ *   rho_s = fl(a / b) if b > 0, else 0, with a = fl(fl(c.re c.re) + fl(c.im c.im)), b = fl(E_s E_p)
+ * A test passes when rho >= theta; a NaN rho fails every test.  The best position of the window around e is the
+ * s in [e - W, e + W] with the largest rho_s (NaN lowest), ties to the smallest |s - e|, then to the earlier s.
+ * Rotation r(c) in [0, M), sgn(-0) = +1: M = 2: c.re >= 0 ? 0 : 1;  M = 4: q = |c.re| >= |c.im| ? (c.re >= 0 ? 0 : 2)
+ * : (c.im >= 0 ? 1 : 3);  M = 8: q as for M = 4, c' = c (-i)^q (exact), t = fl(K c'.re) with K = f32(sqrt 2 - 1),
+ * o = c'.im > t ? 1 : (c'.im < -t ? -1 : 0), r = (2 q + o) mod 8.
+ * Derotation D_r(x) = x e^{-2 pi i r / M}: sign changes and swaps for M = 2 and 4; for M = 8 and odd r first
+ * x <- (fl(fl(x.re + x.im) h), fl(fl(x.im - x.re) h)) with h = f32(1 / sqrt 2), then x (-i)^floor(r / 2), exact.
+ * State machine, per channel, decisions in increasing position order, each made once the symbols it needs are in:
+ *   SEARCH from sigma: the first s >= sigma with rho_s >= th_search: HIT.  V = 0: LOCK at once, emit the frame at s,
+ *           R = r(c_s), e = s + F.  Else VERIFY with e = s + F, v = 0.
+ *   VERIFY: s* = the best position around e.  Pass (rho >= th_check): VERIFY_PASS, v += 1; at v = V: LOCK, emit the
+ *           frame at s*, R = r(c_s*); either way e = s* + F.  Fail: VERIFY_FAIL, SEARCH from sigma = e + W + 1.
+ *   LOCK:   s* = the best position around e.  Pass: LOCK_PASS, R = r(c_s*), m = 0, emit the frame at s*, e = s* + F.
+ *           Fail: m += 1; m < max_miss: LOCK_MISS, emit the frame at e with R unchanged (flywheel), e += F;
+ *           else LOCK_LOST, SEARCH from sigma = e + W + 1.
+ * Emitting the frame at s appends D_R(z_t), t = s + Lp .. s + F - 1, to the channel's payload stream as those symbols
+ * arrive: every emitted frame carries F - Lp symbols, and a frame's payload is complete before the next decision.
+ * The search never rewinds: positions passed over while verifying are not searched again (the word repeats, so this
+ * costs at most one more frame of acquisition).
+ * Records (sdr_fsync_record_t), one per decision: pos = s* for HIT and passes, e for fails, misses and losses;
+ * out_index = the payload index of the emitted frame's first symbol, or UINT64_MAX when no frame is emitted; corr and
+ * rho of the best (or hit) position in every case; rot = the R a frame is emitted with, else r(corr); kind.
+ * Bounds (sdr_fsync_max_output, host only): for n_in = n > 0 symbols after T consumed, with G = F - W + 1 and
+ * m = 1 if Lp >= W else 2,  payload <= m (n + min(T, Lp + 2 W - 1)),  records <= min(n, 2 floor((n - 1) / G) + 2).
+ * Proof: each symbol completes at most one decision; after a fail or a loss the next decision is a HIT, after which
+ * the next one completes at least F + W symbols later; after any other decision the next one completes at least
+ * F - W symbols later, so any two consecutive gaps sum to at least G.  Emitted frames start at least F - W apart, so
+ * a symbol lies in at most m payloads; a call emits its own symbols and, at decisions, carried ones.
+ * A call whose out_cap (or rec_cap, when recs is not NULL) is below the largest bound returns
+ * SDR_ERR_OUTPUT_TOO_SMALL before any state changes.  Counts depend on the data: like sdr_tsync_process_dev,
+ * sdr_fsync_process_dev enqueues its work, copies the C counts back and synchronises the handle's stream.
+ * Rows: C input rows of n_in[k] symbols at in_stride (>= the longest row when C > 1); C payload rows at out_stride
+ * (>= the largest payload bound when C > 1); recs may be NULL, else C rows of rec_stride records (>= the largest
+ * record bound when C > 1); n_rec may be NULL.  Symbol totals stay below 2^62 (else SDR_ERR_INVALID_ARG).
+ * Carried per channel: fewer than Lp + 2 W symbols, the state, the totals.  reset returns every channel to SEARCH
+ * from 0 with nothing consumed; clone copies the current state, device part included.  A call is one launch, one
+ * small upload of the counts and one copy of the C output counts back.  The state machine is a recurrence, so the
+ * bank shards by channel only.  Device pointers need 8-byte alignment.
+ * ====================================================================================== */
+#define SDR_FSYNC_SEARCH 0
+#define SDR_FSYNC_VERIFY 1
+#define SDR_FSYNC_LOCK 2
+
+#define SDR_FSYNC_HIT 1
+#define SDR_FSYNC_VERIFY_PASS 2
+#define SDR_FSYNC_VERIFY_FAIL 3
+#define SDR_FSYNC_LOCK_PASS 4
+#define SDR_FSYNC_LOCK_MISS 5
+#define SDR_FSYNC_LOCK_LOST 6
+
+typedef struct {
+    uint32_t period;        /* F: frame period in symbols, word included; Lp + 2 W < F <= 2^24 */
+    uint32_t order;         /* M: 2, 4 or 8 */
+    float thresh_search;    /* th_search in (0, 1] */
+    float thresh_check;     /* th_check in (0, 1] */
+    uint32_t verify;        /* V <= 8 */
+    uint32_t max_miss;      /* 1..255 */
+    uint32_t window;        /* W <= 32 */
+} sdr_fsync_params_t;
+
+typedef struct {
+    size_t word_len;                  /* Lp, 8..1024 */
+    const float *words;               /* n_words rows of Lp c64 */
+    size_t n_words;                   /* 1 (shared) or n_channels */
+    const sdr_fsync_params_t *params; /* n_params parameter sets */
+    size_t n_params;                  /* 1 (shared) or n_channels */
+    size_t n_channels;                /* C, 1..65536 */
+    int device;
+    void *stream;
+} sdr_fsync_config_t;
+
+typedef struct {
+    uint64_t pos;       /* s* for HIT and passes; e for fails, misses and losses */
+    uint64_t out_index; /* payload index of the emitted frame's first symbol, or UINT64_MAX */
+    float corr[2];      /* c of the best (or hit) position */
+    float rho;          /* its rho */
+    uint16_t rot;       /* R of the emitted frame, else r(corr) */
+    uint16_t kind;      /* SDR_FSYNC_HIT .. SDR_FSYNC_LOCK_LOST */
+} sdr_fsync_record_t;
+
+typedef struct {
+    uint32_t state;     /* SDR_FSYNC_SEARCH, _VERIFY or _LOCK */
+    uint32_t count;     /* v (VERIFY) or m (LOCK) */
+    uint64_t pos;       /* sigma (SEARCH) or e */
+    uint32_t rot;       /* R */
+    uint32_t pad;
+    uint64_t consumed;  /* symbols since create or reset */
+    uint64_t payload;   /* payload symbols emitted (counting the current frame whole) */
+} sdr_fsync_state_t;
+
+typedef struct sdr_fsync sdr_fsync_t;
+sdr_fsync_t *sdr_fsync_create(const sdr_fsync_config_t *cfg, int *err);
+void sdr_fsync_destroy(sdr_fsync_t *);
+int sdr_fsync_reset(sdr_fsync_t *); /* every channel to SEARCH from 0, nothing consumed */
+sdr_fsync_t *sdr_fsync_clone(const sdr_fsync_t *, int *err);
+/* host only: pay_caps[k], rec_caps[k] = the bounds above for the next n_in[k] symbols of channel k */
+int sdr_fsync_max_output(const sdr_fsync_t *, const size_t *n_in, size_t *pay_caps, size_t *rec_caps);
+int sdr_fsync_process(sdr_fsync_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                      size_t out_cap, size_t out_stride, size_t *n_out, sdr_fsync_record_t *recs, size_t rec_cap,
+                      size_t rec_stride, size_t *n_rec);
+/* device pointers; returns after the counts are copied back (synchronises the handle's stream) */
+int sdr_fsync_process_dev(sdr_fsync_t *, const float *in_c64, const size_t *n_in, size_t in_stride, float *out_c64,
+                          size_t out_cap, size_t out_stride, size_t *n_out, sdr_fsync_record_t *recs, size_t rec_cap,
+                          size_t rec_stride, size_t *n_rec);
+/* one channel's state; synchronises */
+int sdr_fsync_get_state(sdr_fsync_t *, size_t channel, sdr_fsync_state_t *state);
+
 #ifdef __cplusplus
 }
 #endif

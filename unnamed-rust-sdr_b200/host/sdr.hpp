@@ -1355,6 +1355,66 @@ class Vit : public Handle<sdr_vit_t, sdr_vit_destroy, sdr_vit_clone> {
     void reset() { check(sdr_vit_reset(h_), "Vit::reset"); }
 };
 
+// frame synchronizer bank: per channel, finds the sync word, locks to the frames and emits their payloads derotated
+class Fsync : public Handle<sdr_fsync_t, sdr_fsync_destroy, sdr_fsync_clone> {
+    size_t c_ = 0;
+
+  public:
+    struct Out {
+        std::vector<std::vector<Complex>> payload;
+        std::vector<std::vector<sdr_fsync_record_t>> records;
+    };
+    // words: one row of Lp symbols (shared) or one per channel; params: one (shared) or one per channel
+    Fsync(size_t channels, size_t word_len, const std::vector<Complex> &words,
+          const std::vector<sdr_fsync_params_t> &params)
+        : c_(channels) {
+        sdr_fsync_config_t cfg{};
+        cfg.word_len = word_len;
+        cfg.words = reinterpret_cast<const float *>(words.data());
+        cfg.n_words = word_len ? words.size() / word_len : 0;
+        cfg.params = params.data();
+        cfg.n_params = params.size();
+        cfg.n_channels = c_;
+        int err = 0;
+        h_ = sdr_fsync_create(&cfg, &err);
+        if (!h_) throw sdr::Error(err, "Fsync::new");
+    }
+    size_t channels() const { return c_; }
+    // (payload, record) bounds per channel for the next n_in[k] symbols
+    std::pair<std::vector<size_t>, std::vector<size_t>> max_output(const std::vector<size_t> &n_in) const {
+        std::vector<size_t> p(c_), r(c_);
+        check(sdr_fsync_max_output(h_, n_in.data(), p.data(), r.data()), "Fsync::max_output");
+        return {p, r};
+    }
+    sdr_fsync_state_t state(size_t k) {
+        sdr_fsync_state_t s{};
+        check(sdr_fsync_get_state(h_, k, &s), "Fsync::state");
+        return s;
+    }
+    // in: channels rows, row k of n_in[k] symbols at row stride in_stride (>= the longest row)
+    Out process(const Complex *in, const std::vector<size_t> &n_in, size_t in_stride) {
+        const auto caps = max_output(n_in);
+        const size_t cap = std::max<size_t>(1, *std::max_element(caps.first.begin(), caps.first.end()));
+        const size_t rcap = std::max<size_t>(1, *std::max_element(caps.second.begin(), caps.second.end()));
+        std::vector<Complex> pay(cap * c_);
+        std::vector<sdr_fsync_record_t> rec(rcap * c_);
+        std::vector<size_t> got(c_), rgot(c_);
+        check(sdr_fsync_process(h_, reinterpret_cast<const float *>(in), n_in.data(), in_stride,
+                                reinterpret_cast<float *>(pay.data()), cap, cap, got.data(), rec.data(), rcap, rcap,
+                                rgot.data()),
+              "Fsync::process");
+        Out o;
+        o.payload.resize(c_);
+        o.records.resize(c_);
+        for (size_t k = 0; k < c_; ++k) {
+            o.payload[k].assign(pay.begin() + k * cap, pay.begin() + k * cap + got[k]);
+            o.records[k].assign(rec.begin() + k * rcap, rec.begin() + k * rcap + rgot[k]);
+        }
+        return o;
+    }
+    void reset() { check(sdr_fsync_reset(h_), "Fsync::reset"); }
+};
+
 }  // namespace fec
 
 // =========================================================================================

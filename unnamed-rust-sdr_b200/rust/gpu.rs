@@ -891,6 +891,74 @@ impl Drop for GpuVit {
     fn drop(&mut self) { unsafe { sdr_vit_destroy(self.h) } }
 }
 
+/// frame synchronizer bank: per channel, finds the sync word, locks to the frames and emits their payloads derotated
+pub struct GpuFsync {
+    h: *mut sdr_fsync_t,
+    c: usize,
+}
+unsafe impl Send for GpuFsync {}
+
+impl GpuFsync {
+    /// words: one row of word_len symbols (shared) or one per channel; params: one (shared) or one per channel
+    pub fn new(channels: usize, word_len: usize, words: &[Complex<f32>], params: &[sdr_fsync_params_t])
+               -> Result<Self, Error> {
+        let cfg = sdr_fsync_config_t {
+            word_len, words: words.as_ptr() as *const f32, n_words: if word_len > 0 { words.len() / word_len } else { 0 },
+            params: params.as_ptr(), n_params: params.len(), n_channels: channels, device: 0,
+            stream: std::ptr::null_mut(),
+        };
+        let mut err = 0;
+        let h = unsafe { sdr_fsync_create(&cfg, &mut err) };
+        if h.is_null() { return Err(Error(err)); }
+        Ok(GpuFsync { h, c: channels })
+    }
+    /// (payload, record) bounds per channel for the next n_in[k] symbols
+    pub fn max_output(&self, n_in: &[usize]) -> Result<(Vec<usize>, Vec<usize>), Error> {
+        assert!(n_in.len() == self.c);
+        let (mut p, mut r) = (vec![0usize; self.c], vec![0usize; self.c]);
+        check(unsafe { sdr_fsync_max_output(self.h, n_in.as_ptr(), p.as_mut_ptr(), r.as_mut_ptr()) })?;
+        Ok((p, r))
+    }
+    pub fn state(&mut self, k: usize) -> Result<sdr_fsync_state_t, Error> {
+        let mut s = sdr_fsync_state_t::default();
+        check(unsafe { sdr_fsync_get_state(self.h, k, &mut s) })?;
+        Ok(s)
+    }
+    /// input: one row per channel, row k of n_in[k] symbols at a row stride of `stride` (>= the longest row);
+    /// channel k's payload symbols and records are appended to payload[k] and records[k]
+    pub fn process(&mut self, input: &[Complex<f32>], n_in: &[usize], stride: usize,
+                   payload: &mut [Vec<Complex<f32>>], records: &mut [Vec<sdr_fsync_record_t>]) -> Result<(), Error> {
+        let (p, r) = self.max_output(n_in)?;
+        let cap = p.iter().copied().max().unwrap_or(0).max(1);
+        let rcap = r.iter().copied().max().unwrap_or(0).max(1);
+        let mut out = vec![Complex::new(0.0f32, 0.0); cap * self.c];
+        let mut rec = vec![sdr_fsync_record_t::default(); rcap * self.c];
+        let (mut got, mut rgot) = (vec![0usize; self.c], vec![0usize; self.c]);
+        check(unsafe {
+            sdr_fsync_process(self.h, input.as_ptr() as *const f32, n_in.as_ptr(), stride,
+                              out.as_mut_ptr() as *mut f32, cap, cap, got.as_mut_ptr(), rec.as_mut_ptr(), rcap, rcap,
+                              rgot.as_mut_ptr())
+        })?;
+        for k in 0..self.c {
+            payload[k].extend_from_slice(&out[k * cap..k * cap + got[k]]);
+            records[k].extend_from_slice(&rec[k * rcap..k * rcap + rgot[k]]);
+        }
+        Ok(())
+    }
+    pub fn reset(&mut self) -> Result<(), Error> { check(unsafe { sdr_fsync_reset(self.h) }) }
+}
+impl Clone for GpuFsync {
+    fn clone(&self) -> Self {
+        let mut err = 0;
+        let h = unsafe { sdr_fsync_clone(self.h, &mut err) };
+        assert!(!h.is_null(), "sdr_fsync_clone failed: {}", Error(err));
+        GpuFsync { h, c: self.c }
+    }
+}
+impl Drop for GpuFsync {
+    fn drop(&mut self) { unsafe { sdr_fsync_destroy(self.h) } }
+}
+
 /// body of fft::fft after `let mut data: Vec<_> = input.iter().collect();` (src/fft.rs:8-27)
 pub fn fft_shifted(data: &[Complex<f32>], rate: f32) -> Result<Vec<(f32, Complex<f32>)>, Error> {
     if data.is_empty() { return Ok(vec![]); }

@@ -51,6 +51,7 @@ pub enum sdr_tsync_t {}
 pub enum sdr_csync_t {}
 pub enum sdr_eq_t {}
 pub enum sdr_vit_t {}
+pub enum sdr_fsync_t {}
 pub enum sdr_channelizer_t {}
 /// same role as libsamplerate's SRC_STATE (src/resample.rs:12)
 pub enum SDR_SRC_STATE {}
@@ -332,6 +333,63 @@ pub struct sdr_vit_config_t {
     pub stream: *mut c_void,
 }
 
+pub const SDR_FSYNC_SEARCH: u32 = 0;
+pub const SDR_FSYNC_VERIFY: u32 = 1;
+pub const SDR_FSYNC_LOCK: u32 = 2;
+pub const SDR_FSYNC_HIT: u16 = 1;
+pub const SDR_FSYNC_VERIFY_PASS: u16 = 2;
+pub const SDR_FSYNC_VERIFY_FAIL: u16 = 3;
+pub const SDR_FSYNC_LOCK_PASS: u16 = 4;
+pub const SDR_FSYNC_LOCK_MISS: u16 = 5;
+pub const SDR_FSYNC_LOCK_LOST: u16 = 6;
+
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct sdr_fsync_params_t {
+    pub period: u32,
+    pub order: u32,
+    pub thresh_search: c_float,
+    pub thresh_check: c_float,
+    pub verify: u32,
+    pub max_miss: u32,
+    pub window: u32,
+}
+
+#[repr(C)]
+pub struct sdr_fsync_config_t {
+    pub word_len: size_t,
+    pub words: *const c_float,
+    pub n_words: size_t,
+    pub params: *const sdr_fsync_params_t,
+    pub n_params: size_t,
+    pub n_channels: size_t,
+    pub device: c_int,
+    pub stream: *mut c_void,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct sdr_fsync_record_t {
+    pub pos: u64,
+    pub out_index: u64,
+    pub corr: [c_float; 2],
+    pub rho: c_float,
+    pub rot: u16,
+    pub kind: u16,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct sdr_fsync_state_t {
+    pub state: u32,
+    pub count: u32,
+    pub pos: u64,
+    pub rot: u32,
+    pub pad: u32,
+    pub consumed: u64,
+    pub payload: u64,
+}
+
 #[repr(C)]
 pub struct sdr_fm_config_t {
     pub n_stations: size_t,
@@ -554,6 +612,21 @@ extern "C" {
                           n_out: *mut size_t) -> c_int;
     pub fn sdr_vit_finish_dev(h: *mut sdr_vit_t, which: *const u8, terminated: c_int, out: *mut u8,
                               out_stride: size_t, n_out: *mut size_t) -> c_int;
+    pub fn sdr_fsync_create(cfg: *const sdr_fsync_config_t, err: *mut c_int) -> *mut sdr_fsync_t;
+    pub fn sdr_fsync_destroy(h: *mut sdr_fsync_t);
+    pub fn sdr_fsync_reset(h: *mut sdr_fsync_t) -> c_int;
+    pub fn sdr_fsync_clone(h: *const sdr_fsync_t, err: *mut c_int) -> *mut sdr_fsync_t;
+    pub fn sdr_fsync_max_output(h: *const sdr_fsync_t, n_in: *const size_t, pay_caps: *mut size_t,
+                                rec_caps: *mut size_t) -> c_int;
+    pub fn sdr_fsync_process(h: *mut sdr_fsync_t, in_c64: *const c_float, n_in: *const size_t, in_stride: size_t,
+                             out_c64: *mut c_float, out_cap: size_t, out_stride: size_t, n_out: *mut size_t,
+                             recs: *mut sdr_fsync_record_t, rec_cap: size_t, rec_stride: size_t,
+                             n_rec: *mut size_t) -> c_int;
+    pub fn sdr_fsync_process_dev(h: *mut sdr_fsync_t, in_c64: *const c_float, n_in: *const size_t,
+                                 in_stride: size_t, out_c64: *mut c_float, out_cap: size_t, out_stride: size_t,
+                                 n_out: *mut size_t, recs: *mut sdr_fsync_record_t, rec_cap: size_t,
+                                 rec_stride: size_t, n_rec: *mut size_t) -> c_int;
+    pub fn sdr_fsync_get_state(h: *mut sdr_fsync_t, channel: size_t, state: *mut sdr_fsync_state_t) -> c_int;
 
     // drop-in for libsamplerate_sys::{src_new, src_process, ...} used by src/resample.rs
     pub fn sdr_src_new(converter_type: c_int, channels: c_int, error: *mut c_int) -> *mut SDR_SRC_STATE;

@@ -145,6 +145,21 @@ class VitConfig(C.Structure):
                 ("zero_start", i32), ("n_channels", sz), ("device", i32), ("stream", vp)]
 
 
+class FsyncParams(C.Structure):
+    _fields_ = [("period", C.c_uint32), ("order", C.c_uint32), ("thresh_search", C.c_float),
+                ("thresh_check", C.c_float), ("verify", C.c_uint32), ("max_miss", C.c_uint32), ("window", C.c_uint32)]
+
+
+class FsyncConfig(C.Structure):
+    _fields_ = [("word_len", sz), ("words", vp), ("n_words", sz), ("params", vp), ("n_params", sz),
+                ("n_channels", sz), ("device", i32), ("stream", vp)]
+
+
+class FsyncState(C.Structure):
+    _fields_ = [("state", C.c_uint32), ("count", C.c_uint32), ("pos", C.c_uint64), ("rot", C.c_uint32),
+                ("pad", C.c_uint32), ("consumed", C.c_uint64), ("payload", C.c_uint64)]
+
+
 class SrcData(C.Structure):
     _fields_ = [("data_in", vp), ("data_out", vp), ("input_frames", C.c_long), ("output_frames", C.c_long),
                 ("input_frames_used", C.c_long), ("output_frames_gen", C.c_long),
@@ -295,6 +310,14 @@ PROTOTYPES = {
     "sdr_vit_process_dev": (i32, [vp, vp, vp, sz, vp, sz, vp]),
     "sdr_vit_finish": (i32, [vp, vp, i32, vp, sz, vp]),
     "sdr_vit_finish_dev": (i32, [vp, vp, i32, vp, sz, vp]),
+    "sdr_fsync_create": (vp, [C.POINTER(FsyncConfig), C.POINTER(i32)]),
+    "sdr_fsync_destroy": (None, [vp]),
+    "sdr_fsync_reset": (i32, [vp]),
+    "sdr_fsync_clone": (vp, [vp, C.POINTER(i32)]),
+    "sdr_fsync_max_output": (i32, [vp, vp, vp, vp]),
+    "sdr_fsync_process": (i32, [vp, vp, vp, sz, vp, sz, sz, vp, vp, sz, sz, vp]),
+    "sdr_fsync_process_dev": (i32, [vp, vp, vp, sz, vp, sz, sz, vp, vp, sz, sz, vp]),
+    "sdr_fsync_get_state": (i32, [vp, sz, C.POINTER(FsyncState)]),
     "sdr_fm_create": (vp, [C.POINTER(FmConfig), C.POINTER(i32)]),
     "sdr_fm_destroy": (None, [vp]),
     "sdr_fm_reset": (i32, [vp]),

@@ -1318,6 +1318,88 @@ class Vit(_Handle):
         return got.astype(np.int64)
 
 
+FSYNC_RECORD = np.dtype([("pos", "<u8"), ("out_index", "<u8"), ("corr", "<f4", (2,)), ("rho", "<f4"),
+                         ("rot", "<u2"), ("kind", "<u2")])
+
+
+class Fsync(_Handle):
+    """Frame synchronizer bank (sdr_fsync): per channel, finds a known sync word by correlation, tracks frames with a
+    search -> verify -> lock -> flywheel state machine and emits each frame's payload derotated by the rotation read
+    from the correlation's phase.  words: Lp complex values (shared) or [C, Lp]; params: one
+    (F, M, th_search, th_check, V, max_miss, W) or one per channel.  process returns the payload symbols and the
+    decision records (FSYNC_RECORD: pos, out_index, corr, rho, rot, kind); see include/sdr_b200.h."""
+
+    _abi = "fsync"
+    SEARCH, VERIFY, LOCK = 0, 1, 2
+    HIT, VERIFY_PASS, VERIFY_FAIL, LOCK_PASS, LOCK_MISS, LOCK_LOST = 1, 2, 3, 4, 5, 6
+
+    def __init__(self, words, params, n_channels=None, device=0, stream=None):
+        w = np.ascontiguousarray(words, np.complex64)
+        w = w[None] if w.ndim == 1 else w
+        prm = [params] if np.ndim(params[0]) == 0 else list(params)
+        c = int(n_channels) if n_channels is not None else max(len(w), len(prm))
+        self.n_channels, self.word_len = c, int(w.shape[1])
+        self._words = w
+        self._params = (F.FsyncParams * len(prm))(*[F.FsyncParams(int(p[0]), int(p[1]), float(p[2]), float(p[3]),
+                                                                   int(p[4]), int(p[5]), int(p[6])) for p in prm])
+        cfg = F.FsyncConfig(self.word_len, w.ctypes.data, len(w), C.addressof(self._params), len(prm), c, device,
+                            _stream_ptr(stream))
+        self._create(cfg)
+
+    def _counts(self, n_in):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(n_in, np.int64), (self.n_channels,)), np.uintp)
+
+    def max_output(self, n_in):
+        """(payload bounds, record bounds): numpy arrays of C for the next n_in symbols (an int, or one per channel)"""
+        n = self._counts(n_in)
+        pc, rc = np.zeros(self.n_channels, np.uintp), np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_fsync_max_output(self.h, n.ctypes.data, pc.ctypes.data, rc.ctypes.data),
+              "sdr_fsync_max_output")
+        return pc.astype(np.int64), rc.astype(np.int64)
+
+    def state(self, k):
+        """(state, v or m, sigma or e, R, symbols consumed, payload total) of channel k"""
+        s = F.FsyncState()
+        check(lib().sdr_fsync_get_state(self.h, int(k), C.byref(s)), "sdr_fsync_get_state")
+        return s.state, s.count, s.pos, s.rot, s.consumed, s.payload
+
+    def process(self, rows, records=True):
+        """rows: complex64 [C, n] or a list of C rows of any lengths -> (payloads, records): lists of C complex64
+        arrays and C FSYNC_RECORD arrays (None when records is False)"""
+        if isinstance(rows, np.ndarray) and rows.ndim == 1 and self.n_channels == 1:
+            rows = rows[None]
+        rows = [np.ascontiguousarray(r, np.complex64).ravel() for r in rows]
+        if len(rows) != self.n_channels:
+            raise ValueError("rows: %d channels expected" % self.n_channels)
+        n = np.array([r.size for r in rows], np.uintp)
+        stride = max(int(n.max()), 1)
+        x = np.zeros((self.n_channels, stride), np.complex64)
+        for k, r in enumerate(rows):
+            x[k, :r.size] = r
+        pc, rc = self.max_output(n)
+        cap, rcap = max(int(pc.max()), 1), max(int(rc.max()), 1)
+        y = np.empty((self.n_channels, cap), np.complex64)
+        rec = np.empty((self.n_channels, rcap), FSYNC_RECORD) if records else None
+        got, rgot = np.zeros(self.n_channels, np.uintp), np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_fsync_process(self.h, x.ctypes.data, n.ctypes.data, stride, y.ctypes.data, cap, cap,
+                                      got.ctypes.data, None if rec is None else rec.ctypes.data, rcap, rcap,
+                                      rgot.ctypes.data), "sdr_fsync_process")
+        return ([y[k, :int(got[k])].copy() for k in range(self.n_channels)],
+                None if rec is None else [rec[k, :int(rgot[k])].copy() for k in range(self.n_channels)])
+
+    def process_dev(self, d_in, n_in, in_stride, d_out, out_cap, out_stride, d_rec=None, rec_cap=0, rec_stride=0):
+        """device-resident: d_in C rows of in_stride complex64, row k of n_in (an int, or C counts) symbols; d_out C
+        rows of out_stride complex64 (out_cap >= the payload bound); d_rec (C rows of rec_stride 32-byte records, e.g.
+        a uint8 tensor [C, rec_stride, 32]) may be None.  Returns (payload counts, record counts), numpy arrays of C,
+        once they are known, which synchronises the handle's stream."""
+        n = self._counts(n_in)
+        got, rgot = np.zeros(self.n_channels, np.uintp), np.zeros(self.n_channels, np.uintp)
+        check(lib().sdr_fsync_process_dev(self.h, _ptr(d_in), n.ctypes.data, in_stride, _ptr(d_out), out_cap,
+                                          out_stride, got.ctypes.data, _ptr(d_rec), rec_cap, rec_stride,
+                                          rgot.ctypes.data), "sdr_fsync_process_dev")
+        return got.astype(np.int64), rgot.astype(np.int64)
+
+
 class FmStereo:
     """The FM broadcast stereo receiver of src/main.rs:32-81 for a batch of stations, device-resident end to end:
     u8 IQ -> Pll demodulator -> /75000 -> SincFastest to 144 kHz -> pilot Pll + (mono, diff) -> SincBest to 48 kHz ->
